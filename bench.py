@@ -4,6 +4,7 @@
     python bench.py [--gpus N] [--steps K] [--warmup W]            # N=1 directly; N>1 under torchrun (or self-spawned)
     python bench.py --impl reference ...                           # the reference's CPU path (oracle port) on host cores
     python bench.py --config {0,1,2,3}                             # the other BASELINE.json configurations
+    python bench.py --dump-outputs DIR ...                         # also save the last timed step's outputs as DIR/*.npy
 
 Default workload = BASELINE.json configs[3] (the configuration the images/s metric is quoted on): SDXL UNet (LCM-LoRA fused) +
 ControlNet-Canny small + fp16-fix VAE topology, fp16, 8 synthetic 1024x1024 images per GPU per step, 4 LCM steps at strength 0.5
@@ -34,7 +35,8 @@ sys.path.insert(0, ROOT)
 
 TFLOP_PER_IMAGE = {"sdxl": 44.45, "ssd-1b": 34.22}      # BASELINE.md section 3 (CN-small, 2 executed steps)
 VAE_TFLOP_PER_IMAGE = 4.887 + 10.486                     # encode + decode
-REF_BUDGET_S = float(os.environ.get("FIE_REF_BUDGET_S", "170"))   # wall budget of the timed CPU edits (at least one always runs)
+_budget = os.environ.get("FIE_REF_BUDGET_S")
+REF_BUDGET_S = float(_budget) if _budget else None       # optional wall budget of the timed CPU edits; unset: exactly --steps edits
 
 
 def parse():
@@ -47,9 +49,11 @@ def parse():
     ap.add_argument("--model", default=None, choices=["sdxl", "ssd-1b"])
     ap.add_argument("--batch", type=int, default=None, help="images per GPU per step")
     ap.add_argument("--no-cpu-baseline", action="store_true")
-    ap.add_argument("--metrics-eval", action="store_true", help="time the evaluation metrics (MetricsCalculator, DESIGN 3.10) instead of the edit")
+    ap.add_argument("--metrics-eval", action="store_true", help="time the evaluation metrics (MetricsCalculator, DESIGN 3.10) instead of the edit; a step = 4 image pairs")
     ap.add_argument("--no-graph", action="store_true", help="launch the ~2000 kernels of an edit eagerly instead of replaying one CUDA graph")
     ap.add_argument("--profile-out", default=None, help="write the per-kernel-family breakdown JSON here")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step returned as DIR/<name>.npy (float32 or float64)")
     a = ap.parse_args()
     if a.config == 0:
         a.impl = "reference"
@@ -57,6 +61,10 @@ def parse():
         a.model = "ssd-1b" if a.config in (0, 2) else "sdxl"
     if a.batch is None:
         a.batch = {0: 1, 1: 32, 2: 1, 3: 8}[a.config]
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl == "reference":
+        ap.error("--dump-outputs needs a B200 path (the reference arm returns no outputs)")
     return a
 
 
@@ -134,17 +142,18 @@ def cpu_model_name():
     return "unknown"
 
 
-def timed_cpu_edits(state, max_edits: int, threads: int):
-    """One untimed 64x64 warm-up (thread pools, oneDNN primitive caches), then full 1024x1024 edits until ``max_edits`` or the wall
-    budget REF_BUDGET_S is reached (at least one).  -> (list of seconds, stage split of the first)."""
+def timed_cpu_edits(state, edits: int, threads: int):
+    """One untimed 64x64 warm-up (thread pools, oneDNN primitive caches), then ``edits`` full 1024x1024 edits; only when the
+    FIE_REF_BUDGET_S wall budget is set, fewer (at least one) once another edit would overrun it.
+    -> (list of seconds, stage split of the first)."""
     cpu_reference_edit(state, 64, threads)
     times, stages0 = [], None
     t_begin = time.perf_counter()
-    while len(times) < max(max_edits, 1):
+    while len(times) < edits:
         t, st = cpu_reference_edit(state, 1024, threads)
         times.append(t)
         stages0 = stages0 or st
-        if (time.perf_counter() - t_begin) + t > REF_BUDGET_S:      # another edit would overrun the budget
+        if REF_BUDGET_S is not None and (time.perf_counter() - t_begin) + t > REF_BUDGET_S:
             break
     return times, stages0
 
@@ -161,9 +170,10 @@ def run_reference(a):
     times, stages = timed_cpu_edits(state, a.steps, threads)
     t = sum(times) / len(times)
     value = 1.0 / t
+    bound = "" if REF_BUDGET_S is None else f", bounded by a {REF_BUDGET_S:.0f} s wall budget (FIE_REF_BUDGET_S)"
     sample = (f"{len(times)} timed full fp32 oracle edit(s) of ONE 1024x1024 image each (Canny + VAE encode + 2 x (ControlNet + UNet CFG pair) + "
               f"VAE decode, {a.model} + ControlNet-small widths, LoRA unfused as in the reference) on {threads} host threads "
-              f"({cpu_model_name()}), after one untimed 64x64 warm-up; {a.steps} steps requested, bounded by a {REF_BUDGET_S:.0f} s wall budget; "
+              f"({cpu_model_name()}), after one untimed 64x64 warm-up; {a.steps} steps requested{bound}; "
               f"nothing is extrapolated")
     line = {"impl": "reference", "metric": "1024x1024 4-step edit images/sec", "value": value, "unit": "images/s", "n_gpus": a.gpus,
             "steps": len(times), "steps_requested": a.steps, "warmup": 1, "ms_per_step": t * 1e3, "higher_is_better": True, "scaling": "weak",
@@ -201,6 +211,25 @@ def load_peaks():
         return {}
 
 
+DUMP_MAX_ELEMENTS = 4 << 20      # per array: 16 MB of float32, so the few arrays of a dump stay far below 64 MB
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes each array of ``arrays`` (name -> numpy array) as ``out_dir/<name>.npy``: float64 stays float64, everything else
+    becomes float32 (exact for the uint8 and fp16 outputs).  An array of more than DUMP_MAX_ELEMENTS elements is replaced by
+    the flattened values at DUMP_MAX_ELEMENTS sorted positions drawn by a generator seeded with 0, so two runs with the same
+    arguments sample the same positions and their files compare element for element."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    for name, x in arrays.items():
+        x = np.asarray(x)
+        x = x.astype(np.float64 if x.dtype == np.float64 else np.float32)
+        if x.size > DUMP_MAX_ELEMENTS:
+            pick = np.sort(np.random.default_rng(0).choice(x.size, DUMP_MAX_ELEMENTS, replace=False))
+            x = x.reshape(-1)[pick]
+        np.save(os.path.join(out_dir, f"{name}.npy"), x)
+
+
 def latest_profile_json(pattern):
     import glob
     files = sorted(glob.glob(os.path.join(ROOT, "profiles", pattern)))
@@ -226,7 +255,7 @@ def run_metrics_eval(a):
     import warnings
     import numpy as np
     import torch
-    pairs = max(a.steps, 1) * 4
+    pairs = a.steps * 4                 # one step = one pass over the 4 image pairs
     from PIL import Image
     from fast_image_editing_with_generative_models_b200 import ops
     from fast_image_editing_with_generative_models_b200.metrics import MetricsCalculator
@@ -241,11 +270,13 @@ def run_metrics_eval(a):
     torch.cuda.synchronize()
     launches0 = ops.LAUNCHES
     t0 = time.perf_counter()
-    for i in range(pairs):
-        calc.calculate_all_metrics(src[i % 4], edited[i % 4], prompt)
+    for _ in range(a.steps):
+        metrics = [calc.calculate_all_metrics(src[i], edited[i], prompt) for i in range(4)]
     torch.cuda.synchronize()
     per_pair = (time.perf_counter() - t0) / pairs
     launches = (ops.LAUNCHES - launches0) / pairs
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, {k: np.array([m[k] for m in metrics], np.float64) for k in metrics[0]})   # [4] per metric
     split = {}
     for name, fn in (("ssim", lambda: calc.calculate_ssim(src[0], edited[0])), ("lpips", lambda: calc.calculate_lpips(src[0], edited[0])),
                      ("clip_score", lambda: calc.calculate_clip_score(edited[0], prompt)), ("psnr", lambda: calc.calculate_psnr(src[0], edited[0])),
@@ -259,7 +290,7 @@ def run_metrics_eval(a):
         split[name] = round((time.perf_counter() - t0) / 10 * 1e3, 3)
     out = {"metric": "evaluated image pairs per second (all six metrics, PIL in -> floats out)", "value": round(1.0 / per_pair, 2), "unit": "pairs/s", "n_gpus": 1,
            "higher_is_better": True, "ms_per_pair": round(per_pair * 1e3, 2),
-           "gpu_launches_per_pair": launches, "ms_per_metric": split, "weights": "synthetic (seeded random init)", "pairs": pairs,
+           "gpu_launches_per_pair": launches, "ms_per_metric": split, "weights": "synthetic (seeded random init)", "steps": a.steps, "pairs": pairs,
            "device": torch.cuda.get_device_name(0)}
     if not a.no_cpu_baseline:
         from oracle import metrics_oracle as MO
@@ -374,9 +405,13 @@ def main():
     if a.config == 1:
         return run_config1(a, eng, imgs, dev, rank, world, peak_tf, peak_hbm, peak_src, timed, ClockSampler(local))
 
+    last = {}
+
     def step():
         out = eng.edit_batch(imgs, pe_d, pl_d, nz_d, **EDIT)
-        return sweep.gather_outputs(out.images) if world > 1 else out.images
+        last["images"] = sweep.gather_outputs(out.images) if world > 1 else out.images
+        last["edges"] = out.edges              # gathered after the timed region, for --dump-outputs only
+        return last["images"]
 
     W = max(a.warmup, 3)
     for _ in range(W):
@@ -389,6 +424,12 @@ def main():
     launches = ops.LAUNCHES - l0
     clocks = sampler.stop()
     value = world * B * a.steps / (ms * 1e-3)
+    if a.dump_outputs:
+        # before any further edit: with graph replay the outputs are the graph's static buffers, which the next call overwrites.
+        # With several ranks rank 0 writes every rank's images and edges (the gather is collective, so every rank takes part).
+        edges = sweep.gather_outputs(last["edges"])         # the local tensor itself with one rank
+        if rank == 0:
+            dump_outputs(a.dump_outputs, {"images": last["images"].cpu().numpy(), "edges": edges.cpu().numpy()})
 
     # ---- end-to-end through the plugin API: FastEditor.edit_many on host PIL images and prompt strings -> host PIL images ----
     pil = [Image.fromarray(imgs_np[i]) for i in range(B)]
@@ -507,6 +548,7 @@ def run_config1(a, eng, imgs, dev, rank, world, peak_tf, peak_hbm, peak_src, tim
     CH = 8
     vae = eng.vae
     lat = [torch.randn((CH, 128, 128, 4), device=dev, generator=torch.Generator(dev).manual_seed(i)).half() for i in range(B // CH)]
+    last = {}
 
     def step():
         edges = ops.canny(imgs, 100, 200, out_channels=3)
@@ -514,6 +556,7 @@ def run_config1(a, eng, imgs, dev, rank, world, peak_tf, peak_hbm, peak_src, tim
         for c in range(B // CH):
             vae.encode_moments(ops.preprocess_pad8(imgs[c * CH:(c + 1) * CH], True))
             outs.append(ops.postprocess(vae.decode(lat[c])))
+        last["edges"], last["images"] = edges, outs
         return edges, outs
 
     W = max(a.warmup, 3)
@@ -524,6 +567,12 @@ def run_config1(a, eng, imgs, dev, rank, world, peak_tf, peak_hbm, peak_src, tim
     ms = timed(step, a.steps, 0)
     launches = ops.LAUNCHES - l0
     clocks = sampler.stop()
+    if a.dump_outputs:
+        from fast_image_editing_with_generative_models_b200 import sweep
+        got = {"edges": last["edges"], "images": torch.cat(last["images"])}
+        got = {k: sweep.gather_outputs(v) for k, v in got.items()}      # collective (every rank takes part); local with one rank
+        if rank == 0:
+            dump_outputs(a.dump_outputs, {k: v.cpu().numpy() for k, v in got.items()})
     ops.PROFILE = []
     step()
     fam = ops.profile_summary()

@@ -1,10 +1,15 @@
 """CLIP BPE tokenizer (SURVEY 8(f)-1) pinned against transformers.CLIPTokenizer on a vocabulary learned here (the real
-vocab.json / merges.txt are not available offline)."""
+vocab.json / merges.txt are not available offline): against its ids stored in tests/golden, and against transformers itself where
+it is installed."""
 import collections
+import os
+import zlib
 
+import numpy as np
 import pytest
 
 from fast_image_editing_with_generative_models_b200.tokenizer import BOS, EOS, CLIPBPETokenizer, byte_alphabet
+from tests.util import GOLDEN
 
 CORPUS = ("a photo of a cat sitting on a wooden bench in the park . a watercolor painting of mountains at sunset , highly detailed . "
           "the quick brown fox jumps over the lazy dog's back ; it's raining cats and dogs ! we've got 2 apples , 37 oranges and 1000 grapes . "
@@ -57,13 +62,25 @@ PROMPTS = ["", "a photo of a cat", "A Photo   of\ta CAT!!", "it's raining; we've
 
 @pytest.fixture(scope="module")
 def toks():
-    transformers = pytest.importorskip("transformers")
+    """(this tokenizer, transformers.CLIPTokenizer or None where transformers is not installed, vocabulary)."""
     vocab, merges = _learn()
+    try:
+        import transformers
+    except ImportError:
+        return CLIPBPETokenizer(vocab, merges), None, vocab
     try:
         ref = transformers.CLIPTokenizer(vocab=vocab, merges=[tuple(m) for m in merges])
     except Exception:
         ref = transformers.CLIPTokenizer(vocab=vocab, merges=[" ".join(m) for m in merges])
     return CLIPBPETokenizer(vocab, merges), ref, vocab
+
+
+@pytest.fixture(scope="module")
+def transformers_ids():
+    """transformers' ids of PROMPTS, stored by tests/golden/make_tokenizer_golden.py."""
+    z = np.load(os.path.join(GOLDEN, "clip_tokenizer_golden.npz"))
+    assert [zlib.crc32(p.encode("utf-8")) for p in PROMPTS] == z["prompt_crc"].tolist(), "PROMPTS changed: regenerate the fixture"
+    return z["ids"].tolist()
 
 
 def test_byte_alphabet_is_a_bijection_on_printables():
@@ -72,11 +89,13 @@ def test_byte_alphabet_is_a_bijection_on_printables():
 
 
 @pytest.mark.parametrize("i", range(len(PROMPTS)))
-def test_ids_match_transformers(toks, i):
+def test_ids_match_transformers(toks, transformers_ids, i):
     mine, ref, _ = toks
-    want = ref(PROMPTS[i], padding="max_length", max_length=77, truncation=True).input_ids
+    want = transformers_ids[i]
+    if ref is not None:
+        assert list(ref(PROMPTS[i], padding="max_length", max_length=77, truncation=True).input_ids) == want
     got = mine(PROMPTS[i])[0]
-    assert len(got) == 77 and got == list(want), (PROMPTS[i], got[:20], list(want)[:20])
+    assert len(got) == 77 and got == want, (PROMPTS[i], got[:20], want[:20])
 
 
 def test_batch_and_pad_token(toks):

@@ -7,11 +7,11 @@ GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
 KINDS = ["shapes", "noise", "smooth"]
 
 
-def canny_golden_cases():
-    """Yields (img_u8 [h,w,3], low, high, edges_u8 [h,w]) from the committed cv2 fixture."""
+def canny_golden_cases(name="canny_golden.npz"):
+    """Yields (img_u8 [h,w,3], low, high, edges_u8 [h,w], crc32 of the gray image) from a committed cv2 fixture."""
     import zlib
     from oracle.canny_oracle import synthetic_image
-    z = np.load(os.path.join(GOLDEN, "canny_golden.npz"))
+    z = np.load(os.path.join(GOLDEN, name))
     i = 0
     while f"case{i}_meta" in z:
         seed, h, w, kind, lo, hi, crc = [int(v) for v in z[f"case{i}_meta"]]
