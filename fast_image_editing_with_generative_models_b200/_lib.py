@@ -12,7 +12,9 @@ import subprocess
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("FIE_LIB") or os.path.join(_HERE, "libfie_b200.so")   # FIE_LIB: experiment builds only
 
-c_void_p, c_int, c_ll, c_float, c_size_t = ctypes.c_void_p, ctypes.c_int, ctypes.c_longlong, ctypes.c_float, ctypes.c_size_t
+DT_F16, DT_BF16, DT_F32 = 0, 1, 2       # out_dtype of the *_bf16 entry points (FIE_DT_*)
+
+c_void_p, c_int, c_ll, c_float, c_size_t =ctypes.c_void_p, ctypes.c_int, ctypes.c_longlong, ctypes.c_float, ctypes.c_size_t
 
 
 class Epilogue(ctypes.Structure):
@@ -86,7 +88,20 @@ SIGNATURES = {
     "fie_attention_d64_causal_f16": (c_int, [c_void_p, c_ll, c_void_p, c_ll, c_void_p, c_ll, c_void_p, c_ll, c_int, c_int, c_int, c_int, c_float, c_void_p]),
     "fie_embed_tokens_f16": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_ll, c_int, c_int, c_int, c_void_p]),
     "fie_vae_sample_add_noise": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_ll, c_float, c_float, c_float, c_void_p]),
-    "fie_cfg_lcm_step": (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_ll] + [c_float] * 7 + [c_int, c_void_p]),
+    "fie_gemm_bf16": (c_int, [c_void_p, c_ll, c_void_p, c_ll, c_int, c_void_p, c_void_p, c_ll, c_ll, c_int, c_int, ctypes.POINTER(Epilogue), c_int, c_void_p]),
+    "fie_conv3x3_bf16": (c_int, [c_void_p, c_void_p, c_void_p, c_ll, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int, ctypes.POINTER(Epilogue), c_int,
+                                 c_void_p]),
+    "fie_conv_up2x_bf16": (c_int, [c_void_p, c_void_p, c_void_p, c_ll, c_int, c_int, c_int, c_int, c_int, ctypes.POINTER(Epilogue), c_int, c_void_p]),
+    "fie_conv3x3_c8_bf16": (c_int, [c_void_p, c_void_p, c_void_p, c_ll, c_int, c_int, c_int, c_int, c_int, ctypes.POINTER(Epilogue), c_int, c_void_p]),
+    "fie_groupnorm_bf16_workspace_bytes": (c_size_t, [c_int, c_ll, c_int, c_int]),
+    "fie_groupnorm_bf16": (c_int, [c_void_p, c_int, c_void_p, c_int, c_void_p, c_int, c_ll, c_int, c_void_p, c_void_p, c_float, c_int, c_void_p, c_size_t,
+                                   c_void_p]),
+    "fie_softmax_rows_f32_to_bf16": (c_int, [c_void_p, c_ll, c_void_p, c_ll, c_ll, c_int, c_float, c_void_p]),
+    "fie_attn_vae_d512_bf16": (c_int, [c_void_p, c_ll, c_void_p, c_ll, c_void_p, c_void_p, c_ll, c_int, c_int, c_float, c_int, c_void_p, c_size_t, c_void_p]),
+    "fie_pack_conv3x3_bf16": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p]),
+    "fie_pack_conv_up2x_bf16": (c_int, [c_void_p, c_void_p, c_int, c_int, c_void_p]),
+    "fie_pack_rows_bf16": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_void_p]),
+    "fie_cfg_lcm_step":(c_int, [c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_ll] + [c_float] * 7 + [c_int, c_void_p]),
 }
 
 _lib = None

@@ -70,7 +70,8 @@ def controlnet_config_from_json(d: Dict, name: str = "controlnet") -> C.ControlN
 def vae_config_from_json(d: Dict, name: str = "vae") -> C.VAEConfig:
     return C.VAEConfig(name=name, block_out_channels=tuple(d["block_out_channels"]), layers_per_block=d.get("layers_per_block", 2),
                        latent_channels=d.get("latent_channels", 4), norm_groups=d.get("norm_num_groups", 32), norm_eps=1e-6,
-                       scaling_factor=d.get("scaling_factor", 0.13025))
+                       scaling_factor=d.get("scaling_factor", 0.13025),
+                       force_upcast=bool(d["force_upcast"]) if d.get("force_upcast") is not None else None)
 
 
 def _weights_file(folder: str) -> str:

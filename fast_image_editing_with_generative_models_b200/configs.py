@@ -103,6 +103,9 @@ class VAEConfig:
     scaling_factor: float = 0.13025
     conv_out_gain: float = 1.0  # synthetic recipe: decoder conv_out gain so image std ~0.3-0.5
     seed: int = 15
+    # diffusers' AutoencoderKL ``force_upcast`` (config.json): True = the VAE's activations do not fit fp16 (the original SDXL VAE);
+    # None = the key is absent.  FastEditor(vae_dtype=None) runs such a VAE in bf16.
+    force_upcast: Optional[bool] = None
 
 
 def tiny_vae_config() -> VAEConfig:

@@ -59,3 +59,30 @@ extern "C" int fie_attn_vae_d512_f16(const void* q, long long ldq, const void* k
     }
     return FIE_OK;
 }
+
+// bf16 twin (the bf16 VAE): the same three passes with bf16 operands; the logits always stay fp32 between the passes, and P is written
+// as bf16 so that both operands of the P V product are bf16.
+extern "C" int fie_attn_vae_d512_bf16(const void* q, long long ldq, const void* k, long long ldk, const void* vt, void* out, long long ldo,
+                                      int ntok, int d, float scale, int chunk_rows, void* workspace, size_t workspace_bytes, void* stream) {
+    using namespace fie;
+    FIE_REQUIRE(q && k && vt && out && workspace, "fie_attn_vae_d512_bf16: null pointer");
+    FIE_REQUIRE(ntok > 0 && d > 0 && (d % 64) == 0 && (ntok % 8) == 0, "fie_attn_vae_d512_bf16: d %% 64 and ntok %% 8 required (d=%d ntok=%d)", d, ntok);
+    if (chunk_rows <= 0 || chunk_rows > ntok) chunk_rows = ntok;
+    FIE_REQUIRE(workspace_bytes >= fie_attn_vae_workspace_bytes(ntok, chunk_rows, 1), "fie_attn_vae_d512_bf16: workspace too small");
+    FIE_REQUIRE((reinterpret_cast<uintptr_t>(workspace) & 255) == 0, "fie_attn_vae_d512_bf16: workspace must be 256-byte aligned");
+    uint8_t* ws = (uint8_t*)workspace;
+    void* scores = ws;
+    void* probs = ws + (((size_t)chunk_rows * ntok * 4) + 255) / 256 * 256;
+    for (int r0 = 0; r0 < ntok; r0 += chunk_rows) {
+        const int rows = ntok - r0 < chunk_rows ? ntok - r0 : chunk_rows;
+        fie_epilogue e1 = {};
+        e1.rows_per_group = 1; e1.scale = 1.0f; e1.out_f32 = 1;
+        int rc = fie_gemm_bf16((const uint16_t*)q + (size_t)r0 * ldq, ldq, nullptr, 0, 0, k, scores, ntok, rows, ntok, d, &e1, FIE_DT_F32, stream);
+        if (rc) return rc;
+        if ((rc = fie_softmax_rows_f32_to_bf16(scores, ntok, probs, ntok, rows, ntok, scale, stream))) return rc;
+        fie_epilogue e2 = {};
+        e2.rows_per_group = 1; e2.scale = 1.0f;
+        if ((rc = fie_gemm_bf16(probs, ntok, nullptr, 0, 0, vt, (uint16_t*)out + (size_t)r0 * ldo, ldo, rows, d, ntok, &e2, FIE_DT_BF16, stream))) return rc;
+    }
+    return FIE_OK;
+}

@@ -133,12 +133,13 @@ __device__ __forceinline__ float to_f(__half v) { return __half2float(v); }
 
 // Single-pass form for rows of at most 256 x 4 x NV columns: the row lives in registers (NV independent vector loads in flight
 // per thread), one block reduction for the max and one for the sum.
-template <typename T, int NV>
-__global__ void __launch_bounds__(256) k_softmax_rows_reg(const T* __restrict__ s, long long ld_in, __half* __restrict__ p, long long ld_out, int cols, float scale) {
+// OBF: the probabilities are stored as bf16 instead of fp16 (the bf16 VAE).
+template <typename T, int NV, bool OBF = false>
+__global__ void __launch_bounds__(256) k_softmax_rows_reg(const T* __restrict__ s, long long ld_in, uint16_t* __restrict__ p, long long ld_out, int cols, float scale) {
     __shared__ float red[8];
     __shared__ float bc;
     const T* row = s + (long long)blockIdx.x * ld_in;
-    __half* orow = p + (long long)blockIdx.x * ld_out;
+    uint16_t* orow = p + (long long)blockIdx.x * ld_out;
     const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
     float4 v[NV];
 #pragma unroll
@@ -173,8 +174,7 @@ __global__ void __launch_bounds__(256) k_softmax_rows_reg(const T* __restrict__ 
     for (int k = 0; k < NV; ++k) {
         const int i = (k * 256 + tid) * 4;
         if (i + 4 <= cols) {
-            __half2 a = __floats2half2_rn(v[k].x * inv, v[k].y * inv), b = __floats2half2_rn(v[k].z * inv, v[k].w * inv);
-            uint2 u; u.x = *reinterpret_cast<uint32_t*>(&a); u.y = *reinterpret_cast<uint32_t*>(&b);
+            uint2 u; u.x = pack_h2<OBF>(v[k].x * inv, v[k].y * inv); u.y = pack_h2<OBF>(v[k].z * inv, v[k].w * inv);
             *reinterpret_cast<uint2*>(orow + i) = u;
         }
     }
@@ -231,12 +231,12 @@ __global__ void __launch_bounds__(256, 4) k_softmax_rows_exp(const __half* __res
     if (tid == 0) { float t = 0; for (int i = 0; i < 8; ++i) t += red[i]; inv_sum[blockIdx.x] = 1.0f / t; }
 }
 
-template <typename T>
-__global__ void __launch_bounds__(256) k_softmax_rows(const T* __restrict__ s, long long ld_in, __half* __restrict__ p, long long ld_out, int cols, float scale) {
+template <typename T, bool OBF = false>
+__global__ void __launch_bounds__(256) k_softmax_rows(const T* __restrict__ s, long long ld_in, uint16_t* __restrict__ p, long long ld_out, int cols, float scale) {
     __shared__ float red[8];
     __shared__ float bc;
     const T* row = s + (long long)blockIdx.x * ld_in;
-    __half* orow = p + (long long)blockIdx.x * ld_out;
+    uint16_t* orow = p + (long long)blockIdx.x * ld_out;
     const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
     float mx = -INFINITY;
     for (int i = tid * 4; i < cols; i += 1024) {
@@ -265,11 +265,11 @@ __global__ void __launch_bounds__(256) k_softmax_rows(const T* __restrict__ s, l
     for (int i = tid * 4; i < cols; i += 1024) {
         if (i + 4 <= cols) {
             float4 v = Vec4<T>::ld(row + i);
-            __half2 a = __floats2half2_rn(exp2f((v.x - mx) * sl2) * inv, exp2f((v.y - mx) * sl2) * inv);
-            __half2 b = __floats2half2_rn(exp2f((v.z - mx) * sl2) * inv, exp2f((v.w - mx) * sl2) * inv);
-            uint2 u; u.x = *reinterpret_cast<uint32_t*>(&a); u.y = *reinterpret_cast<uint32_t*>(&b);
+            uint2 u;
+            u.x = pack_h2<OBF>(exp2f((v.x - mx) * sl2) * inv, exp2f((v.y - mx) * sl2) * inv);
+            u.y = pack_h2<OBF>(exp2f((v.z - mx) * sl2) * inv, exp2f((v.w - mx) * sl2) * inv);
             *reinterpret_cast<uint2*>(orow + i) = u;
-        } else for (int j = i; j < cols; ++j) orow[j] = __float2half_rn(exp2f((to_f(row[j]) - mx) * sl2) * inv);
+        } else for (int j = i; j < cols; ++j) orow[j] = f_to_h<OBF>(exp2f((to_f(row[j]) - mx) * sl2) * inv);
     }
 }
 
@@ -375,14 +375,20 @@ extern "C" int fie_sincos_embedding(const float* host_vals, int count, int dim, 
 }
 extern "C" int fie_softmax_rows_f32_to_f16(const void* s, long long ld_in, void* p, long long ld_out, long long rows, int cols, float scale, void* stream) {
     FIE_REQUIRE(s && p && rows > 0 && rows < (1ll << 31) && cols > 0 && (ld_in % 4) == 0 && (ld_out % 4) == 0, "fie_softmax_rows: bad args");
-    if ((cols % 4) == 0 && cols <= 16384) k_softmax_rows_reg<float, 16><<<(unsigned)rows, 256, 0, (cudaStream_t)stream>>>((const float*)s, ld_in, (__half*)p, ld_out, cols, scale);
-    else k_softmax_rows<float><<<(unsigned)rows, 256, 0, (cudaStream_t)stream>>>((const float*)s, ld_in, (__half*)p, ld_out, cols, scale);
+    if ((cols % 4) == 0 && cols <= 16384) k_softmax_rows_reg<float, 16><<<(unsigned)rows, 256, 0, (cudaStream_t)stream>>>((const float*)s, ld_in, (uint16_t*)p, ld_out, cols, scale);
+    else k_softmax_rows<float><<<(unsigned)rows, 256, 0, (cudaStream_t)stream>>>((const float*)s, ld_in, (uint16_t*)p, ld_out, cols, scale);
     return check_launch("fie_softmax_rows_f32_to_f16");
+}
+extern "C" int fie_softmax_rows_f32_to_bf16(const void* s, long long ld_in, void* p, long long ld_out, long long rows, int cols, float scale, void* stream) {
+    FIE_REQUIRE(s && p && rows > 0 && rows < (1ll << 31) && cols > 0 && (ld_in % 4) == 0 && (ld_out % 4) == 0, "fie_softmax_rows_f32_to_bf16: bad args");
+    if ((cols % 4) == 0 && cols <= 16384) k_softmax_rows_reg<float, 16, true><<<(unsigned)rows, 256, 0, (cudaStream_t)stream>>>((const float*)s, ld_in, (uint16_t*)p, ld_out, cols, scale);
+    else k_softmax_rows<float, true><<<(unsigned)rows, 256, 0, (cudaStream_t)stream>>>((const float*)s, ld_in, (uint16_t*)p, ld_out, cols, scale);
+    return check_launch("fie_softmax_rows_f32_to_bf16");
 }
 extern "C" int fie_softmax_rows_f16(const void* s, long long ld_in, void* p, long long ld_out, long long rows, int cols, float scale, void* stream) {
     FIE_REQUIRE(s && p && rows > 0 && rows < (1ll << 31) && cols > 0 && (ld_in % 4) == 0 && (ld_out % 4) == 0, "fie_softmax_rows_f16: bad args");
-    if ((cols % 4) == 0 && cols <= 16384) k_softmax_rows_reg<__half, 16><<<(unsigned)rows, 256, 0, (cudaStream_t)stream>>>((const __half*)s, ld_in, (__half*)p, ld_out, cols, scale);
-    else k_softmax_rows<__half><<<(unsigned)rows, 256, 0, (cudaStream_t)stream>>>((const __half*)s, ld_in, (__half*)p, ld_out, cols, scale);
+    if ((cols % 4) == 0 && cols <= 16384) k_softmax_rows_reg<__half, 16><<<(unsigned)rows, 256, 0, (cudaStream_t)stream>>>((const __half*)s, ld_in, (uint16_t*)p, ld_out, cols, scale);
+    else k_softmax_rows<__half><<<(unsigned)rows, 256, 0, (cudaStream_t)stream>>>((const __half*)s, ld_in, (uint16_t*)p, ld_out, cols, scale);
     return check_launch("fie_softmax_rows_f16");
 }
 extern "C" int fie_softmax_rows_exp_f16(const void* s, long long ld_in, void* p, long long ld_out, float* inv_sum, long long rows, int cols, float scale, void* stream) {

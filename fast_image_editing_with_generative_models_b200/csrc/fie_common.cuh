@@ -2,6 +2,7 @@
 #pragma once
 #include <cuda_runtime.h>
 #include <cuda_fp16.h>
+#include <cuda_bf16.h>
 #include <stdint.h>
 #include <stdio.h>
 #include <stdarg.h>
@@ -75,6 +76,24 @@ __device__ __forceinline__ void silu2(float& y0, float& y1) {
 }
 
 __device__ __forceinline__ float quick_gelu_f(float x) { return __fdividef(x, 1.0f + __expf(-1.702f * x)); }
+
+// Two 16-bit floats in one 32-bit word: fp16 (BF = false) or bf16 (BF = true), round to nearest even.
+template <bool BF> __device__ __forceinline__ uint32_t pack_h2(float a, float b) {
+    if constexpr (BF) { const __nv_bfloat162 h = __floats2bfloat162_rn(a, b); return *reinterpret_cast<const uint32_t*>(&h); }
+    else { const __half2 h = __floats2half2_rn(a, b); return *reinterpret_cast<const uint32_t*>(&h); }
+}
+template <bool BF> __device__ __forceinline__ float2 unpack_h2(uint32_t u) {
+    if constexpr (BF) return __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&u));
+    else return __half22float2(*reinterpret_cast<const __half2*>(&u));
+}
+template <bool BF> __device__ __forceinline__ float h_to_f(uint16_t u) {
+    if constexpr (BF) return __bfloat162float(__ushort_as_bfloat16(u));
+    else return __half2float(__ushort_as_half(u));
+}
+template <bool BF> __device__ __forceinline__ uint16_t f_to_h(float v) {
+    if constexpr (BF) return __bfloat16_as_ushort(__float2bfloat16_rn(v));
+    else return __half_as_ushort(__float2half_rn(v));
+}
 
 __device__ __forceinline__ float warp_sum(float v) {
 #pragma unroll

@@ -1,6 +1,6 @@
 // Persistent, warp-specialised tcgen05 GEMM / implicit-GEMM 3x3 convolution for sm_100a.
 //
-//   D[M, N] = epilogue( A[M, K] * B[N, K]^T )     fp16 operands, fp32 accumulators in TMEM
+//   D[M, N] = epilogue( A[M, K] * B[N, K]^T )     fp16 (or bf16) operands, fp32 accumulators in TMEM
 //
 // Replaces F.linear / F.conv2d (cuBLASLt / cuDNN) in every diffusers module on the reference's edit path
 // (UNet2DConditionModel, ControlNetModel, AutoencoderKL; reference call site src/pipeline.py:261-272).
@@ -13,7 +13,7 @@
 //   B tile = 2-D box {64 k, block_n rows} of the packed weight matrix [N][K].
 // Math: one elected thread issues tcgen05.mma (M=128, N=block_n, K=16) into a double-buffered TMEM accumulator.
 // Epilogue: 4 warps read TMEM (tcgen05.ld 32x32b), fuse bias / time-embedding broadcast / SiLU / GEGLU /
-//           scale / residual, and store fp16 (or fp32) rows.
+//           scale / residual, and store fp16 (or bf16 / fp32) rows.
 //
 // Warp roles (384 threads): w0-7 epilogue, w8 TMA producer, w9 MMA issuer, w10 TMEM allocator, w11 idle.
 #include "tc_common.cuh"
@@ -77,11 +77,13 @@ struct GemmParams {
     long long rows_per_group;
     long long ld_row_bias;
     const float* m_bias;
-    const __half* residual;
+    const __half* residual;         // in the output's 16-bit type (fp16, or bf16 when out_bf16)
     long long ld_res;
     float scale;
     int act;
     int out_f32;
+    int out_bf16;                   // 16-bit output (and residual) is bf16 (kernel variant OBF = 1)
+    int ab_bf16;                    // A and B are bf16 (instruction-descriptor operand formats and TMA maps)
     unsigned long long* gn_stats;   // optional GroupNorm statistics of the output [images][groups][2], 2^-20 fixed point
     int gn_cpg, gn_groups;          // channels per group (divides 32), groups
     long long gn_rows;              // rows per image
@@ -102,6 +104,7 @@ __device__ __forceinline__ long long out_row(const GemmParams& p, long long m) {
     return ((long long)n * 2 * p.OH + 2 * h + p.up_a) * (2 * p.OW) + 2 * w + p.up_b;
 }
 
+template <bool OBF>
 __device__ __forceinline__ void store_chunk(const GemmParams& p, long long m, int n0, const float (&v)[32]) {
     // stores v[0..31] to output row m, columns n0..n0+31 (masked by n_store)
     if (p.out_f32) {
@@ -113,19 +116,17 @@ __device__ __forceinline__ void store_chunk(const GemmParams& p, long long m, in
             for (int i = 0; i < 32; ++i) if (n0 + i < p.n_store) d[i] = v[i];
         }
     } else {
-        __half* d = reinterpret_cast<__half*>(p.D) + out_row(p, m) * p.ldd + n0;
+        uint16_t* d = reinterpret_cast<uint16_t*>(p.D) + out_row(p, m) * p.ldd + n0;
         if (n0 + 32 <= p.n_store && (p.ldd & 7) == 0) {
 #pragma unroll
             for (int i = 0; i < 4; ++i) {
                 uint4 u;
-                __half2 h0 = __floats2half2_rn(v[8 * i], v[8 * i + 1]), h1 = __floats2half2_rn(v[8 * i + 2], v[8 * i + 3]);
-                __half2 h2 = __floats2half2_rn(v[8 * i + 4], v[8 * i + 5]), h3 = __floats2half2_rn(v[8 * i + 6], v[8 * i + 7]);
-                u.x = *reinterpret_cast<uint32_t*>(&h0); u.y = *reinterpret_cast<uint32_t*>(&h1);
-                u.z = *reinterpret_cast<uint32_t*>(&h2); u.w = *reinterpret_cast<uint32_t*>(&h3);
+                u.x = pack_h2<OBF>(v[8 * i], v[8 * i + 1]); u.y = pack_h2<OBF>(v[8 * i + 2], v[8 * i + 3]);
+                u.z = pack_h2<OBF>(v[8 * i + 4], v[8 * i + 5]); u.w = pack_h2<OBF>(v[8 * i + 6], v[8 * i + 7]);
                 reinterpret_cast<uint4*>(d)[i] = u;
             }
         } else {
-            for (int i = 0; i < 32; ++i) if (n0 + i < p.n_store) d[i] = __float2half_rn(v[i]);
+            for (int i = 0; i < 32; ++i) if (n0 + i < p.n_store) d[i] = f_to_h<OBF>(v[i]);
         }
     }
 }
@@ -164,6 +165,7 @@ __device__ __forceinline__ void gn_stats_chunk(const float (&v)[32], bool row_ok
 
 // Out-of-line generic epilogue for one 32-column chunk of one accumulator row per thread: partial chunks at the N edge,
 // fp32 output, unaligned leading dimensions.  Rare; kept out of the hot loop on purpose.
+template <bool OBF>
 __device__ __noinline__ void epi_slow_chunk(const GemmParams& p, uint32_t taddr, uint32_t taddr_gate, int ngate, long long m, bool row_ok,
                                             int nacc, int nout, float mb, const float* rb) {
     uint32_t r[32];
@@ -199,15 +201,14 @@ __device__ __noinline__ void epi_slow_chunk(const GemmParams& p, uint32_t taddr,
     for (int i = 0; i < 32; ++i) v[i] *= p.scale;
     if (row_ok && nout < p.n_store) {
         if (p.residual) {
-            const __half* rp = p.residual + m * p.ld_res + nout;
-            for (int i = 0; i < 32; ++i) if (nout + i < p.n_store) v[i] += __half2float(rp[i]);
+            const uint16_t* rp = reinterpret_cast<const uint16_t*>(p.residual) + m * p.ld_res + nout;
+            for (int i = 0; i < 32; ++i) if (nout + i < p.n_store) v[i] += h_to_f<OBF>(rp[i]);
         }
         if (!p.out_f32 && !p.up2 && nout == 0 && p.n_store <= 4 && p.ldd == 4 && (reinterpret_cast<uintptr_t>(p.D) & 7) == 0) {
             // <= 4 output channels in a 4-wide row (decoder conv_out: 3 of 4): one 8-byte store per pixel; the spare lane gets 0
-            const __half2 h0 = __floats2half2_rn(v[0], p.n_store > 1 ? v[1] : 0.f), h1 = __floats2half2_rn(p.n_store > 2 ? v[2] : 0.f, p.n_store > 3 ? v[3] : 0.f);
-            uint2 u; u.x = *reinterpret_cast<const uint32_t*>(&h0); u.y = *reinterpret_cast<const uint32_t*>(&h1);
-            *reinterpret_cast<uint2*>(reinterpret_cast<__half*>(p.D) + m * 4) = u;
-        } else store_chunk(p, m, nout, v);
+            uint2 u; u.x = pack_h2<OBF>(v[0], p.n_store > 1 ? v[1] : 0.f); u.y = pack_h2<OBF>(p.n_store > 2 ? v[2] : 0.f, p.n_store > 3 ? v[3] : 0.f);
+            *reinterpret_cast<uint2*>(reinterpret_cast<uint16_t*>(p.D) + m * 4) = u;
+        } else store_chunk<OBF>(p, m, nout, v);
     }
 }
 
@@ -220,7 +221,8 @@ __device__ __noinline__ void epi_slow_chunk(const GemmParams& p, uint32_t taddr,
 // CG = 1: one CTA per tile (M = 128).  CG = 2: CTA pair (cta_group::2), tile M = 256, each CTA loads half of B.
 // KPS = 64-wide K blocks per pipeline stage (per producer/consumer mbarrier handshake).
 // MT = 128-row M sub-tiles per CTA that share every B tile (narrow-N problems: twice the MMA work per handshake).
-template <int CG, int KPS, int MT, int GEGLU>
+// OBF = 1: 16-bit outputs and residuals are bf16 (the bf16 VAE); the operand format is a run-time field of the instruction descriptor.
+template <int CG, int KPS, int MT, int GEGLU, int OBF>
 __global__ void __launch_bounds__(384, 1) k_gemm_conv(const __grid_constant__ GemmParams p) {
     extern __shared__ __align__(1024) uint8_t smem_raw[];
     // dynamic smem base is only guaranteed 16-byte aligned by the ABI; round up to 1024 for the 128B swizzle
@@ -362,7 +364,7 @@ __global__ void __launch_bounds__(384, 1) k_gemm_conv(const __grid_constant__ Ge
         }
     } else if (warp == W_MMA && leader) {
         // ===================== MMA issuer (leader CTA of the pair) =====================
-        const uint32_t idesc = umma_idesc_f16(BLOCK_M * CG, block_n);
+        const uint32_t idesc = umma_idesc_f16(BLOCK_M * CG, block_n) | (p.ab_bf16 ? kIdescABBF16 : 0u);
         int stage = 0; uint32_t phase = 0; int it = 0;
         if (p.mode == 2) {
             int ab = 0; uint32_t aph = 0;
@@ -589,7 +591,7 @@ __global__ void __launch_bounds__(384, 1) k_gemm_conv(const __grid_constant__ Ge
                         issue_res(t_, m_, c_, prf0, prf1);
                     }
                     if (!chunk_fast(n_blk, c)) {
-                        epi_slow_chunk(p, tacc + (uint32_t)(c * 32), GEGLU ? tacc + (uint32_t)((block_n >> 1) + c * 32) : 0u, GEGLU ? nacc + (block_n >> 1) : 0,
+                        epi_slow_chunk<OBF>(p, tacc + (uint32_t)(c * 32), GEGLU ? tacc + (uint32_t)((block_n >> 1) + c * 32) : 0u, GEGLU ? nacc + (block_n >> 1) : 0,
                                        m, row_ok, nacc, nout, mb, rb);
                         continue;
                     }
@@ -643,8 +645,8 @@ __global__ void __launch_bounds__(384, 1) k_gemm_conv(const __grid_constant__ Ge
                     if (res_fast && row_ok) {
 #pragma unroll
                         for (int i = 0; i < 8; ++i) {
-                            float2 f = __half22float2(*reinterpret_cast<const __half2*>(&res0[i])); v[2 * i] += f.x; v[2 * i + 1] += f.y;
-                            f = __half22float2(*reinterpret_cast<const __half2*>(&res1[i])); v[16 + 2 * i] += f.x; v[16 + 2 * i + 1] += f.y;
+                            float2 f = unpack_h2<OBF>(res0[i]); v[2 * i] += f.x; v[2 * i + 1] += f.y;
+                            f = unpack_h2<OBF>(res1[i]); v[16 + 2 * i] += f.x; v[16 + 2 * i + 1] += f.y;
                         }
                     }
                     if (p.ln_out) {                                     // LayerNorm statistics of this row of the (fp16-rounded) output
@@ -683,10 +685,7 @@ __global__ void __launch_bounds__(384, 1) k_gemm_conv(const __grid_constant__ Ge
                     } else if (row_ok) {
                         uint32_t o0[8], o1[8];
 #pragma unroll
-                        for (int i = 0; i < 8; ++i) {
-                            __half2 h = __floats2half2_rn(v[2 * i], v[2 * i + 1]); o0[i] = *reinterpret_cast<uint32_t*>(&h);
-                            h = __floats2half2_rn(v[16 + 2 * i], v[16 + 2 * i + 1]); o1[i] = *reinterpret_cast<uint32_t*>(&h);
-                        }
+                        for (int i = 0; i < 8; ++i) { o0[i] = pack_h2<OBF>(v[2 * i], v[2 * i + 1]); o1[i] = pack_h2<OBF>(v[16 + 2 * i], v[16 + 2 * i + 1]); }
                         stg256(orow + nout, o0); stg256(orow + nout + 16, o1);
                     }
                 }
@@ -732,14 +731,14 @@ static PFN_encodeTiled get_encode() {
     return fn;
 }
 
-int make_tmap_f16(CUtensorMap* out, const void* base, int rank, const uint64_t* dims, const uint64_t* strides_bytes, const uint32_t* box) {
+int make_tmap_f16(CUtensorMap* out, const void* base, int rank, const uint64_t* dims, const uint64_t* strides_bytes, const uint32_t* box, bool bf16) {
     PFN_encodeTiled enc = get_encode();
     if (!enc) { set_error("cuTensorMapEncodeTiled not available (driver too old?)"); return FIE_ERR_CUDA; }
     if ((reinterpret_cast<uintptr_t>(base) & 15) != 0) { set_error("TMA base pointer %p not 16-byte aligned", base); return FIE_ERR_INVALID; }
     cuuint64_t gd[5]; cuuint64_t gs[4]; cuuint32_t bx[5]; cuuint32_t es[5];
     for (int i = 0; i < rank; ++i) { gd[i] = dims[i]; bx[i] = box[i]; es[i] = 1; if (box[i] > 256 || box[i] == 0) { set_error("TMA box dim %d = %u out of range", i, box[i]); return FIE_ERR_INVALID; } }
     for (int i = 0; i + 1 < rank; ++i) { gs[i] = strides_bytes[i]; if (gs[i] & 15) { set_error("TMA stride %d = %llu not a multiple of 16 bytes", i, (unsigned long long)gs[i]); return FIE_ERR_INVALID; } }
-    CUresult r = enc(out, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, (cuuint32_t)rank, const_cast<void*>(base), gd, gs, bx, es,
+    CUresult r = enc(out, bf16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT16, (cuuint32_t)rank, const_cast<void*>(base), gd, gs, bx, es,
                      CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                      CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     if (r != CUDA_SUCCESS) { set_error("cuTensorMapEncodeTiled failed with CUresult %d (rank %d dims %llu,%llu box %u,%u)", (int)r, rank,
@@ -787,15 +786,26 @@ static void pick_config(long long M, int N, bool geglu, int* cg_out, int* bn_out
     *cg_out = best_cg; *bn_out = best_bn; *mt_out = best_mt;
 }
 
-static int fill_epilogue(GemmParams& p, const fie_epilogue* ep, long long M, int N, void* D, long long ldd) {
+static int out_dtype_of(const fie_epilogue* ep) { return (ep && ep->out_f32) ? FIE_DT_F32 : FIE_DT_F16; }
+
+// Validation of the explicit output type of the *_bf16 entry points (before any CUDA call).
+static int check_out_dtype(const char* fn, const fie_epilogue* ep, int out_dtype) {
+    FIE_REQUIRE(out_dtype == FIE_DT_F16 || out_dtype == FIE_DT_BF16 || out_dtype == FIE_DT_F32, "%s: bad out_dtype %d", fn, out_dtype);
+    FIE_REQUIRE(!(ep && ep->out_f32 && out_dtype != FIE_DT_F32), "%s: fie_epilogue.out_f32 needs out_dtype FIE_DT_F32", fn);
+    return FIE_OK;
+}
+
+static int fill_epilogue(GemmParams& p, const fie_epilogue* ep, long long M, int N, void* D, long long ldd, int out_dtype) {
     static const fie_epilogue kDefault = {nullptr, nullptr, 1, 0, nullptr, nullptr, 0, 1.0f, FIE_ACT_NONE, 0, nullptr, 0, 0, nullptr, nullptr, 0.0f, 0, nullptr};
     if (!ep) ep = &kDefault;
     p.D = D; p.ldd = ldd;
     p.col_bias = ep->col_bias; p.row_bias = ep->row_bias; p.rows_per_group = ep->rows_per_group > 0 ? ep->rows_per_group : 1;
     p.ld_row_bias = ep->ld_row_bias > 0 ? ep->ld_row_bias : N;
     p.m_bias = ep->m_bias; p.residual = (const __half*)ep->residual; p.ld_res = ep->ld_res;
-    p.scale = ep->scale; p.act = ep->act; p.out_f32 = ep->out_f32;
+    p.scale = ep->scale; p.act = ep->act; p.out_f32 = out_dtype == FIE_DT_F32; p.out_bf16 = out_dtype == FIE_DT_BF16;
     FIE_REQUIRE(p.act >= 0 && p.act <= FIE_ACT_RELU, "epilogue: bad act %d", p.act);
+    FIE_REQUIRE(!(p.out_bf16 && (ep->gn_stats || ep->ln_stats_out || p.act == FIE_ACT_GEGLU)),
+                "epilogue: gn_stats, ln_stats_out and GEGLU need fp16 output (not supported with bf16 output)");
     FIE_REQUIRE(!(p.act == FIE_ACT_GEGLU && (N % 64)), "GEGLU needs N %% 64 == 0");
     FIE_REQUIRE(!(p.residual && p.ld_res <= 0), "epilogue: residual needs ld_res");
     p.gn_stats = (unsigned long long*)ep->gn_stats; p.gn_groups = ep->gn_groups; p.gn_rows = ep->gn_rows_per_image; p.gn_cpg = 0;
@@ -852,20 +862,20 @@ static int launch(GemmParams& p, cudaStream_t stream) {
     size_t smem = (size_t)SMEM_BUDGET + EPI_STAGE_BYTES + 1024;
     // (>113 KiB of dynamic smem: one CTA per SM, so a 512-column TMEM allocation can never deadlock)
     typedef void (*KernelFn)(GemmParams);
-#define FIE_K(cg, kps, mt) {k_gemm_conv<cg, kps, mt, 0>, k_gemm_conv<cg, kps, mt, 1>}
-    static const KernelFn kernels[2][2][2][2] = {{{FIE_K(1, 1, 1), FIE_K(1, 1, 2)}, {FIE_K(1, 2, 1), FIE_K(1, 2, 2)}},
+#define FIE_K(cg, kps, mt) {k_gemm_conv<cg, kps, mt, 0, 0>, k_gemm_conv<cg, kps, mt, 1, 0>, k_gemm_conv<cg, kps, mt, 0, 1>}
+    static const KernelFn kernels[2][2][2][3] = {{{FIE_K(1, 1, 1), FIE_K(1, 1, 2)}, {FIE_K(1, 2, 1), FIE_K(1, 2, 2)}},
                                                  {{FIE_K(2, 1, 1), FIE_K(2, 1, 2)}, {FIE_K(2, 2, 1), FIE_K(2, 2, 2)}}};
 #undef FIE_K
     static bool attr_set_dev[kMaxDevices] = {false};          // cudaFuncSetAttribute is per device
     bool& attr_set = attr_set_dev[current_device()];
     if (!attr_set) {
-        for (int a = 0; a < 2; ++a) for (int b = 0; b < 2; ++b) for (int c = 0; c < 2; ++c) for (int d = 0; d < 2; ++d) {
+        for (int a = 0; a < 2; ++a) for (int b = 0; b < 2; ++b) for (int c = 0; c < 2; ++c) for (int d = 0; d < 3; ++d) {
             cudaError_t e = cudaFuncSetAttribute(kernels[a][b][c][d], cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BUDGET + EPI_STAGE_BYTES + 1024);
             if (e != cudaSuccess) { set_error("cudaFuncSetAttribute(k_gemm_conv): %s", cudaGetErrorString(e)); return FIE_ERR_CUDA; }
         }
         attr_set = true;
     }
-    KernelFn fn = kernels[cg - 1][kps - 1][mt - 1][p.act == FIE_ACT_GEGLU ? 1 : 0];
+    KernelFn fn = kernels[cg - 1][kps - 1][mt - 1][p.act == FIE_ACT_GEGLU ? 1 : (p.out_bf16 ? 2 : 0)];
     const int tiles = p.num_m_blocks * p.num_n_blocks;
     const int slots = num_sms() / cg;
     const int grid = cg * (tiles < slots ? tiles : slots);
@@ -899,19 +909,19 @@ extern "C" void fie_gemm_trace(long long* device_buf) { fie::g_trace = device_bu
 
 extern "C" int fie_geglu_block_n(int N) { return (N % 256) == 0 ? 256 : ((N % 128) == 0 ? 128 : 64); }
 
-extern "C" int fie_gemm_f16(const void* A, long long lda, const void* A1, long long lda1, int k_split,
-                            const void* B, void* D, long long ldd, long long M, int N, int K,
-                            const fie_epilogue* ep, void* stream) {
-    FIE_REQUIRE(A && B && D, "fie_gemm_f16: null pointer");
-    FIE_REQUIRE(M > 0 && N > 0 && K > 0, "fie_gemm_f16: bad shape M=%lld N=%d K=%d", M, N, K);
-    FIE_REQUIRE(M < (1ll << 31), "fie_gemm_f16: M too large");
-    FIE_REQUIRE((lda % 8) == 0 && (K % 8) == 0 && lda >= (A1 ? k_split : K), "fie_gemm_f16: lda/K must be multiples of 8");
+static int gemm_impl(const char* fn, const void* A, long long lda, const void* A1, long long lda1, int k_split,
+                     const void* B, void* D, long long ldd, long long M, int N, int K,
+                     const fie_epilogue* ep, int ab_bf16, int out_dtype, void* stream) {
+    FIE_REQUIRE(A && B && D, "%s: null pointer", fn);
+    FIE_REQUIRE(M > 0 && N > 0 && K > 0, "%s: bad shape M=%lld N=%d K=%d", fn, M, N, K);
+    FIE_REQUIRE(M < (1ll << 31), "%s: M too large", fn);
+    FIE_REQUIRE((lda % 8) == 0 && (K % 8) == 0 && lda >= (A1 ? k_split : K), "%s: lda/K must be multiples of 8", fn);
     GemmParams p;
     memset(&p, 0, sizeof(p));
-    int rc = fill_epilogue(p, ep, M, N, D, ldd);
+    int rc = fill_epilogue(p, ep, M, N, D, ldd, out_dtype);
     if (rc) return rc;
     const bool geglu = p.act == FIE_ACT_GEGLU;
-    p.mode = 0; p.M = M; p.N = N;
+    p.mode = 0; p.M = M; p.N = N; p.ab_bf16 = ab_bf16;
     pick_config(M, N, geglu, &p.cg, &p.block_n, &p.mt);
     p.num_m_blocks = (int)((M + BLOCK_M * p.cg * p.mt - 1) / (BLOCK_M * p.cg * p.mt));
     p.num_n_blocks = (N + p.block_n - 1) / p.block_n;
@@ -920,49 +930,49 @@ extern "C" int fie_gemm_f16(const void* A, long long lda, const void* A1, long l
     p.n_store = geglu ? N / 2 : N;
     uint64_t dims[2], strides[1]; uint32_t box[2];
     if (A1) {
-        FIE_REQUIRE(k_split > 0 && k_split < K && (k_split % BLOCK_K) == 0 && (lda1 % 8) == 0 && lda1 >= K - k_split, "fie_gemm_f16: bad two-source split");
+        FIE_REQUIRE(k_split > 0 && k_split < K && (k_split % BLOCK_K) == 0 && (lda1 % 8) == 0 && lda1 >= K - k_split, "%s: bad two-source split", fn);
         p.kb_split = k_split / BLOCK_K;
         dims[0] = (uint64_t)k_split; dims[1] = (uint64_t)M; strides[0] = (uint64_t)lda * 2; box[0] = BLOCK_K; box[1] = BLOCK_M;
-        if ((rc = make_tmap_f16(&p.a_maps[0], A, 2, dims, strides, box))) return rc;
+        if ((rc = make_tmap_f16(&p.a_maps[0], A, 2, dims, strides, box, ab_bf16 != 0))) return rc;
         dims[0] = (uint64_t)(K - k_split); strides[0] = (uint64_t)lda1 * 2;
-        if ((rc = make_tmap_f16(&p.a_maps[1], A1, 2, dims, strides, box))) return rc;
+        if ((rc = make_tmap_f16(&p.a_maps[1], A1, 2, dims, strides, box, ab_bf16 != 0))) return rc;
     } else {
         dims[0] = (uint64_t)K; dims[1] = (uint64_t)M; strides[0] = (uint64_t)lda * 2; box[0] = BLOCK_K; box[1] = BLOCK_M;
-        if ((rc = make_tmap_f16(&p.a_maps[0], A, 2, dims, strides, box))) return rc;
+        if ((rc = make_tmap_f16(&p.a_maps[0], A, 2, dims, strides, box, ab_bf16 != 0))) return rc;
         p.a_maps[1] = p.a_maps[0];
     }
     p.a_maps[2] = p.a_maps[0]; p.a_maps[3] = p.a_maps[0];
     dims[0] = (uint64_t)K; dims[1] = (uint64_t)N; strides[0] = (uint64_t)K * 2; box[0] = BLOCK_K; box[1] = (uint32_t)(p.block_n / p.cg);
-    if ((rc = make_tmap_f16(&p.b_map, B, 2, dims, strides, box))) return rc;
+    if ((rc = make_tmap_f16(&p.b_map, B, 2, dims, strides, box, ab_bf16 != 0))) return rc;
     return launch(p, (cudaStream_t)stream);
 }
 
-extern "C" int fie_conv3x3_f16(const void* x, const void* wgt, void* out, long long ldd, int n, int h, int w, int cin, int cout,
-                               int cout_valid, int stride, int pad_mode, const fie_epilogue* ep, void* stream) {
-    FIE_REQUIRE(x && wgt && out, "fie_conv3x3_f16: null pointer");
-    FIE_REQUIRE(n > 0 && h > 0 && w > 0 && cin > 0 && cout > 0, "fie_conv3x3_f16: bad shape");
-    FIE_REQUIRE((cin % BLOCK_K) == 0, "fie_conv3x3_f16: cin=%d must be a multiple of 64", cin);
-    FIE_REQUIRE((cout % 32) == 0, "fie_conv3x3_f16: cout=%d (weight rows) must be a multiple of 32", cout);
-    FIE_REQUIRE(stride == 1 || stride == 2, "fie_conv3x3_f16: stride must be 1 or 2");
-    FIE_REQUIRE(stride == 1 || ((h % 2) == 0 && (w % 2) == 0), "fie_conv3x3_f16: stride 2 needs even h, w");
+static int conv3x3_impl(const char* fn, const void* x, const void* wgt, void* out, long long ldd, int n, int h, int w, int cin, int cout,
+                        int cout_valid, int stride, int pad_mode, const fie_epilogue* ep, int ab_bf16, int out_dtype, void* stream) {
+    FIE_REQUIRE(x && wgt && out, "%s: null pointer", fn);
+    FIE_REQUIRE(n > 0 && h > 0 && w > 0 && cin > 0 && cout > 0, "%s: bad shape", fn);
+    FIE_REQUIRE((cin % BLOCK_K) == 0, "%s: cin=%d must be a multiple of 64", fn, cin);
+    FIE_REQUIRE((cout % 32) == 0, "%s: cout=%d (weight rows) must be a multiple of 32", fn, cout);
+    FIE_REQUIRE(stride == 1 || stride == 2, "%s: stride must be 1 or 2", fn);
+    FIE_REQUIRE(stride == 1 || ((h % 2) == 0 && (w % 2) == 0), "%s: stride 2 needs even h, w", fn);
     const int OH = h / stride, OW = w / stride;
     int bw, bh, bn;
-    if (OW >= 128) { FIE_REQUIRE((OW % 128) == 0, "fie_conv3x3_f16: output width %d must be a multiple of 128", OW); bw = 128; bh = 1; bn = 1; }
+    if (OW >= 128) { FIE_REQUIRE((OW % 128) == 0, "%s: output width %d must be a multiple of 128", fn, OW); bw = 128; bh = 1; bn = 1; }
     else {
-        FIE_REQUIRE((128 % OW) == 0, "fie_conv3x3_f16: output width %d must divide 128", OW);
+        FIE_REQUIRE((128 % OW) == 0, "%s: output width %d must divide 128", fn, OW);
         bw = OW; bh = 128 / OW;
-        if (bh <= OH) { FIE_REQUIRE((OH % bh) == 0, "fie_conv3x3_f16: output height %d not a multiple of %d", OH, bh); bn = 1; }
-        else { FIE_REQUIRE((bh % OH) == 0, "fie_conv3x3_f16: output height %d must divide %d", OH, bh); bn = bh / OH; bh = OH; }
+        if (bh <= OH) { FIE_REQUIRE((OH % bh) == 0, "%s: output height %d not a multiple of %d", fn, OH, bh); bn = 1; }
+        else { FIE_REQUIRE((bh % OH) == 0, "%s: output height %d must divide %d", fn, OH, bh); bn = bh / OH; bh = OH; }
     }
     GemmParams p;
     memset(&p, 0, sizeof(p));
     const long long M = (long long)n * OH * OW;
-    int rc = fill_epilogue(p, ep, M, cout, out, ldd);
+    int rc = fill_epilogue(p, ep, M, cout, out, ldd, out_dtype);
     if (rc) return rc;
-    FIE_REQUIRE(p.act != FIE_ACT_GEGLU, "fie_conv3x3_f16: GEGLU epilogue not supported for conv");
+    FIE_REQUIRE(p.act != FIE_ACT_GEGLU, "%s: GEGLU epilogue not supported for conv", fn);
     if (g_halo < 0) { const char* e = getenv("FIE_CONV_HALO"); g_halo = e ? atoi(e) : 1; }
     const bool halo = g_halo > 0 && stride == 1 && (OW % BLOCK_M) == 0 && cout <= g_halo_max_cout;
-    p.mode = halo ? 2 : 1; p.M = M; p.N = cout; p.OH = OH; p.OW = OW;
+    p.mode = halo ? 2 : 1; p.M = M; p.N = cout; p.OH = OH; p.OW = OW; p.ab_bf16 = ab_bf16;
     pick_config(M, cout, false, &p.cg, &p.block_n, &p.mt, halo ? 1 : 2);
     p.num_m_blocks = (int)((M + BLOCK_M * p.cg * p.mt - 1) / (BLOCK_M * p.cg * p.mt));
     p.num_n_blocks = (cout + p.block_n - 1) / p.block_n;
@@ -974,7 +984,7 @@ extern "C" int fie_conv3x3_f16(const void* x, const void* wgt, void* out, long l
     if (stride == 1) {
         const uint64_t dims[4] = {(uint64_t)cin, (uint64_t)w, (uint64_t)h, (uint64_t)n};
         const uint64_t strides[3] = {(uint64_t)cin * 2, (uint64_t)w * cin * 2, (uint64_t)h * w * cin * 2};
-        if ((rc = make_tmap_f16(&p.a_maps[0], x, 4, dims, strides, box))) return rc;
+        if ((rc = make_tmap_f16(&p.a_maps[0], x, 4, dims, strides, box, ab_bf16 != 0))) return rc;
         p.a_maps[1] = p.a_maps[0]; p.a_maps[2] = p.a_maps[0]; p.a_maps[3] = p.a_maps[0];
         for (int t = 0; t < 9; ++t) { p.tap_map[t] = 0; p.tap_dh[t] = (int8_t)(t / 3 - 1); p.tap_dw[t] = (int8_t)(t % 3 - 1); }
     } else {
@@ -984,7 +994,7 @@ extern "C" int fie_conv3x3_f16(const void* x, const void* wgt, void* out, long l
         for (int hp = 0; hp < 2; ++hp)
             for (int wp = 0; wp < 2; ++wp) {
                 const uint8_t* base = (const uint8_t*)x + ((size_t)hp * w + wp) * cin * 2;
-                if ((rc = make_tmap_f16(&p.a_maps[hp * 2 + wp], base, 4, dims, strides, box))) return rc;
+                if ((rc = make_tmap_f16(&p.a_maps[hp * 2 + wp], base, 4, dims, strides, box, ab_bf16 != 0))) return rc;
             }
         // input row = 2*oh + k - pad:  pad 1: k=0 -> (parity 1, shift -1), k=1 -> (0, 0), k=2 -> (1, 0)
         //                              pad 0 (asymmetric (0,1) padding): k=0 -> (0, 0), k=1 -> (1, 0), k=2 -> (0, +1)
@@ -998,7 +1008,7 @@ extern "C" int fie_conv3x3_f16(const void* x, const void* wgt, void* out, long l
     const uint64_t bdims[2] = {(uint64_t)9 * cin, (uint64_t)cout};
     const uint64_t bstr[1] = {(uint64_t)9 * cin * 2};
     const uint32_t bbox[2] = {BLOCK_K, (uint32_t)(p.block_n / p.cg)};
-    if ((rc = make_tmap_f16(&p.b_map, wgt, 2, bdims, bstr, bbox))) return rc;
+    if ((rc = make_tmap_f16(&p.b_map, wgt, 2, bdims, bstr, bbox, ab_bf16 != 0))) return rc;
     return launch(p, (cudaStream_t)stream);
 }
 
@@ -1006,27 +1016,27 @@ extern "C" int fie_conv3x3_f16(const void* x, const void* wgt, void* out, long l
 // conv3x3).  Output pixel (2i+a, 2j+b) only ever sees a 2x2 neighbourhood of the input, with the 3x3 taps that land on the
 // same input pixel pre-summed by the host: four phase convolutions with 2x2 taps = 16/36 of the FLOPs and no upsampled
 // tensor in HBM.  wgt: fp16 [4 phases (a*2+b)][cout][2][2][cin].
-extern "C" int fie_conv_up2x_f16(const void* x, const void* wgt, void* out, long long ldd, int n, int h, int w, int cin, int cout,
-                                 const fie_epilogue* ep, void* stream) {
-    FIE_REQUIRE(x && wgt && out, "fie_conv_up2x_f16: null pointer");
-    FIE_REQUIRE(n > 0 && h > 0 && w > 0 && cin > 0 && cout > 0, "fie_conv_up2x_f16: bad shape");
-    FIE_REQUIRE((cin % BLOCK_K) == 0 && (cout % 32) == 0, "fie_conv_up2x_f16: cin %% 64 and cout %% 32 required");
+static int conv_up2x_impl(const char* fn, const void* x, const void* wgt, void* out, long long ldd, int n, int h, int w, int cin, int cout,
+                          const fie_epilogue* ep, int ab_bf16, int out_dtype, void* stream) {
+    FIE_REQUIRE(x && wgt && out, "%s: null pointer", fn);
+    FIE_REQUIRE(n > 0 && h > 0 && w > 0 && cin > 0 && cout > 0, "%s: bad shape", fn);
+    FIE_REQUIRE((cin % BLOCK_K) == 0 && (cout % 32) == 0, "%s: cin %% 64 and cout %% 32 required", fn);
     int bw, bh, bn;
-    if (w >= 128) { FIE_REQUIRE((w % 128) == 0, "fie_conv_up2x_f16: width %d must be a multiple of 128", w); bw = 128; bh = 1; bn = 1; }
+    if (w >= 128) { FIE_REQUIRE((w % 128) == 0, "%s: width %d must be a multiple of 128", fn, w); bw = 128; bh = 1; bn = 1; }
     else {
-        FIE_REQUIRE((128 % w) == 0, "fie_conv_up2x_f16: width %d must divide 128", w);
+        FIE_REQUIRE((128 % w) == 0, "%s: width %d must divide 128", fn, w);
         bw = w; bh = 128 / w;
-        if (bh <= h) { FIE_REQUIRE((h % bh) == 0, "fie_conv_up2x_f16: height %d not a multiple of %d", h, bh); bn = 1; }
-        else { FIE_REQUIRE((bh % h) == 0, "fie_conv_up2x_f16: height %d must divide %d", h, bh); bn = bh / h; bh = h; }
+        if (bh <= h) { FIE_REQUIRE((h % bh) == 0, "%s: height %d not a multiple of %d", fn, h, bh); bn = 1; }
+        else { FIE_REQUIRE((bh % h) == 0, "%s: height %d must divide %d", fn, h, bh); bn = bh / h; bh = h; }
     }
     const long long M = (long long)n * h * w;
     for (int ph = 0; ph < 4; ++ph) {
         GemmParams p;
         memset(&p, 0, sizeof(p));
-        int rc = fill_epilogue(p, ep, M, cout, out, ldd);
+        int rc = fill_epilogue(p, ep, M, cout, out, ldd, out_dtype);
         if (rc) return rc;
-        FIE_REQUIRE(p.act != FIE_ACT_GEGLU && !p.residual && !p.out_f32, "fie_conv_up2x_f16: unsupported epilogue");
-        p.mode = 1; p.M = M; p.N = cout; p.OH = h; p.OW = w;
+        FIE_REQUIRE(p.act != FIE_ACT_GEGLU && !p.residual && !p.out_f32, "%s: unsupported epilogue", fn);
+        p.mode = 1; p.M = M; p.N = cout; p.OH = h; p.OW = w; p.ab_bf16 = ab_bf16;
         p.up2 = 1; p.up_a = ph >> 1; p.up_b = ph & 1;
         pick_config(M, cout, false, &p.cg, &p.block_n, &p.mt);
         p.num_m_blocks = (int)((M + BLOCK_M * p.cg * p.mt - 1) / (BLOCK_M * p.cg * p.mt));
@@ -1038,7 +1048,7 @@ extern "C" int fie_conv_up2x_f16(const void* x, const void* wgt, void* out, long
         const uint32_t box[4] = {BLOCK_K, (uint32_t)bw, (uint32_t)bh, (uint32_t)bn};
         const uint64_t dims[4] = {(uint64_t)cin, (uint64_t)w, (uint64_t)h, (uint64_t)n};
         const uint64_t strides[3] = {(uint64_t)cin * 2, (uint64_t)w * cin * 2, (uint64_t)h * w * cin * 2};
-        if ((rc = make_tmap_f16(&p.a_maps[0], x, 4, dims, strides, box))) return rc;
+        if ((rc = make_tmap_f16(&p.a_maps[0], x, 4, dims, strides, box, ab_bf16 != 0))) return rc;
         p.a_maps[1] = p.a_maps[0]; p.a_maps[2] = p.a_maps[0]; p.a_maps[3] = p.a_maps[0];
         for (int t = 0; t < 4; ++t) {   // tap (ty, tx): input row i + ty - 1 + a, column j + tx - 1 + b
             p.tap_map[t] = 0; p.tap_dh[t] = (int8_t)((t >> 1) - 1 + p.up_a); p.tap_dw[t] = (int8_t)((t & 1) - 1 + p.up_b);
@@ -1047,7 +1057,7 @@ extern "C" int fie_conv_up2x_f16(const void* x, const void* wgt, void* out, long
         const uint64_t bstr[1] = {(uint64_t)4 * cin * 2};
         const uint32_t bbox[2] = {BLOCK_K, (uint32_t)(p.block_n / p.cg)};
         const uint8_t* wp = (const uint8_t*)wgt + (size_t)ph * cout * 4 * cin * 2;
-        if ((rc = make_tmap_f16(&p.b_map, wp, 2, bdims, bstr, bbox))) return rc;
+        if ((rc = make_tmap_f16(&p.b_map, wp, 2, bdims, bstr, bbox, ab_bf16 != 0))) return rc;
         if ((rc = launch(p, (cudaStream_t)stream))) return rc;
     }
     return FIE_OK;
@@ -1060,24 +1070,24 @@ extern "C" int fie_conv_up2x_f16(const void* x, const void* wgt, void* out, long
 // (8 padded pixels, of which the first 3 carry non-zero weights), dimension 1 = start pixel with a 16-byte stride.  K = 3 kernel
 // rows x 64, so the generic implicit-GEMM kernel runs unchanged with 3 "taps" of one K block each.
 // wgt: fp16 [cout][3][2][64]: per kernel row a hi and a lo block (w = hi + lo to ~2^-22), element kw*8 + c = w[co][c][kh][kw].
-extern "C" int fie_conv3x3_c8_f16(const void* xp, const void* wgt, void* out, long long ldd, int n, int h, int w, int cout,
-                                  int cout_valid, const fie_epilogue* ep, void* stream) {
-    FIE_REQUIRE(xp && wgt && out, "fie_conv3x3_c8_f16: null pointer");
-    FIE_REQUIRE(n > 0 && h > 0 && w > 0 && cout > 0 && (cout % 32) == 0, "fie_conv3x3_c8_f16: bad shape (cout must be a multiple of 32)");
+static int conv3x3_c8_impl(const char* fn, const void* xp, const void* wgt, void* out, long long ldd, int n, int h, int w, int cout,
+                           int cout_valid, const fie_epilogue* ep, int out_dtype, void* stream) {
+    FIE_REQUIRE(xp && wgt && out, "%s: null pointer", fn);
+    FIE_REQUIRE(n > 0 && h > 0 && w > 0 && cout > 0 && (cout % 32) == 0, "%s: bad shape (cout must be a multiple of 32)", fn);
     int bw, bh, bn;
-    if (w >= 128) { FIE_REQUIRE((w % 128) == 0, "fie_conv3x3_c8_f16: width %d must be a multiple of 128", w); bw = 128; bh = 1; bn = 1; }
+    if (w >= 128) { FIE_REQUIRE((w % 128) == 0, "%s: width %d must be a multiple of 128", fn, w); bw = 128; bh = 1; bn = 1; }
     else {
-        FIE_REQUIRE((128 % w) == 0, "fie_conv3x3_c8_f16: width %d must divide 128", w);
+        FIE_REQUIRE((128 % w) == 0, "%s: width %d must divide 128", fn, w);
         bw = w; bh = 128 / w;
-        if (bh <= h) { FIE_REQUIRE((h % bh) == 0, "fie_conv3x3_c8_f16: height %d not a multiple of %d", h, bh); bn = 1; }
-        else { FIE_REQUIRE((bh % h) == 0, "fie_conv3x3_c8_f16: height %d must divide %d", h, bh); bn = bh / h; bh = h; }
+        if (bh <= h) { FIE_REQUIRE((h % bh) == 0, "%s: height %d not a multiple of %d", fn, h, bh); bn = 1; }
+        else { FIE_REQUIRE((bh % h) == 0, "%s: height %d must divide %d", fn, h, bh); bn = bh / h; bh = h; }
     }
     GemmParams p;
     memset(&p, 0, sizeof(p));
     const long long M = (long long)n * h * w;
-    int rc = fill_epilogue(p, ep, M, cout, out, ldd);
+    int rc = fill_epilogue(p, ep, M, cout, out, ldd, out_dtype);
     if (rc) return rc;
-    FIE_REQUIRE(p.act != FIE_ACT_GEGLU, "fie_conv3x3_c8_f16: GEGLU epilogue not supported for conv");
+    FIE_REQUIRE(p.act != FIE_ACT_GEGLU, "%s: GEGLU epilogue not supported for conv", fn);
     p.mode = 1; p.M = M; p.N = cout; p.OH = h; p.OW = w;
     pick_config(M, cout, false, &p.cg, &p.block_n, &p.mt);
     p.num_m_blocks = (int)((M + BLOCK_M * p.cg * p.mt - 1) / (BLOCK_M * p.cg * p.mt));
@@ -1096,4 +1106,48 @@ extern "C" int fie_conv3x3_c8_f16(const void* xp, const void* wgt, void* out, lo
     const uint32_t bbox[2] = {BLOCK_K, (uint32_t)(p.block_n / p.cg)};
     if ((rc = make_tmap_f16(&p.b_map, wgt, 2, bdims, bstr, bbox))) return rc;
     return launch(p, (cudaStream_t)stream);
+}
+
+extern "C" int fie_gemm_f16(const void* A, long long lda, const void* A1, long long lda1, int k_split, const void* B, void* D, long long ldd,
+                            long long M, int N, int K, const fie_epilogue* ep, void* stream) {
+    return gemm_impl("fie_gemm_f16", A, lda, A1, lda1, k_split, B, D, ldd, M, N, K, ep, 0, out_dtype_of(ep), stream);
+}
+
+extern "C" int fie_gemm_bf16(const void* A, long long lda, const void* A1, long long lda1, int k_split, const void* B, void* D, long long ldd,
+                             long long M, int N, int K, const fie_epilogue* ep, int out_dtype, void* stream) {
+    if (int rc = check_out_dtype("fie_gemm_bf16", ep, out_dtype)) return rc;
+    return gemm_impl("fie_gemm_bf16", A, lda, A1, lda1, k_split, B, D, ldd, M, N, K, ep, 1, out_dtype, stream);
+}
+
+extern "C" int fie_conv3x3_f16(const void* x, const void* wgt, void* out, long long ldd, int n, int h, int w, int cin, int cout,
+                               int cout_valid, int stride, int pad_mode, const fie_epilogue* ep, void* stream) {
+    return conv3x3_impl("fie_conv3x3_f16", x, wgt, out, ldd, n, h, w, cin, cout, cout_valid, stride, pad_mode, ep, 0, out_dtype_of(ep), stream);
+}
+
+extern "C" int fie_conv3x3_bf16(const void* x, const void* wgt, void* out, long long ldd, int n, int h, int w, int cin, int cout,
+                                int cout_valid, int stride, int pad_mode, const fie_epilogue* ep, int out_dtype, void* stream) {
+    if (int rc = check_out_dtype("fie_conv3x3_bf16", ep, out_dtype)) return rc;
+    return conv3x3_impl("fie_conv3x3_bf16", x, wgt, out, ldd, n, h, w, cin, cout, cout_valid, stride, pad_mode, ep, 1, out_dtype, stream);
+}
+
+extern "C" int fie_conv_up2x_f16(const void* x, const void* wgt, void* out, long long ldd, int n, int h, int w, int cin, int cout,
+                                 const fie_epilogue* ep, void* stream) {
+    return conv_up2x_impl("fie_conv_up2x_f16", x, wgt, out, ldd, n, h, w, cin, cout, ep, 0, out_dtype_of(ep), stream);
+}
+
+extern "C" int fie_conv_up2x_bf16(const void* x, const void* wgt, void* out, long long ldd, int n, int h, int w, int cin, int cout,
+                                  const fie_epilogue* ep, int out_dtype, void* stream) {
+    if (int rc = check_out_dtype("fie_conv_up2x_bf16", ep, out_dtype)) return rc;
+    return conv_up2x_impl("fie_conv_up2x_bf16", x, wgt, out, ldd, n, h, w, cin, cout, ep, 1, out_dtype, stream);
+}
+
+extern "C" int fie_conv3x3_c8_f16(const void* xp, const void* wgt, void* out, long long ldd, int n, int h, int w, int cout,
+                                  int cout_valid, const fie_epilogue* ep, void* stream) {
+    return conv3x3_c8_impl("fie_conv3x3_c8_f16", xp, wgt, out, ldd, n, h, w, cout, cout_valid, ep, out_dtype_of(ep), stream);
+}
+
+extern "C" int fie_conv3x3_c8_bf16(const void* xp, const void* wgt, void* out, long long ldd, int n, int h, int w, int cout,
+                                   int cout_valid, const fie_epilogue* ep, int out_dtype, void* stream) {
+    if (int rc = check_out_dtype("fie_conv3x3_c8_bf16", ep, out_dtype)) return rc;
+    return conv3x3_c8_impl("fie_conv3x3_c8_bf16", xp, wgt, out, ldd, n, h, w, cout, cout_valid, ep, out_dtype, stream);
 }

@@ -9,17 +9,20 @@
 //   fie_pack_rows_f16         [N,K] fp32 -> fp16 [N,K] with an optional row permutation (GEGLU tile interleave) and bias gather
 //   fie_fold_layernorm_f16    LayerNorm(gamma, beta) folded into the following Linear: W'' = centred(W * gamma) fp16, b'' = b + W beta
 //   fie_fuse_lora_f32         W += scale * B A  (LCM-LoRA fuse, fp32; conv weights viewed as [O, I*k*k])
+//   fie_pack_{conv3x3,conv_up2x,rows}_bf16: the same layouts with bf16 elements (the bf16 VAE)
 #include "fie_common.cuh"
 
 namespace fie {
 
-__global__ void __launch_bounds__(256) k_pack_conv3x3(const float* __restrict__ w, __half* __restrict__ out, int O, int I, int Op, int Ip) {
+// OBF: bf16 elements instead of fp16 (the bf16 VAE); same layouts.
+template <bool OBF>
+__global__ void __launch_bounds__(256) k_pack_conv3x3(const float* __restrict__ w, uint16_t* __restrict__ out, int O, int I, int Op, int Ip) {
     const long long total = (long long)Op * 9 * Ip;
     for (long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x; e < total; e += (long long)gridDim.x * blockDim.x) {
         const int i = (int)(e % Ip), t = (int)((e / Ip) % 9), o = (int)(e / ((long long)9 * Ip));
         float v = 0.f;
         if (o < O && i < I) v = w[(((long long)o * I + i) * 9) + t];          // OIHW: tap t = kh * 3 + kw
-        out[e] = __float2half_rn(v);
+        out[e] = f_to_h<OBF>(v);
     }
 }
 
@@ -37,7 +40,8 @@ __global__ void __launch_bounds__(256) k_pack_conv3x3_c8(const float* __restrict
     }
 }
 
-__global__ void __launch_bounds__(256) k_pack_conv_up2x(const float* __restrict__ w, __half* __restrict__ out, int O, int I) {
+template <bool OBF>
+__global__ void __launch_bounds__(256) k_pack_conv_up2x(const float* __restrict__ w, uint16_t* __restrict__ out, int O, int I) {
     // phase (a, b), tap (ty, tx): sum of the 3x3 taps that land on input pixel (i + ty - 1 + a, j + tx - 1 + b) of the 2x-upsampled conv.
     // a = 0: ty 0 <- kh {0}, ty 1 <- kh {1, 2};  a = 1: ty 0 <- kh {0, 1}, ty 1 <- kh {2}; identically for columns.
     const long long total = (long long)4 * O * 4 * I;
@@ -56,17 +60,18 @@ __global__ void __launch_bounds__(256) k_pack_conv_up2x(const float* __restrict_
             acc = first_col ? r : acc + r;
             first_col = false;
         }
-        out[e] = __float2half_rn(acc);
+        out[e] = f_to_h<OBF>(acc);
     }
 }
 
+template <bool OBF>
 __global__ void __launch_bounds__(256) k_pack_rows(const float* __restrict__ w, const float* __restrict__ b, const int* __restrict__ perm,
-                                                   __half* __restrict__ out_w, float* __restrict__ out_b, int N, int K) {
+                                                   uint16_t* __restrict__ out_w, float* __restrict__ out_b, int N, int K) {
     const long long total = (long long)N * K;
     for (long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x; e < total; e += (long long)gridDim.x * blockDim.x) {
         const int n = (int)(e / K), k = (int)(e % K);
         const int src = perm ? perm[n] : n;
-        out_w[e] = __float2half_rn(w[(long long)src * K + k]);
+        out_w[e] = f_to_h<OBF>(w[(long long)src * K + k]);
         if (k == 0 && b && out_b) out_b[n] = b[src];
     }
 }
@@ -134,8 +139,14 @@ using namespace fie;
 
 extern "C" int fie_pack_conv3x3_f16(const float* w, void* out, int cout, int cin, int cout_pad, int cin_pad, void* stream) {
     FIE_REQUIRE(w && out && cout > 0 && cin > 0 && cout_pad >= cout && cin_pad >= cin, "fie_pack_conv3x3_f16: bad arguments");
-    k_pack_conv3x3<<<grid_for((long long)cout_pad * 9 * cin_pad), 256, 0, (cudaStream_t)stream>>>(w, (__half*)out, cout, cin, cout_pad, cin_pad);
+    k_pack_conv3x3<false><<<grid_for((long long)cout_pad * 9 * cin_pad), 256, 0, (cudaStream_t)stream>>>(w, (uint16_t*)out, cout, cin, cout_pad, cin_pad);
     return check_launch("fie_pack_conv3x3_f16");
+}
+
+extern "C" int fie_pack_conv3x3_bf16(const float* w, void* out, int cout, int cin, int cout_pad, int cin_pad, void* stream) {
+    FIE_REQUIRE(w && out && cout > 0 && cin > 0 && cout_pad >= cout && cin_pad >= cin, "fie_pack_conv3x3_bf16: bad arguments");
+    k_pack_conv3x3<true><<<grid_for((long long)cout_pad * 9 * cin_pad), 256, 0, (cudaStream_t)stream>>>(w, (uint16_t*)out, cout, cin, cout_pad, cin_pad);
+    return check_launch("fie_pack_conv3x3_bf16");
 }
 
 extern "C" int fie_pack_conv3x3_c8_f16(const float* w, void* out, int cout, int cin, int cout_pad, void* stream) {
@@ -146,14 +157,26 @@ extern "C" int fie_pack_conv3x3_c8_f16(const float* w, void* out, int cout, int 
 
 extern "C" int fie_pack_conv_up2x_f16(const float* w, void* out, int cout, int cin, void* stream) {
     FIE_REQUIRE(w && out && cout > 0 && cin > 0, "fie_pack_conv_up2x_f16: bad arguments");
-    k_pack_conv_up2x<<<grid_for((long long)16 * cout * cin), 256, 0, (cudaStream_t)stream>>>(w, (__half*)out, cout, cin);
+    k_pack_conv_up2x<false><<<grid_for((long long)16 * cout * cin), 256, 0, (cudaStream_t)stream>>>(w, (uint16_t*)out, cout, cin);
     return check_launch("fie_pack_conv_up2x_f16");
+}
+
+extern "C" int fie_pack_conv_up2x_bf16(const float* w, void* out, int cout, int cin, void* stream) {
+    FIE_REQUIRE(w && out && cout > 0 && cin > 0, "fie_pack_conv_up2x_bf16: bad arguments");
+    k_pack_conv_up2x<true><<<grid_for((long long)16 * cout * cin), 256, 0, (cudaStream_t)stream>>>(w, (uint16_t*)out, cout, cin);
+    return check_launch("fie_pack_conv_up2x_bf16");
 }
 
 extern "C" int fie_pack_rows_f16(const float* w, const float* bias, const int* perm, void* out_w, float* out_bias, int n, int k, void* stream) {
     FIE_REQUIRE(w && out_w && n > 0 && k > 0 && (!bias || out_bias), "fie_pack_rows_f16: bad arguments");
-    k_pack_rows<<<grid_for((long long)n * k), 256, 0, (cudaStream_t)stream>>>(w, bias, perm, (__half*)out_w, out_bias, n, k);
+    k_pack_rows<false><<<grid_for((long long)n * k), 256, 0, (cudaStream_t)stream>>>(w, bias, perm, (uint16_t*)out_w, out_bias, n, k);
     return check_launch("fie_pack_rows_f16");
+}
+
+extern "C" int fie_pack_rows_bf16(const float* w, const float* bias, const int* perm, void* out_w, float* out_bias, int n, int k, void* stream) {
+    FIE_REQUIRE(w && out_w && n > 0 && k > 0 && (!bias || out_bias), "fie_pack_rows_bf16: bad arguments");
+    k_pack_rows<true><<<grid_for((long long)n * k), 256, 0, (cudaStream_t)stream>>>(w, bias, perm, (uint16_t*)out_w, out_bias, n, k);
+    return check_launch("fie_pack_rows_bf16");
 }
 
 extern "C" int fie_fold_layernorm_f16(const float* w, const float* bias, const float* gamma, const float* beta, void* out_w, float* out_bias,

@@ -259,9 +259,12 @@ __device__ __forceinline__ uint64_t umma_desc_sw128(uint32_t smem_addr, uint32_t
 __host__ __device__ constexpr uint32_t umma_idesc_f16(int M, int N, int a_mn_major = 0, int b_mn_major = 0) {
     return (1u << 4) | ((uint32_t)a_mn_major << 15) | ((uint32_t)b_mn_major << 16) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
 }
+// OR-ed into it: A format (bits 7-9) and B format (bits 10-12) = 1 (BF16).  Same MMA rate; both operands always share the type.
+constexpr uint32_t kIdescABBF16 = (1u << 7) | (1u << 10);
 
 // ---------------- host: TMA descriptors ----------------
-// Encodes a tiled fp16 tensor map with 128B swizzle. dims/strides innermost-first; strides (bytes) for dims 1..rank-1.
-int make_tmap_f16(CUtensorMap* out, const void* base, int rank, const uint64_t* dims, const uint64_t* strides_bytes, const uint32_t* box);
+// Encodes a tiled fp16 (bf16 = true: bf16) tensor map with 128B swizzle. dims/strides innermost-first; strides (bytes) for dims 1..rank-1.
+int make_tmap_f16(CUtensorMap* out, const void* base, int rank, const uint64_t* dims, const uint64_t* strides_bytes, const uint32_t* box,
+                  bool bf16 = false);
 
 }  // namespace fie

@@ -15,6 +15,7 @@ Differences, all forced by the environment and stated in DESIGN.md:
 * compute is fp16 with fp32 accumulation on the GPU.  ``use_full_precision=True`` is accepted and ``.dtype`` reports
   ``torch.float32`` like the reference (callers only use it for naming), but the kernels stay fp16 and a warning says so;
   ``.compute_dtype`` is always ``torch.float16``.  ``enable_cpu_offload`` is a no-op on a 180 GB part.
+  The VAE alone may run in bf16 (``vae_dtype``, ``.vae_dtype``): by default whenever its ``config.json`` says ``"force_upcast": true``.
 """
 from __future__ import annotations
 
@@ -57,6 +58,26 @@ def expand_checkpoints(root: str, controlnet: Optional[str], vae: Optional[str] 
     return ck
 
 
+def resolve_vae_dtype(vae_dtype: Optional[torch.dtype], force_upcast: Optional[bool]) -> torch.dtype:
+    """``FastEditor(vae_dtype=...)``: None -> bf16 when the VAE config says ``force_upcast: true`` (activations beyond the fp16 range),
+    else fp16; ``torch.float16`` / ``torch.bfloat16`` force the choice."""
+    if vae_dtype is None:
+        return torch.bfloat16 if force_upcast else torch.float16
+    if vae_dtype not in (torch.float16, torch.bfloat16):
+        raise ValueError(f"vae_dtype must be None, torch.float16 or torch.bfloat16, not {vae_dtype}")
+    return vae_dtype
+
+
+def vae_fp16_warning(real_weights: bool, vae_dtype: torch.dtype, force_upcast: Optional[bool]) -> Optional[str]:
+    """The RuntimeWarning text when a loaded VAE checkpoint runs in fp16 without its config stating ``force_upcast: false`` (diffusers
+    treats a missing key as true and upcasts), else None."""
+    if not real_weights or vae_dtype != torch.float16 or force_upcast is False:
+        return None
+    return ("FastEditor: the VAE runs in fp16, but its config.json does not state \"force_upcast\": false; a VAE whose activations exceed "
+            "the fp16 range (e.g. stabilityai/sdxl-vae) gives inf/NaN images in fp16.  Use the fp16-fix VAE (madebyollin/sdxl-vae-fp16-fix, "
+            "--vae_dir) or FastEditor(vae_dtype=torch.bfloat16) (--vae_dtype bf16).")
+
+
 class _PipeShim:
     """What callers touch on ``editor.pipe``: ``run_batch.py:157-158`` calls ``set_progress_bar_config(disable=True)``."""
 
@@ -91,7 +112,7 @@ class FastEditor:
     def __init__(self, model_name="sdxl", device="cuda", dtype=torch.float16, enable_cpu_offload=True, use_full_precision=False,
                  use_full_controlnet=False, *, state: Optional[Dict] = None, prompt_encoder: Optional[Callable] = None, tiny: bool = False,
                  text_encoders: bool = False, checkpoints: Optional[Dict[str, str]] = None, tokenizers: Optional[Sequence[str]] = None,
-                 verbose: bool = True):
+                 verbose: bool = True, vae_dtype: Optional[torch.dtype] = None):
         if model_name not in self.MODEL_CONFIGS:
             raise ValueError(f"Unknown model: {model_name}. Choose from {list(self.MODEL_CONFIGS.keys())}")
         self.model_name = model_name
@@ -132,6 +153,13 @@ class FastEditor:
         if use_full_precision:
             # the one fp32 lever the engine has: VAE mid-block attention logits kept in fp32 between the passes (engine._VAEAttention)
             state = dict(state, vae_scores_f32=True)
+        force_upcast = getattr(state["vae_cfg"], "force_upcast", None)
+        self.vae_dtype = resolve_vae_dtype(vae_dtype, force_upcast)
+        msg = vae_fp16_warning(bool(checkpoints) and not self.synthetic_weights, self.vae_dtype, force_upcast)
+        if msg:
+            warnings.warn(msg, RuntimeWarning, stacklevel=2)
+        state = dict(state, vae_dtype=self.vae_dtype)
+        self._say(f"[FastEditor] VAE dtype: {self.vae_dtype}")
         with torch.cuda.device(self._dev):
             self._engine = model_zoo.build_engine(state, self._dev)
         self._engine.use_graphs = True      # every edit has the same shapes: replay it as one CUDA graph after the first call

@@ -43,8 +43,9 @@ def _pad64(n: int) -> int:
 class _Packer:
     """Pulls tensors out of a diffusers-style state dict, applies the LoRA fuse, moves them to the device."""
 
-    def __init__(self, params: Params, device, lora: Optional[Params] = None, lora_scale: float = 1.0, prefix: str = ""):
+    def __init__(self, params: Params, device, lora: Optional[Params] = None, lora_scale: float = 1.0, prefix: str = "", dtype=torch.float16):
         self.p, self.dev, self.lora, self.ls, self.prefix = params, device, lora, lora_scale, prefix
+        self.dtype = dtype        # element type of the packed GEMM / convolution weights (fp16, or bf16 for the bf16 VAE)
 
     def w(self, name: str) -> Tensor:
         """fp32 weight on the device with the LoRA delta (if any) fused."""
@@ -61,10 +62,10 @@ class _Packer:
         return (self.prefix + name + ".weight") in self.p
 
     def linear(self, name: str) -> Tuple[Tensor, Optional[Tensor]]:
-        return cast_f16(self.w(name)), self.b(name)
+        return cast_f16(self.w(name), self.dtype), self.b(name)
 
     def conv3(self, name: str, pad_cout_to=None, pad_cin_to=None) -> Tuple[Tensor, Optional[Tensor]]:
-        w = pack_conv3x3(self.w(name), pad_cout_to, pad_cin_to)
+        w = pack_conv3x3(self.w(name), pad_cout_to, pad_cin_to, self.dtype)
         b = self.b(name)
         if b is not None and pad_cout_to and pad_cout_to > b.numel():
             bp = torch.zeros(pad_cout_to, dtype=torch.float32, device=self.dev)
@@ -74,11 +75,11 @@ class _Packer:
 
     def conv_up(self, name: str) -> Tuple[Tensor, Optional[Tensor]]:
         """Upsample2D conv: phase-decomposed weights for the fused nearest-2x upsample + conv3x3 kernel."""
-        return pack_conv_up2x(self.w(name)), self.b(name)
+        return pack_conv_up2x(self.w(name), self.dtype), self.b(name)
 
     def conv1(self, name: str) -> Tuple[Tensor, Optional[Tensor]]:
         w = self.w(name)
-        return cast_f16(w.reshape(w.shape[0], w.shape[1])), self.b(name)
+        return cast_f16(w.reshape(w.shape[0], w.shape[1]), self.dtype), self.b(name)
 
     def cin4(self, name: str) -> Tuple[Tensor, Optional[Tensor]]:
         """[Cout, Cin<=4, 3, 3] -> fp32 [Cout, 3, 3, 4] for the CUDA-core conv_in kernel."""
@@ -88,7 +89,8 @@ class _Packer:
         return out.contiguous(), self.b(name)
 
     def c8(self, name: str, pad_cout_to=None) -> Tuple[Tensor, Optional[Tensor]]:
-        """[Cout, Cin<=8, 3, 3] -> fp16 [Cout_p, 192] for the tensor-core conv_in on a zero-padded 8-channel image."""
+        """[Cout, Cin<=8, 3, 3] -> fp16 [Cout_p, 192] for the tensor-core conv_in on a zero-padded 8-channel image (fp16 also for the
+        bf16 VAE: its inputs are bounded, only its output is bf16)."""
         w = pack_conv3x3_c8(self.w(name), pad_cout_to)
         b = self.b(name)
         if b is not None and pad_cout_to and pad_cout_to > b.numel():
@@ -129,11 +131,12 @@ class Resnet:
     def __call__(self, x: Tensor, temb_all: Optional[Tensor] = None, skip: Optional[Tensor] = None) -> Tensor:
         n, h, w, _ = x.shape
         hcur = ops.groupnorm(x, self.n1[0], self.n1[1], self.eps, True, self.groups, skip)
+        gn = self.groups if self.w1.dtype == torch.float16 else 0      # bf16: no producer-side GroupNorm statistics
         if self.temb_off is not None:
             rb = temb_all[:, self.temb_off:self.temb_off + self.cout]
-            hcur = ops.conv3x3(hcur, self.w1, row_bias=rb, rows_per_group=h * w, gn_groups=self.groups)
+            hcur = ops.conv3x3(hcur, self.w1, row_bias=rb, rows_per_group=h * w, gn_groups=gn)
         else:
-            hcur = ops.conv3x3(hcur, self.w1, col_bias=self.b1, gn_groups=self.groups)
+            hcur = ops.conv3x3(hcur, self.w1, col_bias=self.b1, gn_groups=gn)
         hcur = ops.groupnorm(hcur, self.n2[0], self.n2[1], self.eps, True, self.groups)
         if self.sc is not None:
             res = ops.gemm(x, self.sc[0], a1=skip, col_bias=self.sc[1])
@@ -451,10 +454,13 @@ class _VAEAttention:
 
     @staticmethod
     def _attention_unfused(q, k, vt, ntok, c, scale, chunk, f32):
-        o = torch.empty((ntok, c), dtype=torch.float16, device=q.device)
+        o = torch.empty((ntok, c), dtype=q.dtype, device=q.device)
         for r0 in range(0, ntok, chunk):
             r1 = min(r0 + chunk, ntok)
-            if not f32 and ntok % 4 == 0 and ntok <= 16384:
+            if q.dtype == torch.bfloat16:                                  # bf16 VAE: fp32 logits, bf16 P for the P V GEMM
+                s = ops.gemm(q[r0:r1], k, out_f32=True)
+                ops.gemm(ops.softmax_rows(s, scale, out_dtype=torch.bfloat16), vt, out=o[r0:r1])
+            elif not f32 and ntok % 4 == 0 and ntok <= 16384:
                 s = ops.gemm(q[r0:r1], k, scale=scale)                     # [rows, ntok] fp16, already scaled
                 p, inv = ops.softmax_rows_exp(s, 1.0, out=s)               # exp only, in place; 1 / rowsum on the side
                 ops.gemm(p, vt, out=o[r0:r1], row_scale=inv)               # ... applied in fp32 by the P V epilogue
@@ -468,9 +474,15 @@ class _VAEAttention:
 
 
 class VAE:
-    def __init__(self, params: Params, cfg: VAEConfig, device, attention_scores_f32: bool = False):
-        pk = _Packer(params, device)
-        self.cfg, self.dev = cfg, device
+    """AutoencoderKL.  ``dtype=torch.bfloat16`` (VAE checkpoints whose activations leave the fp16 range, DESIGN.md 3.11): bf16
+    weights and stored activations, fp32 accumulation and fp32 attention logits, no producer-side GroupNorm statistics.  The interface
+    does not depend on it: ``encode_moments`` returns fp16 moments and ``decode`` an fp16 image either way."""
+
+    def __init__(self, params: Params, cfg: VAEConfig, device, attention_scores_f32: bool = False, dtype=torch.float16):
+        if dtype not in (torch.float16, torch.bfloat16):
+            raise ValueError(f"VAE dtype must be torch.float16 or torch.bfloat16, not {dtype}")
+        pk = _Packer(params, device, dtype=dtype)
+        self.cfg, self.dev, self.dtype = cfg, device, dtype
         g, eps = cfg.norm_groups, cfg.norm_eps
         ch = list(cfg.block_out_channels)
         L = cfg.latent_channels
@@ -501,19 +513,21 @@ class VAE:
             self.d_up.append((res, us))
         self.d_norm = pk.norm("decoder.conv_norm_out")
         self.d_out = pk.conv3("decoder.conv_out", pad_cout_to=32)
-        # every block output of the VAE is consumed by a GroupNorm: let the producing epilogue accumulate its statistics
+        # every block output of the VAE is consumed by a GroupNorm: let the producing epilogue accumulate its statistics (fp16 only:
+        # the bf16 GroupNorm computes range-safe statistics itself)
+        bf = dtype == torch.bfloat16
         for res, _ in self.e_down + self.d_up:
             for r in res:
-                r.out_gn = g
+                r.out_gn = 0 if bf else g
         for blk in (self.e_mid, self.d_mid):
-            blk[0].out_gn = g; blk[2].out_gn = g
-        self.gn_groups = g
+            blk[0].out_gn = blk[2].out_gn = 0 if bf else g
+        self.gn_groups = 0 if bf else g
         self.e_mid[1].scores_f32 = self.d_mid[1].scores_f32 = bool(attention_scores_f32)
 
     def encode_moments(self, xp8: Tensor) -> Tensor:
         """xp8: zero-padded [N,H+2,W+8,8] fp16 image in [-1,1] (ops.preprocess_pad8) -> moments [N,H/8,W/8,2L] fp16."""
         cfg = self.cfg
-        h = ops.conv3x3_c8(xp8, self.e_in[0], col_bias=self.e_in[1], gn_groups=self.gn_groups)
+        h = ops.conv3x3_c8(xp8, self.e_in[0], col_bias=self.e_in[1], gn_groups=self.gn_groups, out_dtype=self.dtype)
         for res, ds in self.e_down:
             for r in res:
                 h = r(h)
@@ -525,14 +539,14 @@ class VAE:
         h = ops.groupnorm(h, self.e_norm[0], self.e_norm[1], cfg.norm_eps, True, cfg.norm_groups)
         h = ops.conv3x3(h, self.e_out[0], cout_valid=2 * cfg.latent_channels, col_bias=self.e_out[1])
         n, hh, ww, c = h.shape
-        return ops.gemm(h.view(n * hh * ww, c), self.quant[0], col_bias=self.quant[1]).view(n, hh, ww, c)
+        return ops.gemm(h.view(n * hh * ww, c), self.quant[0], col_bias=self.quant[1], out_dtype=torch.float16).view(n, hh, ww, c)
 
     def decode(self, z: Tensor) -> Tensor:
         """z [N,h,w,4] fp16 latents (scaled) -> image [N,8h,8w,4] fp16 (3 valid channels) in ~[-1,1]."""
         cfg = self.cfg
         L = cfg.latent_channels
         h = ops.conv3x3_cin4(z, self.pq[0], self.pq[1], L, ld_out=4)
-        h = ops.conv3x3_c8(ops.pad8(h), self.d_in[0], col_bias=self.d_in[1], gn_groups=self.gn_groups)
+        h = ops.conv3x3_c8(ops.pad8(h), self.d_in[0], col_bias=self.d_in[1], gn_groups=self.gn_groups, out_dtype=self.dtype)
         h = self.d_mid[0](h)
         h = self.d_mid[1](h)
         h = self.d_mid[2](h)

@@ -37,4 +37,5 @@ def synthetic_state(model_name: str, full_controlnet: bool = False, tiny: bool =
 def build_engine(state: Dict, device="cuda", pack_on_host: bool = False):
     from .pipeline import EditEngine
     return EditEngine(state["unet"], state["unet_cfg"], state["cn"], state["cn_cfg"], state["vae"], state["vae_cfg"], device,
-                      state.get("lora"), state.get("lora_scale", 1.0), pack_on_host=pack_on_host, vae_scores_f32=bool(state.get("vae_scores_f32", False)))
+                      state.get("lora"), state.get("lora_scale", 1.0), pack_on_host=pack_on_host, vae_scores_f32=bool(state.get("vae_scores_f32", False)),
+                      vae_dtype=state.get("vae_dtype", torch.float16))

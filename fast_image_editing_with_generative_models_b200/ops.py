@@ -1,6 +1,8 @@
 """Thin Python wrappers over the C-ABI: torch owns device memory and streams, the kernels do the work.
 
 Activations are NHWC / token-major fp16 tensors.  Every wrapper raises if the CUDA library is unavailable.
+The GEMM / convolution / GroupNorm / softmax / VAE-attention wrappers also take bf16 tensors (the bf16 VAE, DESIGN.md 3.11): a bf16
+input goes to the ``*_bf16`` entry points, an fp16 input to the fp16 ones exactly as before.
 """
 from __future__ import annotations
 
@@ -80,6 +82,9 @@ def profile_summary(by_tag: bool = False):
         d["ms"] += e0.elapsed_time(e1)
         d["work"] += work
     return out
+
+
+_DT = {torch.float16: _lib.DT_F16, torch.bfloat16: _lib.DT_BF16, torch.float32: _lib.DT_F32}
 
 
 def _stream() -> int:
@@ -446,16 +451,20 @@ def sincos_embedding(vals, dim: int, device) -> torch.Tensor:
     return out
 
 
-def softmax_rows(s: torch.Tensor, scale: float, out: Optional[torch.Tensor] = None) -> torch.Tensor:
-    """Row softmax of fp32 scores (scaled here) or fp16 scores (pre-scaled by the GEMM epilogue: pass scale = 1) -> fp16."""
+def softmax_rows(s: torch.Tensor, scale: float, out: Optional[torch.Tensor] = None, out_dtype=torch.float16) -> torch.Tensor:
+    """Row softmax of fp32 scores (scaled here) or fp16 scores (pre-scaled by the GEMM epilogue: pass scale = 1) -> fp16
+    (fp32 scores: or bf16, by ``out_dtype`` or the dtype of ``out``)."""
     if s.dtype not in (torch.float32, torch.float16):
         raise _lib.FieError("softmax_rows: fp32 or fp16 scores expected")
     _req(s, s.dtype, "softmax_rows")
     rows, cols = s.shape
-    out = torch.empty((rows, cols), dtype=torch.float16, device=s.device) if out is None else out
+    out = torch.empty((rows, cols), dtype=out_dtype, device=s.device) if out is None else out
     f16 = s.dtype == torch.float16
+    if out.dtype not in (torch.float16, torch.bfloat16) or (f16 and out.dtype != torch.float16):
+        raise _lib.FieError("softmax_rows: fp16 output, or bf16 output of fp32 scores")
     with _prof("softmax_rows", (4.0 if f16 else 6.0) * rows * cols, "B"):
-        fn = _lib.lib().fie_softmax_rows_f16 if f16 else _lib.lib().fie_softmax_rows_f32_to_f16
+        fn = _lib.lib().fie_softmax_rows_f16 if f16 else (_lib.lib().fie_softmax_rows_f32_to_bf16 if out.dtype == torch.bfloat16
+                                                           else _lib.lib().fie_softmax_rows_f32_to_f16)
         check(fn(_p(s), s.stride(0), _p(out), out.stride(0), rows, cols, float(scale), _stream()), "fie_softmax_rows")
     _count()
     return out
@@ -502,7 +511,10 @@ def zeros_i64(shape, device) -> torch.Tensor:
 def groupnorm(x0: torch.Tensor, gamma: torch.Tensor, beta: torch.Tensor, eps: float, silu: bool, groups: int = 32,
               x1: Optional[torch.Tensor] = None) -> torch.Tensor:
     """x0 [N,H,W,C0] (+ optional concatenated x1 [N,H,W,C1]) -> [N,H,W,C0+C1] normalised (+SiLU).  If x0 was produced by a
-    GEMM / conv call with ``gn_groups=groups``, its statistics already exist and only the apply pass runs."""
+    GEMM / conv call with ``gn_groups=groups``, its statistics already exist and only the apply pass runs.  bf16 inputs take the
+    range-safe statistics of fie_groupnorm_bf16."""
+    if x0.dtype == torch.bfloat16:
+        return _groupnorm_bf16(x0, gamma, beta, eps, silu, groups, x1)
     _req(x0, torch.float16, "groupnorm")
     n = x0.shape[0]
     c0 = x0.shape[-1]
@@ -523,6 +535,28 @@ def groupnorm(x0: torch.Tensor, gamma: torch.Tensor, beta: torch.Tensor, eps: fl
     cpg = (c0 + c1) // groups
     slab = (not ready) and cpg % 2 == 0 and hw >= 64 and hw * cpg * 2 <= 192 * 1024 and os.environ.get("FIE_GN_SLAB", "1") != "0"
     _count(1 if (ready or slab) else 2)
+    return out
+
+
+def _groupnorm_bf16(x0, gamma, beta, eps, silu, groups, x1):
+    _req(x0, torch.bfloat16, "groupnorm")
+    n = x0.shape[0]
+    c0 = x0.shape[-1]
+    hw = x0.numel() // (n * c0)
+    c1 = 0
+    if x1 is not None:
+        _req(x1, torch.bfloat16, "groupnorm")
+        c1 = x1.shape[-1]
+    out = torch.empty(tuple(x0.shape[:-1]) + (c0 + c1,), dtype=torch.bfloat16, device=x0.device)
+    L = _lib.lib()
+    nbytes = L.fie_groupnorm_bf16_workspace_bytes(n, hw, c0 + c1, groups)
+    ws = torch.empty(max(nbytes, 256), dtype=torch.uint8, device=x0.device)
+    with _prof("groupnorm", 4.0 * out.numel(), "B", f"[{n},{hw},{c0}+{c1}] bf16"):
+        check(L.fie_groupnorm_bf16(_p(x0), c0, _p(x1), c1, _p(out), n, hw, groups, _p(gamma), _p(beta), float(eps), int(silu), _p(ws), ws.numel(),
+                                   _stream()), "fie_groupnorm_bf16")
+    cpg = (c0 + c1) // groups
+    slab = cpg % 2 == 0 and hw >= 64 and hw * cpg * 2 <= 192 * 1024 and os.environ.get("FIE_GN_SLAB", "1") != "0"
+    _count(1 if slab else 2)
     return out
 
 
@@ -559,11 +593,16 @@ def _epilogue(col_bias=None, row_bias=None, rows_per_group=1, m_bias=None, resid
 def gemm(a: torch.Tensor, w: torch.Tensor, *, a1: Optional[torch.Tensor] = None, out: Optional[torch.Tensor] = None, n_valid: Optional[int] = None,
          col_bias=None, row_bias=None, rows_per_group=1, m_bias=None, residual=None, scale=1.0, act=ACT_NONE, out_f32=False,
          gn_groups: int = 0, gn_rows: int = 0, ln_out: Optional[torch.Tensor] = None, ln_in=None,
-         row_scale: Optional[torch.Tensor] = None) -> torch.Tensor:
+         row_scale: Optional[torch.Tensor] = None, out_dtype: Optional[torch.dtype] = None) -> torch.Tensor:
     """D = epilogue(A @ W^T).  a: [..., K] fp16 rows (row stride may exceed K), w: [N, K] fp16; optional a1 continues K.
     ln_out: zeroed int64 [M, 2] that receives the LayerNorm statistics of the output rows.  ln_in = (stats, eps): the A rows are
-    layer-normalised on the fly (w / col_bias from weights.fold_layernorm)."""
-    if a.dtype != torch.float16 or w.dtype != torch.float16 or not a.is_cuda:
+    layer-normalised on the fly (w / col_bias from weights.fold_layernorm).
+    bf16 a / w (/ a1): fie_gemm_bf16, whose output is bf16 by default, else ``out_dtype`` / the dtype of ``out`` (fp16, bf16, fp32)."""
+    bf = a.dtype == torch.bfloat16
+    if bf:
+        if w.dtype != torch.bfloat16 or (a1 is not None and a1.dtype != torch.bfloat16) or not a.is_cuda:
+            raise _lib.FieError("gemm: bf16 A needs bf16 W (and A1) CUDA tensors")
+    elif a.dtype != torch.float16 or w.dtype != torch.float16 or not a.is_cuda:
         raise _lib.FieError("gemm: fp16 CUDA tensors required")
     k0 = a.shape[-1]
     m = a.numel() // k0
@@ -577,11 +616,16 @@ def gemm(a: torch.Tensor, w: torch.Tensor, *, a1: Optional[torch.Tensor] = None,
     else:
         assert k0 == k, (k0, k)
     n_out = n // 2 if act == ACT_GEGLU else n
+    if not bf and out_dtype not in (None, torch.float16):
+        raise _lib.FieError("gemm: fp16 operands give fp16 (or, with out_f32, fp32) output")
     if out is None:
-        out = torch.empty(tuple(a.shape[:-1]) + (n_out,), dtype=torch.float32 if out_f32 else torch.float16, device=a.device)
+        odt = torch.float32 if out_f32 else (out_dtype or a.dtype)
+        out = torch.empty(tuple(a.shape[:-1]) + (n_out,), dtype=odt, device=a.device)
+    if bf:
+        out_f32 = out.dtype == torch.float32
     ldd = out.stride(-2) if out.dim() >= 2 else n_out
     gn = None
-    if gn_groups and gn_rows and not out_f32 and m % gn_rows == 0 and _gn_stats_ok(n_out, gn_groups, gn_rows, ldd):
+    if gn_groups and gn_rows and not out_f32 and not bf and m % gn_rows == 0 and _gn_stats_ok(n_out, gn_groups, gn_rows, ldd):
         gn = (_gn_stats_alloc(out, m // gn_rows, gn_groups), gn_groups, gn_rows)
     if ln_out is not None and (ln_out.dtype != torch.int64 or ln_out.numel() != 2 * m or not ln_out.is_contiguous()):
         raise _lib.FieError("gemm: ln_out must be a contiguous int64 [M, 2] tensor")
@@ -591,70 +635,100 @@ def gemm(a: torch.Tensor, w: torch.Tensor, *, a1: Optional[torch.Tensor] = None,
         raise _lib.FieError("gemm: row_scale must be a contiguous fp32 [M] tensor")
     ep = _epilogue(col_bias, row_bias, rows_per_group, m_bias, residual, scale, act, out_f32, gn, ln_out, ln_in, row_scale)
     ep.ln_dim = k
-    with _prof("gemm", 2.0 * m * n * k, "FLOP", f"M{m} N{n} K{k} act{act} res{int(residual is not None)} f32{int(out_f32)}"):
-        check(_lib.lib().fie_gemm_f16(_p(a), lda, _p(a1), lda1, k_split, _p(w), _p(out), ldd, m, n, k, ctypes.byref(ep), _stream()), "fie_gemm_f16")
+    with _prof("gemm", 2.0 * m * n * k, "FLOP", f"M{m} N{n} K{k} act{act} res{int(residual is not None)} f32{int(out_f32)}" + (" bf16" if bf else "")):
+        if bf:
+            check(_lib.lib().fie_gemm_bf16(_p(a), lda, _p(a1), lda1, k_split, _p(w), _p(out), ldd, m, n, k, ctypes.byref(ep), _DT[out.dtype], _stream()),
+                  "fie_gemm_bf16")
+        else:
+            check(_lib.lib().fie_gemm_f16(_p(a), lda, _p(a1), lda1, k_split, _p(w), _p(out), ldd, m, n, k, ctypes.byref(ep), _stream()), "fie_gemm_f16")
     _count()
     return out
+
+
+def _req_any(x: torch.Tensor, w: torch.Tensor, name: str) -> bool:
+    """Activation and packed weight both fp16 (-> False) or both bf16 (-> True)."""
+    if x.dtype == torch.bfloat16:
+        _req(x, torch.bfloat16, name)
+        if w.dtype != torch.bfloat16:
+            raise _lib.FieError(f"{name}: bf16 activations need bf16 weights")
+        return True
+    _req(x, torch.float16, name)
+    return False
 
 
 def conv3x3(x: torch.Tensor, w: torch.Tensor, *, stride: int = 1, pad_mode: int = 0, cout_valid: Optional[int] = None,
             out: Optional[torch.Tensor] = None, col_bias=None, row_bias=None, rows_per_group=1, residual=None, scale=1.0, act=ACT_NONE,
             gn_groups: int = 0) -> torch.Tensor:
-    """x [N,H,W,Cin] fp16, w packed [Cout, 9*Cin] fp16 -> [N,H/stride,W/stride,cout_valid]."""
-    _req(x, torch.float16, "conv3x3")
+    """x [N,H,W,Cin] fp16, w packed [Cout, 9*Cin] fp16 -> [N,H/stride,W/stride,cout_valid].  bf16 x / w: fie_conv3x3_bf16, output in
+    the dtype of ``out`` (default bf16); GroupNorm statistics are then left to the GroupNorm kernel."""
+    bf = _req_any(x, w, "conv3x3")
     n, h, wd, cin = x.shape
     cout = w.shape[0]
     assert w.shape[1] == 9 * cin, (w.shape, cin)
     cv = cout if cout_valid is None else cout_valid
     if out is None:
-        out = torch.empty((n, h // stride, wd // stride, cv), dtype=torch.float16, device=x.device)
+        out = torch.empty((n, h // stride, wd // stride, cv), dtype=x.dtype, device=x.device)
     gn = None
     ohw = (h // stride) * (wd // stride)
-    if gn_groups and cv == cout and _gn_stats_ok(cout, gn_groups, ohw, out.stride(-2)):
+    if gn_groups and not bf and cv == cout and _gn_stats_ok(cout, gn_groups, ohw, out.stride(-2)):
         gn = (_gn_stats_alloc(out, n, gn_groups), gn_groups, ohw)
     ep = _epilogue(col_bias, row_bias, rows_per_group, None, residual, scale, act, False, gn)
-    with _prof("conv3x3", 2.0 * n * (h // stride) * (wd // stride) * cv * 9 * cin, "FLOP", f"[{n},{h},{wd},{cin}]->{cv} s{stride}"):
-        check(_lib.lib().fie_conv3x3_f16(_p(x), _p(w), _p(out), out.stride(-2), n, h, wd, cin, cout, cv, stride, pad_mode, ctypes.byref(ep), _stream()),
-              "fie_conv3x3_f16")
+    with _prof("conv3x3", 2.0 * n * (h // stride) * (wd // stride) * cv * 9 * cin, "FLOP", f"[{n},{h},{wd},{cin}]->{cv} s{stride}" + (" bf16" if bf else "")):
+        if bf:
+            check(_lib.lib().fie_conv3x3_bf16(_p(x), _p(w), _p(out), out.stride(-2), n, h, wd, cin, cout, cv, stride, pad_mode, ctypes.byref(ep),
+                                              _DT[out.dtype], _stream()), "fie_conv3x3_bf16")
+        else:
+            check(_lib.lib().fie_conv3x3_f16(_p(x), _p(w), _p(out), out.stride(-2), n, h, wd, cin, cout, cv, stride, pad_mode, ctypes.byref(ep), _stream()),
+                  "fie_conv3x3_f16")
     _count()
     return out
 
 
 def conv_up2x(x: torch.Tensor, w4: torch.Tensor, *, col_bias=None, out: Optional[torch.Tensor] = None, gn_groups: int = 0) -> torch.Tensor:
-    """Fused nearest-2x upsample + conv3x3.  x [N,H,W,Cin], w4 packed [4, Cout, 4*Cin] (weights.pack_conv_up2x) -> [N,2H,2W,Cout]."""
-    _req(x, torch.float16, "conv_up2x")
+    """Fused nearest-2x upsample + conv3x3.  x [N,H,W,Cin], w4 packed [4, Cout, 4*Cin] (weights.pack_conv_up2x) -> [N,2H,2W,Cout].
+    bf16 x / w4: fie_conv_up2x_bf16 (output dtype of ``out``, default bf16)."""
+    bf = _req_any(x, w4, "conv_up2x")
     n, h, wd, cin = x.shape
     cout = w4.shape[1]
     assert w4.shape[0] == 4 and w4.shape[2] == 4 * cin, (w4.shape, cin)
     if out is None:
-        out = torch.empty((n, 2 * h, 2 * wd, cout), dtype=torch.float16, device=x.device)
+        out = torch.empty((n, 2 * h, 2 * wd, cout), dtype=x.dtype, device=x.device)
     gn = None
-    if gn_groups and _gn_stats_ok(cout, gn_groups, h * wd, out.stride(-2)):
+    if gn_groups and not bf and _gn_stats_ok(cout, gn_groups, h * wd, out.stride(-2)):
         gn = (_gn_stats_alloc(out, n, gn_groups), gn_groups, h * wd)       # rows of each phase launch are INPUT pixels: h*w per image
     ep = _epilogue(col_bias, gn=gn)
-    with _prof("conv_up2x", 2.0 * n * 4 * h * wd * cout * 4 * cin, "FLOP", f"[{n},{h},{wd},{cin}]->{cout}"):
-        check(_lib.lib().fie_conv_up2x_f16(_p(x), _p(w4), _p(out), out.stride(-2), n, h, wd, cin, cout, ctypes.byref(ep), _stream()), "fie_conv_up2x_f16")
+    with _prof("conv_up2x", 2.0 * n * 4 * h * wd * cout * 4 * cin, "FLOP", f"[{n},{h},{wd},{cin}]->{cout}" + (" bf16" if bf else "")):
+        if bf:
+            check(_lib.lib().fie_conv_up2x_bf16(_p(x), _p(w4), _p(out), out.stride(-2), n, h, wd, cin, cout, ctypes.byref(ep), _DT[out.dtype], _stream()),
+                  "fie_conv_up2x_bf16")
+        else:
+            check(_lib.lib().fie_conv_up2x_f16(_p(x), _p(w4), _p(out), out.stride(-2), n, h, wd, cin, cout, ctypes.byref(ep), _stream()), "fie_conv_up2x_f16")
     _count(4)
     return out
 
 
 def conv3x3_c8(xp: torch.Tensor, w: torch.Tensor, *, cout_valid: Optional[int] = None, col_bias=None, act=ACT_NONE, gn_groups: int = 0,
-               residual: Optional[torch.Tensor] = None) -> torch.Tensor:
+               residual: Optional[torch.Tensor] = None, out_dtype=torch.float16) -> torch.Tensor:
     """Tensor-core conv_in.  xp: zero-padded [N,H+2,W+8,8] fp16 (:func:`preprocess_pad8`), w: [Cout, 384] (weights.pack_conv3x3_c8)
-    -> [N,H,W,cout_valid]."""
+    -> [N,H,W,cout_valid] fp16, or bf16 with ``out_dtype=torch.bfloat16`` (fie_conv3x3_c8_bf16: the operands stay fp16)."""
     _req(xp, torch.float16, "conv3x3_c8")
     n, hp, wp, c = xp.shape
     assert c == 8 and w.shape[1] == 384, (xp.shape, w.shape)
     h, wd = hp - 2, wp - 8
     cout = w.shape[0]
     cv = cout if cout_valid is None else cout_valid
-    out = torch.empty((n, h, wd, cv), dtype=torch.float16, device=xp.device)
+    bf = out_dtype == torch.bfloat16
+    out = torch.empty((n, h, wd, cv), dtype=out_dtype, device=xp.device)
     gn = None
-    if gn_groups and cv == cout and _gn_stats_ok(cout, gn_groups, h * wd, out.stride(-2)):
+    if gn_groups and not bf and cv == cout and _gn_stats_ok(cout, gn_groups, h * wd, out.stride(-2)):
         gn = (_gn_stats_alloc(out, n, gn_groups), gn_groups, h * wd)
     ep = _epilogue(col_bias, act=act, gn=gn, residual=residual)
-    with _prof("conv_in_c8", 2.0 * out.numel() + 2.0 * xp.numel(), "B", f"[{n},{h},{wd},8]->{cv}"):
-        check(_lib.lib().fie_conv3x3_c8_f16(_p(xp), _p(w), _p(out), out.stride(-2), n, h, wd, cout, cv, ctypes.byref(ep), _stream()), "fie_conv3x3_c8_f16")
+    with _prof("conv_in_c8", 2.0 * out.numel() + 2.0 * xp.numel(), "B", f"[{n},{h},{wd},8]->{cv}" + (" bf16" if bf else "")):
+        if bf:
+            check(_lib.lib().fie_conv3x3_c8_bf16(_p(xp), _p(w), _p(out), out.stride(-2), n, h, wd, cout, cv, ctypes.byref(ep), _DT[out.dtype], _stream()),
+                  "fie_conv3x3_c8_bf16")
+        else:
+            check(_lib.lib().fie_conv3x3_c8_f16(_p(xp), _p(w), _p(out), out.stride(-2), n, h, wd, cout, cv, ctypes.byref(ep), _stream()), "fie_conv3x3_c8_f16")
     _count()
     return out
 
@@ -694,12 +768,15 @@ _VAE_WS = {}
 def attention_vae(q: torch.Tensor, k: torch.Tensor, vt: torch.Tensor, scale: float, out: Optional[torch.Tensor] = None, f32_scores: bool = False,
                   chunk_rows: int = 0) -> torch.Tensor:
     """softmax(scale q k^T) v for ONE image of the VAE mid-block attention (1 head): q, k [ntok, d] fp16, vt [d, ntok] fp16 (V transposed)
-    -> [ntok, d].  One C-ABI call (fie_attn_vae_d512_f16); the score workspace is cached per (device, shape)."""
+    -> [ntok, d].  One C-ABI call (fie_attn_vae_d512_f16); the score workspace is cached per (device, shape).  bf16 q, k, vt:
+    fie_attn_vae_d512_bf16, bf16 output, always fp32 scores."""
+    bf = q.dtype == torch.bfloat16
     for t in (q, k, vt):
-        _req(t, torch.float16, "attention_vae")
+        _req(t, torch.bfloat16 if bf else torch.float16, "attention_vae")
+    f32_scores = f32_scores or bf
     ntok, d = q.shape
     if out is None:
-        out = torch.empty((ntok, d), dtype=torch.float16, device=q.device)
+        out = torch.empty((ntok, d), dtype=q.dtype, device=q.device)
     L = _lib.lib()
     nbytes = L.fie_attn_vae_workspace_bytes(ntok, int(chunk_rows), int(f32_scores))
     key = (str(q.device), nbytes)
@@ -709,9 +786,13 @@ def attention_vae(q: torch.Tensor, k: torch.Tensor, vt: torch.Tensor, scale: flo
         if not torch.cuda.is_current_stream_capturing():
             _VAE_WS.clear()
             _VAE_WS[key] = ws
-    with _prof("vae_attention", 4.0 * ntok * ntok * d, "FLOP", f"ntok{ntok} d{d} f32{int(f32_scores)}"):
-        check(L.fie_attn_vae_d512_f16(_p(q), q.stride(0), _p(k), k.stride(0), _p(vt), _p(out), out.stride(0), ntok, d, float(scale), int(f32_scores),
-                                      int(chunk_rows), _p(ws), nbytes, _stream()), "fie_attn_vae_d512_f16")
+    with _prof("vae_attention", 4.0 * ntok * ntok * d, "FLOP", f"ntok{ntok} d{d} f32{int(f32_scores)}" + (" bf16" if bf else "")):
+        if bf:
+            check(L.fie_attn_vae_d512_bf16(_p(q), q.stride(0), _p(k), k.stride(0), _p(vt), _p(out), out.stride(0), ntok, d, float(scale), int(chunk_rows),
+                                           _p(ws), nbytes, _stream()), "fie_attn_vae_d512_bf16")
+        else:
+            check(L.fie_attn_vae_d512_f16(_p(q), q.stride(0), _p(k), k.stride(0), _p(vt), _p(out), out.stride(0), ntok, d, float(scale), int(f32_scores),
+                                          int(chunk_rows), _p(ws), nbytes, _stream()), "fie_attn_vae_d512_f16")
     nchunks = 1 if chunk_rows <= 0 else -(-ntok // chunk_rows)
     _count(3 * nchunks)
     return out

@@ -56,10 +56,12 @@ class EditEngine:
     """Owns the packed weights of one (UNet, ControlNet, VAE) triple on one GPU and runs batched edits."""
 
     def __init__(self, unet_params, unet_cfg: UNetConfig, cn_params, cn_cfg: ControlNetConfig, vae_params, vae_cfg: VAEConfig,
-                 device="cuda", lora=None, lora_scale: float = 1.0, pack_on_host: bool = False, vae_scores_f32: bool = False):
+                 device="cuda", lora=None, lora_scale: float = 1.0, pack_on_host: bool = False, vae_scores_f32: bool = False,
+                 vae_dtype=torch.float16):
         """Load-time weight packing (layout transforms, LoRA fuse, LayerNorm fold; cold path, reference ``src/pipeline.py:45-181``)
         uses plain torch tensor ops: by default on the GPU (ATen / cuBLAS kernels, seconds for SDXL), with ``pack_on_host`` on the
-        CPU followed by plain H2D copies — then no library kernel is ever launched on the device, only ours (``smoke()``)."""
+        CPU followed by plain H2D copies — then no library kernel is ever launched on the device, only ours (``smoke()``).
+        ``vae_dtype=torch.bfloat16`` runs the VAE with bf16 weights and activations (engine.VAE); its interface stays fp16."""
         self.dev = torch.device(device)
         if self.dev.type != "cuda":
             raise RuntimeError("EditEngine runs on CUDA (sm_100a) only; there is no CPU path")
@@ -67,7 +69,7 @@ class EditEngine:
             pdev = torch.device("cpu") if pack_on_host else self.dev
             self.unet = UNet(unet_params, unet_cfg, pdev, lora, lora_scale)
             self.cn = ControlNet(cn_params, cn_cfg, pdev)
-            self.vae = VAE(vae_params, vae_cfg, pdev, attention_scores_f32=vae_scores_f32)   # fp32 VAE attention logits: real checkpoints
+            self.vae = VAE(vae_params, vae_cfg, pdev, attention_scores_f32=vae_scores_f32, dtype=vae_dtype)   # fp32 VAE attention logits: real checkpoints
             if pack_on_host:
                 for m in (self.unet, self.cn, self.vae):
                     _move_to(m, self.dev)

@@ -4,7 +4,8 @@ reference ``src/pipeline.py:45-181``): conv weights to [Cout][kh][kw][Cin], GEGL
 Every transform has two implementations with the same result: on CUDA tensors the library's own kernels (``csrc/pack.cu``,
 ``fie_pack_* / fie_fold_layernorm_f16 / fie_fuse_lora_f32`` — SURVEY 8(b) ``fie_pack_weights_*``; no ATen / cuBLAS compute kernel
 runs at load time), on CPU tensors plain torch ops (``EditEngine(pack_on_host=True)`` and the CPU tests, which are also what
-``tests/test_gpu_kernels.py`` checks the kernels against)."""
+``tests/test_gpu_kernels.py`` checks the kernels against).  ``dtype=torch.bfloat16`` gives the same layouts with bf16 elements (the bf16
+VAE; ``fie_pack_*_bf16``)."""
 from __future__ import annotations
 
 from typing import Optional, Tuple
@@ -26,31 +27,41 @@ def _f32(t: torch.Tensor) -> torch.Tensor:
     return t if (t.dtype == torch.float32 and t.is_contiguous()) else t.float().contiguous()
 
 
-def cast_f16(w: torch.Tensor) -> torch.Tensor:
-    """fp32 [N, K] -> fp16 [N, K] (a Linear / 1x1-conv weight as the GEMM's B operand)."""
+def _bf(dtype) -> bool:
+    if dtype not in (torch.float16, torch.bfloat16):
+        raise ValueError(f"packed weights are fp16 or bf16, not {dtype}")
+    return dtype == torch.bfloat16
+
+
+def cast_f16(w: torch.Tensor, dtype=torch.float16) -> torch.Tensor:
+    """fp32 [N, K] -> fp16 (or bf16) [N, K] (a Linear / 1x1-conv weight as the GEMM's B operand)."""
+    bf = _bf(dtype)
     if not (w.is_cuda and NATIVE):
-        return w.to(torch.float16).contiguous()
+        return w.to(dtype).contiguous()
     w = _f32(w)
     n, k = w.shape[0], w.numel() // w.shape[0]
-    out = torch.empty(w.shape, dtype=torch.float16, device=w.device)
+    out = torch.empty(w.shape, dtype=dtype, device=w.device)
+    fn = "fie_pack_rows_bf16" if bf else "fie_pack_rows_f16"
     with torch.cuda.device(w.device):
-        _lib.check(_lib.lib().fie_pack_rows_f16(w.data_ptr(), None, None, out.data_ptr(), None, n, k, _stream(w)), "fie_pack_rows_f16")
+        _lib.check(getattr(_lib.lib(), fn)(w.data_ptr(), None, None, out.data_ptr(), None, n, k, _stream(w)), fn)
     return out
 
 
-def pack_conv3x3(w: torch.Tensor, pad_cout_to: Optional[int] = None, pad_cin_to: Optional[int] = None) -> torch.Tensor:
-    """[Cout, Cin, 3, 3] -> fp16 [Cout_p, 9*Cin_p] with K order (kh, kw, cin); zero padding of channels on request."""
+def pack_conv3x3(w: torch.Tensor, pad_cout_to: Optional[int] = None, pad_cin_to: Optional[int] = None, dtype=torch.float16) -> torch.Tensor:
+    """[Cout, Cin, 3, 3] -> fp16 (or bf16) [Cout_p, 9*Cin_p] with K order (kh, kw, cin); zero padding of channels on request."""
+    bf = _bf(dtype)
     cout, cin = w.shape[:2]
     cp = pad_cin_to or cin
     op = pad_cout_to or cout
     if w.is_cuda and NATIVE:
         w = _f32(w)
-        out = torch.empty((op, 9 * cp), dtype=torch.float16, device=w.device)
+        out = torch.empty((op, 9 * cp), dtype=dtype, device=w.device)
+        fn = "fie_pack_conv3x3_bf16" if bf else "fie_pack_conv3x3_f16"
         with torch.cuda.device(w.device):
-            _lib.check(_lib.lib().fie_pack_conv3x3_f16(w.data_ptr(), out.data_ptr(), cout, cin, op, cp, _stream(w)), "fie_pack_conv3x3_f16")
+            _lib.check(getattr(_lib.lib(), fn)(w.data_ptr(), out.data_ptr(), cout, cin, op, cp, _stream(w)), fn)
         return out
-    out = torch.zeros((op, 3, 3, cp), dtype=torch.float16, device=w.device)
-    out[:cout, :, :, :cin] = w.permute(0, 2, 3, 1).to(torch.float16)
+    out = torch.zeros((op, 3, 3, cp), dtype=dtype, device=w.device)
+    out[:cout, :, :, :cin] = w.permute(0, 2, 3, 1).to(dtype)
     return out.reshape(op, 9 * cp).contiguous()
 
 
@@ -76,16 +87,18 @@ def pack_conv3x3_c8(w: torch.Tensor, pad_cout_to: Optional[int] = None) -> torch
     return out.reshape(op, 3 * 2 * 64).contiguous()
 
 
-def pack_conv_up2x(w: torch.Tensor) -> torch.Tensor:
-    """[Cout, Cin, 3, 3] -> fp16 [4, Cout, 4*Cin]: phase (a, b) weights of nearest-2x-upsample + conv3x3.
+def pack_conv_up2x(w: torch.Tensor, dtype=torch.float16) -> torch.Tensor:
+    """[Cout, Cin, 3, 3] -> fp16 (or bf16) [4, Cout, 4*Cin]: phase (a, b) weights of nearest-2x-upsample + conv3x3.
     Output row 2i+a reads input rows {i-1, i} (a = 0) or {i, i+1} (a = 1); the 3x3 taps that fall on the same input row are
     summed (in fp32): a=0 -> [W0, W1+W2], a=1 -> [W0+W1, W2]; identically for columns.  K order (ty, tx, cin)."""
+    bf = _bf(dtype)
     if w.is_cuda and NATIVE:
         w = _f32(w)
         cout, cin = w.shape[:2]
-        out = torch.empty((4, cout, 4 * cin), dtype=torch.float16, device=w.device)
+        out = torch.empty((4, cout, 4 * cin), dtype=dtype, device=w.device)
+        fn = "fie_pack_conv_up2x_bf16" if bf else "fie_pack_conv_up2x_f16"
         with torch.cuda.device(w.device):
-            _lib.check(_lib.lib().fie_pack_conv_up2x_f16(w.data_ptr(), out.data_ptr(), cout, cin, _stream(w)), "fie_pack_conv_up2x_f16")
+            _lib.check(getattr(_lib.lib(), fn)(w.data_ptr(), out.data_ptr(), cout, cin, _stream(w)), fn)
         return out
     w = w.float()
     rows = {0: [w[:, :, 0], w[:, :, 1] + w[:, :, 2]], 1: [w[:, :, 0] + w[:, :, 1], w[:, :, 2]]}   # each [Cout, Cin, 3(kw)]
@@ -98,7 +111,7 @@ def pack_conv_up2x(w: torch.Tensor) -> torch.Tensor:
                 cols = [r[:, :, 0], r[:, :, 1] + r[:, :, 2]] if b == 0 else [r[:, :, 0] + r[:, :, 1], r[:, :, 2]]
                 taps += cols                                   # (ty, tx) order, each [Cout, Cin]
             out.append(torch.stack(taps, dim=1).reshape(w.shape[0], -1))
-    return torch.stack(out, 0).to(torch.float16).contiguous()
+    return torch.stack(out, 0).to(dtype).contiguous()
 
 
 def pack_geglu(w: torch.Tensor, b: Optional[torch.Tensor]) -> Tuple[torch.Tensor, Optional[torch.Tensor]]:

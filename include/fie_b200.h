@@ -249,6 +249,43 @@ int fie_conv3x3_cin4_f16(const void* x, const float* wgt, const float* bias, voi
 int fie_conv3x3_c8_f16(const void* xp, const void* wgt, void* out, long long ldd, int n, int h, int w, int cout,
                        int cout_valid, const fie_epilogue* ep, void* stream);
 
+/* ---- bf16 VAE (DESIGN.md 3.11): the same tensor-core kernels with bf16 operands, for VAE checkpoints whose activations leave the
+ * fp16 range (config.json "force_upcast": true, e.g. the original SDXL VAE).  Operands and fie_epilogue are as for the fp16 entry
+ * points above, with every fp16 activation and weight replaced by bf16; accumulation stays fp32.  out_dtype selects the output
+ * (FIE_DT_F16, FIE_DT_BF16 or FIE_DT_F32; fie_epilogue.out_f32 may only be set together with FIE_DT_F32); a residual is read in
+ * the output's type.  GroupNorm statistics in the producing epilogue (gn_stats), ln_stats_out and GEGLU need fp16 output and are
+ * rejected with FIE_ERR_INVALID for bf16 output. ---- */
+enum { FIE_DT_F16 = 0, FIE_DT_BF16 = 1, FIE_DT_F32 = 2 };
+int fie_gemm_bf16(const void* A, long long lda, const void* A1, long long lda1, int k_split,
+                  const void* B, void* D, long long ldd, long long M, int N, int K,
+                  const fie_epilogue* ep, int out_dtype, void* stream);
+int fie_conv3x3_bf16(const void* x, const void* wgt, void* out, long long ldd, int n, int h, int w, int cin, int cout,
+                     int cout_valid, int stride, int pad_mode, const fie_epilogue* ep, int out_dtype, void* stream);
+int fie_conv_up2x_bf16(const void* x, const void* wgt, void* out, long long ldd, int n, int h, int w, int cin, int cout,
+                       const fie_epilogue* ep, int out_dtype, void* stream);
+/* conv_in at image / latent resolution: the operands stay fp16 (pad8 input and hi/lo weights exactly as fie_conv3x3_c8_f16, whose
+ * inputs are bounded: an image in [-1, 1] or latents / scaling_factor); only the output type is selectable. */
+int fie_conv3x3_c8_bf16(const void* xp, const void* wgt, void* out, long long ldd, int n, int h, int w, int cout,
+                        int cout_valid, const fie_epilogue* ep, int out_dtype, void* stream);
+/* GroupNorm(+SiLU) of bf16 NHWC activations (x0, optional concatenated x1, out as fie_groupnorm_f16).  Range-safe and deterministic:
+ * slabs that fit one CTA take the single-pass two-pass-variance kernel (the fie_groupnorm_f16 rule); otherwise per-chunk
+ * (count, mean, M2) partials over a fixed row partition are merged in a fixed order with Chan's formula (no fixed point, no
+ * floating-point atomics).  workspace: fie_groupnorm_bf16_workspace_bytes(n, hw, c0 + c1, groups) bytes, 256-byte aligned. */
+size_t fie_groupnorm_bf16_workspace_bytes(int n, long long hw, int c, int groups);
+int fie_groupnorm_bf16(const void* x0, int c0, const void* x1, int c1, void* out, int n, long long hw, int groups,
+                       const float* gamma, const float* beta, float eps, int fuse_silu, void* workspace, size_t workspace_bytes, void* stream);
+/* row softmax of fp32 scores * scale -> bf16 probabilities */
+int fie_softmax_rows_f32_to_bf16(const void* s_f32, long long ld_in, void* p_bf16, long long ld_out,
+                                 long long rows, int cols, float scale, void* stream);
+/* fie_attn_vae_d512_f16 with bf16 q, k, vt and out; the logits always stay fp32 between the passes
+ * (workspace: fie_attn_vae_workspace_bytes(ntok, chunk_rows, 1)). */
+int fie_attn_vae_d512_bf16(const void* q, long long ldq, const void* k, long long ldk, const void* vt, void* out, long long ldo,
+                           int ntok, int d, float scale, int chunk_rows, void* workspace, size_t workspace_bytes, void* stream);
+/* bf16 twins of the load-time packers below (same layouts, bf16 elements) */
+int fie_pack_conv3x3_bf16(const float* w, void* out, int cout, int cin, int cout_pad, int cin_pad, void* stream);
+int fie_pack_conv_up2x_bf16(const float* w, void* out, int cout, int cin, void* stream);
+int fie_pack_rows_bf16(const float* w, const float* bias, const int* perm, void* out_w, float* out_bias, int n, int k, void* stream);
+
 /* ---- VAE mid-block attention: 1 head, d = C (512), ntok = H*W tokens (16 384 at 1024^2) — SURVEY 8(b) `fie_attn_vae_d512` ----
  * Replaces Attention / AttnProcessor2_0 of the AutoencoderKL UNetMidBlock2D.  q, k: fp16 [ntok, d]; vt: fp16 [d, ntok] (V transposed, so
  * that P V is a K-major GEMM); out: fp16 [ntok, d].  One call = softmax(scale q k^T) v for one image, computed as three passes of the

@@ -75,6 +75,14 @@ def add_checkpoint_args(p):
     p.add_argument("--vae_dir", type=str, default=None, help="VAE folder (e.g. sdxl-vae-fp16-fix); default <checkpoints>/vae")
     p.add_argument("--unet_dir", type=str, default=None, help="UNet folder override (SSD-1B: the lcm-ssd-1b UNet)")
     p.add_argument("--lcm_lora", type=str, default=None, help="LCM-LoRA safetensors file (SDXL)")
+    p.add_argument("--vae_dtype", choices=("auto", "fp16", "bf16"), default="auto",
+                   help="VAE storage type: auto = bf16 if the VAE config.json says force_upcast: true (e.g. stabilityai/sdxl-vae), else fp16")
+
+
+def vae_dtype_from_args(args):
+    """--vae_dtype -> FastEditor(vae_dtype=...): None (auto), torch.float16 or torch.bfloat16."""
+    import torch
+    return {"auto": None, "fp16": torch.float16, "bf16": torch.bfloat16}[args.vae_dtype]
 
 
 def checkpoints_from_args(args):
@@ -119,7 +127,7 @@ def main(argv=None):
     device = f"cuda:{local}" if world > 1 else "cuda"
     editor = FastEditor(model_name=args.model, device=device, enable_cpu_offload=not args.no_cpu_offload,
                         use_full_precision=args.full_precision, use_full_controlnet=args.full_controlnet, verbose=rank == 0,
-                        checkpoints=checkpoints_from_args(args))
+                        checkpoints=checkpoints_from_args(args), vae_dtype=vae_dtype_from_args(args))
     if hasattr(editor, "pipe"):
         editor.pipe.set_progress_bar_config(disable=True)
     processed = skipped = failed = 0

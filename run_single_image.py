@@ -12,7 +12,7 @@ from datetime import datetime
 
 from PIL import Image
 
-from run_batch import checkpoints_from_args
+from run_batch import checkpoints_from_args, vae_dtype_from_args
 from src.pipeline import FastEditor
 
 
@@ -70,7 +70,7 @@ def main(argv=None):
     print("\n[2/4] Initializing FastEditor...")
     editor = FastEditor(model_name=args.model, device="cuda", enable_cpu_offload=not args.no_cpu_offload,
                         use_full_precision=args.full_precision, use_full_controlnet=args.full_controlnet,
-                        checkpoints=checkpoints_from_args(args))
+                        checkpoints=checkpoints_from_args(args), vae_dtype=vae_dtype_from_args(args))
     mem = editor.get_memory_usage()
     print(f"      GPU Memory: {mem['allocated_gb']:.2f}GB allocated, {mem['reserved_gb']:.2f}GB reserved")
     print("\n[3/4] Running image editing...")
