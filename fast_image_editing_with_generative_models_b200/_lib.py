@@ -70,6 +70,7 @@ SIGNATURES = {
     "fie_gemm_trace": (None, [c_void_p]),
     "fie_attention_trace": (None, [c_void_p]),
     "fie_tune_conv_halo": (None, [c_int, c_int]),
+    "fie_tune_conv_im2col": (None, [c_int]),
     "fie_tune_groupnorm_slab": (None, [c_int]),
     "fie_pack_conv3x3_f16": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p]),
     "fie_pack_conv3x3_c8_f16": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_void_p]),

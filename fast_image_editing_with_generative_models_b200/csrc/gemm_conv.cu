@@ -10,6 +10,9 @@
 //   CONV mode:  A tile = 4-D box {64 ch, bw, bh, bn} (bw*bh*bn = 128 output pixels) of the NHWC activation,
 //               shifted by the filter tap; zero padding comes from TMA out-of-bounds fill, so im2col is never
 //               materialised.  Stride-2 convolutions read four parity-split views of the input.
+//   CONV im2col mode (widths the box cannot tile: not a multiple of 128 and not a divisor of 128): A tile = 128 consecutive
+//               output pixels in raster order (n, y, x), wrapping across rows and images, loaded by TMA im2col mode with the
+//               tap as the im2col offset; the map's bounding box gives the zero padding.
 //   B tile = 2-D box {64 k, block_n rows} of the packed weight matrix [N][K].
 // Math: one elected thread issues tcgen05.mma (M=128, N=block_n, K=16) into a double-buffered TMEM accumulator.
 // Epilogue: 4 warps read TMEM (tcgen05.ld 32x32b), fuse bias / time-embedding broadcast / SiLU / GEGLU /
@@ -50,7 +53,8 @@ constexpr int EPI_STAGE_BYTES = 8 * 1024;      // per-epilogue-warp bias staging
 struct GemmParams {
     CUtensorMap a_maps[4];
     CUtensorMap b_map;
-    int mode;         // 0 = GEMM, 1 = CONV (one shifted A tile per tap), 2 = CONV halo (A slabs shared by the 9 taps)
+    int mode;         // 0 = GEMM, 1 = CONV (one shifted A tile per tap), 2 = CONV halo (A slabs shared by the 9 taps),
+                      // 3 = CONV im2col (one raster run of 128 output pixels per tap; a_maps are im2col maps)
     int num_kb;       // K blocks of 64
     int kb_per_tap;   // CONV: cin/64
     int kb_split;     // GEMM: k-blocks taken from a_maps[0]; the rest from a_maps[1]
@@ -317,7 +321,7 @@ __global__ void __launch_bounds__(384, 1) k_gemm_conv(const __grid_constant__ Ge
                 for (int mt = 0; mt < MT; ++mt) {
                     m0[mt] = (((long long)m_blk * MT + mt) * CG + cta_rank) * BLOCK_M;
                     n0i[mt] = 0; h0[mt] = 0; w0[mt] = 0;
-                    if (p.mode == 1) {
+                    if (p.mode == 1 || p.mode == 3) {
                         const long long pix = (long long)p.OH * p.OW;
                         n0i[mt] = (int)(m0[mt] / pix);
                         const int rem = (int)(m0[mt] % pix);
@@ -344,6 +348,16 @@ __global__ void __launch_bounds__(384, 1) k_gemm_conv(const __grid_constant__ Ge
                                     const CUtensorMap* am = first ? &p.a_maps[0] : &p.a_maps[1];
                                     const int kc = (first ? kb : kb - p.kb_split) * BLOCK_K;
                                     if (CG == 1) tma_load_2d(am, &full_bar[stage], sa, kc, (int)m0[mt]); else tma_load_2d_2sm(am, &full_bar[stage], sa, kc, (int)m0[mt]);
+                                } else if (p.mode == 3) {
+                                    // the run starts at input pixel (x - 1, y - 1) of the bounding box; tap (dh, dw) reads it at (+dw+1, +dh+1).
+                                    // Past the last K block the B tile is zero-filled, so any in-bounds A block adds nothing (tap 0, chunk 0).
+                                    const bool pad_kb = kb >= p.num_kb;
+                                    const int tap = pad_kb ? 0 : kb / p.kb_per_tap;
+                                    const int c0 = pad_kb ? 0 : (kb - tap * p.kb_per_tap) * BLOCK_K;
+                                    const CUtensorMap* am = &p.a_maps[p.tap_map[tap]];
+                                    const uint16_t ow = (uint16_t)(p.tap_dw[tap] + 1), oh = (uint16_t)(p.tap_dh[tap] + 1);
+                                    if (CG == 1) tma_load_im2col_4d(am, &full_bar[stage], sa, c0, w0[mt] - 1, h0[mt] - 1, n0i[mt], ow, oh);
+                                    else tma_load_im2col_4d_2sm(am, &full_bar[stage], sa, c0, w0[mt] - 1, h0[mt] - 1, n0i[mt], ow, oh);
                                 } else {
                                     int tap = kb / p.kb_per_tap;
                                     int c0 = (kb - tap * p.kb_per_tap) * BLOCK_K;
@@ -656,7 +670,10 @@ __global__ void __launch_bounds__(384, 1) k_gemm_conv(const __grid_constant__ Ge
                             lo_s += f.x + f.y; lo_q = fmaf(f.x, f.x, fmaf(f.y, f.y, lo_q));
                         }
                     }
-                    if (p.gn_stats) {                                   // GroupNorm statistics of the (fp16-rounded) output for the consumer
+                    // GroupNorm statistics of the (fp16-rounded) output for the consumer.  Only warps whose rows start below M: a warp of the
+                    // last, partial tile that lies wholly past M would key image n, one block past the [n][groups][2] buffer.  (gn_rows is a
+                    // multiple of 32 and divides M, so a warp is either wholly inside or wholly past M, and never spans two images.)
+                    if (p.gn_stats && m - lane < p.M) {
                         const long long key = ((m - lane) / p.gn_rows) * p.num_n_blocks + n_blk;
                         if (key != gn_key) { gn_flush(); gn_key = key; }
                         float vr[32];
@@ -746,7 +763,48 @@ int make_tmap_f16(CUtensorMap* out, const void* base, int rank, const uint64_t* 
     return FIE_OK;
 }
 
+typedef CUresult (*PFN_encodeIm2col)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*, const int*,
+                                     const int*, cuuint32_t, cuuint32_t, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
+                                     CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
+
+int make_tmap_im2col_f16(CUtensorMap* out, const void* base, const uint64_t* dims, const uint64_t* strides_bytes, const int* lower,
+                         const int* upper, bool bf16) {
+    static PFN_encodeIm2col enc = nullptr;
+    if (!enc) {
+        void* fp = nullptr;
+        cudaDriverEntryPointQueryResult q;
+        if (cudaGetDriverEntryPoint("cuTensorMapEncodeIm2col", &fp, cudaEnableDefault, &q) == cudaSuccess && q == cudaDriverEntryPointSuccess)
+            enc = (PFN_encodeIm2col)fp;
+    }
+    if (!enc) { set_error("cuTensorMapEncodeIm2col not available (driver too old?)"); return FIE_ERR_CUDA; }
+    if ((reinterpret_cast<uintptr_t>(base) & 15) != 0) { set_error("TMA base pointer %p not 16-byte aligned", base); return FIE_ERR_INVALID; }
+    cuuint64_t gd[4]; cuuint64_t gs[3]; const cuuint32_t es[4] = {1, 1, 1, 1};
+    for (int i = 0; i < 4; ++i) gd[i] = dims[i];
+    for (int i = 0; i < 3; ++i) { gs[i] = strides_bytes[i]; if (gs[i] & 15) { set_error("TMA stride %d = %llu not a multiple of 16 bytes", i, (unsigned long long)gs[i]); return FIE_ERR_INVALID; } }
+    CUresult r = enc(out, bf16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 4, const_cast<void*>(base), gd, gs, lower, upper,
+                     (cuuint32_t)BLOCK_K, (cuuint32_t)BLOCK_M, es, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
+                     CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    if (r != CUDA_SUCCESS) { set_error("cuTensorMapEncodeIm2col failed with CUresult %d (dims %llu,%llu,%llu,%llu)", (int)r, (unsigned long long)dims[0],
+                                       (unsigned long long)dims[1], (unsigned long long)dims[2], (unsigned long long)dims[3]); return FIE_ERR_CUDA; }
+    return FIE_OK;
+}
+
 static int num_sms() { return device_sm_count(); }
+
+static int g_force_im2col = 0;      // test / measurement hook (fie_tune_conv_im2col): im2col mode on shapes the box also tiles
+
+// The rectangular A box {64 ch, bw, bh, bn} of 128 output pixels for an OH x OW output, or false when no such box tiles it (the
+// width is neither a multiple nor a divisor of 128, or the rows do not stack into whole boxes): those shapes run in im2col mode.
+static bool box_tile(int OW, int OH, int* bw, int* bh, int* bn) {
+    if (g_force_im2col) return false;
+    if (OW >= BLOCK_M) { *bw = BLOCK_M; *bh = 1; *bn = 1; return (OW % BLOCK_M) == 0; }
+    if ((BLOCK_M % OW) != 0) return false;
+    *bw = OW; *bh = BLOCK_M / OW; *bn = 1;
+    if (*bh <= OH) return (OH % *bh) == 0;
+    if ((*bh % OH) != 0) return false;
+    *bn = *bh / OH; *bh = OH;
+    return true;
+}
 
 // Tile configuration.  Measured on B200 (scripts/gemm_bench.py, scripts/gemm_dbg.py): the producer/consumer mbarrier
 // handshake costs ~300 ns per pipeline stage regardless of tile width, so the kernel runs 2 K-blocks per stage (KPS = 2)
@@ -814,7 +872,8 @@ static int fill_epilogue(GemmParams& p, const fie_epilogue* ep, long long M, int
         FIE_REQUIRE(p.gn_groups > 0 && (n_out % p.gn_groups) == 0, "epilogue: gn_groups must divide the output channels");
         p.gn_cpg = n_out / p.gn_groups;
         FIE_REQUIRE(p.gn_cpg <= 32 && (32 % p.gn_cpg) == 0 && p.gn_cpg >= 4, "epilogue: fused GroupNorm statistics need channels/group in {4, 8, 16, 32} (got %d)", p.gn_cpg);
-        FIE_REQUIRE(p.gn_rows > 0 && (p.gn_rows % 32) == 0, "epilogue: gn_rows_per_image must be a positive multiple of 32");
+        FIE_REQUIRE(p.gn_rows > 0 && (p.gn_rows % 32) == 0 && (M % p.gn_rows) == 0,
+                    "epilogue: gn_rows_per_image must be a positive multiple of 32 that divides the rows");
         FIE_REQUIRE(!p.out_f32 && (n_out % 32) == 0 && (ldd % 16) == 0 && (reinterpret_cast<uintptr_t>(D) & 31) == 0 &&
                     (!p.residual || ((p.ld_res % 16) == 0 && (reinterpret_cast<uintptr_t>(p.residual) & 31) == 0)) &&
                     (!p.row_bias || (p.rows_per_group % 32) == 0),
@@ -833,7 +892,6 @@ static int fill_epilogue(GemmParams& p, const fie_epilogue* ep, long long M, int
         FIE_REQUIRE(!p.ln_in || (ep->ln_dim > 0 && p.ln_eps >= 0.0f && !p.row_bias && !p.m_bias), "epilogue: ln_stats_in needs ln_dim > 0, ln_eps >= 0 and no row / m bias");
         FIE_REQUIRE(!(p.ln_out && p.act == FIE_ACT_GEGLU), "epilogue: ln_stats_out is not supported with the GEGLU epilogue");
     }
-    (void)M;
     return FIE_OK;
 }
 
@@ -900,6 +958,8 @@ using namespace fie;
 
 extern "C" void fie_tune_conv_halo(int enable, int max_cout) { fie::g_halo = enable; if (max_cout > 0) fie::g_halo_max_cout = max_cout; }
 
+extern "C" void fie_tune_conv_im2col(int force) { fie::g_force_im2col = force != 0; }
+
 extern "C" void fie_tune_gemm(int force_cg, int force_block_n) { fie::g_force_cg = force_cg & 3; fie::g_force_kps = (force_cg >> 2) & 3; fie::g_dbg = (force_cg >> 4) & 15; fie::g_force_mt = (force_cg >> 8) & 3; fie::g_force_bn = force_block_n; }
 
 // Debug: install (or clear, with NULL) a device buffer of 8 x int64 per CTA that the next GEMM launches fill with
@@ -956,14 +1016,8 @@ static int conv3x3_impl(const char* fn, const void* x, const void* wgt, void* ou
     FIE_REQUIRE(stride == 1 || stride == 2, "%s: stride must be 1 or 2", fn);
     FIE_REQUIRE(stride == 1 || ((h % 2) == 0 && (w % 2) == 0), "%s: stride 2 needs even h, w", fn);
     const int OH = h / stride, OW = w / stride;
-    int bw, bh, bn;
-    if (OW >= 128) { FIE_REQUIRE((OW % 128) == 0, "%s: output width %d must be a multiple of 128", fn, OW); bw = 128; bh = 1; bn = 1; }
-    else {
-        FIE_REQUIRE((128 % OW) == 0, "%s: output width %d must divide 128", fn, OW);
-        bw = OW; bh = 128 / OW;
-        if (bh <= OH) { FIE_REQUIRE((OH % bh) == 0, "%s: output height %d not a multiple of %d", fn, OH, bh); bn = 1; }
-        else { FIE_REQUIRE((bh % OH) == 0, "%s: output height %d must divide %d", fn, OH, bh); bn = bh / OH; bh = OH; }
-    }
+    int bw = 0, bh = 0, bn = 0;
+    const bool boxed = box_tile(OW, OH, &bw, &bh, &bn);
     GemmParams p;
     memset(&p, 0, sizeof(p));
     const long long M = (long long)n * OH * OW;
@@ -971,8 +1025,8 @@ static int conv3x3_impl(const char* fn, const void* x, const void* wgt, void* ou
     if (rc) return rc;
     FIE_REQUIRE(p.act != FIE_ACT_GEGLU, "%s: GEGLU epilogue not supported for conv", fn);
     if (g_halo < 0) { const char* e = getenv("FIE_CONV_HALO"); g_halo = e ? atoi(e) : 1; }
-    const bool halo = g_halo > 0 && stride == 1 && (OW % BLOCK_M) == 0 && cout <= g_halo_max_cout;
-    p.mode = halo ? 2 : 1; p.M = M; p.N = cout; p.OH = OH; p.OW = OW; p.ab_bf16 = ab_bf16;
+    const bool halo = boxed && g_halo > 0 && stride == 1 && (OW % BLOCK_M) == 0 && cout <= g_halo_max_cout;
+    p.mode = halo ? 2 : (boxed ? 1 : 3); p.M = M; p.N = cout; p.OH = OH; p.OW = OW; p.ab_bf16 = ab_bf16;
     pick_config(M, cout, false, &p.cg, &p.block_n, &p.mt, halo ? 1 : 2);
     p.num_m_blocks = (int)((M + BLOCK_M * p.cg * p.mt - 1) / (BLOCK_M * p.cg * p.mt));
     p.num_n_blocks = (cout + p.block_n - 1) / p.block_n;
@@ -981,10 +1035,12 @@ static int conv3x3_impl(const char* fn, const void* x, const void* wgt, void* ou
     p.kb_split = p.num_kb;
     p.n_store = cout_valid > 0 ? cout_valid : cout;
     const uint32_t box[4] = {BLOCK_K, (uint32_t)(halo ? HALO_PX : bw), (uint32_t)(halo ? 1 : bh), (uint32_t)(halo ? 1 : bn)};
+    static const int lower[2] = {-1, -1}, upper[2] = {-1, -1};    // im2col: one run position per output pixel of the view
     if (stride == 1) {
         const uint64_t dims[4] = {(uint64_t)cin, (uint64_t)w, (uint64_t)h, (uint64_t)n};
         const uint64_t strides[3] = {(uint64_t)cin * 2, (uint64_t)w * cin * 2, (uint64_t)h * w * cin * 2};
-        if ((rc = make_tmap_f16(&p.a_maps[0], x, 4, dims, strides, box, ab_bf16 != 0))) return rc;
+        if ((rc = boxed ? make_tmap_f16(&p.a_maps[0], x, 4, dims, strides, box, ab_bf16 != 0)
+                        : make_tmap_im2col_f16(&p.a_maps[0], x, dims, strides, lower, upper, ab_bf16 != 0))) return rc;
         p.a_maps[1] = p.a_maps[0]; p.a_maps[2] = p.a_maps[0]; p.a_maps[3] = p.a_maps[0];
         for (int t = 0; t < 9; ++t) { p.tap_map[t] = 0; p.tap_dh[t] = (int8_t)(t / 3 - 1); p.tap_dw[t] = (int8_t)(t % 3 - 1); }
     } else {
@@ -994,7 +1050,8 @@ static int conv3x3_impl(const char* fn, const void* x, const void* wgt, void* ou
         for (int hp = 0; hp < 2; ++hp)
             for (int wp = 0; wp < 2; ++wp) {
                 const uint8_t* base = (const uint8_t*)x + ((size_t)hp * w + wp) * cin * 2;
-                if ((rc = make_tmap_f16(&p.a_maps[hp * 2 + wp], base, 4, dims, strides, box, ab_bf16 != 0))) return rc;
+                if ((rc = boxed ? make_tmap_f16(&p.a_maps[hp * 2 + wp], base, 4, dims, strides, box, ab_bf16 != 0)
+                                : make_tmap_im2col_f16(&p.a_maps[hp * 2 + wp], base, dims, strides, lower, upper, ab_bf16 != 0))) return rc;
             }
         // input row = 2*oh + k - pad:  pad 1: k=0 -> (parity 1, shift -1), k=1 -> (0, 0), k=2 -> (1, 0)
         //                              pad 0 (asymmetric (0,1) padding): k=0 -> (0, 0), k=1 -> (1, 0), k=2 -> (0, +1)
@@ -1021,14 +1078,8 @@ static int conv_up2x_impl(const char* fn, const void* x, const void* wgt, void* 
     FIE_REQUIRE(x && wgt && out, "%s: null pointer", fn);
     FIE_REQUIRE(n > 0 && h > 0 && w > 0 && cin > 0 && cout > 0, "%s: bad shape", fn);
     FIE_REQUIRE((cin % BLOCK_K) == 0 && (cout % 32) == 0, "%s: cin %% 64 and cout %% 32 required", fn);
-    int bw, bh, bn;
-    if (w >= 128) { FIE_REQUIRE((w % 128) == 0, "%s: width %d must be a multiple of 128", fn, w); bw = 128; bh = 1; bn = 1; }
-    else {
-        FIE_REQUIRE((128 % w) == 0, "%s: width %d must divide 128", fn, w);
-        bw = w; bh = 128 / w;
-        if (bh <= h) { FIE_REQUIRE((h % bh) == 0, "%s: height %d not a multiple of %d", fn, h, bh); bn = 1; }
-        else { FIE_REQUIRE((bh % h) == 0, "%s: height %d must divide %d", fn, h, bh); bn = bh / h; bh = h; }
-    }
+    int bw = 0, bh = 0, bn = 0;
+    const bool boxed = box_tile(w, h, &bw, &bh, &bn);
     const long long M = (long long)n * h * w;
     for (int ph = 0; ph < 4; ++ph) {
         GemmParams p;
@@ -1036,7 +1087,7 @@ static int conv_up2x_impl(const char* fn, const void* x, const void* wgt, void* 
         int rc = fill_epilogue(p, ep, M, cout, out, ldd, out_dtype);
         if (rc) return rc;
         FIE_REQUIRE(p.act != FIE_ACT_GEGLU && !p.residual && !p.out_f32, "%s: unsupported epilogue", fn);
-        p.mode = 1; p.M = M; p.N = cout; p.OH = h; p.OW = w; p.ab_bf16 = ab_bf16;
+        p.mode = boxed ? 1 : 3; p.M = M; p.N = cout; p.OH = h; p.OW = w; p.ab_bf16 = ab_bf16;
         p.up2 = 1; p.up_a = ph >> 1; p.up_b = ph & 1;
         pick_config(M, cout, false, &p.cg, &p.block_n, &p.mt);
         p.num_m_blocks = (int)((M + BLOCK_M * p.cg * p.mt - 1) / (BLOCK_M * p.cg * p.mt));
@@ -1048,7 +1099,9 @@ static int conv_up2x_impl(const char* fn, const void* x, const void* wgt, void* 
         const uint32_t box[4] = {BLOCK_K, (uint32_t)bw, (uint32_t)bh, (uint32_t)bn};
         const uint64_t dims[4] = {(uint64_t)cin, (uint64_t)w, (uint64_t)h, (uint64_t)n};
         const uint64_t strides[3] = {(uint64_t)cin * 2, (uint64_t)w * cin * 2, (uint64_t)h * w * cin * 2};
-        if ((rc = make_tmap_f16(&p.a_maps[0], x, 4, dims, strides, box, ab_bf16 != 0))) return rc;
+        static const int lower[2] = {-1, -1}, upper[2] = {-1, -1};
+        if ((rc = boxed ? make_tmap_f16(&p.a_maps[0], x, 4, dims, strides, box, ab_bf16 != 0)
+                        : make_tmap_im2col_f16(&p.a_maps[0], x, dims, strides, lower, upper, ab_bf16 != 0))) return rc;
         p.a_maps[1] = p.a_maps[0]; p.a_maps[2] = p.a_maps[0]; p.a_maps[3] = p.a_maps[0];
         for (int t = 0; t < 4; ++t) {   // tap (ty, tx): input row i + ty - 1 + a, column j + tx - 1 + b
             p.tap_map[t] = 0; p.tap_dh[t] = (int8_t)((t >> 1) - 1 + p.up_a); p.tap_dw[t] = (int8_t)((t & 1) - 1 + p.up_b);
@@ -1074,21 +1127,15 @@ static int conv3x3_c8_impl(const char* fn, const void* xp, const void* wgt, void
                            int cout_valid, const fie_epilogue* ep, int out_dtype, void* stream) {
     FIE_REQUIRE(xp && wgt && out, "%s: null pointer", fn);
     FIE_REQUIRE(n > 0 && h > 0 && w > 0 && cout > 0 && (cout % 32) == 0, "%s: bad shape (cout must be a multiple of 32)", fn);
-    int bw, bh, bn;
-    if (w >= 128) { FIE_REQUIRE((w % 128) == 0, "%s: width %d must be a multiple of 128", fn, w); bw = 128; bh = 1; bn = 1; }
-    else {
-        FIE_REQUIRE((128 % w) == 0, "%s: width %d must divide 128", fn, w);
-        bw = w; bh = 128 / w;
-        if (bh <= h) { FIE_REQUIRE((h % bh) == 0, "%s: height %d not a multiple of %d", fn, h, bh); bn = 1; }
-        else { FIE_REQUIRE((bh % h) == 0, "%s: height %d must divide %d", fn, h, bh); bn = bh / h; bh = h; }
-    }
+    int bw = 0, bh = 0, bn = 0;
+    const bool boxed = box_tile(w, h, &bw, &bh, &bn);
     GemmParams p;
     memset(&p, 0, sizeof(p));
     const long long M = (long long)n * h * w;
     int rc = fill_epilogue(p, ep, M, cout, out, ldd, out_dtype);
     if (rc) return rc;
     FIE_REQUIRE(p.act != FIE_ACT_GEGLU, "%s: GEGLU epilogue not supported for conv", fn);
-    p.mode = 1; p.M = M; p.N = cout; p.OH = h; p.OW = w;
+    p.mode = boxed ? 1 : 3; p.M = M; p.N = cout; p.OH = h; p.OW = w;
     pick_config(M, cout, false, &p.cg, &p.block_n, &p.mt);
     p.num_m_blocks = (int)((M + BLOCK_M * p.cg * p.mt - 1) / (BLOCK_M * p.cg * p.mt));
     p.num_n_blocks = (cout + p.block_n - 1) / p.block_n;
@@ -1098,7 +1145,10 @@ static int conv3x3_c8_impl(const char* fn, const void* xp, const void* wgt, void
     const uint64_t wp = (uint64_t)w + 8, hp = (uint64_t)h + 2;
     const uint64_t dims[4] = {BLOCK_K, (uint64_t)w, hp, (uint64_t)n};
     const uint64_t strides[3] = {16, wp * 16, hp * wp * 16};
-    if ((rc = make_tmap_f16(&p.a_maps[0], xp, 4, dims, strides, box))) return rc;
+    // im2col: the run walks the w start pixels of the h output rows (the view has h + 2 rows); the taps add the kernel row
+    static const int lower[2] = {-1, -1}, upper[2] = {-1, -3};
+    if ((rc = boxed ? make_tmap_f16(&p.a_maps[0], xp, 4, dims, strides, box) : make_tmap_im2col_f16(&p.a_maps[0], xp, dims, strides, lower, upper)))
+        return rc;
     p.a_maps[1] = p.a_maps[0]; p.a_maps[2] = p.a_maps[0]; p.a_maps[3] = p.a_maps[0];
     for (int t = 0; t < 6; ++t) { p.tap_map[t] = 0; p.tap_dh[t] = (int8_t)(t >> 1); p.tap_dw[t] = 0; }   // padded row y + kh, padded pixel x
     const uint64_t bdims[2] = {(uint64_t)6 * BLOCK_K, (uint64_t)cout};

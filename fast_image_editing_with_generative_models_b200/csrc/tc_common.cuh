@@ -93,6 +93,23 @@ __device__ __forceinline__ void tma_load_4d_2sm(const CUtensorMap* m, uint64_t* 
         ::"r"(smem_u32(dst)), "l"(reinterpret_cast<uint64_t>(m)), "r"(smem_u32(bar) & kPeerBitMask), "r"(c0), "r"(c1), "r"(c2), "r"(c3) : "memory");
 }
 
+// Im2col-mode loads of an NHWC map (make_tmap_im2col_f16): the channelsPerPixel x pixelsPerColumn block that starts at pixel
+// (c1, c2, c3) = (w, h, n) and walks the map's bounding box in raster order (w, then h, then n), every pixel read at (+ow, +oh).
+__device__ __forceinline__ void tma_load_im2col_4d(const CUtensorMap* m, uint64_t* bar, void* dst, int c0, int c1, int c2, int c3,
+                                                   uint16_t ow, uint16_t oh) {
+    asm volatile(
+        "cp.async.bulk.tensor.4d.shared::cluster.global.im2col.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], [%2], {%7, %8};"
+        ::"r"(smem_u32(dst)), "l"(reinterpret_cast<uint64_t>(m)), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2), "r"(c3), "h"(ow), "h"(oh)
+        : "memory");
+}
+__device__ __forceinline__ void tma_load_im2col_4d_2sm(const CUtensorMap* m, uint64_t* bar, void* dst, int c0, int c1, int c2, int c3,
+                                                       uint16_t ow, uint16_t oh) {
+    asm volatile(
+        "cp.async.bulk.tensor.4d.cta_group::2.shared::cluster.global.im2col.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5, %6}], [%2], {%7, %8};"
+        ::"r"(smem_u32(dst)), "l"(reinterpret_cast<uint64_t>(m)), "r"(smem_u32(bar) & kPeerBitMask), "r"(c0), "r"(c1), "r"(c2), "r"(c3),
+          "h"(ow), "h"(oh) : "memory");
+}
+
 // One elected lane of a fully converged warp (elect.sync).  Together with a shuffle-broadcast warp index this keeps the
 // TMA / MMA issue loops in uniform control flow, so their descriptors live in uniform registers instead of being moved
 // there (R2UR + vote loops) before every tcgen05.mma / cp.async.bulk.tensor.
@@ -266,5 +283,9 @@ constexpr uint32_t kIdescABBF16 = (1u << 7) | (1u << 10);
 // Encodes a tiled fp16 (bf16 = true: bf16) tensor map with 128B swizzle. dims/strides innermost-first; strides (bytes) for dims 1..rank-1.
 int make_tmap_f16(CUtensorMap* out, const void* base, int rank, const uint64_t* dims, const uint64_t* strides_bytes, const uint32_t* box,
                   bool bf16 = false);
+// Encodes a rank-4 im2col map {C, W, H, N} with 128B swizzle that loads 64 channels x 128 pixels.  lower / upper: {W, H} corners
+// of the bounding box the pixels are walked in: [lower, dim - 1 + upper]; reads outside the tensor are zero-filled.
+int make_tmap_im2col_f16(CUtensorMap* out, const void* base, const uint64_t* dims, const uint64_t* strides_bytes, const int* lower,
+                         const int* upper, bool bf16 = false);
 
 }  // namespace fie

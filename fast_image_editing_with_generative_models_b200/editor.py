@@ -4,7 +4,9 @@ Same constructor, ``edit`` / ``preprocess_image`` / ``clear_memory`` / ``get_mem
 (``model_name, device, dtype, config, controlnet, pipe``) and error behaviour (``ValueError`` for an unknown model and for
 an invalid ``strength``, Python exceptions per image, usable after a failed call) as the reference; the arithmetic runs in
 the hand-written CUDA kernels behind ``include/fie_b200.h``.  One addition: :meth:`FastEditor.edit_many`, the batched form
-of ``edit`` (micro-batches of 8 images per GPU, SURVEY 8(e)) that ``run_batch.py`` uses.
+of ``edit`` (micro-batches of 8 images per GPU, SURVEY 8(e)) that ``run_batch.py`` uses.  ``edit``, ``edit_many`` and ``warm_up`` take a
+keyword-only ``size``: ``None`` (the reference's 1024 x 1024), a ``(width, height)`` or ``"auto"`` (the SDXL aspect-ratio bucket
+closest to the input's shape, ``FastEditor.SDXL_BUCKETS``).
 
 Differences, all forced by the environment and stated in DESIGN.md:
 
@@ -78,6 +80,40 @@ def vae_fp16_warning(real_weights: bool, vae_dtype: torch.dtype, force_upcast: O
             "--vae_dir) or FastEditor(vae_dtype=torch.bfloat16) (--vae_dtype bf16).")
 
 
+MAX_PIXELS = 1024 * 1024        # VAE mid-block attention: at most 16384 latent tokens (fie_softmax_rows_exp_f16)
+
+
+def resolve_size(size, image_size) -> tuple:
+    """``size`` argument -> (width, height) of the edit for an input of PIL size ``image_size`` = (width, height).
+
+    ``None``: 1024 x 1024.  ``(width, height)``: each side a multiple of 64 in [256, 2048] and width * height <= 1024^2.
+    ``"auto"``: the entry of :data:`FastEditor.SDXL_BUCKETS` whose aspect ratio is closest to the input's in log space (ties: the
+    earlier one)."""
+    if size is None:
+        return (FastEditor.OUT_SIZE, FastEditor.OUT_SIZE)
+    if isinstance(size, str):
+        if size != "auto":
+            raise ValueError(f"size must be None, (width, height) or 'auto', not {size!r}")
+        iw, ih = image_size
+        if iw <= 0 or ih <= 0:
+            raise ValueError(f"size='auto' needs a non-empty image, got {image_size}")
+        r = np.log(iw) - np.log(ih)
+        # log w - log h: exactly antisymmetric, so transposed buckets are exactly equidistant from a square input; min keeps the first
+        return min(FastEditor.SDXL_BUCKETS, key=lambda b: abs(np.log(b[0]) - np.log(b[1]) - r))
+    try:
+        w, h = size
+    except (TypeError, ValueError):
+        raise ValueError(f"size must be None, (width, height) or 'auto', not {size!r}") from None
+    if not all(isinstance(v, (int, np.integer)) and not isinstance(v, bool) for v in (w, h)):
+        raise ValueError(f"size sides must be integers, got {size!r}")
+    w, h = int(w), int(h)
+    if w % 64 or h % 64 or not (256 <= w <= 2048 and 256 <= h <= 2048):
+        raise ValueError(f"size {w}x{h}: each side must be a multiple of 64 in [256, 2048]")
+    if w * h > MAX_PIXELS:
+        raise ValueError(f"size {w}x{h}: at most {MAX_PIXELS} pixels (1024 x 1024)")
+    return (w, h)
+
+
 class _PipeShim:
     """What callers touch on ``editor.pipe``: ``run_batch.py:157-158`` calls ``set_progress_bar_config(disable=True)``."""
 
@@ -107,7 +143,9 @@ class FastEditor:
         },
     }
     MICRO_BATCH = 8            # images per GPU per engine call in edit_many (SURVEY 8(e))
-    OUT_SIZE = 1024            # the reference resizes every input to 1024 x 1024 (src/pipeline.py:251)
+    OUT_SIZE = 1024            # the reference resizes every input to 1024 x 1024 (src/pipeline.py:251); the default of ``size``
+    # size="auto": SDXL / SSD-1B training resolutions of about one megapixel, (width, height)
+    SDXL_BUCKETS = ((1024, 1024), (1152, 896), (896, 1152), (1216, 832), (832, 1216), (1344, 768), (768, 1344), (1536, 640), (640, 1536))
 
     def __init__(self, model_name="sdxl", device="cuda", dtype=torch.float16, enable_cpu_offload=True, use_full_precision=False,
                  use_full_controlnet=False, *, state: Optional[Dict] = None, prompt_encoder: Optional[Callable] = None, tiny: bool = False,
@@ -268,33 +306,38 @@ class FastEditor:
                              f"{n_exec} which is < 1 and not appropriate for this pipeline.")
         return n_exec
 
-    def _draw_noises(self, seed, n_exec: int) -> List[torch.Tensor]:
-        """Reference RNG order for one image: posterior sample, init noise, then one draw per non-final executed step."""
+    def _draw_noises(self, seed, n_exec: int, size=(OUT_SIZE, OUT_SIZE)) -> List[torch.Tensor]:
+        """Reference RNG order for one image of ``size`` = (width, height): posterior sample, init noise, then one draw per non-final
+        executed step, each [1, 4, height/8, width/8]."""
         gen = torch.Generator(device=self._dev)
         if seed is not None:
             gen.manual_seed(int(seed))
         else:
             gen.seed()
-        h = self.OUT_SIZE // 8
-        return [torch.randn((1, 4, h, h), generator=gen, device=self._dev, dtype=torch.float16) for _ in range(2 + max(n_exec - 1, 0))]
+        shape = (1, 4, size[1] // 8, size[0] // 8)
+        return [torch.randn(shape, generator=gen, device=self._dev, dtype=torch.float16) for _ in range(2 + max(n_exec - 1, 0))]
 
-    def _to_device_1024(self, image) -> torch.Tensor:
-        """PIL image of any size -> uint8 [1,1024,1024,3] on the GPU; ``image.resize((1024, 1024), Image.LANCZOS)`` of the reference
-        (src/pipeline.py:251) runs on the GPU, bit-identical to Pillow."""
+    def _to_device(self, image, size=(OUT_SIZE, OUT_SIZE)) -> torch.Tensor:
+        """PIL image of any size -> uint8 [1,height,width,3] on the GPU; ``image.resize(size, Image.LANCZOS)`` of the reference
+        (src/pipeline.py:251, there with size = (1024, 1024)) runs on the GPU, bit-identical to Pillow."""
         arr = np.ascontiguousarray(np.array(image.convert("RGB")))
         img = torch.from_numpy(arr[None]).pin_memory().to(self._dev, non_blocking=True)      # pinned staging: the copy does not block the host
-        if img.shape[1] != self.OUT_SIZE or img.shape[2] != self.OUT_SIZE:
-            img = ops.resize_lanczos(img, self.OUT_SIZE, self.OUT_SIZE)
+        w, h = size
+        if img.shape[1] != h or img.shape[2] != w:
+            img = ops.resize_lanczos(img, h, w)
         return img
 
     def edit(self, image, prompt, negative_prompt="", strength=0.80, num_inference_steps=4, guidance_scale=1.5,
-             controlnet_conditioning_scale=0.5, canny_low_threshold=100, canny_high_threshold=200, seed=None, *, canny_gaussian_blur=False):
-        """Edit an image with a text prompt, preserving structure via Canny conditioning -> PIL RGB 1024x1024."""
+             controlnet_conditioning_scale=0.5, canny_low_threshold=100, canny_high_threshold=200, seed=None, *, canny_gaussian_blur=False,
+             size=None):
+        """Edit an image with a text prompt, preserving structure via Canny conditioning -> PIL RGB image of ``size`` (default
+        1024x1024; see :func:`resolve_size`)."""
+        wh = resolve_size(size, image.size)
         n_exec = self._executed_steps(strength, num_inference_steps)
         with torch.cuda.device(self._dev):
-            img = self._to_device_1024(image)
+            img = self._to_device(image, wh)
             pe, pl = self._encode_prompt(prompt, negative_prompt)
-            noises = self._draw_noises(seed, n_exec)
+            noises = self._draw_noises(seed, n_exec, wh)
             out = self._engine.edit_batch(img, pe, pl, noises, strength=strength, num_inference_steps=num_inference_steps,
                                           guidance_scale=guidance_scale, controlnet_conditioning_scale=controlnet_conditioning_scale,
                                           canny_low=int(np.floor(canny_low_threshold)), canny_high=int(np.floor(canny_high_threshold)),
@@ -304,7 +347,7 @@ class FastEditor:
     def edit_many(self, images: Sequence, prompts: Union[str, Sequence[str]], negative_prompt: Union[str, Sequence[str]] = "", strength=0.80,
                   num_inference_steps=4, guidance_scale=1.5, controlnet_conditioning_scale=0.5, canny_low_threshold=100, canny_high_threshold=200,
                   seed=None, seeds: Optional[Sequence[Optional[int]]] = None, micro_batch: Optional[int] = None,
-                  canny_gaussian_blur: bool = False, output: str = "pil", jpeg_quality: int = 75) -> List:
+                  canny_gaussian_blur: bool = False, output: str = "pil", jpeg_quality: int = 75, *, size=None) -> List:
         """Batched ``edit``: ``[edit(images[i], prompts[i], ..., seed=seeds[i]) for i]`` — same per-image semantics (each image gets its
         own generator seeded with ``seeds[i]``, or ``seed`` for all, drawing in the reference's order; the results are the ones the
         per-image calls give) but run in micro-batches of ``micro_batch`` (default 8) images per engine call.
@@ -312,6 +355,9 @@ class FastEditor:
         ``output="jpeg"``: returns the edited images as JPEG files (``bytes``, what ``image.save("x.jpg")`` would write — byte-identical
         to Pillow's encoder at ``jpeg_quality``), encoded on the GPU: ~0.1-0.3 MB instead of 3 MB per image cross PCIe and the host
         does no pixel work at all.
+
+        ``size`` as in :meth:`edit`.  With ``"auto"`` the images are grouped by their bucket; each group runs in its own micro-batches
+        and the results come back in input order.
 
         The host side is pipelined: while the GPU runs micro-batch *i* (one CUDA-graph replay), the host converts the outputs of
         micro-batch *i-1* to PIL images and stages the inputs of *i+1* (pinned buffers, asynchronous copies)."""
@@ -330,12 +376,15 @@ class FastEditor:
         n_exec = self._executed_steps(strength, num_inference_steps)
         mb = int(micro_batch or self.MICRO_BATCH)
         lo, hi = int(np.floor(canny_low_threshold)), int(np.floor(canny_high_threshold))
-        S_ = self.OUT_SIZE
+        sizes = [resolve_size(size, im.size) for im in images]
+        by_size: Dict[tuple, List[int]] = {}
+        for i, wh in enumerate(sizes):
+            by_size.setdefault(wh, []).append(i)
+        chunks = [(wh, idx[b0:b0 + mb]) for wh, idx in by_size.items() for b0 in range(0, len(idx), mb)]
         results: List[Optional[Image.Image]] = [None] * n
         pending = None                                   # (index list, pinned output buffer, event) of the micro-batch in flight
         with torch.cuda.device(self._dev):
             stream = torch.cuda.current_stream(self._dev)
-            bufs = self._host_buffers(mb)
 
             def finalize(p):
                 idx, host_out, ev = p
@@ -361,13 +410,12 @@ class FastEditor:
                     trace.append((name, _time.perf_counter() - t0))
                 return _time.perf_counter()
 
-            for k, b0 in enumerate(range(0, n, mb)):
+            for k, (wh, idx) in enumerate(chunks):
                 t_ = _time.perf_counter()
-                idx = list(range(b0, min(b0 + mb, n)))
                 nb = len(idx)
                 pad_to = mb if nb * 2 >= mb else 1 << (nb - 1).bit_length()       # ragged tail: reuse the full-size graph, or the next power of two
-                host_in, host_out = bufs[k & 1]
-                same = all(images[i].size == (S_, S_) for i in idx)
+                host_in, host_out = self._host_buffers(mb, wh)[k & 1]
+                same = all(images[i].size == wh for i in idx)
                 if same:
                     for j, i in enumerate(idx):
                         host_in[j].copy_(torch.from_numpy(np.array(images[i].convert("RGB"))))
@@ -375,13 +423,13 @@ class FastEditor:
                         host_in[j].copy_(host_in[nb - 1])
                     d_img = host_in[:pad_to].to(self._dev, non_blocking=True)
                 else:
-                    parts = [self._to_device_1024(images[i]) for i in idx]
+                    parts = [self._to_device(images[i], wh) for i in idx]
                     d_img = torch.cat(parts + [parts[-1]] * (pad_to - nb), 0)
                 t_ = mark("stage images (PIL->pinned->H2D)", t_)
                 pad = [idx[-1]] * (pad_to - nb)
                 pe, pl = self._encode_prompts([prompts[i] for i in idx + pad], [negs[i] for i in idx + pad])      # [B,2,77,D], [B,2,P]
                 t_ = mark("encode prompts (launch)", t_)
-                per_img = [self._draw_noises(seeds[i], n_exec) for i in idx]
+                per_img = [self._draw_noises(seeds[i], n_exec, wh) for i in idx]
                 per_img += [per_img[-1]] * (pad_to - nb)
                 noises = [torch.cat([p[d] for p in per_img], 0) for d in range(len(per_img[0]))]
                 t_ = mark("noise draws (launch)", t_)
@@ -418,31 +466,40 @@ class FastEditor:
                 finalize(pending)
         return results  # type: ignore[return-value]
 
-    def warm_up(self, micro_batch: Optional[int] = None, **edit_kwargs) -> float:
+    def warm_up(self, micro_batch: Optional[int] = None, *, size=None, **edit_kwargs) -> float:
         """Runs one dummy micro-batch with the given ``edit`` arguments so that the CUDA graph for that shape / schedule is captured and
-        the pinned staging buffers exist before the first real call (sweeps call this during initialisation).  Returns the seconds spent."""
+        the pinned staging buffers exist before the first real call (sweeps call this during initialisation).  ``size`` as in
+        :meth:`edit`; ``"auto"`` warms up the square bucket.  Returns the seconds spent."""
         import time
         t0 = time.perf_counter()
         mb = int(micro_batch or self.MICRO_BATCH)
-        dummy = [Image.new("RGB", (self.OUT_SIZE, self.OUT_SIZE), (127, 127, 127))] * mb
-        self.edit_many(dummy, "warm-up", seed=0, micro_batch=mb, **edit_kwargs)
+        wh = resolve_size(size, (self.OUT_SIZE, self.OUT_SIZE))
+        dummy = [Image.new("RGB", wh, (127, 127, 127))] * mb
+        self.edit_many(dummy, "warm-up", seed=0, micro_batch=mb, size=wh, **edit_kwargs)
         torch.cuda.synchronize(self._dev)
         return time.perf_counter() - t0
 
-    def _host_buffers(self, mb: int):
-        """Two (input, output) pairs of pinned uint8 staging buffers [mb,1024,1024,3] (allocated once per micro-batch size)."""
+    def _host_buffers(self, mb: int, size=(OUT_SIZE, OUT_SIZE)):
+        """Two (input, output) pairs of pinned uint8 staging buffers [mb,height,width,3] (allocated once per micro-batch size and image
+        size = (width, height))."""
         cache = self.__dict__.setdefault("_pinned", {})
-        if mb not in cache:
-            S_ = self.OUT_SIZE
-            cache[mb] = [(torch.empty((mb, S_, S_, 3), dtype=torch.uint8).pin_memory(), torch.empty((mb, S_, S_, 3), dtype=torch.uint8).pin_memory())
-                         for _ in range(2)]
-        return cache[mb]
+        w, h = size
+        key = (mb, h, w)
+        if key not in cache:
+            cache[key] = [(torch.empty((mb, h, w, 3), dtype=torch.uint8).pin_memory(), torch.empty((mb, h, w, 3), dtype=torch.uint8).pin_memory())
+                          for _ in range(2)]
+        self._pinned_last = key
+        return cache[key]
 
     def clear_memory(self):
         """Clear GPU memory cache (reference ``src/pipeline.py:276-279``).  Also drops every captured CUDA graph except the most
-        recently used one (each holds a private memory pool), so a parameter sweep cannot grow memory without bound."""
+        recently used one (each holds a private memory pool) and the pinned staging buffers of every image size but the most recently
+        used one (about 100 MB per size at 8 images per micro-batch), so a parameter sweep cannot grow memory without bound."""
         if str(self.device).startswith("cuda"):
             self._engine.release_graphs(keep=1)
+            pinned = self.__dict__.get("_pinned", {})
+            for key in [k for k in pinned if isinstance(k[0], int) and k != getattr(self, "_pinned_last", None)]:
+                del pinned[key]
             with torch.cuda.device(self._dev):
                 torch.cuda.empty_cache()
 

@@ -28,6 +28,12 @@ class EditOutput:
     extras: Optional[Dict] = None
 
 
+def sdxl_time_ids(height: int, width: int) -> List[float]:
+    """SDXL micro-conditioning of an uncropped image edited at its own size: original size, crop corner (0, 0), target size, each as
+    (height, width), as diffusers' ``_get_add_time_ids``."""
+    return [float(height), float(width), 0.0, 0.0, float(height), float(width)]
+
+
 def _move_to(obj, dev, seen=None):
     """Recursively moves every tensor reachable from ``obj`` (attributes, lists, tuples, dicts) to ``dev``; returns the moved object."""
     seen = set() if seen is None else seen
@@ -184,7 +190,7 @@ class EditEngine:
         rows = [0, 1] if do_cfg else [1]
         ctx = torch.cat([pe[:, r] for r in rows], 0).contiguous()
         te = torch.cat([pl[:, r] for r in rows], 0).contiguous()
-        time_ids = [float(H), float(W), 0.0, 0.0, float(H), float(W)]
+        time_ids = sdxl_time_ids(H, W)
         nctx = ctx.shape[1]
         ps_cn = self.cn.prepare_prompt(ctx, te, time_ids)
         ps_un = self.unet.prepare_prompt(ctx, te, time_ids)

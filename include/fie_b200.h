@@ -175,7 +175,8 @@ typedef struct {
     int out_f32;             /* 1: D is fp32, else fp16 */
     /* Optional GroupNorm statistics of the OUTPUT, accumulated by the epilogue so that the following fie_groupnorm_f16 can
      * skip its statistics pass (stats_ready = 1): int64 [images][gn_groups][2] (sum, sum of squares; 2^-20 fixed point),
-     * zeroed by the caller.  Requires channels-per-group = N_out / gn_groups dividing 32, gn_rows_per_image % 32 == 0 and a
+     * zeroed by the caller.  Requires channels-per-group = N_out / gn_groups dividing 32, gn_rows_per_image % 32 == 0 and
+     * dividing the rows (M = images * gn_rows_per_image; fie_conv_up2x_*: rows are input pixels), and a
      * launch that stays on the fast epilogue path (fp16 output, N_out % 32 == 0, 32-byte aligned rows); else FIE_ERR_INVALID. */
     void* gn_stats;          /* or NULL */
     int gn_groups;
@@ -206,6 +207,9 @@ void fie_tune_gemm(int force_cg, int force_block_n);
 /* Tuning / test hook: enable (1) / disable (0) the halo form of the stride-1 3x3 convolution (input rows loaded once per channel
  * chunk and shared by the 9 taps) and set the widest cout it is used for (0 = keep).  Not needed in production. */
 void fie_tune_conv_halo(int enable, int max_cout);
+/* Test / measurement hook: force (1) the im2col form of fie_conv3x3_*, fie_conv_up2x_* and fie_conv3x3_c8_* on shapes that the
+ * rectangular-box form also tiles (0 = choose by shape, the default).  Not needed in production. */
+void fie_tune_conv_im2col(int force);
 /* GroupNorm: largest thread-block cluster the single-pass shared-memory kernel (k_gn_slab) may use; 0 = always the two-kernel path,
  * default 1 (env FIE_GN_SLAB) — see the measurement note in csrc/norm.cu.  Experiments / tests only. */
 void fie_tune_groupnorm_slab(int max_cluster);
@@ -228,11 +232,16 @@ int fie_gemm_f16(const void* A, long long lda, const void* A1, long long lda1, i
 /* 3x3 convolution as implicit GEMM, NHWC fp16.  x: [n,h,w,cin] (cin multiple of 64), wgt: [cout][3][3][cin],
  * out: [n,oh,ow,cout].  stride 1: pad 1.  stride 2: pad_mode 0 = symmetric pad 1 (UNet Downsample2D),
  * pad_mode 1 = F.pad(0,1,0,1) then pad 0 (VAE encoder Downsample2D).  cout_valid <= cout columns are stored
- * (weights may be zero-padded to a multiple of 32 output channels). */
+ * (weights may be zero-padded to a multiple of 32 output channels).
+ * Shapes: any n, h, w (stride 2: even h, w).  An output width that is a multiple of 128, or a divisor of 128 whose rows stack into
+ * whole 128-pixel boxes, loads the A operand as a rectangular TMA box (stride 1 with >= 128-pixel rows: the halo form); every other
+ * shape (e.g. widths 152, 76, 38, 576, 288, 144 of the 1216x832 / 1152x896 SDXL buckets) loads 128 consecutive output pixels in
+ * raster order with TMA im2col mode.  The choice depends on the shape only; fie_conv_up2x_* and fie_conv3x3_c8_* follow the same
+ * rule with the input width. */
 int fie_conv3x3_f16(const void* x, const void* wgt, void* out, long long ldd, int n, int h, int w, int cin, int cout,
                     int cout_valid, int stride, int pad_mode, const fie_epilogue* ep, void* stream);
 
-/* Nearest-2x upsample fused with the following 3x3 convolution (diffusers Upsample2D).  x: [n,h,w,cin] -> out [n,2h,2w,cout].
+/* Nearest-2x upsample fused with the following 3x3 convolution (diffusers Upsample2D).  x: [n,h,w,cin] -> out [n,2h,2w,cout], any n, h, w.
  * wgt: fp16 [4][cout][2][2][cin] phase weights (host pre-sums the 3x3 taps that hit the same input pixel, see weights.py). */
 int fie_conv_up2x_f16(const void* x, const void* wgt, void* out, long long ldd, int n, int h, int w, int cin, int cout,
                       const fie_epilogue* ep, void* stream);
@@ -245,7 +254,7 @@ int fie_conv3x3_cin4_f16(const void* x, const float* wgt, const float* bias, voi
 /* 3x3 convolution (pad 1) of an image-like input with <= 8 channels on the tensor cores: conv_in of the VAE encoder and of
  * the ControlNet conditioning embedding at full resolution.  xp: fp16 zero-padded [n,h+2,w+8,8] (fie_preprocess_u8_to_f16_pad8);
  * wgt: fp16 [cout][3][2][64]: per kernel row a hi block and a lo block (w = hi + lo keeps the fp32 weights to ~2^-22), element
- * kw*8 + c = w[co][c][kh][kw], zeros elsewhere; out: [n,h,w,cout_valid..] rows of ldd. */
+ * kw*8 + c = w[co][c][kh][kw], zeros elsewhere; out: [n,h,w,cout_valid..] rows of ldd.  Any n, h, w (see fie_conv3x3_f16). */
 int fie_conv3x3_c8_f16(const void* xp, const void* wgt, void* out, long long ldd, int n, int h, int w, int cout,
                        int cout_valid, const fie_epilogue* ep, void* stream);
 

@@ -64,7 +64,27 @@ def build_parser():
     p.add_argument("--no_gpu_jpeg", action="store_true", help="encode *.jpg outputs with PIL on the host instead of the GPU encoder "
                    "(the files are byte-identical either way)")
     add_checkpoint_args(p)
+    add_size_arg(p)
     return p
+
+
+def add_size_arg(p):
+    p.add_argument("--size", type=parse_size, default=(1024, 1024), metavar="{WxH|auto}",
+                   help="output size: WIDTHxHEIGHT (multiples of 64 in [256, 2048], at most 1024x1024 pixels) or auto = the SDXL "
+                        "aspect-ratio bucket closest to each input (default 1024x1024)")
+
+
+def parse_size(text):
+    """--size value -> FastEditor(size=...): 'auto' or (width, height)."""
+    import argparse
+    from fast_image_editing_with_generative_models_b200.editor import resolve_size
+    if text == "auto":
+        return "auto"
+    try:
+        w, h = (int(v) for v in text.lower().split("x"))
+        return resolve_size((w, h), (w, h))
+    except ValueError as e:
+        raise argparse.ArgumentTypeError(f"--size {text!r}: expected WIDTHxHEIGHT or auto ({e})") from None
 
 
 def add_checkpoint_args(p):
@@ -90,6 +110,25 @@ def checkpoints_from_args(args):
     if not args.checkpoints:
         return None           # FastEditor then consults the environment variables
     return expand_checkpoints(args.checkpoints, args.controlnet_dir, args.vae_dir, args.lcm_lora, args.unet_dir)
+
+
+def micro_batches(work, mb, size):
+    """Work items -> groups of at most ``mb`` for edit_many.  With ``size="auto"`` the items are first grouped by their bucket (first-seen
+    order; only the image header is read), so that each group holds one size: full micro-batches and one CUDA graph per bucket,
+    instead of small padded chunks of every bucket in each group.  An unreadable image goes to a group of its own kind; loading it
+    reports the error."""
+    if size != "auto":
+        return [work[i:i + mb] for i in range(0, len(work), mb)]
+    from fast_image_editing_with_generative_models_b200.editor import resolve_size
+    by_bucket = {}
+    for it in work:
+        try:
+            with Image.open(it[2]) as im:
+                key = resolve_size("auto", im.size)
+        except Exception:
+            key = None
+        by_bucket.setdefault(key, []).append(it)
+    return [items[i:i + mb] for items in by_bucket.values() for i in range(0, len(items), mb)]
 
 
 def select_entries(mapping, args):
@@ -156,9 +195,10 @@ def main(argv=None):
             print(f"\n      Error processing {image_id} ({type(e).__name__}): {e}")
             failed += 1
     mb = max(int(args.micro_batch), 1)
-    groups = [work[i:i + mb] for i in range(0, len(work), mb)]
+    groups = micro_batches(work, mb, args.size)
     edit_kw = dict(negative_prompt=args.negative_prompt, strength=args.strength, num_inference_steps=args.steps, guidance_scale=args.guidance,
-                   controlnet_conditioning_scale=args.control_scale, canny_low_threshold=args.canny_low, canny_high_threshold=args.canny_high)
+                   controlnet_conditioning_scale=args.control_scale, canny_low_threshold=args.canny_low, canny_high_threshold=args.canny_high,
+                   size=args.size)
 
     def load(item):
         return Image.open(item[2]).convert("RGB")
@@ -230,7 +270,7 @@ def main(argv=None):
             editor.clear_memory()
         processed += sum(o is not None for o in outs)
         if rank == 0:
-            print(f"\r      Editing[{rank}]: {min((gi + 1) * mb, len(work))}/{len(work)}", end="", flush=True)
+            print(f"\r      Editing[{rank}]: {sum(len(g) for g in groups[:gi + 1])}/{len(work)}", end="", flush=True)
     for it, fut in saves:
         try:
             fut.result()

@@ -36,8 +36,9 @@ def build_parser():
     p.add_argument("--full_controlnet", action="store_true")
     p.add_argument("--compute_metrics", action="store_true")
     p.add_argument("--show_plot", action="store_true")
-    from run_batch import add_checkpoint_args
+    from run_batch import add_checkpoint_args, add_size_arg
     add_checkpoint_args(p)
+    add_size_arg(p)
     return p
 
 
@@ -79,7 +80,7 @@ def main(argv=None):
     t0 = time.time()
     edited_img = editor.edit(image=source_img, prompt=args.prompt, negative_prompt=args.negative_prompt, strength=args.strength,
                              num_inference_steps=args.steps, guidance_scale=args.guidance, controlnet_conditioning_scale=args.control_scale,
-                             canny_low_threshold=args.canny_low, canny_high_threshold=args.canny_high, seed=args.seed)
+                             canny_low_threshold=args.canny_low, canny_high_threshold=args.canny_high, seed=args.seed, size=args.size)
     elapsed = time.time() - t0
     print(f"      Editing completed in {elapsed:.2f} seconds")
     mem = editor.get_memory_usage()
