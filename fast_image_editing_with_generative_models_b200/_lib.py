@@ -68,7 +68,6 @@ SIGNATURES = {
     "fie_geglu_block_n": (c_int, [c_int]),
     "fie_tune_gemm": (None, [c_int, c_int]),
     "fie_gemm_trace": (None, [c_void_p]),
-    "fie_attention_trace": (None, [c_void_p]),
     "fie_tune_conv_halo": (None, [c_int, c_int]),
     "fie_tune_conv_im2col": (None, [c_int]),
     "fie_tune_groupnorm_slab": (None, [c_int]),

@@ -2,7 +2,7 @@
 // Replaces F.scaled_dot_product_attention (AttnProcessor2_0) for the UNet / ControlNet self- and cross-attention
 // of the reference's edit path (diffusers call at reference src/pipeline.py:261-272).  No mask, scale 1/sqrt(d).
 //
-// One CTA = TWO 128-row Q tiles of one (batch, head) sharing every K/V tile (3-stage TMA ring of 128-row tiles).
+// One work item = TWO 128-row Q tiles of one (batch, head) sharing every K/V tile (3-stage TMA ring of 128-row tiles).
 // Per Q tile q and K/V tile j:
 //   S_q = Q_q K_j^T   tcgen05.mma 128x128x64 -> TMEM columns [128q, 128q+128)
 //   softmax           one warpgroup per Q tile, one thread per row (TMEM lane == row: no cross-thread reductions),
@@ -18,14 +18,11 @@
 // The two warpgroups ping-pong: while one does its softmax the tensor core serves the other (FlashAttention-4 style).
 // Warp roles (384 threads): w0 TMA producer, w1 MMA issuer, w2 TMEM allocator, w3 idle, w4-7 softmax(q=0), w8-11 softmax(q=1).
 #include "tc_common.cuh"
-#include <stdlib.h>
 #include <type_traits>
 
-#ifndef FIE_ATT_EMU
-#define FIE_ATT_EMU 2          // exponentials per 8 evaluated without MUFU in the self-attention softmax
-#endif
-
 namespace fie {
+
+constexpr int ATT_EMU = 2;     // exponentials per 8 evaluated without MUFU in the self-attention softmax
 
 // 2^x for x <= 127 without the MUFU unit: x = n + f (add with round-down against 1.5 * 2^23 leaves n in the low mantissa bits),
 // 2^f by a cubic on [0, 1) (relative error ~1e-4), exponent patched in with an integer add.  Inputs below -126 give ~1e-38.
@@ -82,11 +79,8 @@ __device__ __forceinline__ void store_o_row(__half* orow, const uint32_t (&r)[64
     }
 }
 
-constexpr int ATT_BM = 128, ATT_BN = 128, ATT_D = 64, ATT_QT = 2, ATT_KV_STAGES = 3;
+constexpr int ATT_BM = 128, ATT_BN = 128, ATT_D = 64, ATT_QT = 2;
 constexpr int ATT_TILE_BYTES = 128 * 64 * 2;                                   // 16 KiB (Q, K or V tile)
-constexpr int ATT_OFF_KV = ATT_QT * ATT_TILE_BYTES;                            // after Q0, Q1
-constexpr int ATT_OFF_BAR = ATT_OFF_KV + ATT_KV_STAGES * 2 * ATT_TILE_BYTES;   // after the K/V ring (P lives in TMEM)
-constexpr int ATT_SMEM = ATT_OFF_BAR + 256;
 
 struct AttnParams {
     CUtensorMap q_map, k_map, v_map;
@@ -95,283 +89,20 @@ struct AttnParams {
     int nq, nkv;
     float scale_log2;
     int causal;       // (kv1 kernel only) key j is visible to query row i iff j <= i
-    long long* trace; // debug: per-CTA wait-cycle accounting [grid][16] (fie_attention_trace), or NULL
 };
 
-#define ATT_TIMED(acc, stmt) do { if (p.trace) { const long long t0_ = clock64(); stmt; (acc) += clock64() - t0_; } else { stmt; } } while (0)
-
-__global__ void __launch_bounds__(384, 1) k_attention_d64(const __grid_constant__ AttnParams p) {
-    extern __shared__ __align__(1024) uint8_t smem[];     // no static smem in this kernel: base is 1024-aligned
-    uint8_t* sQ = smem;
-    uint8_t* sKV = smem + ATT_OFF_KV;                     // stage s: K at s*32K, V at s*32K + 16K
-    uint64_t* bars = reinterpret_cast<uint64_t*>(smem + ATT_OFF_BAR);
-    uint64_t* q_full = bars;                 // [1]
-    uint64_t* kv_full = bars + 1;            // [3]
-    uint64_t* kv_empty = bars + 4;           // [3]
-    uint64_t* s_full = bars + 7;             // [2]
-    uint64_t* p_full = bars + 9;             // [2]
-    uint64_t* o_full = bars + 11;            // [2]
-    uint64_t* s_free = bars + 13;            // [2]  S_q has been read into registers: the next Q K^T may overwrite it
-    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 15);
-    if ((smem_u32(smem) & 1023u) != 0) { if (threadIdx.x == 0) printf("fie: attention smem base misaligned\n"); __trap(); }
-
-    const int warp = warp_idx_uniform(), lane = threadIdx.x & 31;
-    const int qt0 = blockIdx.x * ATT_QT, head = blockIdx.y, b = blockIdx.z;
-    const int n_tiles = (p.nkv + ATT_BN - 1) / ATT_BN;
-
-    if (threadIdx.x == 0) {
-        mbar_init(q_full, 1);
-        for (int s = 0; s < ATT_KV_STAGES; ++s) { mbar_init(&kv_full[s], 1); mbar_init(&kv_empty[s], 1); }
-        for (int q = 0; q < ATT_QT; ++q) { mbar_init(&s_full[q], 1); mbar_init(&p_full[q], 128); mbar_init(&o_full[q], 1); mbar_init(&s_free[q], 128); }
-        mbar_fence_init();
-    }
-    if (warp == 0 && lane == 0) { tma_prefetch_desc(&p.q_map); tma_prefetch_desc(&p.k_map); tma_prefetch_desc(&p.v_map); }
-    if (warp == 2) tmem_alloc(tmem_slot, 512);
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    asm volatile("griddepcontrol.wait;" ::: "memory");      // programmatic dependent launch: the prologue above overlaps the previous kernel's tail
-    const uint32_t tmem = *tmem_slot;
-
-    if (warp == 0) {
-        if (elect_one_sync()) {
-            mbar_arrive_expect_tx(q_full, ATT_QT * ATT_TILE_BYTES);
-            for (int q = 0; q < ATT_QT; ++q) tma_load_3d(&p.q_map, q_full, sQ + q * ATT_TILE_BYTES, head * ATT_D, (qt0 + q) * ATT_BM, b);
-            int s = 0; uint32_t ph = 0;
-            for (int j = 0; j < n_tiles; ++j) {
-                mbar_wait(&kv_empty[s], ph ^ 1);
-                mbar_arrive_expect_tx(&kv_full[s], 2 * ATT_TILE_BYTES);
-                tma_load_3d(&p.k_map, &kv_full[s], sKV + s * 2 * ATT_TILE_BYTES, head * ATT_D, j * ATT_BN, b);
-                tma_load_3d(&p.v_map, &kv_full[s], sKV + s * 2 * ATT_TILE_BYTES + ATT_TILE_BYTES, head * ATT_D, j * ATT_BN, b);
-                if (++s == ATT_KV_STAGES) { s = 0; ph ^= 1; }
-            }
-        }
-    } else if (warp == 1) {
-        const uint32_t idesc_qk = umma_idesc_f16(ATT_BM, ATT_BN, 0, 0);
-        const uint32_t idesc_pv = umma_idesc_f16(ATT_BM, ATT_D, 0, 1);   // B (= V) is MN-major
-        const uint32_t aQ = smem_u32(sQ), aKV = smem_u32(sKV);
-        auto issue_qk = [&](int q, int s) {        // S_q = Q_q K_s^T
-            if (elect_one_sync()) {
-                const uint64_t ad = umma_desc_sw128(aQ + q * ATT_TILE_BYTES), bd = umma_desc_sw128(aKV + s * 2 * ATT_TILE_BYTES);
-#pragma unroll
-                for (int k = 0; k < ATT_D / 16; ++k) umma_f16(tmem + q * 128, ad + 2 * k, bd + 2 * k, idesc_qk, k ? 1u : 0u);
-                umma_commit(&s_full[q]);
-            }
-            __syncwarp();
-        };
-        long long tw_kv = 0, tw_sfree = 0, tw_pfull = 0; const long long t_begin = p.trace ? clock64() : 0;
-        mbar_wait(q_full, 0);
-        mbar_wait(&kv_full[0], 0);
-        tc_fence_after();
-        issue_qk(0, 0);
-        issue_qk(1, 0);
-        int s = 0; uint32_t ph = 0;                 // stage / phase of tile j
-        for (int j = 0; j < n_tiles; ++j) {
-            int sn = s + 1; uint32_t phn = ph; if (sn == ATT_KV_STAGES) { sn = 0; phn ^= 1; }
-            // S_q(j+1) = Q_q K_{j+1}^T is issued as soon as the softmax warps hold S_q(j) in registers, i.e. while they are
-            // still exponentiating it: the next scores are ready when P_q(j) is, and the softmax never waits on the tensor pipe.
-            if (j + 1 < n_tiles) {
-                ATT_TIMED(tw_kv, mbar_wait(&kv_full[sn], phn));
-                for (int q = 0; q < ATT_QT; ++q) {
-                    ATT_TIMED(tw_sfree, mbar_wait(&s_free[q], (uint32_t)(j & 1)));
-                    tc_fence_after();
-                    issue_qk(q, sn);
-                }
-            }
-            for (int q = 0; q < ATT_QT; ++q) {
-                ATT_TIMED(tw_pfull, mbar_wait(&p_full[q], (uint32_t)(j & 1)));
-                tc_fence_after();
-                if (elect_one_sync()) {
-                    const uint32_t aV = aKV + s * 2 * ATT_TILE_BYTES + ATT_TILE_BYTES;
-#pragma unroll
-                    for (int k = 0; k < ATT_BN / 16; ++k) {
-                        const uint64_t bd = umma_desc_sw128(aV + k * 2048, 1024, 1024);
-                        umma_f16_ts(tmem + 256 + q * 64, tmem + 384 + q * 64 + k * 8, bd, idesc_pv, (j | k) ? 1u : 0u);   // O accumulates in TMEM across K/V tiles
-                    }
-                    umma_commit(&o_full[q]);
-                    if (q == ATT_QT - 1) umma_commit(&kv_empty[s]);
-                }
-                __syncwarp();
-            }
-            s = sn; ph = phn;
-        }
-        if (p.trace && lane == 0) {
-            long long* t = p.trace + ((long long)(blockIdx.z * gridDim.y + blockIdx.y) * gridDim.x + blockIdx.x) * 16;
-            t[0] = clock64() - t_begin; t[1] = tw_kv; t[2] = tw_sfree; t[3] = tw_pfull;
-        }
-    } else if (warp >= 4) {
-        // ===================== softmax / epilogue: warpgroup = Q tile, thread = row =====================
-        const int q = (warp - 4) >> 2;
-        const int wq = warp & 3;                          // TMEM lane quadrant of this warp
-        const int row = wq * 32 + lane;
-        const uint32_t lane_addr = (uint32_t)(wq * 32) << 16;
-        const uint32_t tS = tmem + q * 128 + lane_addr, tO = tmem + 256 + q * 64 + lane_addr, tP = tmem + 384 + q * 64 + lane_addr;
-        float m_run = -INFINITY, l_run = 0.f;
-        const float sl2 = p.scale_log2;
-        const bool wide_o = (p.ldo & 15) == 0 && (reinterpret_cast<uintptr_t>(p.out) & 31) == 0;   // 32-byte aligned output rows
-        // exp2 of one 64-column half against the reference max folded into mneg -> packed fp16 in pp (the A operand layout of
-        // P V: two columns per 32-bit TMEM column); returns the row sum of the half.  FULL: no column masking.  WITH_MAX: also
-        // folds the raw scores into the four running-max accumulators mx[] (one FMNMX3 per column pair), so that the maximum
-        // search rides in the issue slots the MUFU-bound exponentials leave free.
-        auto exp_cols = [&](const uint32_t* r, int col0, float mneg, int kv_left, auto full_c, auto max_c, auto nu_c, uint32_t* pp, float (&mx)[4]) -> float {
-            constexpr bool FULL = decltype(full_c)::value;
-            constexpr bool WITH_MAX = decltype(max_c)::value;
-            constexpr int NU = decltype(nu_c)::value;           // units of 8 columns: 8 (a 64-column half) or 4
-            f32x2 psa = 0ull, psb = 0ull;                       // four partial row sums as two packed accumulators (0 bits == +0.f pair)
-            const f32x2 sl22 = pack2(sl2, sl2), mneg2 = pack2(mneg, mneg);
-#pragma unroll
-            for (int u = 0; u < NU; ++u) {
-#pragma unroll
-                for (int i = 0; i < 4; ++i) {
-                    const int c = u * 8 + 2 * i;
-                    // The MUFU unit (16 ex2 / clk / SM) and the issue slots are this kernel's limits: FIE_ATT_EMU of every 8
-                    // exponentials run on the FMA / ALU pipes instead (Cody-Waite split + cubic, ~1e-4 relative: below the fp16
-                    // rounding of P), as packed column pairs.
-                    if (WITH_MAX) {
-                        if (FULL) mx[i] = fmaxf(fmaxf(mx[i], __uint_as_float(r[c])), __uint_as_float(r[c + 1]));
-                        else { if (col0 + c < kv_left) mx[i] = fmaxf(mx[i], __uint_as_float(r[c])); if (col0 + c + 1 < kv_left) mx[i] = fmaxf(mx[i], __uint_as_float(r[c + 1])); }
-                    }
-                    const f32x2 x2 = ffma2(pack2u(r[c], r[c + 1]), sl22, mneg2);
-                    float x0, x1, p0, p1;
-                    unpack2(x2, x0, x1);
-                    if (2 * i >= 8 - FIE_ATT_EMU) ex2_emulated2(pack2(fmaxf(x0, -126.0f), fmaxf(x1, -126.0f)), p0, p1);
-                    else { p0 = ex2_approx(x0); p1 = ex2_approx(x1); }
-                    if (!FULL) { if (col0 + c >= kv_left) p0 = 0.f; if (col0 + c + 1 >= kv_left) p1 = 0.f; }
-                    if (i & 1) psb = fadd2(psb, pack2(p0, p1)); else psa = fadd2(psa, pack2(p0, p1));
-                    __half2 h = __floats2half2_rn(p0, p1);
-                    pp[4 * u + i] = *reinterpret_cast<uint32_t*>(&h);
-                }
-            }
-            float s0, s1;
-            unpack2(fadd2(psa, psb), s0, s1);
-            return s0 + s1;
-        };
-        auto half_max = [&](const uint32_t (&r)[64], int hf, int kv_left, bool full_tile, float (&mx)[4]) {
-            if (full_tile) {
-#pragma unroll
-                for (int i = 0; i < 64; i += 8) {                      // 3-input max (FMNMX3): two columns per instruction
-                    mx[0] = fmaxf(fmaxf(mx[0], __uint_as_float(r[i])), __uint_as_float(r[i + 1])); mx[1] = fmaxf(fmaxf(mx[1], __uint_as_float(r[i + 2])), __uint_as_float(r[i + 3]));
-                    mx[2] = fmaxf(fmaxf(mx[2], __uint_as_float(r[i + 4])), __uint_as_float(r[i + 5])); mx[3] = fmaxf(fmaxf(mx[3], __uint_as_float(r[i + 6])), __uint_as_float(r[i + 7]));
-                }
-            } else {
-#pragma unroll
-                for (int i = 0; i < 64; ++i) if (hf * 64 + i < kv_left) mx[0] = fmaxf(mx[0], __uint_as_float(r[i]));
-            }
-        };
-        const std::true_type yes{}; const std::false_type no{};
-        const std::integral_constant<int, 8> n8{}; const std::integral_constant<int, 4> n4{};
-        long long tw_sfull = 0, tw_ofull = 0, tw_st = 0; const long long t_begin = p.trace ? clock64() : 0;
-        for (int j = 0; j < n_tiles; ++j) {
-            ATT_TIMED(tw_sfull, mbar_wait(&s_full[q], (uint32_t)(j & 1)));
-            tc_fence_after();
-            const int kv_left = p.nkv - j * ATT_BN;     // valid columns in this tile
-            const bool full_tile = kv_left >= ATT_BN;
-            // Optimistic single pass: the exponentials of the first half are taken against the CURRENT reference max while the
-            // tile's row maximum is still being searched.  The reference only has to move when a row maximum outgrows it by more
-            // than 2^8 in the exponent domain (P = exp2((s - m_run) * scale) <= 256 still fits fp16, and O / l stays exact because
-            // both are accumulated against the same reference) -- after the first tile that is rare, and then the first half is
-            // simply redone.
-            float mx4[4] = {-INFINITY, -INFINITY, -INFINITY, -INFINITY};
-            uint32_t pp0[32];
-            float psum = 0.f;
-            {
-                uint32_t ra[64];
-                tmem_ld_32x64(tS, ra);
-                tmem_ld_wait();
-                if (j == 0) half_max(ra, 0, kv_left, full_tile, mx4);
-                else if (full_tile) psum = exp_cols(ra, 0, -m_run * sl2, kv_left, yes, yes, n8, pp0, mx4);
-                else psum = exp_cols(ra, 0, -m_run * sl2, kv_left, no, yes, n8, pp0, mx4);
-            }
-            uint32_t rb[64];
-            tmem_ld_32x64(tS + 64, rb);
-            tmem_ld_wait();
-            half_max(rb, 1, kv_left, full_tile, mx4);
-            const float mx = fmaxf(fmaxf(mx4[0], mx4[1]), fmaxf(mx4[2], mx4[3]));
-            const bool move = (j == 0) || ((mx - m_run) * sl2 > 8.0f);
-            float alpha = 1.0f;
-            if (j > 0) {
-                // P_q and O_q are free once PV(q, j-1) has completed
-                ATT_TIMED(tw_ofull, mbar_wait(&o_full[q], (uint32_t)((j - 1) & 1)));
-                tc_fence_after();
-            }
-            if (__any_sync(0xffffffffu, move)) {
-                // the reference max of some row of this warp moves (always on the first tile): rescale O_q, which lives in TMEM,
-                // by exp2(m_old - m_new), and (re)do the first half against the new reference
-                if (move) { alpha = ex2_approx((m_run - fmaxf(mx, m_run)) * sl2); m_run = fmaxf(mx, m_run); }      // first tile: exp2(-inf) = 0
-                // (32 columns at a time: this rare path must not raise the register pressure of the common one)
-                if (j > 0) {
-#pragma unroll 1
-                    for (int hq = 0; hq < 2; ++hq) {
-                        uint32_t ro[32];
-                        tmem_ld_32x32(tO + (uint32_t)(hq * 32), ro);
-                        tmem_ld_wait();
-#pragma unroll
-                        for (int i = 0; i < 32; ++i) ro[i] = __float_as_uint(__uint_as_float(ro[i]) * alpha);
-                        tmem_st_32x32(tO + (uint32_t)(hq * 32), ro);
-                    }
-                }
-                float dummy[4];
-                psum = 0.f;
-#pragma unroll
-                for (int hq = 0; hq < 2; ++hq) {
-                    uint32_t rq[32];
-                    tmem_ld_32x32(tS + (uint32_t)(hq * 32), rq);
-                    tmem_ld_wait();
-                    if (full_tile) psum += exp_cols(rq, hq * 32, -m_run * sl2, kv_left, yes, no, n4, pp0 + hq * 16, dummy);
-                    else psum += exp_cols(rq, hq * 32, -m_run * sl2, kv_left, no, no, n4, pp0 + hq * 16, dummy);
-                }
-            }
-            tmem_st_32x32(tP, pp0);
-            tc_fence_before();
-            mbar_arrive(&s_free[q]);                      // S_q has been consumed: Q_q K_{j+1}^T may be issued now
-            {
-                uint32_t pp1[32];
-                float dummy[4];
-                if (full_tile) psum += exp_cols(rb, 64, -m_run * sl2, kv_left, yes, no, n8, pp1, dummy);
-                else psum += exp_cols(rb, 64, -m_run * sl2, kv_left, no, no, n8, pp1, dummy);
-                tmem_st_32x32(tP + 32u, pp1);
-            }
-            l_run = l_run * alpha + psum;
-            ATT_TIMED(tw_st, tmem_st_wait());
-            tc_fence_before();
-            mbar_arrive(&p_full[q]);
-        }
-        if (p.trace && wq == 0 && lane == 0) {
-            long long* t = p.trace + ((long long)(blockIdx.z * gridDim.y + blockIdx.y) * gridDim.x + blockIdx.x) * 16 + 4 + q * 4;
-            t[0] = clock64() - t_begin; t[1] = tw_sfull; t[2] = tw_ofull; t[3] = tw_st;
-        }
-        mbar_wait(&o_full[q], (uint32_t)((n_tiles - 1) & 1));
-        tc_fence_after();
-        const float inv_l = 1.0f / l_run;
-        const int qrow = (qt0 + q) * ATT_BM + row;
-        __half* orow = p.out + ((long long)b * p.nq + qrow) * p.ldo + head * ATT_D;
-        {
-            uint32_t r[64];
-            tmem_ld_32x64(tO, r);
-            tmem_ld_wait();
-            if (qrow < p.nq) store_o_row(orow, r, inv_l, wide_o);
-        }
-        tc_fence_before();
-    }
-    __syncthreads();
-    if (warp == 2) { tc_fence_after(); tmem_dealloc(tmem, 512); }
-}
-
 // ------------------------------------------------------------------------------------------------
-// Persistent form of k_attention_d64 (round 2).  With 1024 keys a CTA lives for 8 K/V steps (~12 us of steady state) and pays ~5 us
-// of set-up and drain around them: block scheduling, barrier init, the 512-column TMEM allocation, the first Q / K / V round trip,
-// the O read-out and store.  Here <= 148 CTAs each walk a strided list of (batch, head, 256-row query block) items with everything
-// allocated once: the producer runs ahead across items (Q is double-buffered, the K/V ring simply continues), the MMA warp issues
-// S = Q K^T for the FIRST tile of the next item as soon as the last tile of the current one has been consumed, and a softmax
-// warpgroup goes from the epilogue of one item straight into scores that are already waiting in TMEM.
+// Self-attention (nkv > 128), persistent.  With 1024 keys a CTA per (batch, head, 256-row query block) item would live for 8 K/V
+// steps (~12 us of steady state) and pay ~5 us of set-up and drain around them: block scheduling, barrier init, the 512-column TMEM
+// allocation, the first Q / K / V round trip, the O read-out and store.  Here <= 148 CTAs each walk a strided list of items with
+// everything allocated once: the producer runs ahead across items (Q is double-buffered, the K/V ring simply continues), the MMA
+// warp issues S = Q K^T for the FIRST tile of the next item as soon as the last tile of the current one has been consumed, and a
+// softmax warpgroup goes from the epilogue of one item straight into scores that are already waiting in TMEM.
 // Barrier parities follow GLOBAL counters (tiles processed by this CTA), not per-item ones.  No extra barrier protects O_q / P_q across
 // items: a softmax warpgroup reads O_q of item n (epilogue) before it arrives on p_full for the first tile of item n + 1, and the MMA
 // warp only overwrites O_q / reads P_q after that arrival.
 // ------------------------------------------------------------------------------------------------
-#ifndef FIE_ATTP_STAGES
-#define FIE_ATTP_STAGES 3
-#endif
-constexpr int ATTP_KV_STAGES = FIE_ATTP_STAGES;                                    // K/V ring depth (prefetch distance across items)
+constexpr int ATTP_KV_STAGES = 3;                                                 // K/V ring depth (prefetch distance across items)
 constexpr int ATTP_OFF_KV = 2 * ATT_QT * ATT_TILE_BYTES;                          // after Q[2 buffers][2 tiles]
 constexpr int ATTP_OFF_BAR = ATTP_OFF_KV + ATTP_KV_STAGES * 2 * ATT_TILE_BYTES;
 constexpr int ATTP_SMEM = ATTP_OFF_BAR + 256;
@@ -460,6 +191,8 @@ __global__ void __launch_bounds__(384, 1) k_attention_d64_p(const __grid_constan
         for (int n = 0; n < my_items; ++n) {
             for (int j = 0; j < n_tiles; ++j, ++g) {
                 int sn = s + 1; uint32_t phn = ph; if (sn == ATTP_KV_STAGES) { sn = 0; phn ^= 1; }
+                // S_q(j+1) = Q_q K_{j+1}^T is issued as soon as the softmax warps hold S_q(j) in registers, i.e. while they are
+                // still exponentiating it: the next scores are ready when P_q(j) is, and the softmax never waits on the tensor pipe.
                 const bool next_same = j + 1 < n_tiles, next_item = !next_same && n + 1 < my_items;
                 if (next_same || next_item) {
                     const int un = next_same ? (n & 1) : ((n + 1) & 1);
@@ -491,25 +224,32 @@ __global__ void __launch_bounds__(384, 1) k_attention_d64_p(const __grid_constan
             }
         }
     } else if (warp >= 4) {
-        // ===================== softmax / epilogue: warpgroup = Q tile, thread = row (same arithmetic as k_attention_d64) =====================
+        // ===================== softmax / epilogue: warpgroup = Q tile, thread = row =====================
         const int q = (warp - 4) >> 2;
-        const int wq = warp & 3;
+        const int wq = warp & 3;                          // TMEM lane quadrant of this warp
         const int row = wq * 32 + lane;
         const uint32_t lane_addr = (uint32_t)(wq * 32) << 16;
         const uint32_t tS = tmem + q * 128 + lane_addr, tO = tmem + 256 + q * 64 + lane_addr, tP = tmem + 384 + q * 64 + lane_addr;
         const float sl2 = p.scale_log2;
         const bool wide_o = (p.ldo & 15) == 0 && (reinterpret_cast<uintptr_t>(p.out) & 31) == 0;   // 32-byte aligned output rows
+        // exp2 of one 64-column half against the reference max folded into mneg -> packed fp16 in pp (the A operand layout of
+        // P V: two columns per 32-bit TMEM column); returns the row sum of the half.  FULL: no column masking.  WITH_MAX: also
+        // folds the raw scores into the four running-max accumulators mx[] (one FMNMX3 per column pair), so that the maximum
+        // search rides in the issue slots the MUFU-bound exponentials leave free.
         auto exp_cols = [&](const uint32_t* r, int col0, float mneg, int kv_left, auto full_c, auto max_c, auto nu_c, uint32_t* pp, float (&mx)[4]) -> float {
             constexpr bool FULL = decltype(full_c)::value;
             constexpr bool WITH_MAX = decltype(max_c)::value;
-            constexpr int NU = decltype(nu_c)::value;
-            f32x2 psa = 0ull, psb = 0ull;
+            constexpr int NU = decltype(nu_c)::value;           // units of 8 columns: 8 (a 64-column half) or 4
+            f32x2 psa = 0ull, psb = 0ull;                       // four partial row sums as two packed accumulators (0 bits == +0.f pair)
             const f32x2 sl22 = pack2(sl2, sl2), mneg2 = pack2(mneg, mneg);
 #pragma unroll
             for (int u = 0; u < NU; ++u) {
 #pragma unroll
                 for (int i = 0; i < 4; ++i) {
                     const int c = u * 8 + 2 * i;
+                    // The MUFU unit (16 ex2 / clk / SM) and the issue slots are this kernel's limits: ATT_EMU of every 8
+                    // exponentials run on the FMA / ALU pipes instead (Cody-Waite split + cubic, ~1e-4 relative: below the fp16
+                    // rounding of P), as packed column pairs.
                     if (WITH_MAX) {
                         if (FULL) mx[i] = fmaxf(fmaxf(mx[i], __uint_as_float(r[c])), __uint_as_float(r[c + 1]));
                         else { if (col0 + c < kv_left) mx[i] = fmaxf(mx[i], __uint_as_float(r[c])); if (col0 + c + 1 < kv_left) mx[i] = fmaxf(mx[i], __uint_as_float(r[c + 1])); }
@@ -517,7 +257,7 @@ __global__ void __launch_bounds__(384, 1) k_attention_d64_p(const __grid_constan
                     const f32x2 x2 = ffma2(pack2u(r[c], r[c + 1]), sl22, mneg2);
                     float x0, x1, p0, p1;
                     unpack2(x2, x0, x1);
-                    if (2 * i >= 8 - FIE_ATT_EMU) ex2_emulated2(pack2(fmaxf(x0, -126.0f), fmaxf(x1, -126.0f)), p0, p1);
+                    if (2 * i >= 8 - ATT_EMU) ex2_emulated2(pack2(fmaxf(x0, -126.0f), fmaxf(x1, -126.0f)), p0, p1);
                     else { p0 = ex2_approx(x0); p1 = ex2_approx(x1); }
                     if (!FULL) { if (col0 + c >= kv_left) p0 = 0.f; if (col0 + c + 1 >= kv_left) p1 = 0.f; }
                     if (i & 1) psb = fadd2(psb, pack2(p0, p1)); else psa = fadd2(psa, pack2(p0, p1));
@@ -532,7 +272,7 @@ __global__ void __launch_bounds__(384, 1) k_attention_d64_p(const __grid_constan
         auto half_max = [&](const uint32_t (&r)[64], int hf, int kv_left, bool full_tile, float (&mx)[4]) {
             if (full_tile) {
 #pragma unroll
-                for (int i = 0; i < 64; i += 8) {
+                for (int i = 0; i < 64; i += 8) {                      // 3-input max (FMNMX3): two columns per instruction
                     mx[0] = fmaxf(fmaxf(mx[0], __uint_as_float(r[i])), __uint_as_float(r[i + 1])); mx[1] = fmaxf(fmaxf(mx[1], __uint_as_float(r[i + 2])), __uint_as_float(r[i + 3]));
                     mx[2] = fmaxf(fmaxf(mx[2], __uint_as_float(r[i + 4])), __uint_as_float(r[i + 5])); mx[3] = fmaxf(fmaxf(mx[3], __uint_as_float(r[i + 6])), __uint_as_float(r[i + 7]));
                 }
@@ -551,8 +291,13 @@ __global__ void __launch_bounds__(384, 1) k_attention_d64_p(const __grid_constan
             for (int j = 0; j < n_tiles; ++j, ++g) {
                 mbar_wait(&s_full[q], g & 1u);
                 tc_fence_after();
-                const int kv_left = p.nkv - j * ATT_BN;
+                const int kv_left = p.nkv - j * ATT_BN;     // valid columns in this tile
                 const bool full_tile = kv_left >= ATT_BN;
+                // Optimistic single pass: the exponentials of the first half are taken against the CURRENT reference max while the
+                // tile's row maximum is still being searched.  The reference only has to move when a row maximum outgrows it by more
+                // than 2^8 in the exponent domain (P = exp2((s - m_run) * scale) <= 256 still fits fp16, and O / l stays exact because
+                // both are accumulated against the same reference) -- after the first tile that is rare, and then the first half is
+                // simply redone.
                 float mx4[4] = {-INFINITY, -INFINITY, -INFINITY, -INFINITY};
                 uint32_t pp0[32];
                 float psum = 0.f;
@@ -576,7 +321,10 @@ __global__ void __launch_bounds__(384, 1) k_attention_d64_p(const __grid_constan
                     tc_fence_after();
                 }
                 if (__any_sync(0xffffffffu, move)) {
-                    if (move) { alpha = ex2_approx((m_run - fmaxf(mx, m_run)) * sl2); m_run = fmaxf(mx, m_run); }
+                    // the reference max of some row of this warp moves (always on the first tile): rescale O_q, which lives in TMEM,
+                    // by exp2(m_old - m_new), and (re)do the first half against the new reference
+                    if (move) { alpha = ex2_approx((m_run - fmaxf(mx, m_run)) * sl2); m_run = fmaxf(mx, m_run); }      // first tile: exp2(-inf) = 0
+                    // (32 columns at a time: this rare path must not raise the register pressure of the common one)
                     if (j > 0) {
 #pragma unroll 1
                         for (int hq = 0; hq < 2; ++hq) {
@@ -601,7 +349,7 @@ __global__ void __launch_bounds__(384, 1) k_attention_d64_p(const __grid_constan
                 }
                 tmem_st_32x32(tP, pp0);
                 tc_fence_before();
-                mbar_arrive(&s_free[q]);
+                mbar_arrive(&s_free[q]);                      // S_q has been consumed: Q_q K_{j+1}^T may be issued now
                 {
                     uint32_t pp1[32];
                     float dummy[4];
@@ -636,10 +384,10 @@ __global__ void __launch_bounds__(384, 1) k_attention_d64_p(const __grid_constan
 
 // ------------------------------------------------------------------------------------------------
 // Cross-attention form (nkv <= 128: the 77 prompt tokens): one K/V tile, so the work per (batch, head, 256 query rows) is a
-// short latency chain (Q K^T -> softmax -> P V -> store) and one CTA per item, as above, spends most of its life in set-up.
+// short latency chain (Q K^T -> softmax -> P V -> store) and one CTA per item would spend most of its life in set-up.
 // Here 148 persistent CTAs each walk a contiguous range of items; the producer keeps the next item's Q / K / V in flight in a
 // second shared-memory buffer, and TMEM allocation, barrier set-up and descriptor fetches are paid once per CTA.
-// Same warp roles as k_attention_d64.  Barriers flip once per item (parity = item counter & 1).
+// Same warp roles as k_attention_d64_p.  Barriers flip once per item (parity = item counter & 1).
 // ------------------------------------------------------------------------------------------------
 constexpr int ATT1_OFF_KV = 2 * ATT_QT * ATT_TILE_BYTES;                       // after Q[2 buffers][2 tiles]
 constexpr int ATT1_OFF_P = ATT1_OFF_KV + 2 * 2 * ATT_TILE_BYTES;               // after K/V[2 buffers]
@@ -802,11 +550,6 @@ __global__ void __launch_bounds__(384, 1) k_attention_d64_kv1(const __grid_const
 }  // namespace fie
 using namespace fie;
 
-static long long* g_att_trace = nullptr;
-// Debug: per-CTA [16] int64: [0] MMA warp total cycles, [1] blocked on K/V tiles, [2] on "S in registers", [3] on "P ready";
-// [4 + 4q ..]: softmax warpgroup q total, blocked on "S ready", on "P V done", on the TMEM store of P.  NULL switches it off.
-extern "C" void fie_attention_trace(long long* device_buf) { g_att_trace = device_buf; }
-
 static int attention_d64(const void* q, long long ldq, const void* k, long long ldk, const void* v, long long ldv,
                          void* out, long long ldo, int b, int heads, int nq, int nkv, float scale, int causal, void* stream) {
     FIE_REQUIRE(q && k && v && out, "fie_attention_d64_f16: null pointer");
@@ -832,66 +575,39 @@ static int attention_d64(const void* q, long long ldq, const void* k, long long 
     p.out = (__half*)out; p.ldo = ldo; p.nq = nq; p.nkv = nkv;
     p.scale_log2 = scale * 1.4426950408889634f;
     p.causal = causal;
-    p.trace = g_att_trace;
     FIE_REQUIRE(!causal || nkv <= ATT_BN, "fie_attention_d64_causal_f16: nkv must be <= 128");
-    static bool attr_dev[kMaxDevices] = {false};               // cudaFuncSetAttribute is per device
-    bool& attr = attr_dev[current_device()];
-    if (!attr) {
-        cudaError_t e = cudaFuncSetAttribute(k_attention_d64, cudaFuncAttributeMaxDynamicSharedMemorySize, ATT_SMEM);
-        if (e != cudaSuccess) { set_error("cudaFuncSetAttribute(k_attention_d64): %s", cudaGetErrorString(e)); return FIE_ERR_CUDA; }
-        attr = true;
-    }
-    static int pdl = -1;                                 // FIE_PDL=0: plain stream-ordered launches (see gemm_conv.cu)
-    if (pdl < 0) { const char* e = getenv("FIE_PDL"); pdl = e ? atoi(e) : 1; }
-    cudaLaunchAttribute pdl_attr[1];
+    cudaLaunchAttribute pdl_attr[1];                      // programmatic dependent launch (see gemm_conv.cu)
     pdl_attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     pdl_attr[0].val.programmaticStreamSerializationAllowed = 1;
-    static int kv1 = -1;
-    if (kv1 < 0) { const char* e = getenv("FIE_ATT_KV1"); kv1 = e ? atoi(e) : 1; }
-    if ((kv1 || causal) && nkv <= ATT_BN) {
-        // cross-attention: persistent CTAs over (batch, head, 256-row query block) items
-        static bool attr1_dev[kMaxDevices] = {false};
+    const long long items = (long long)b * heads * ((nq + ATT_QT * ATT_BM - 1) / (ATT_QT * ATT_BM));
+    const int sms = device_sm_count();
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = dim3((unsigned)(items < sms ? items : sms)); cfg.blockDim = dim3(384); cfg.stream = (cudaStream_t)stream;
+    cfg.attrs = pdl_attr; cfg.numAttrs = 1;
+    if (nkv <= ATT_BN) {
+        // cross-attention: one K/V tile per item
+        static bool attr1_dev[kMaxDevices] = {false};               // cudaFuncSetAttribute is per device
         bool& attr1 = attr1_dev[current_device()];
         if (!attr1) {
             cudaError_t e = cudaFuncSetAttribute(k_attention_d64_kv1, cudaFuncAttributeMaxDynamicSharedMemorySize, ATT1_SMEM);
             if (e != cudaSuccess) { set_error("cudaFuncSetAttribute(k_attention_d64_kv1): %s", cudaGetErrorString(e)); return FIE_ERR_CUDA; }
             attr1 = true;
         }
-        const long long items = (long long)b * heads * ((nq + ATT_QT * ATT_BM - 1) / (ATT_QT * ATT_BM));
-        const int sms = device_sm_count();
-        const int grid1 = (int)(items < sms ? items : sms);
-        cudaLaunchConfig_t cfg = {};
-        cfg.gridDim = dim3((unsigned)grid1); cfg.blockDim = dim3(384); cfg.dynamicSmemBytes = ATT1_SMEM; cfg.stream = (cudaStream_t)stream;
-        cfg.attrs = pdl_attr; cfg.numAttrs = pdl ? 1 : 0;
+        cfg.dynamicSmemBytes = ATT1_SMEM;
         cudaError_t e = cudaLaunchKernelEx(&cfg, k_attention_d64_kv1, p, heads, b);
         if (e != cudaSuccess) { set_error("cudaLaunchKernelEx(k_attention_d64_kv1): %s", cudaGetErrorString(e)); cudaGetLastError(); return FIE_ERR_CUDA; }
         return check_launch("fie_attention_d64_f16");
     }
-    static int persist = -1;                             // FIE_ATT_PERSIST=0: one CTA per (batch, head, query block) as in round 1
-    if (persist < 0) { const char* e = getenv("FIE_ATT_PERSIST"); persist = e ? atoi(e) : 1; }
-    if (persist && !g_att_trace) {
-        static bool attrp_dev[kMaxDevices] = {false};
-        bool& attrp = attrp_dev[current_device()];
-        if (!attrp) {
-            cudaError_t e = cudaFuncSetAttribute(k_attention_d64_p, cudaFuncAttributeMaxDynamicSharedMemorySize, ATTP_SMEM);
-            if (e != cudaSuccess) { set_error("cudaFuncSetAttribute(k_attention_d64_p): %s", cudaGetErrorString(e)); return FIE_ERR_CUDA; }
-            attrp = true;
-        }
-        const long long items = (long long)b * heads * ((nq + ATT_QT * ATT_BM - 1) / (ATT_QT * ATT_BM));
-        const int sms = device_sm_count();
-        cudaLaunchConfig_t cfgp = {};
-        cfgp.gridDim = dim3((unsigned)(items < sms ? items : sms)); cfgp.blockDim = dim3(384); cfgp.dynamicSmemBytes = ATTP_SMEM; cfgp.stream = (cudaStream_t)stream;
-        cfgp.attrs = pdl_attr; cfgp.numAttrs = pdl ? 1 : 0;
-        cudaError_t e = cudaLaunchKernelEx(&cfgp, k_attention_d64_p, p, heads, b);
-        if (e != cudaSuccess) { set_error("cudaLaunchKernelEx(k_attention_d64_p): %s", cudaGetErrorString(e)); cudaGetLastError(); return FIE_ERR_CUDA; }
-        return check_launch("fie_attention_d64_f16");
+    static bool attrp_dev[kMaxDevices] = {false};
+    bool& attrp = attrp_dev[current_device()];
+    if (!attrp) {
+        cudaError_t e = cudaFuncSetAttribute(k_attention_d64_p, cudaFuncAttributeMaxDynamicSharedMemorySize, ATTP_SMEM);
+        if (e != cudaSuccess) { set_error("cudaFuncSetAttribute(k_attention_d64_p): %s", cudaGetErrorString(e)); return FIE_ERR_CUDA; }
+        attrp = true;
     }
-    dim3 grid((nq + ATT_QT * ATT_BM - 1) / (ATT_QT * ATT_BM), heads, b);
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = grid; cfg.blockDim = dim3(384); cfg.dynamicSmemBytes = ATT_SMEM; cfg.stream = (cudaStream_t)stream;
-    cfg.attrs = pdl_attr; cfg.numAttrs = pdl ? 1 : 0;
-    cudaError_t e = cudaLaunchKernelEx(&cfg, k_attention_d64, p);
-    if (e != cudaSuccess) { set_error("cudaLaunchKernelEx(k_attention_d64): %s", cudaGetErrorString(e)); cudaGetLastError(); return FIE_ERR_CUDA; }
+    cfg.dynamicSmemBytes = ATTP_SMEM;
+    cudaError_t e = cudaLaunchKernelEx(&cfg, k_attention_d64_p, p, heads, b);
+    if (e != cudaSuccess) { set_error("cudaLaunchKernelEx(k_attention_d64_p): %s", cudaGetErrorString(e)); cudaGetLastError(); return FIE_ERR_CUDA; }
     return check_launch("fie_attention_d64_f16");
 }
 

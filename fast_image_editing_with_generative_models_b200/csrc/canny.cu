@@ -13,7 +13,6 @@
 // The hysteresis result is the unique closure of strong pixels through candidates, so the union-find
 // formulation is bit-exact with OpenCV's stack-based flood fill without any host round trip.
 #include "fie_common.cuh"
-#include <stdlib.h>
 
 namespace fie {
 
@@ -516,10 +515,8 @@ extern "C" int fie_canny_u8(const void* img, void* edges, int n, int h, int w, i
     uint8_t* state = gray + pxr;
     uint32_t* parent = (uint32_t*)(state + pxr);
     (void)gray;                                   // (the gray plane is no longer materialised: k_nms<3> converts on the fly)
-    static int fast_env = -1;                       // FIE_CANNY_FAST=0: the generic kernels for every shape (A/B, debugging)
-    if (fast_env < 0) { const char* e = getenv("FIE_CANNY_FAST"); fast_env = e ? atoi(e) : 1; }
     dim3 g1(ceil_div(w, TW), ceil_div(h, TH), n);
-    const bool fast_tile = fast_env && in_channels == 3 && (w % TW) == 0 && (h % TH) == 0 && low >= 0 && high < 8192 &&
+    const bool fast_tile = in_channels == 3 && (w % TW) == 0 && (h % TH) == 0 && low >= 0 && high < 8192 &&
                            ((reinterpret_cast<uintptr_t>(img) | reinterpret_cast<uintptr_t>(state)) & 3) == 0;
     if (fast_tile) k_nms_rgb_fast<<<g1, 256, 0, stream>>>((const uint8_t*)img, state, parent, h, w, low, high);
     else if (in_channels == 3) k_nms<3><<<g1, 256, 0, stream>>>((const uint8_t*)img, state, parent, h, w, low, high);

@@ -21,19 +21,12 @@
 // Warp roles (384 threads): w0-7 epilogue, w8 TMA producer, w9 MMA issuer, w10 TMEM allocator, w11 idle.
 #include "tc_common.cuh"
 
-#ifndef FIE_GEMM_SETMAXNREG
-#define FIE_GEMM_SETMAXNREG 1
-#endif
-
 namespace fie {
 
 // Warp roles.  The epilogue warps get the LOW warp ids: the SM's warp scheduler favours higher ids among ready warps, and the
 // single-thread TMA producer / MMA issuer must never wait behind eight ALU-busy epilogue warps.
-#ifndef FIE_GEMM_ROLES_HIGH
-#define FIE_GEMM_ROLES_HIGH 1
-#endif
-constexpr int W_EPI0 = FIE_GEMM_ROLES_HIGH ? 0 : 4;        // first of the 8 epilogue warps
-constexpr int W_PROD = FIE_GEMM_ROLES_HIGH ? 8 : 0, W_MMA = W_PROD + 1, W_ALLOC = W_PROD + 2;
+constexpr int W_EPI0 = 0;        // first of the 8 epilogue warps
+constexpr int W_PROD = 8, W_MMA = W_PROD + 1, W_ALLOC = W_PROD + 2;
 
 constexpr int BLOCK_M = 128;
 constexpr int BLOCK_K = 64;
@@ -272,9 +265,7 @@ __global__ void __launch_bounds__(384, 1) k_gemm_conv(const __grid_constant__ Ge
     // Register re-partition (384 threads x 168 at launch): the producer / MMA / allocator warpgroup keeps 56 registers per
     // thread, the two epilogue warpgroups get 224 so that the epilogue math has the ILP to stay off the critical path.
     if (warp >= W_PROD && warp < W_PROD + 4) {
-#if FIE_GEMM_SETMAXNREG
     asm volatile("setmaxnreg.dec.sync.aligned.u32 56;");
-#endif
     if (warp == W_PROD) {
         // ===================== TMA producer =====================
         const bool prod_lane = elect_one_sync();
@@ -456,9 +447,7 @@ __global__ void __launch_bounds__(384, 1) k_gemm_conv(const __grid_constant__ Ge
         if (p.trace && elect_one_sync()) { p.trace[blockIdx.x * 8 + 2] = tr_wait; p.trace[blockIdx.x * 8 + 3] = tr_wait2; p.trace[blockIdx.x * 8 + 4] = clock64() - tr_start; }
     }
     } else {
-#if FIE_GEMM_SETMAXNREG
         asm volatile("setmaxnreg.inc.sync.aligned.u32 224;");
-#endif
         // ===================== Epilogue: 8 warps, two per TMEM lane quadrant (even / odd 32-column chunks) =====================
         // Work item = one 32-row x 32-column chunk of the accumulator; a thread owns one row of it (TMEM lane == row), i.e.
         // 64 contiguous bytes of fp16 output, moved as two 256-bit global accesses (full 32-byte sectors, no shared-memory
@@ -811,16 +800,15 @@ static bool box_tile(int OW, int OH, int* bw, int* bh, int* bn) {
 // and prefers the CTA-pair form (cta_group::2: 256-row tiles, B split across the pair) with the widest accumulator that
 // does not waste columns: time per tile and K-block ~ (290 + block_n).  Waves are quantised over 74 CTA pairs.
 // fie_tune_gemm() can force the form for experiments.
-static int g_force_cg = -1;
+static int g_force_cg = 0;
 static int g_force_bn = 0;
 static int g_dbg = 0;
 static int g_force_kps = 0;
 static int g_force_mt = 0;
 static long long* g_trace = nullptr;
-static int g_halo = -1;             // FIE_CONV_HALO=0 disables the halo convolution path
+static int g_halo = 1;              // fie_tune_conv_halo(0, ...) disables the halo convolution path
 static int g_halo_max_cout = 640;   // wider outputs reuse each A tile enough for the per-tap form to win
 static void pick_config(long long M, int N, bool geglu, int* cg_out, int* bn_out, int* mt_out, int max_mt = 2) {
-    if (g_force_cg < 0) { const char* s = getenv("FIE_GEMM_CG"); g_force_cg = s ? atoi(s) : 0; }
     const int sms = num_sms();
     double best_cost = 1e30; int best_cg = 2, best_bn = 32, best_mt = 1;
     for (int cg = 2; cg >= 1; --cg) {
@@ -939,14 +927,12 @@ static int launch(GemmParams& p, cudaStream_t stream) {
     const int grid = cg * (tiles < slots ? tiles : slots);
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3(grid); cfg.blockDim = dim3(384); cfg.dynamicSmemBytes = smem; cfg.stream = stream;
-    static int pdl = -1;                               // FIE_PDL=0: plain stream-ordered launches
-    if (pdl < 0) { const char* e = getenv("FIE_PDL"); pdl = e ? atoi(e) : 1; }
     cudaLaunchAttribute at[2];
     at[0].id = cudaLaunchAttributeClusterDimension;
     at[0].val.clusterDim.x = cg; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
     at[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     at[1].val.programmaticStreamSerializationAllowed = 1;
-    cfg.attrs = at; cfg.numAttrs = pdl ? 2 : 1;
+    cfg.attrs = at; cfg.numAttrs = 2;
     cudaError_t e = cudaLaunchKernelEx(&cfg, fn, p);
     if (e != cudaSuccess) { set_error("cudaLaunchKernelEx(k_gemm_conv): %s", cudaGetErrorString(e)); cudaGetLastError(); return FIE_ERR_CUDA; }
     return check_launch("k_gemm_conv");
@@ -1024,7 +1010,6 @@ static int conv3x3_impl(const char* fn, const void* x, const void* wgt, void* ou
     int rc = fill_epilogue(p, ep, M, cout, out, ldd, out_dtype);
     if (rc) return rc;
     FIE_REQUIRE(p.act != FIE_ACT_GEGLU, "%s: GEGLU epilogue not supported for conv", fn);
-    if (g_halo < 0) { const char* e = getenv("FIE_CONV_HALO"); g_halo = e ? atoi(e) : 1; }
     const bool halo = boxed && g_halo > 0 && stride == 1 && (OW % BLOCK_M) == 0 && cout <= g_halo_max_cout;
     p.mode = halo ? 2 : (boxed ? 1 : 3); p.M = M; p.N = cout; p.OH = OH; p.OW = OW; p.ab_bf16 = ab_bf16;
     pick_config(M, cout, false, &p.cg, &p.block_n, &p.mt, halo ? 1 : 2);

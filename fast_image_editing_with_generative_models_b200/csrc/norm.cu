@@ -9,7 +9,6 @@
 //   LayerNorm: one warp per row, row kept in registers, two-pass mean / variance in fp32.
 // Replaces F.group_norm / F.silu / F.layer_norm in diffusers ResnetBlock2D, Transformer2DModel, BasicTransformerBlock.
 #include "fie_common.cuh"
-#include <stdlib.h>
 #include <string.h>
 #include <type_traits>
 
@@ -424,28 +423,26 @@ __global__ void __launch_bounds__(256) k_layernorm(const uint4* __restrict__ x, 
     }
 }
 
-static int g_gn_slab_mode = -1;
+// Largest cluster size the single-pass slab kernel may use (0: always the two-kernel path); fie_tune_groupnorm_slab sets it.
+// Measured on B200 (scripts/gn_bench.py, SDXL batch-8 shapes): with one CTA the slab kernel wins (82.6 -> 57.4 us on
+// [16,1024,1280+640], 90 -> 75 us on [16,4096,640]); clusters of 4-8 CTAs (one CTA per SM, barrier-separated phases) LOSE
+// against the streaming two-kernel path (309 -> 644 us on [16,16384,640+320]), so by default only slabs that fit one CTA take it.
+static int g_gn_slab_mode = 1;
 
-// Single-pass slab kernel when the (image, group) slab of every image fits the shared memory of <= FIE_GN_SLAB CTAs.
+// Single-pass slab kernel when the (image, group) slab of every image fits the shared memory of <= g_gn_slab_mode CTAs.
 // Returns FIE_OK when it launched, an error code, or 1 when the shape does not qualify (the caller takes the two-kernel path).
 template <bool BF>
 static int gn_try_slab(const void* x0, int c0, const void* x1, int c1, void* out, int n, long long hw, int groups,
                        const float* gamma, const float* beta, float eps, int fuse_silu, cudaStream_t stream) {
-    // FIE_GN_SLAB = largest cluster size the single-pass kernel may use (0: always the two-kernel path).  Measured on B200
-    // (scripts/gn_bench.py, SDXL batch-8 shapes): with one CTA the slab kernel wins (82.6 -> 57.4 us on [16,1024,1280+640],
-    // 90 -> 75 us on [16,4096,640]); clusters of 4-8 CTAs (one CTA per SM, barrier-separated phases) LOSE against the streaming
-    // two-kernel path (309 -> 644 us on [16,16384,640+320]), so by default only slabs that fit one CTA take it.
-    int& slab_mode = g_gn_slab_mode;
-    if (slab_mode < 0) { const char* e = getenv("FIE_GN_SLAB"); slab_mode = e ? atoi(e) : 1; }
     const int c = c0 + c1;
     const int cpg = c / groups;
     const long long slab_bytes = hw * cpg * 2;
     constexpr long long kCtaBytes = 192 * 1024;
-    if (!(slab_mode && (cpg % 2) == 0 && (c0 % 2) == 0 && (c1 % 2) == 0 && slab_bytes <= 8 * kCtaBytes && hw >= 64 &&
+    if (!(g_gn_slab_mode && (cpg % 2) == 0 && (c0 % 2) == 0 && (c1 % 2) == 0 && slab_bytes <= 8 * kCtaBytes && hw >= 64 &&
           ((reinterpret_cast<uintptr_t>(gamma) | reinterpret_cast<uintptr_t>(beta)) & 7) == 0))
         return 1;
     int nranks = 1; while ((long long)nranks * kCtaBytes < slab_bytes) nranks <<= 1;
-    if (nranks > slab_mode) return 1;
+    if (nranks > g_gn_slab_mode) return 1;
     GNSlabArgs g;
     g.x0 = (const __half2*)x0; g.x1 = (const __half2*)x1; g.out = (__half2*)out;
     g.c0h = c0 / 2; g.c1h = c1 / 2; g.ch = c / 2; g.cpgh = cpg / 2; g.hw = hw;

@@ -15,7 +15,6 @@ NHWC fp16 activations through the hand-written kernels in ``csrc/``.  Weights ar
 from __future__ import annotations
 
 import math
-import os
 from typing import Dict, List, Optional, Sequence, Tuple
 
 import torch
@@ -26,10 +25,6 @@ from .weights import cast_f16, fold_layernorm, fuse_lora, pack_conv3x3, pack_con
 
 Tensor = torch.Tensor
 Params = Dict[str, Tensor]
-
-
-# Fold the transformer blocks' LayerNorms into the neighbouring GEMMs (FIE_FOLD_LN=0: separate fie_layernorm_f16 launches)
-FOLD_LN = os.environ.get("FIE_FOLD_LN", "1") != "0"
 
 
 def _pad32(n: int) -> int:
@@ -147,14 +142,13 @@ class Resnet:
 
 
 class TransformerBlock:
-    """BasicTransformerBlock.  With FOLD_LN the three LayerNorms never run as kernels: the GEMM that produces each residual
+    """BasicTransformerBlock.  The three LayerNorms never run as kernels: the GEMM that produces each residual
     stream also accumulates its row statistics (ln_out), and the GEMM that consumes LN(x) runs on the raw rows with gamma, beta
     and the mean subtraction folded into its weights (weights.fold_layernorm) and scales by 1/sigma in its epilogue (ln_in)."""
     LN_EPS = 1e-5
 
     def __init__(self, pk: _Packer, pre: str, c: int, kv_slot: List):
         self.c = c
-        self.fold = FOLD_LN
         ln1, ln2, ln3 = pk.norm(pre + ".norm1"), pk.norm(pre + ".norm2"), pk.norm(pre + ".norm3")
         wqkv = torch.cat([pk.w(f"{pre}.attn1.{n}") for n in ("to_q", "to_k", "to_v")], 0)
         self.wo1 = pk.linear(pre + ".attn1.to_out.0")
@@ -162,42 +156,24 @@ class TransformerBlock:
         kv_slot.append(cast_f16(torch.cat([pk.w(pre + ".attn2.to_k"), pk.w(pre + ".attn2.to_v")], 0)))
         self.wo2 = pk.linear(pre + ".attn2.to_out.0")
         self.wf = pk.linear(pre + ".ff.net.2")
-        if self.fold:
-            self.wqkv, self.bqkv = fold_layernorm(wqkv, None, *ln1)
-            self.wq2, self.bq2 = fold_layernorm(pk.w(pre + ".attn2.to_q"), pk.b(pre + ".attn2.to_q"), *ln2)
-            self.wg, self.bg = pack_geglu(*fold_layernorm(pk.w(pre + ".ff.net.0.proj"), pk.b(pre + ".ff.net.0.proj"), *ln3))
-        else:
-            self.ln1, self.ln2, self.ln3 = ln1, ln2, ln3
-            self.wqkv = cast_f16(wqkv)
-            self.wq2 = pk.linear(pre + ".attn2.to_q")[0]
-            self.wg, self.bg = pack_geglu(*pk.linear(pre + ".ff.net.0.proj"))
+        self.wqkv, self.bqkv = fold_layernorm(wqkv, None, *ln1)
+        self.wq2, self.bq2 = fold_layernorm(pk.w(pre + ".attn2.to_q"), pk.b(pre + ".attn2.to_q"), *ln2)
+        self.wg, self.bg = pack_geglu(*fold_layernorm(pk.w(pre + ".ff.net.0.proj"), pk.b(pre + ".ff.net.0.proj"), *ln3))
 
-    def __call__(self, h: Tensor, b: int, ntok: int, ctx_kv: Tensor, nctx: int, st: Optional[Tensor] = None, st_next: Optional[Tensor] = None) -> Tensor:
+    def __call__(self, h: Tensor, b: int, ntok: int, ctx_kv: Tensor, nctx: int, st: Tensor, st_next: Optional[Tensor] = None) -> Tensor:
         """st: int64 [3, M, 2] row statistics (st[0] already holds those of h); st_next receives those of the result."""
         c, heads = self.c, self.c // 64
         k = ctx_kv[:, self.kv_off:self.kv_off + c]
         v = ctx_kv[:, self.kv_off + c:self.kv_off + 2 * c]
-        if self.fold:
-            eps = self.LN_EPS
-            qkv = ops.gemm(h, self.wqkv, col_bias=self.bqkv, ln_in=(st[0], eps))
-            a = ops.attention_d64(qkv[:, :c], qkv[:, c:2 * c], qkv[:, 2 * c:], b, heads, ntok, ntok)
-            h = ops.gemm(a, self.wo1[0], col_bias=self.wo1[1], residual=h, ln_out=st[1])
-            q = ops.gemm(h, self.wq2, col_bias=self.bq2, ln_in=(st[1], eps))
-            a = ops.attention_d64(q, k, v, b, heads, ntok, nctx)
-            h = ops.gemm(a, self.wo2[0], col_bias=self.wo2[1], residual=h, ln_out=st[2])
-            g = ops.gemm(h, self.wg, col_bias=self.bg, act=ops.ACT_GEGLU, ln_in=(st[2], eps))
-            return ops.gemm(g, self.wf[0], col_bias=self.wf[1], residual=h, ln_out=st_next)
-        n1 = ops.layernorm(h, *self.ln1)
-        qkv = ops.gemm(n1, self.wqkv)
+        eps = self.LN_EPS
+        qkv = ops.gemm(h, self.wqkv, col_bias=self.bqkv, ln_in=(st[0], eps))
         a = ops.attention_d64(qkv[:, :c], qkv[:, c:2 * c], qkv[:, 2 * c:], b, heads, ntok, ntok)
-        h = ops.gemm(a, self.wo1[0], col_bias=self.wo1[1], residual=h)
-        n2 = ops.layernorm(h, *self.ln2)
-        q = ops.gemm(n2, self.wq2)
+        h = ops.gemm(a, self.wo1[0], col_bias=self.wo1[1], residual=h, ln_out=st[1])
+        q = ops.gemm(h, self.wq2, col_bias=self.bq2, ln_in=(st[1], eps))
         a = ops.attention_d64(q, k, v, b, heads, ntok, nctx)
-        h = ops.gemm(a, self.wo2[0], col_bias=self.wo2[1], residual=h)
-        n3 = ops.layernorm(h, *self.ln3)
-        g = ops.gemm(n3, self.wg, col_bias=self.bg, act=ops.ACT_GEGLU)
-        return ops.gemm(g, self.wf[0], col_bias=self.wf[1], residual=h)
+        h = ops.gemm(a, self.wo2[0], col_bias=self.wo2[1], residual=h, ln_out=st[2])
+        g = ops.gemm(h, self.wg, col_bias=self.bg, act=ops.ACT_GEGLU, ln_in=(st[2], eps))
+        return ops.gemm(g, self.wf[0], col_bias=self.wf[1], residual=h, ln_out=st_next)
 
 
 class Transformer2D:
@@ -212,15 +188,12 @@ class Transformer2D:
         n, hh, ww, c = x.shape
         ntok = hh * ww
         h = ops.groupnorm(x, self.norm[0], self.norm[1], 1e-6, False, self.groups)
-        fold = bool(self.blocks) and self.blocks[0].fold
+        fold = bool(self.blocks)
         # one zero-fill for the row statistics of all 3 x depth LayerNorm inputs of this transformer
         st = ops.zeros_i64((3 * len(self.blocks), n * ntok, 2), x.device) if fold else None
         h = ops.gemm(h.view(n * ntok, c), self.pin[0], col_bias=self.pin[1], ln_out=st[0] if fold else None)
         for i, blk in enumerate(self.blocks):
-            if fold:
-                h = blk(h, n, ntok, ctx_kv, nctx, st[3 * i:3 * i + 3], st[3 * i + 3] if i + 1 < len(self.blocks) else None)
-            else:
-                h = blk(h, n, ntok, ctx_kv, nctx)
+            h = blk(h, n, ntok, ctx_kv, nctx, st[3 * i:3 * i + 3], st[3 * i + 3] if i + 1 < len(self.blocks) else None)
         out = ops.gemm(h, self.pout[0], col_bias=self.pout[1], residual=x.view(n * ntok, c))
         return out.view(n, hh, ww, c)
 
@@ -419,28 +392,25 @@ class _VAEAttention:
 
     def __init__(self, pk: _Packer, pre: str, groups: int, eps: float):
         self.groups, self.eps = groups, eps
-        self.scores_f32 = False       # set by VAE(..., attention_scores_f32=True): fp32 logits between the passes
+        # fp16 scores by default (scaled in the GEMM epilogue, exp-only softmax in place, 1 / rowsum applied in fp32 by the P V
+        # epilogue): half the score traffic, parity unchanged on the synthetic weights (1.5e-2).  fp32 scores, set by
+        # VAE(..., attention_scores_f32=True), keep the logits in fp32 between the passes like diffusers' SDPA: the safe choice for
+        # REAL checkpoints, whose VAE logits reach the hundreds.
+        self.scores_f32 = False
         self.norm = pk.norm(pre + ".group_norm")
         self.q, self.k, self.v, self.o = (pk.linear(f"{pre}.{n}") for n in ("to_q", "to_k", "to_v", "to_out.0"))
 
-    # Query rows whose scores are materialised at a time (0 = the whole image: 512 MiB of fp16 scores at 1024^2).  Measured: small
-    # L2-resident chunks lose more in the P V GEMM (M = 1024, N = 512 is 8 tiles on 74 CTA pairs) than they save in HBM traffic; with a
-    # whole image per pass the P V product runs as 128 tiles.
-    CHUNK = int(os.environ.get("FIE_VAE_CHUNK", "0"))
-    # fp16 scores (scaled in the GEMM epilogue, exp-only softmax in place, 1 / rowsum applied in fp32 by the P V epilogue): half the
-    # score traffic, parity unchanged on the synthetic weights (1.5e-2).  fp32 scores (``scores_f32``) keep the logits in fp32 between
-    # the passes like diffusers' SDPA: the safe default for REAL checkpoints, whose VAE logits reach the hundreds.
-    F16_SCORES = os.environ.get("FIE_VAE_F16_SCORES", "1") == "1"
-
-    def __call__(self, x: Tensor, chunk: Optional[int] = None) -> Tensor:
-        chunk = self.CHUNK if chunk is None else chunk
+    # chunk: query rows whose scores are materialised at a time (0 = the whole image: 512 MiB of fp16 scores at 1024^2).  Measured:
+    # small L2-resident chunks lose more in the P V GEMM (M = 1024, N = 512 is 8 tiles on 74 CTA pairs) than they save in HBM traffic;
+    # with a whole image per pass the P V product runs as 128 tiles.
+    def __call__(self, x: Tensor, chunk: int = 0) -> Tensor:
         n, hh, ww, c = x.shape
         ntok = hh * ww
         hn = ops.groupnorm(x, self.norm[0], self.norm[1], self.eps, False, self.groups).view(n, ntok, c)
         xr = x.view(n, ntok, c)
         out = torch.empty_like(xr)
         scale = 1.0 / math.sqrt(c)
-        f32 = self.scores_f32 or not self.F16_SCORES
+        f32 = self.scores_f32
         for i in range(n):
             q = ops.gemm(hn[i], self.q[0], col_bias=self.q[1])
             k = ops.gemm(hn[i], self.k[0], col_bias=self.k[1])

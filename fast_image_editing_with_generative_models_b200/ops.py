@@ -7,7 +7,6 @@ input goes to the ``*_bf16`` entry points, an fp16 input to the fp16 ones exactl
 from __future__ import annotations
 
 import ctypes
-import os
 from typing import Optional
 
 import torch
@@ -494,7 +493,7 @@ def _gn_stats_ok(n_out: int, groups: int, rows_per_image: int, ldd: int) -> bool
 # Channels-per-group for which the producing epilogue accumulates the GroupNorm statistics.  Measured on B200 (SDXL VAE, batch 8):
 # the extra epilogue work costs more than the saved statistics pass for 4 and 8 channels per group (narrow-N convolutions are
 # epilogue-sensitive), and wins for 16 and 32; the kernel supports {4, 8, 16, 32}.
-GN_FUSE_CPG = tuple(int(t) for t in os.environ.get("FIE_GN_FUSE_CPG", "16,32").split(",") if t)    # (8 measured neutral on B200)
+GN_FUSE_CPG = (16, 32)    # (8 measured neutral on B200)
 
 
 def _gn_stats_alloc(out: torch.Tensor, n_img: int, groups: int) -> torch.Tensor:
@@ -533,7 +532,7 @@ def groupnorm(x0: torch.Tensor, gamma: torch.Tensor, beta: torch.Tensor, eps: fl
     # launches: apply only (producer statistics), the single-pass slab kernel (default policy of csrc/norm.cu: the (image, group) slab fits
     # one CTA's shared memory), or statistics + apply
     cpg = (c0 + c1) // groups
-    slab = (not ready) and cpg % 2 == 0 and hw >= 64 and hw * cpg * 2 <= 192 * 1024 and os.environ.get("FIE_GN_SLAB", "1") != "0"
+    slab = (not ready) and cpg % 2 == 0 and hw >= 64 and hw * cpg * 2 <= 192 * 1024
     _count(1 if (ready or slab) else 2)
     return out
 
@@ -555,7 +554,7 @@ def _groupnorm_bf16(x0, gamma, beta, eps, silu, groups, x1):
         check(L.fie_groupnorm_bf16(_p(x0), c0, _p(x1), c1, _p(out), n, hw, groups, _p(gamma), _p(beta), float(eps), int(silu), _p(ws), ws.numel(),
                                    _stream()), "fie_groupnorm_bf16")
     cpg = (c0 + c1) // groups
-    slab = cpg % 2 == 0 and hw >= 64 and hw * cpg * 2 <= 192 * 1024 and os.environ.get("FIE_GN_SLAB", "1") != "0"
+    slab = cpg % 2 == 0 and hw >= 64 and hw * cpg * 2 <= 192 * 1024
     _count(1 if slab else 2)
     return out
 

@@ -12,11 +12,7 @@ from typing import Optional, Tuple
 
 import torch
 
-import os
-
 from . import _lib
-
-NATIVE = os.environ.get("FIE_NATIVE_PACK", "1") != "0"      # 0: torch ops also on CUDA tensors (debugging / A-B)
 
 
 def _stream(t: torch.Tensor) -> int:
@@ -36,7 +32,7 @@ def _bf(dtype) -> bool:
 def cast_f16(w: torch.Tensor, dtype=torch.float16) -> torch.Tensor:
     """fp32 [N, K] -> fp16 (or bf16) [N, K] (a Linear / 1x1-conv weight as the GEMM's B operand)."""
     bf = _bf(dtype)
-    if not (w.is_cuda and NATIVE):
+    if not w.is_cuda:
         return w.to(dtype).contiguous()
     w = _f32(w)
     n, k = w.shape[0], w.numel() // w.shape[0]
@@ -53,7 +49,7 @@ def pack_conv3x3(w: torch.Tensor, pad_cout_to: Optional[int] = None, pad_cin_to:
     cout, cin = w.shape[:2]
     cp = pad_cin_to or cin
     op = pad_cout_to or cout
-    if w.is_cuda and NATIVE:
+    if w.is_cuda:
         w = _f32(w)
         out = torch.empty((op, 9 * cp), dtype=dtype, device=w.device)
         fn = "fie_pack_conv3x3_bf16" if bf else "fie_pack_conv3x3_f16"
@@ -72,7 +68,7 @@ def pack_conv3x3_c8(w: torch.Tensor, pad_cout_to: Optional[int] = None) -> torch
     cout, cin = w.shape[:2]
     assert cin <= 8
     op = pad_cout_to or cout
-    if w.is_cuda and NATIVE:
+    if w.is_cuda:
         w = _f32(w)
         out = torch.empty((op, 384), dtype=torch.float16, device=w.device)
         with torch.cuda.device(w.device):
@@ -92,7 +88,7 @@ def pack_conv_up2x(w: torch.Tensor, dtype=torch.float16) -> torch.Tensor:
     Output row 2i+a reads input rows {i-1, i} (a = 0) or {i, i+1} (a = 1); the 3x3 taps that fall on the same input row are
     summed (in fp32): a=0 -> [W0, W1+W2], a=1 -> [W0+W1, W2]; identically for columns.  K order (ty, tx, cin)."""
     bf = _bf(dtype)
-    if w.is_cuda and NATIVE:
+    if w.is_cuda:
         w = _f32(w)
         cout, cin = w.shape[:2]
         out = torch.empty((4, cout, 4 * cin), dtype=dtype, device=w.device)
@@ -132,7 +128,7 @@ def fold_layernorm(w: torch.Tensor, b: Optional[torch.Tensor], gamma: torch.Tens
     ln_stats_in).  With W' = W (.) gamma and its rows centred over K, W'' = W' - mean_k(W'):
         sum_k x_k W''_nk = sum_k (x_k - mean(x)) W'_nk,   so   LN(x) W^T + b = rstd(x) * (x W''^T) + (b + W beta)
     and the epilogue only has to scale each row by its 1/sigma.  Returns (W'' fp16 [N, K], bias fp32 [N])."""
-    if w.is_cuda and NATIVE:
+    if w.is_cuda:
         w = _f32(w)
         n, k = w.shape
         w16 = torch.empty((n, k), dtype=torch.float16, device=w.device)
@@ -156,7 +152,7 @@ def fold_layernorm(w: torch.Tensor, b: Optional[torch.Tensor], gamma: torch.Tens
 def fuse_lora(w: torch.Tensor, lora_a: torch.Tensor, lora_b: torch.Tensor, scale: float) -> torch.Tensor:
     """W' = W + scale * B A  (re-association of the reference's unfused peft path, src/pipeline.py:154).
     Linear: A [r, in], B [out, r].  Conv: A [r, in, k, k], B [out, r, 1, 1]."""
-    if w.is_cuda and NATIVE:
+    if w.is_cuda:
         out = w.float().clone().contiguous()                       # fp32 master copy, fused in place
         a32, b32 = _f32(lora_a.to(w.device)), _f32(lora_b.to(w.device))
         cout, rank = out.shape[0], a32.shape[0]

@@ -211,16 +211,12 @@ void fie_tune_conv_halo(int enable, int max_cout);
  * rectangular-box form also tiles (0 = choose by shape, the default).  Not needed in production. */
 void fie_tune_conv_im2col(int force);
 /* GroupNorm: largest thread-block cluster the single-pass shared-memory kernel (k_gn_slab) may use; 0 = always the two-kernel path,
- * default 1 (env FIE_GN_SLAB) — see the measurement note in csrc/norm.cu.  Experiments / tests only. */
+ * default 1 — see the measurement note in csrc/norm.cu.  Experiments / tests only. */
 void fie_tune_groupnorm_slab(int max_cluster);
 
 /* Debug hook: device buffer of 8 x int64 per CTA that subsequent GEMM/conv launches fill with per-role wait-cycle
  * accounting (see gemm_conv.cu); NULL switches it off.  Not needed in production. */
 void fie_gemm_trace(long long* device_buf);
-
-/* Debug hook: device buffer of 16 x int64 per CTA that subsequent self-attention launches (nkv > 128) fill with per-role
- * wait-cycle accounting (see attention.cu); NULL switches it off.  Not needed in production. */
-void fie_attention_trace(long long* device_buf);
 
 /* A: fp16 [M, K] with row stride lda (elements, multiple of 8); optional second source A1 supplies
  * K columns [k_split, K) (k_split multiple of 64) — a virtual torch.cat along K.

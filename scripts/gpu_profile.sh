@@ -21,7 +21,7 @@ timeout -k 10 1200 ncu --set full --clock-control none --import-source on -k reg
     -o gpurun_out/prof_gemm_$TAG -f $CMD > gpurun_out/ncu_gemm_$TAG.log 2>&1
 echo "ncu gemm rc=$?"
 timeout -k 10 600 $CMD > gpurun_out/plain3_$TAG.log 2>&1 &&
-timeout -k 10 1200 ncu --set full --clock-control none --import-source on -k regex:'^k_attention_d64$' -s $((3 * 160 + 40)) -c 3 \
+timeout -k 10 1200 ncu --set full --clock-control none --import-source on -k regex:'^k_attention_d64_p$' -s $((3 * 160 + 40)) -c 3 \
     -o gpurun_out/prof_attn_$TAG -f $CMD > gpurun_out/ncu_attn_$TAG.log 2>&1
 echo "ncu attention rc=$?"
 timeout -k 10 1200 ncu --set full --clock-control none --import-source on -k regex:'k_gn_apply|k_gn_stats' -s $((3 * 300 + 20)) -c 6 \

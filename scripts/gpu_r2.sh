@@ -33,7 +33,7 @@ launches)
   timeout -k 10 600 $CMD > gpurun_out/plain_$TAG.log 2>&1 &&
   timeout -k 10 1500 ncu --metrics gpu__time_duration.sum --clock-control none --csv --log-file gpurun_out/launches_$TAG.csv --profile-from-start off python scripts/step_probe.py edit > gpurun_out/ncu_list_$TAG.log 2>&1; echo "launch list rc=$?";;
 full)
-  for K in gemm:k_gemm_conv:400:6 attn:'^k_attention_d64(_p)?$':40:3 norm:'k_gn_apply|k_gn_stats':20:6 vaeattn:k_attn_vae:0:2; do
+  for K in gemm:k_gemm_conv:400:6 attn:'^k_attention_d64_p$':40:3 norm:'k_gn_apply|k_gn_stats':20:6 vaeattn:k_attn_vae:0:2; do
     IFS=: read name rx skip cnt <<< "$K"
     timeout -k 10 1500 ncu --set full --clock-control none --import-source on --profile-from-start off -k regex:"$rx" -s $skip -c $cnt -o gpurun_out/prof_${name}_$TAG -f python scripts/step_probe.py edit > gpurun_out/ncu_${name}_$TAG.log 2>&1; echo "ncu $name rc=$?"
   done;;
