@@ -6,7 +6,7 @@ import pytest
 import torch
 import torch.nn.functional as F
 
-from tests.util import rel_err
+from tests.util import guarded, rel_err
 
 pytestmark = pytest.mark.gpu
 
@@ -431,35 +431,7 @@ def test_conv3x3_c8_latent_input(cuda_dev, n, h, w, cout, res):
     assert rel_err(out, ref) < 1e-3, rel_err(out, ref)
 
 
-# ------------------------------------------------------------------ attention
-@pytest.mark.parametrize("b,heads,nq,nkv", [(1, 1, 128, 128), (2, 2, 256, 256), (2, 10, 1024, 1024), (2, 4, 256, 77), (1, 2, 64, 64), (2, 2, 4096, 4096), (1, 3, 200, 333),
-                                            (16, 20, 1024, 77), (3, 5, 1000, 77), (2, 10, 4096, 77), (1, 1, 300, 1), (4, 7, 520, 128)])
-def test_attention_d64(cuda_dev, b, heads, nq, nkv):
-    ops = _ops()
-    c = heads * 64
-    q = _rand((b * nq, c), cuda_dev, 60).half()
-    k = _rand((b * nkv, c), cuda_dev, 61).half()
-    v = _rand((b * nkv, c), cuda_dev, 62).half()
-    out = ops.attention_d64(q, k, v, b, heads, nq, nkv)
-    qh = q.float().view(b, nq, heads, 64).transpose(1, 2)
-    kh = k.float().view(b, nkv, heads, 64).transpose(1, 2)
-    vh = v.float().view(b, nkv, heads, 64).transpose(1, 2)
-    ref = F.scaled_dot_product_attention(qh, kh, vh).transpose(1, 2).reshape(b * nq, c)
-    err = float((out.float() - ref).abs().max())
-    assert err < 4e-3, err     # P is rounded to fp16 before the PV product
-
-
-def test_attention_fused_qkv_views(cuda_dev):
-    ops = _ops()
-    b, heads, n = 2, 5, 256
-    c = heads * 64
-    qkv = _rand((b * n, 3 * c), cuda_dev, 63).half()
-    out = ops.attention_d64(qkv[:, :c], qkv[:, c:2 * c], qkv[:, 2 * c:], b, heads, n, n)
-    q, k, v = [t.float().reshape(b, n, heads, 64).transpose(1, 2) for t in qkv.chunk(3, dim=-1)]
-    ref = F.scaled_dot_product_attention(q, k, v).transpose(1, 2).reshape(b * n, c)
-    assert float((out.float() - ref).abs().max()) < 4e-3
-
-
+# ------------------------------------------------------------------ softmax (the d=64 attention kernels: test_gpu_attention.py)
 @pytest.mark.parametrize("rows,cols,d", [(300, 1016, 64), (512, 16384, 512), (100, 4096, 128)])
 def test_softmax_exp_with_row_scale_in_the_pv_gemm(cuda_dev, rows, cols, d):
     """VAE mid-block attention path: exp-only softmax (unnormalised fp16 P', 1 / rowsum on the side) + P V GEMM with the row scale in
@@ -482,17 +454,6 @@ def test_softmax_exp_with_row_scale_in_the_pv_gemm(cuda_dev, rows, cols, d):
 
 
 # ------------------------------------------------------------------ guard bands (compute-sanitizer is not available on the GPU pool)
-def _guarded(rows, cols, ld, dev, lead=64, tail=64):
-    """A [rows, cols] view with row stride ld inside a sentinel-filled buffer; returns (view, checker)."""
-    buf = torch.full((lead + rows * ld + tail,), 1234.0, dtype=torch.float16, device=dev)
-    view = buf[lead:lead + rows * ld].view(rows, ld)[:, :cols]
-
-    def untouched():
-        pad = buf[lead:lead + rows * ld].view(rows, ld)[:, cols:]
-        return bool((buf[:lead] == 1234.0).all()) and bool((buf[lead + rows * ld:] == 1234.0).all()) and bool((pad == 1234.0).all())
-    return view, untouched
-
-
 @pytest.mark.parametrize("m,n,k", [(300, 96, 128), (1000, 352, 64), (257, 640, 320), (128, 1280, 1280)])
 def test_gemm_writes_only_its_output(cuda_dev, m, n, k):
     """Ragged M / N with a strided output inside a sentinel-filled buffer: rows >= M, columns >= N and the row padding stay intact
@@ -503,7 +464,7 @@ def test_gemm_writes_only_its_output(cuda_dev, m, n, k):
     bias = _rand((n,), cuda_dev, 72)
     res = _rand((m, n), cuda_dev, 73).half()
     for ld in (n + 16, n + 8):
-        out, ok = _guarded(m, n, ld, cuda_dev)
+        out, ok = guarded(m, n, ld, cuda_dev)
         st = torch.zeros((m + 8, 2), dtype=torch.int64, device=cuda_dev)
         use_ln = n % 32 == 0 and ld % 16 == 0
         ops.gemm(a, w, col_bias=bias, residual=res, out=out, ln_out=st[:m] if use_ln else None)
@@ -513,19 +474,6 @@ def test_gemm_writes_only_its_output(cuda_dev, m, n, k):
         assert int(st[m:].abs().sum()) == 0                              # statistics rows beyond M untouched
         if use_ln:
             assert float((st[:m, 0].double() / 2 ** 20 - out.float().double().sum(1)).abs().max()) < 1e-2
-
-
-@pytest.mark.parametrize("b,heads,nq,nkv", [(2, 3, 200, 333), (1, 2, 130, 77), (2, 2, 256, 256)])
-def test_attention_writes_only_its_output(cuda_dev, b, heads, nq, nkv):
-    ops = _ops()
-    c = heads * 64
-    q = _rand((b * nq, c), cuda_dev, 74).half(); k = _rand((b * nkv, c), cuda_dev, 75).half(); v = _rand((b * nkv, c), cuda_dev, 76).half()
-    out, ok = _guarded(b * nq, c, c + 64, cuda_dev)
-    ops.attention_d64(q, k, v, b, heads, nq, nkv, out=out)
-    torch.cuda.synchronize()
-    assert ok()
-    ref = ops.attention_d64(q, k, v, b, heads, nq, nkv)
-    assert torch.equal(out, ref)
 
 
 def test_conv_and_groupnorm_write_only_their_output(cuda_dev):

@@ -43,3 +43,16 @@ def gauss_golden_cases():
         edges_crc = int(z[f"case{i}_edges_crc"][0]) if f"case{i}_edges_crc" in z else None
         yield src, blur_crc, edges_crc
         i += 1
+
+
+def guarded(rows, cols, ld, dev, lead=64, tail=64):
+    """A [rows, cols] fp16 view with row stride ld, starting lead elements into a sentinel-filled buffer; returns (view, checker):
+    checker() is True while the lead and tail bands and the row padding still hold the sentinel."""
+    import torch
+    buf = torch.full((lead + rows * ld + tail,), 1234.0, dtype=torch.float16, device=dev)
+    view = buf[lead:lead + rows * ld].view(rows, ld)[:, :cols]
+
+    def untouched():
+        pad = buf[lead:lead + rows * ld].view(rows, ld)[:, cols:]
+        return bool((buf[:lead] == 1234.0).all()) and bool((buf[lead + rows * ld:] == 1234.0).all()) and bool((pad == 1234.0).all())
+    return view, untouched
