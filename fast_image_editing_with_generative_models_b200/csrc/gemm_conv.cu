@@ -623,6 +623,10 @@ __global__ void __launch_bounds__(384, 1) k_gemm_conv(const __grid_constant__ Ge
                             v[4 * i] = FIE_LN_LIN(r[4 * i], bv.x); v[4 * i + 1] = FIE_LN_LIN(r[4 * i + 1], bv.y);
                             v[4 * i + 2] = FIE_LN_LIN(r[4 * i + 2], bv.z); v[4 * i + 3] = FIE_LN_LIN(r[4 * i + 3], bv.w);
                         }
+                        if (p.m_bias) {                               // before the activation, as in epi_slow_chunk
+#pragma unroll
+                            for (int i = 0; i < 32; ++i) v[i] += mb;
+                        }
                         if (p.act == FIE_ACT_SILU) {
 #pragma unroll
                             for (int i = 0; i < 32; ++i) v[i] = silu_f(v[i]);
@@ -636,10 +640,6 @@ __global__ void __launch_bounds__(384, 1) k_gemm_conv(const __grid_constant__ Ge
 #pragma unroll
                             for (int i = 0; i < 32; ++i) v[i] = fmaxf(v[i], 0.0f);
                         }
-                    }
-                    if (p.m_bias) {
-#pragma unroll
-                        for (int i = 0; i < 32; ++i) v[i] += mb;        // (GEGLU with a per-row bias is not a supported combination)
                     }
                     if (p.scale != 1.0f) {
 #pragma unroll
@@ -808,7 +808,8 @@ static int g_force_mt = 0;
 static long long* g_trace = nullptr;
 static int g_halo = 1;              // fie_tune_conv_halo(0, ...) disables the halo convolution path
 static int g_halo_max_cout = 640;   // wider outputs reuse each A tile enough for the per-tap form to win
-static void pick_config(long long M, int N, bool geglu, int* cg_out, int* bn_out, int* mt_out, int max_mt = 2) {
+static int pick_config(long long M, int N, bool geglu, int* cg_out, int* bn_out, int* mt_out, int max_mt = 2) {
+    FIE_REQUIRE(g_force_kps != 3, "fie_tune_gemm: forced kps=3 is not a form (1 or 2)");
     const int sms = num_sms();
     double best_cost = 1e30; int best_cg = 2, best_bn = 32, best_mt = 1;
     for (int cg = 2; cg >= 1; --cg) {
@@ -829,7 +830,12 @@ static void pick_config(long long M, int N, bool geglu, int* cg_out, int* bn_out
             }
         }
     }
+    // a form forced through fie_tune_gemm that no candidate matches (mt = 2 with block_n > 128, a GEGLU shape whose packed tile
+    // width the forced form cannot hold, ...) is an error, never a silent fall-back to another form
+    FIE_REQUIRE(best_cost < 1e30, "fie_tune_gemm: forced form cg=%d kps=%d mt=%d block_n=%d has no legal tile for M=%lld N=%d%s",
+                g_force_cg, g_force_kps, g_force_mt, g_force_bn, M, N, geglu ? " (GEGLU)" : "");
     *cg_out = best_cg; *bn_out = best_bn; *mt_out = best_mt;
+    return FIE_OK;
 }
 
 static int out_dtype_of(const fie_epilogue* ep) { return (ep && ep->out_f32) ? FIE_DT_F32 : FIE_DT_F16; }
@@ -853,6 +859,7 @@ static int fill_epilogue(GemmParams& p, const fie_epilogue* ep, long long M, int
     FIE_REQUIRE(!(p.out_bf16 && (ep->gn_stats || ep->ln_stats_out || p.act == FIE_ACT_GEGLU)),
                 "epilogue: gn_stats, ln_stats_out and GEGLU need fp16 output (not supported with bf16 output)");
     FIE_REQUIRE(!(p.act == FIE_ACT_GEGLU && (N % 64)), "GEGLU needs N %% 64 == 0");
+    FIE_REQUIRE(!(p.act == FIE_ACT_GEGLU && p.m_bias), "epilogue: m_bias is not supported with the GEGLU epilogue");
     FIE_REQUIRE(!(p.residual && p.ld_res <= 0), "epilogue: residual needs ld_res");
     p.gn_stats = (unsigned long long*)ep->gn_stats; p.gn_groups = ep->gn_groups; p.gn_rows = ep->gn_rows_per_image; p.gn_cpg = 0;
     if (p.gn_stats) {
@@ -968,7 +975,7 @@ static int gemm_impl(const char* fn, const void* A, long long lda, const void* A
     if (rc) return rc;
     const bool geglu = p.act == FIE_ACT_GEGLU;
     p.mode = 0; p.M = M; p.N = N; p.ab_bf16 = ab_bf16;
-    pick_config(M, N, geglu, &p.cg, &p.block_n, &p.mt);
+    if ((rc = pick_config(M, N, geglu, &p.cg, &p.block_n, &p.mt))) return rc;
     p.num_m_blocks = (int)((M + BLOCK_M * p.cg * p.mt - 1) / (BLOCK_M * p.cg * p.mt));
     p.num_n_blocks = (N + p.block_n - 1) / p.block_n;
     p.num_kb = (K + BLOCK_K - 1) / BLOCK_K;
@@ -1012,7 +1019,7 @@ static int conv3x3_impl(const char* fn, const void* x, const void* wgt, void* ou
     FIE_REQUIRE(p.act != FIE_ACT_GEGLU, "%s: GEGLU epilogue not supported for conv", fn);
     const bool halo = boxed && g_halo > 0 && stride == 1 && (OW % BLOCK_M) == 0 && cout <= g_halo_max_cout;
     p.mode = halo ? 2 : (boxed ? 1 : 3); p.M = M; p.N = cout; p.OH = OH; p.OW = OW; p.ab_bf16 = ab_bf16;
-    pick_config(M, cout, false, &p.cg, &p.block_n, &p.mt, halo ? 1 : 2);
+    if ((rc = pick_config(M, cout, false, &p.cg, &p.block_n, &p.mt, halo ? 1 : 2))) return rc;
     p.num_m_blocks = (int)((M + BLOCK_M * p.cg * p.mt - 1) / (BLOCK_M * p.cg * p.mt));
     p.num_n_blocks = (cout + p.block_n - 1) / p.block_n;
     p.kb_per_tap = cin / BLOCK_K;
@@ -1074,7 +1081,7 @@ static int conv_up2x_impl(const char* fn, const void* x, const void* wgt, void* 
         FIE_REQUIRE(p.act != FIE_ACT_GEGLU && !p.residual && !p.out_f32, "%s: unsupported epilogue", fn);
         p.mode = boxed ? 1 : 3; p.M = M; p.N = cout; p.OH = h; p.OW = w; p.ab_bf16 = ab_bf16;
         p.up2 = 1; p.up_a = ph >> 1; p.up_b = ph & 1;
-        pick_config(M, cout, false, &p.cg, &p.block_n, &p.mt);
+        if ((rc = pick_config(M, cout, false, &p.cg, &p.block_n, &p.mt))) return rc;
         p.num_m_blocks = (int)((M + BLOCK_M * p.cg * p.mt - 1) / (BLOCK_M * p.cg * p.mt));
         p.num_n_blocks = (cout + p.block_n - 1) / p.block_n;
         p.kb_per_tap = cin / BLOCK_K;
@@ -1121,7 +1128,7 @@ static int conv3x3_c8_impl(const char* fn, const void* xp, const void* wgt, void
     if (rc) return rc;
     FIE_REQUIRE(p.act != FIE_ACT_GEGLU, "%s: GEGLU epilogue not supported for conv", fn);
     p.mode = boxed ? 1 : 3; p.M = M; p.N = cout; p.OH = h; p.OW = w;
-    pick_config(M, cout, false, &p.cg, &p.block_n, &p.mt);
+    if ((rc = pick_config(M, cout, false, &p.cg, &p.block_n, &p.mt))) return rc;
     p.num_m_blocks = (int)((M + BLOCK_M * p.cg * p.mt - 1) / (BLOCK_M * p.cg * p.mt));
     p.num_n_blocks = (cout + p.block_n - 1) / p.block_n;
     p.kb_per_tap = 1; p.num_kb = 6; p.kb_split = 6;     // 3 kernel rows x (hi, lo) weight parts, each one 64-wide K block on the same A window

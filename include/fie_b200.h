@@ -161,13 +161,14 @@ enum { FIE_ACT_NONE = 0, FIE_ACT_SILU = 1, FIE_ACT_GEGLU = 2, FIE_ACT_GELU = 3 /
        FIE_ACT_RELU = 5 /* max(x, 0): the SqueezeNet of the LPIPS metric */ };
 
 typedef struct {
-    /* epilogue: v = acc + col_bias[n] + row_bias[m / rows_per_group][n]  (+ chan_bias[m] if per-row bias)
-     *           v = act(v); v *= scale; v += residual[m, n]; store */
+    /* epilogue: v = acc + col_bias[n] + row_bias[m / rows_per_group][n] (+ m_bias[m])
+     *           v = act(v); v *= scale; v += residual[m, n]; store
+     * GEGLU: v = (value + col_bias + row_bias) * gelu_erf(gate + col_bias of the gate column), then scale and residual. */
     const float* col_bias;   /* [N] or NULL */
     const float* row_bias;   /* [ceil(M / rows_per_group), >= N] or NULL (time-embedding broadcast) */
     long long rows_per_group;
     long long ld_row_bias;   /* row stride of row_bias in elements (0 = N) */
-    const float* m_bias;     /* [M] per-output-row bias or NULL (used for transposed projections) */
+    const float* m_bias;     /* [M] per-output-row bias or NULL (used for transposed projections); added before act; not with GEGLU */
     const void* residual;    /* fp16 [M, ld_res] or NULL */
     long long ld_res;
     float scale;             /* applied before the residual add */

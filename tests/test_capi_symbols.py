@@ -92,6 +92,9 @@ def test_argument_validation_reports_errors_without_a_gpu():
     assert L.fie_attn_vae_d512_f16(p, 512, p, 512, p, p, 512, 100, 500, 0.1, 0, 0, p, 1 << 30, None) != 0 and b"d % 64" in L.fie_last_error()
     assert L.fie_ssim_u8(p, p, 1, 8, 8, 3, 11, 1.5, 0.01, 0.03, p, None) != 0 and b"smaller than the window" in L.fie_last_error()
     assert L.fie_patchify_f16(p, 1, p, 1, 30, 32, 16, None, None, None) != 0 and b"patch size" in L.fie_last_error()
+    # the GEGLU epilogue takes no per-row bias (the fast and slow epilogue paths would apply it to different operands)
+    ep = _lib.Epilogue(m_bias=p, scale=1.0, act=2)
+    assert L.fie_gemm_f16(p, 64, None, 0, 0, p, p, 32, 128, 64, 64, ctypes.byref(ep), None) != 0 and b"m_bias" in L.fie_last_error()
     # pure host queries
     assert L.fie_jpeg_header_bytes() == 623 and L.fie_jpeg_max_bytes(1024, 1024) > 3 * 1024 * 1024
     assert L.fie_jpeg_workspace_bytes(8, 1024, 1024) > 8 * 4096 * 384 * 2

@@ -6,7 +6,7 @@ import pytest
 import torch
 import torch.nn.functional as F
 
-from tests.util import guarded, rel_err
+from tests.util import rel_err
 
 pytestmark = pytest.mark.gpu
 
@@ -121,73 +121,7 @@ def test_scheduler_kernels(cuda_dev):
         assert float((got - ref).abs().max()) < 2e-5 and torch.equal(got16, got.half())
 
 
-# ------------------------------------------------------------------ tensor-core GEMM / conv
-@pytest.mark.parametrize("m,n,k", [(128, 64, 64), (256, 160, 320), (300, 320, 640), (2048, 1280, 1280), (77, 640, 2048), (4096, 1920, 640), (2, 1280, 320), (512, 8, 8), (16384, 512, 512)])
-def test_gemm_plain(cuda_dev, m, n, k):
-    ops = _ops()
-    a = _rand((m, k), cuda_dev, 20).half()
-    w = (_rand((n, k), cuda_dev, 21) / math.sqrt(k)).half()
-    bias = _rand((n,), cuda_dev, 22)
-    out = ops.gemm(a, w, col_bias=bias)
-    ref = a.float() @ w.float().t() + bias
-    assert rel_err(out, ref) < 2e-3, rel_err(out, ref)
-
-
-def test_gemm_epilogues(cuda_dev):
-    ops = _ops()
-    m, n, k = 512, 640, 640
-    a = _rand((m, k), cuda_dev, 23).half()
-    w = (_rand((n, k), cuda_dev, 24) / math.sqrt(k)).half()
-    bias = _rand((n,), cuda_dev, 25)
-    res = _rand((m, n), cuda_dev, 26).half()
-    rowb = _rand((2, n), cuda_dev, 27)
-    base = a.float() @ w.float().t()
-    out = ops.gemm(a, w, col_bias=bias, residual=res, scale=0.5)
-    assert rel_err(out, (base + bias) * 0.5 + res.float()) < 2e-3
-    out = ops.gemm(a, w, row_bias=rowb, rows_per_group=256, act=ops.ACT_SILU)
-    ref = F.silu(base + rowb.repeat_interleave(256, dim=0))
-    assert rel_err(out, ref) < 2e-3
-    out = ops.gemm(a, w, out_f32=True)
-    assert out.dtype == torch.float32 and rel_err(out, base) < 1e-5
-    mb = _rand((m,), cuda_dev, 28)
-    out = ops.gemm(a, w, m_bias=mb)
-    assert rel_err(out, base + mb[:, None]) < 2e-3
-    # two-source K (virtual concat)
-    a0, a1 = a[:, :384].contiguous(), a[:, 384:].contiguous()
-    out = ops.gemm(a0, w, a1=a1)
-    assert rel_err(out, base) < 2e-3
-    # strided A view (row stride > K) and strided output
-    big = _rand((m, 3 * k), cuda_dev, 29).half()
-    out = ops.gemm(big[:, k:2 * k], w)
-    assert rel_err(out, big[:, k:2 * k].float() @ w.float().t()) < 2e-3
-
-
-@pytest.mark.parametrize("force_bn", [0, 224, 160, 96])
-def test_gemm_epilogue_persistent_ragged(cuda_dev, force_bn):
-    """Many tiles per CTA, ragged M, N that leaves empty / partial accumulator chunks in the last tile column, bias + residual:
-    exercises the epilogue's cross-item prefetch queues (residual, staged biases) across fast and slow chunks."""
-    ops = _ops()
-    from fast_image_editing_with_generative_models_b200 import _lib
-    m, n, k = 45000, 624, 256
-    a = _rand((m, k), cuda_dev, 33).half()
-    w = (_rand((n, k), cuda_dev, 34) / math.sqrt(k)).half()
-    bias = _rand((n,), cuda_dev, 35)
-    res = _rand((m, n), cuda_dev, 36).half()
-    rowb = _rand((m // 1000, n), cuda_dev, 37)
-    ref = a.float() @ w.float().t() + bias
-    _lib.lib().fie_tune_gemm(0, force_bn)
-    try:
-        out = ops.gemm(a, w, col_bias=bias, residual=res)
-        out2 = ops.gemm(a, w, col_bias=bias, row_bias=rowb, rows_per_group=1000)
-        out3 = ops.gemm(a[:, :k], w, col_bias=bias, row_bias=rowb[:, :n], rows_per_group=1024, residual=res, scale=0.25)
-    finally:
-        _lib.lib().fie_tune_gemm(0, 0)
-    assert rel_err(out, ref + res.float()) < 2e-3
-    assert rel_err(out2, ref + rowb.repeat_interleave(1000, dim=0)) < 2e-3
-    g = torch.arange(m, device=cuda_dev) // 1024
-    assert rel_err(out3, (ref + rowb[g]) * 0.25 + res.float()) < 2e-3
-
-
+# ------------------------------------------------------------------ tensor-core GEMM (epilogue and tile forms: test_gpu_gemm.py) / conv
 @pytest.mark.parametrize("m,c,n", [(16384, 1280, 3840), (4096, 640, 640), (100, 64, 192), (45000, 320, 352), (128, 128, 128)])
 def test_gemm_folded_layernorm(cuda_dev, m, c, n):
     """x = A W0^T + b0 + res (producer writes LayerNorm row statistics) ; y = LN(x) W^T + b without a normalisation pass
@@ -236,22 +170,6 @@ def test_gemm_folded_layernorm_geglu(cuda_dev, m, c):
     wg, bg = pack_geglu(*fold_layernorm(w, b, gamma, beta))
     y = ops.gemm(x, wg, col_bias=bg, act=ops.ACT_GEGLU, ln_in=(st, 1e-5))
     assert rel_err(y, ref) < 3e-3, rel_err(y, ref)
-
-
-@pytest.mark.parametrize("m,c", [(256, 64), (1024, 640), (300, 128)])
-def test_gemm_geglu(cuda_dev, m, c):
-    ops = _ops()
-    from fast_image_editing_with_generative_models_b200.weights import pack_geglu
-    a = _rand((m, c), cuda_dev, 30).half()
-    w = (_rand((8 * c, c), cuda_dev, 31) / math.sqrt(c)).half()
-    b = _rand((8 * c,), cuda_dev, 32) * 0.5
-    wp, bp = pack_geglu(w, b)
-    out = ops.gemm(a, wp, col_bias=bp, act=ops.ACT_GEGLU)
-    h = a.float() @ w.float().t() + b
-    val, gate = h.chunk(2, dim=-1)
-    ref = val * F.gelu(gate)
-    assert out.shape == (m, 4 * c)
-    assert rel_err(out, ref) < 3e-3, rel_err(out, ref)
 
 
 @pytest.mark.parametrize("n,h,w,cin,cout,stride,pad_mode", [
@@ -454,28 +372,6 @@ def test_softmax_exp_with_row_scale_in_the_pv_gemm(cuda_dev, rows, cols, d):
 
 
 # ------------------------------------------------------------------ guard bands (compute-sanitizer is not available on the GPU pool)
-@pytest.mark.parametrize("m,n,k", [(300, 96, 128), (1000, 352, 64), (257, 640, 320), (128, 1280, 1280)])
-def test_gemm_writes_only_its_output(cuda_dev, m, n, k):
-    """Ragged M / N with a strided output inside a sentinel-filled buffer: rows >= M, columns >= N and the row padding stay intact
-    (fast and slow epilogue paths, residual prefetch queue, LayerNorm statistics)."""
-    ops = _ops()
-    a = _rand((m, k), cuda_dev, 70).half()
-    w = (_rand((n, k), cuda_dev, 71) / math.sqrt(k)).half()
-    bias = _rand((n,), cuda_dev, 72)
-    res = _rand((m, n), cuda_dev, 73).half()
-    for ld in (n + 16, n + 8):
-        out, ok = guarded(m, n, ld, cuda_dev)
-        st = torch.zeros((m + 8, 2), dtype=torch.int64, device=cuda_dev)
-        use_ln = n % 32 == 0 and ld % 16 == 0
-        ops.gemm(a, w, col_bias=bias, residual=res, out=out, ln_out=st[:m] if use_ln else None)
-        torch.cuda.synchronize()
-        assert ok(), (m, n, k, ld)
-        assert rel_err(out, a.float() @ w.float().t() + bias + res.float()) < 2e-3
-        assert int(st[m:].abs().sum()) == 0                              # statistics rows beyond M untouched
-        if use_ln:
-            assert float((st[:m, 0].double() / 2 ** 20 - out.float().double().sum(1)).abs().max()) < 1e-2
-
-
 def test_conv_and_groupnorm_write_only_their_output(cuda_dev):
     """Outputs carved out of one sentinel-filled arena, back to back: a kernel that overruns its tensor corrupts the neighbour's guard."""
     ops = _ops()

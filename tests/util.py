@@ -45,14 +45,16 @@ def gauss_golden_cases():
         i += 1
 
 
-def guarded(rows, cols, ld, dev, lead=64, tail=64):
-    """A [rows, cols] fp16 view with row stride ld, starting lead elements into a sentinel-filled buffer; returns (view, checker):
-    checker() is True while the lead and tail bands and the row padding still hold the sentinel."""
+def guarded(rows, cols, ld, dev, lead=64, tail=64, dtype=None):
+    """A [rows, cols] view (fp16 unless dtype is given) with row stride ld, starting lead elements into a sentinel-filled buffer;
+    returns (view, checker): checker() is True while the lead and tail bands and the row padding still hold the sentinel."""
     import torch
-    buf = torch.full((lead + rows * ld + tail,), 1234.0, dtype=torch.float16, device=dev)
+    dtype = dtype or torch.float16
+    s = float(torch.tensor(1234.0, dtype=dtype))          # the sentinel as the type holds it (bf16: 1232)
+    buf = torch.full((lead + rows * ld + tail,), s, dtype=dtype, device=dev)
     view = buf[lead:lead + rows * ld].view(rows, ld)[:, :cols]
 
     def untouched():
         pad = buf[lead:lead + rows * ld].view(rows, ld)[:, cols:]
-        return bool((buf[:lead] == 1234.0).all()) and bool((buf[lead + rows * ld:] == 1234.0).all()) and bool((pad == 1234.0).all())
+        return bool((buf[:lead] == s).all()) and bool((buf[lead + rows * ld:] == s).all()) and bool((pad == s).all())
     return view, untouched
