@@ -102,6 +102,14 @@ SIGNATURES = {
     "fie_pack_conv_up2x_bf16": (c_int, [c_void_p, c_void_p, c_int, c_int, c_void_p]),
     "fie_pack_rows_bf16": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_void_p]),
     "fie_cfg_lcm_step":(c_int, [c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_ll] + [c_float] * 7 + [c_int, c_void_p]),
+    "fie_canny_u8_per_image": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_size_t, c_void_p]),
+    "fie_sincos_embedding_dev": (c_int, [c_void_p, c_int, c_int, c_void_p, c_void_p]),
+    "fie_gemm_f16_ex": (c_int, [c_void_p, c_ll, c_void_p, c_ll, c_int, c_void_p, c_void_p, c_ll, c_ll, c_int, c_int, ctypes.POINTER(Epilogue), c_void_p,
+                                c_void_p]),
+    "fie_gemm_bf16_ex": (c_int, [c_void_p, c_ll, c_void_p, c_ll, c_int, c_void_p, c_void_p, c_ll, c_ll, c_int, c_int, ctypes.POINTER(Epilogue), c_int,
+                                 c_void_p, c_void_p]),
+    "fie_vae_sample_add_noise_batched": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_ll, c_ll, c_float, c_void_p, c_void_p]),
+    "fie_cfg_lcm_step_batched": (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_ll, c_ll, c_void_p, c_int, c_void_p]),
 }
 
 _lib = None

@@ -82,14 +82,16 @@ __device__ __forceinline__ void uf_union(uint32_t* P, uint32_t i, uint32_t j) {
 // component's root is strong iff the component contains a strong pixel).  Global memory only sees the dense state byte and, for candidates,
 // parent[pixel] = the global index of the tile-local root (+ weak bit): every tile-local component leaves as a depth-1 tree, and the global
 // union-find (k_seams) only has to join components across tile seams.
+// thr: per-image (low, high) in device memory, or NULL -> the by-value low, high (the same for every image).
 template <int IN_CH>
 __global__ void __launch_bounds__(256) k_nms(const uint8_t* __restrict__ src, uint8_t* __restrict__ state,
-                                             uint32_t* __restrict__ parent, int H, int W, int low, int high) {
+                                             uint32_t* __restrict__ parent, int H, int W, int low, int high, const int2* __restrict__ thr) {
     __shared__ uint8_t  sg[TH + 4][TW + 4 + 4];
     __shared__ int16_t  sdx[TH + 2][TW + 2], sdy[TH + 2][TW + 2], smg[TH + 2][TW + 2];
     __shared__ uint32_t slab[TH * TW];           // local union-find: label = local index | weak bit
     __shared__ uint8_t  sst[TH * TW];
     const int img = blockIdx.z;
+    if (thr) { const int2 t = __ldg(thr + img); low = t.x; high = t.y; }
     const int x0 = blockIdx.x * TW, y0 = blockIdx.y * TH;
     const uint8_t* g = src + (size_t)img * H * W * IN_CH;
     const int tid = threadIdx.x;
@@ -225,12 +227,13 @@ __device__ __forceinline__ uint32_t mag_class(int dx, int dy) {
 }
 
 __global__ void __launch_bounds__(256, 6) k_nms_rgb_fast(const uint8_t* __restrict__ src, uint8_t* __restrict__ state,
-                                                      uint32_t* __restrict__ parent, int H, int W, int low, int high) {
+                                                      uint32_t* __restrict__ parent, int H, int W, int low, int high, const int2* __restrict__ thr) {
     __shared__ uint32_t sgw[TH + 4][FG];               // gray, 4 px per word, image rows y0-2.., columns x0-4..
     __shared__ __align__(8) uint32_t smc[TH + 2][2 * FG];   // (mag << 2 | class), 2 px per word, image rows y0-1.., columns x0-4..
     __shared__ uint32_t slab[TH * TW];
     __shared__ __align__(4) uint8_t sst[TH * TW];
     const int img = blockIdx.z, x0 = blockIdx.x * TW, y0 = blockIdx.y * TH, tid = threadIdx.x;
+    if (thr) { const int2 t = __ldg(thr + img); low = t.x; high = t.y; }
     const uint8_t* g = src + (size_t)img * H * W * 3;
     const size_t row_bytes = (size_t)W * 3;
     // A
@@ -497,18 +500,19 @@ extern "C" size_t fie_canny_workspace_bytes(int n, int h, int w) {
     return ((px + 255) / 256) * 256 * 2 + px * 4;
 }
 
-extern "C" int fie_canny_u8(const void* img, void* edges, int n, int h, int w, int in_channels, int out_channels,
-                            int low, int high, void* workspace, size_t workspace_bytes, void* stream_) {
+// thr == NULL: (low, high) for every image.  Otherwise the per-image pairs in device memory, which the caller has normalised
+// (swap if low > high, clamp to [0, 2040]); low = 0, high = 2040 then stand for them in the kernel choice.
+static int canny_impl(const char* fn, const void* img, void* edges, int n, int h, int w, int in_channels, int out_channels,
+                      int low, int high, const int2* thr, void* workspace, size_t workspace_bytes, cudaStream_t stream) {
     using namespace fie;
-    cudaStream_t stream = (cudaStream_t)stream_;
-    FIE_REQUIRE(n >= 0 && h > 0 && w > 0, "fie_canny_u8: bad shape n=%d h=%d w=%d", n, h, w);
-    FIE_REQUIRE(in_channels == 1 || in_channels == 3, "fie_canny_u8: in_channels must be 1 or 3");
-    FIE_REQUIRE(out_channels == 1 || out_channels == 3, "fie_canny_u8: out_channels must be 1 or 3");
-    FIE_REQUIRE((long long)h * w < (1ll << 30), "fie_canny_u8: image too large");
-    FIE_REQUIRE(n <= 65535, "fie_canny_u8: batch too large");
+    FIE_REQUIRE(n >= 0 && h > 0 && w > 0, "%s: bad shape n=%d h=%d w=%d", fn, n, h, w);
+    FIE_REQUIRE(in_channels == 1 || in_channels == 3, "%s: in_channels must be 1 or 3", fn);
+    FIE_REQUIRE(out_channels == 1 || out_channels == 3, "%s: out_channels must be 1 or 3", fn);
+    FIE_REQUIRE((long long)h * w < (1ll << 30), "%s: image too large", fn);
+    FIE_REQUIRE(n <= 65535, "%s: batch too large", fn);
     if (n == 0) return FIE_OK;
-    FIE_REQUIRE(img && edges && workspace, "fie_canny_u8: null pointer");
-    FIE_REQUIRE(workspace_bytes >= fie_canny_workspace_bytes(n, h, w), "fie_canny_u8: workspace too small");
+    FIE_REQUIRE(img && edges && workspace, "%s: null pointer", fn);
+    FIE_REQUIRE(workspace_bytes >= fie_canny_workspace_bytes(n, h, w), "%s: workspace too small", fn);
     if (low > high) { int t = low; low = high; high = t; }
     size_t px = (size_t)n * h * w, pxr = ((px + 255) / 256) * 256;
     uint8_t* gray = (uint8_t*)workspace;
@@ -518,9 +522,9 @@ extern "C" int fie_canny_u8(const void* img, void* edges, int n, int h, int w, i
     dim3 g1(ceil_div(w, TW), ceil_div(h, TH), n);
     const bool fast_tile = in_channels == 3 && (w % TW) == 0 && (h % TH) == 0 && low >= 0 && high < 8192 &&
                            ((reinterpret_cast<uintptr_t>(img) | reinterpret_cast<uintptr_t>(state)) & 3) == 0;
-    if (fast_tile) k_nms_rgb_fast<<<g1, 256, 0, stream>>>((const uint8_t*)img, state, parent, h, w, low, high);
-    else if (in_channels == 3) k_nms<3><<<g1, 256, 0, stream>>>((const uint8_t*)img, state, parent, h, w, low, high);
-    else k_nms<1><<<g1, 256, 0, stream>>>((const uint8_t*)img, state, parent, h, w, low, high);
+    if (fast_tile) k_nms_rgb_fast<<<g1, 256, 0, stream>>>((const uint8_t*)img, state, parent, h, w, low, high, thr);
+    else if (in_channels == 3) k_nms<3><<<g1, 256, 0, stream>>>((const uint8_t*)img, state, parent, h, w, low, high, thr);
+    else k_nms<1><<<g1, 256, 0, stream>>>((const uint8_t*)img, state, parent, h, w, low, high, thr);
     const long long seam_px = (long long)((w - 1) / TW) * h + (long long)((h - 1) / TH) * w;
     if (seam_px > 0) k_seams<<<dim3((unsigned)((seam_px + 255) / 256), n), 256, 0, stream>>>(state, parent, h, w);
     const bool fin4 = (w & 3) == 0 && ((reinterpret_cast<uintptr_t>(state) | reinterpret_cast<uintptr_t>(edges)) & 3) == 0;
@@ -528,5 +532,18 @@ extern "C" int fie_canny_u8(const void* img, void* edges, int n, int h, int w, i
     // (measured on B200: 16-pixel / 128-bit and shared-memory-staged variants of this kernel are not faster -- its time is the latency of
     //  the root chains that k_seams leaves behind, paid by every warp that holds a candidate, not the store pattern)
     k_finalize<<<g2, 256, 0, stream>>>(state, parent, (uint8_t*)edges, h, w, out_channels);
-    return check_launch("fie_canny_u8");
+    return check_launch(fn);
+}
+
+extern "C" int fie_canny_u8(const void* img, void* edges, int n, int h, int w, int in_channels, int out_channels,
+                            int low, int high, void* workspace, size_t workspace_bytes, void* stream) {
+    return canny_impl("fie_canny_u8", img, edges, n, h, w, in_channels, out_channels, low, high, nullptr, workspace, workspace_bytes,
+                      (cudaStream_t)stream);
+}
+
+extern "C" int fie_canny_u8_per_image(const void* img, void* edges, int n, int h, int w, int in_channels, int out_channels,
+                                      const int* thresholds, void* workspace, size_t workspace_bytes, void* stream) {
+    FIE_REQUIRE(thresholds || n == 0, "fie_canny_u8_per_image: null thresholds");
+    return canny_impl("fie_canny_u8_per_image", img, edges, n, h, w, in_channels, out_channels, 0, 2040, (const int2*)thresholds, workspace,
+                      workspace_bytes, (cudaStream_t)stream);
 }

@@ -105,13 +105,14 @@ __global__ void __launch_bounds__(256) k_up2x(const uint4* __restrict__ x, uint4
     }
 }
 
+// vals: device array [count], or NULL -> the host values passed by value in a (count <= 64)
 struct SinCosArgs { float vals[64]; };
-__global__ void k_sincos(SinCosArgs a, int count, int dim, __half* __restrict__ out) {
+__global__ void k_sincos(SinCosArgs a, const float* __restrict__ vals, int count, int dim, __half* __restrict__ out) {
     const int half = dim / 2;
     for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < count * half; i += gridDim.x * blockDim.x) {
         int r = i / half, j = i % half;
         float freq = expf(-logf(10000.0f) * (float)j / (float)half);
-        float arg = a.vals[r] * freq;
+        float arg = (vals ? __ldg(vals + r) : a.vals[r]) * freq;
         out[r * dim + j] = __float2half_rn(cosf(arg));
         out[r * dim + half + j] = __float2half_rn(sinf(arg));
     }
@@ -276,10 +277,13 @@ __global__ void __launch_bounds__(256) k_softmax_rows(const T* __restrict__ s, l
 // z0 = (mean + exp(0.5*clamp(logvar,-30,20))*xi)*scaling ; x = sqrt_a*z0 + sqrt_1ma*noise.  The latent STATE is kept in fp32
 // across the scheduler steps (out32); out16 is the fp16 copy the UNet / ControlNet read.  (diffusers keeps the state in the model
 // dtype; the fp32 state removes one fp16 rounding of |x| <= 16, i.e. up to 4e-3, per step from the final latents.)
+// coef: per-image (sqrt_a, sqrt_1ma) [npx / px_per_img] in device memory, or NULL -> the by-value sa, s1.
 __global__ void __launch_bounds__(256) k_vae_sample(const __half* __restrict__ mom, int ld_m, const __half* __restrict__ xi, const __half* __restrict__ noise,
-                                                    float* __restrict__ out32, __half* __restrict__ out16, long long npx, float scaling, float sa, float s1) {
+                                                    float* __restrict__ out32, __half* __restrict__ out16, long long npx, float scaling, float sa, float s1,
+                                                    const float2* __restrict__ coef, long long px_per_img) {
     for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < npx * 4; i += (long long)gridDim.x * blockDim.x) {
         long long px = i >> 2; int c = (int)(i & 3);
+        if (coef) { const float2 k = __ldg(coef + px / px_per_img); sa = k.x; s1 = k.y; }
         const float mean = __half2float(mom[px * ld_m + c]);
         const float logvar = fminf(fmaxf(__half2float(mom[px * ld_m + 4 + c]), -30.0f), 20.0f);
         const float z = (mean + expf(0.5f * logvar) * __half2float(xi[i])) * scaling;
@@ -290,9 +294,14 @@ __global__ void __launch_bounds__(256) k_vae_sample(const __half* __restrict__ m
 
 __global__ void __launch_bounds__(256) k_cfg_lcm(const __half* __restrict__ eu, const __half* __restrict__ ec, int ld_e, const float* __restrict__ x,
                                                  const __half* __restrict__ noise, float* __restrict__ out32, __half* __restrict__ out16, long long npx, float g,
-                                                 float sa, float s1, float c_skip, float c_out, float sap, float s1p, int last) {
+                                                 float sa, float s1, float c_skip, float c_out, float sap, float s1p, int last,
+                                                 const float* __restrict__ coef, long long px_per_img) {
     for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < npx * 4; i += (long long)gridDim.x * blockDim.x) {
         long long px = i >> 2; int c = (int)(i & 3);
+        if (coef) {                                     // per-image (g, sa, s1, c_skip, c_out, sap, s1p) [npx / px_per_img][7]
+            const float* k = coef + (px / px_per_img) * 7;
+            g = __ldg(k); sa = __ldg(k + 1); s1 = __ldg(k + 2); c_skip = __ldg(k + 3); c_out = __ldg(k + 4); sap = __ldg(k + 5); s1p = __ldg(k + 6);
+        }
         float u = __half2float(eu[px * ld_e + c]), cc = __half2float(ec[px * ld_e + c]);
         float eps = u + g * (cc - u);
         float xv = x[i];
@@ -370,8 +379,14 @@ extern "C" int fie_upsample2x_f16(const void* x, void* out, int n, int h, int w,
 extern "C" int fie_sincos_embedding(const float* host_vals, int count, int dim, void* out, void* stream) {
     FIE_REQUIRE(host_vals && out && count > 0 && count <= 64 && dim > 0 && (dim % 2) == 0, "fie_sincos_embedding: bad args");
     SinCosArgs a; for (int i = 0; i < 64; ++i) a.vals[i] = i < count ? host_vals[i] : 0.f;
-    k_sincos<<<ceil_div((long long)count * dim / 2, 128), 128, 0, (cudaStream_t)stream>>>(a, count, dim, (__half*)out);
+    k_sincos<<<ceil_div((long long)count * dim / 2, 128), 128, 0, (cudaStream_t)stream>>>(a, nullptr, count, dim, (__half*)out);
     return check_launch("fie_sincos_embedding");
+}
+extern "C" int fie_sincos_embedding_dev(const float* dev_vals, int count, int dim, void* out, void* stream) {
+    FIE_REQUIRE(dev_vals && out && count > 0 && dim > 0 && (dim % 2) == 0 && (long long)count * (dim / 2) < (1ll << 31), "fie_sincos_embedding_dev: bad args");
+    SinCosArgs a = {};
+    k_sincos<<<ceil_div((long long)count * dim / 2, 128), 128, 0, (cudaStream_t)stream>>>(a, dev_vals, count, dim, (__half*)out);
+    return check_launch("fie_sincos_embedding_dev");
 }
 extern "C" int fie_softmax_rows_f32_to_f16(const void* s, long long ld_in, void* p, long long ld_out, long long rows, int cols, float scale, void* stream) {
     FIE_REQUIRE(s && p && rows > 0 && rows < (1ll << 31) && cols > 0 && (ld_in % 4) == 0 && (ld_out % 4) == 0, "fie_softmax_rows: bad args");
@@ -401,8 +416,17 @@ extern "C" int fie_vae_sample_add_noise(const void* moments, int ld_m, const voi
                                         long long count_px, float scaling, float sqrt_a, float sqrt_1ma, void* stream) {
     FIE_REQUIRE(moments && xi && noise && x_out_f32 && x_out_f16 && count_px > 0 && ld_m >= 8, "fie_vae_sample_add_noise: bad args");
     k_vae_sample<<<grid_for(count_px * 4, 256), 256, 0, (cudaStream_t)stream>>>((const __half*)moments, ld_m, (const __half*)xi, (const __half*)noise,
-                                                                                x_out_f32, (__half*)x_out_f16, count_px, scaling, sqrt_a, sqrt_1ma);
+                                                                                x_out_f32, (__half*)x_out_f16, count_px, scaling, sqrt_a, sqrt_1ma, nullptr, 1);
     return check_launch("fie_vae_sample_add_noise");
+}
+extern "C" int fie_vae_sample_add_noise_batched(const void* moments, int ld_m, const void* xi, const void* noise, float* x_out_f32, void* x_out_f16,
+                                                long long count_px, long long px_per_img, float scaling, const float* coef, void* stream) {
+    FIE_REQUIRE(moments && xi && noise && x_out_f32 && x_out_f16 && coef && count_px > 0 && px_per_img > 0 && (count_px % px_per_img) == 0 && ld_m >= 8,
+                "fie_vae_sample_add_noise_batched: bad args");
+    k_vae_sample<<<grid_for(count_px * 4, 256), 256, 0, (cudaStream_t)stream>>>((const __half*)moments, ld_m, (const __half*)xi, (const __half*)noise,
+                                                                                x_out_f32, (__half*)x_out_f16, count_px, scaling, 0.f, 0.f,
+                                                                                (const float2*)coef, px_per_img);
+    return check_launch("fie_vae_sample_add_noise_batched");
 }
 extern "C" int fie_cfg_lcm_step(const void* eps_u, const void* eps_c, int ld_e, const float* x_f32, const void* noise, float* x_out_f32, void* x_out_f16,
                                 long long count_px, float guidance, float sqrt_a, float sqrt_1ma, float c_skip, float c_out,
@@ -410,6 +434,15 @@ extern "C" int fie_cfg_lcm_step(const void* eps_u, const void* eps_c, int ld_e, 
     FIE_REQUIRE(eps_u && eps_c && x_f32 && x_out_f32 && x_out_f16 && count_px > 0 && ld_e >= 4 && (last || noise), "fie_cfg_lcm_step: bad args");
     k_cfg_lcm<<<grid_for(count_px * 4, 256), 256, 0, (cudaStream_t)stream>>>((const __half*)eps_u, (const __half*)eps_c, ld_e, x_f32,
                                                                               (const __half*)noise, x_out_f32, (__half*)x_out_f16, count_px, guidance, sqrt_a, sqrt_1ma,
-                                                                              c_skip, c_out, sqrt_a_prev, sqrt_1ma_prev, last);
+                                                                              c_skip, c_out, sqrt_a_prev, sqrt_1ma_prev, last, nullptr, 1);
     return check_launch("fie_cfg_lcm_step");
+}
+extern "C" int fie_cfg_lcm_step_batched(const void* eps_u, const void* eps_c, int ld_e, const float* x_f32, const void* noise, float* x_out_f32, void* x_out_f16,
+                                        long long count_px, long long px_per_img, const float* coef, int last, void* stream) {
+    FIE_REQUIRE(eps_u && eps_c && x_f32 && x_out_f32 && x_out_f16 && coef && count_px > 0 && px_per_img > 0 && (count_px % px_per_img) == 0 && ld_e >= 4 &&
+                (last || noise), "fie_cfg_lcm_step_batched: bad args");
+    k_cfg_lcm<<<grid_for(count_px * 4, 256), 256, 0, (cudaStream_t)stream>>>((const __half*)eps_u, (const __half*)eps_c, ld_e, x_f32,
+                                                                              (const __half*)noise, x_out_f32, (__half*)x_out_f16, count_px, 0.f, 0.f, 0.f,
+                                                                              0.f, 0.f, 0.f, 0.f, last, coef, px_per_img);
+    return check_launch("fie_cfg_lcm_step_batched");
 }

@@ -90,6 +90,7 @@ struct GemmParams {
     float ln_eps;
     double ln_inv;                  // 1 / (2^20 * length of the normalised A rows)
     const float* row_scale;         // [M] optional per-row scale of the accumulator (exclusive with ln_in)
+    const float* group_scale;       // [ceil(M / rows_per_group)] optional per-row-group replacement of scale, or NULL
 };
 
 // Output row of accumulator row m (identity, or the strided scatter of one phase of the fused nearest-2x upsample).
@@ -194,8 +195,9 @@ __device__ __noinline__ void epi_slow_chunk(const GemmParams& p, uint32_t taddr,
 #pragma unroll
         for (int i = 0; i < 32; ++i) v[i] = fmaxf(v[i], 0.0f);
     }
+    const float sc = p.group_scale ? (row_ok ? __ldg(p.group_scale + m / p.rows_per_group) : 1.0f) : p.scale;
 #pragma unroll
-    for (int i = 0; i < 32; ++i) v[i] *= p.scale;
+    for (int i = 0; i < 32; ++i) v[i] *= sc;
     if (row_ok && nout < p.n_store) {
         if (p.residual) {
             const uint16_t* rp = reinterpret_cast<const uint16_t*>(p.residual) + m * p.ld_res + nout;
@@ -578,6 +580,7 @@ __global__ void __launch_bounds__(384, 1) k_gemm_conv(const __grid_constant__ Ge
                 const uint32_t tacc = tmem_base + lane_addr + (uint32_t)((buf * MT + mt) * block_n);
                 const float mb = (p.m_bias && row_ok) ? p.m_bias[m] : 0.0f;
                 const float* rb = (p.row_bias && row_ok) ? p.row_bias + (m / p.rows_per_group) * p.ld_row_bias : nullptr;
+                const float gs = p.group_scale ? (row_ok ? __ldg(p.group_scale + m / p.rows_per_group) : 1.0f) : p.scale;
                 __half* orow = reinterpret_cast<__half*>(p.D) + out_row(p, row_ok ? m : 0) * p.ldd;
                 bias_commit();                                         // this group's biases -> staging; then fetch the next group's
                 if (mt + 1 < MT) bias_issue(tile, mt + 1); else bias_issue(tile + tile_step, 0);
@@ -641,9 +644,9 @@ __global__ void __launch_bounds__(384, 1) k_gemm_conv(const __grid_constant__ Ge
                             for (int i = 0; i < 32; ++i) v[i] = fmaxf(v[i], 0.0f);
                         }
                     }
-                    if (p.scale != 1.0f) {
+                    if (p.group_scale || p.scale != 1.0f) {
 #pragma unroll
-                        for (int i = 0; i < 32; ++i) v[i] *= p.scale;
+                        for (int i = 0; i < 32; ++i) v[i] *= gs;
                     }
                     if (res_fast && row_ok) {
 #pragma unroll
@@ -964,7 +967,7 @@ extern "C" int fie_geglu_block_n(int N) { return (N % 256) == 0 ? 256 : ((N % 12
 
 static int gemm_impl(const char* fn, const void* A, long long lda, const void* A1, long long lda1, int k_split,
                      const void* B, void* D, long long ldd, long long M, int N, int K,
-                     const fie_epilogue* ep, int ab_bf16, int out_dtype, void* stream) {
+                     const fie_epilogue* ep, int ab_bf16, int out_dtype, void* stream, const float* group_scale = nullptr) {
     FIE_REQUIRE(A && B && D, "%s: null pointer", fn);
     FIE_REQUIRE(M > 0 && N > 0 && K > 0, "%s: bad shape M=%lld N=%d K=%d", fn, M, N, K);
     FIE_REQUIRE(M < (1ll << 31), "%s: M too large", fn);
@@ -973,6 +976,7 @@ static int gemm_impl(const char* fn, const void* A, long long lda, const void* A
     memset(&p, 0, sizeof(p));
     int rc = fill_epilogue(p, ep, M, N, D, ldd, out_dtype);
     if (rc) return rc;
+    p.group_scale = group_scale;
     const bool geglu = p.act == FIE_ACT_GEGLU;
     p.mode = 0; p.M = M; p.N = N; p.ab_bf16 = ab_bf16;
     if ((rc = pick_config(M, N, geglu, &p.cg, &p.block_n, &p.mt))) return rc;
@@ -1159,6 +1163,17 @@ extern "C" int fie_gemm_bf16(const void* A, long long lda, const void* A1, long 
                              long long M, int N, int K, const fie_epilogue* ep, int out_dtype, void* stream) {
     if (int rc = check_out_dtype("fie_gemm_bf16", ep, out_dtype)) return rc;
     return gemm_impl("fie_gemm_bf16", A, lda, A1, lda1, k_split, B, D, ldd, M, N, K, ep, 1, out_dtype, stream);
+}
+
+extern "C" int fie_gemm_f16_ex(const void* A, long long lda, const void* A1, long long lda1, int k_split, const void* B, void* D, long long ldd,
+                               long long M, int N, int K, const fie_epilogue* ep, const float* group_scale, void* stream) {
+    return gemm_impl("fie_gemm_f16_ex", A, lda, A1, lda1, k_split, B, D, ldd, M, N, K, ep, 0, out_dtype_of(ep), stream, group_scale);
+}
+
+extern "C" int fie_gemm_bf16_ex(const void* A, long long lda, const void* A1, long long lda1, int k_split, const void* B, void* D, long long ldd,
+                                long long M, int N, int K, const fie_epilogue* ep, int out_dtype, const float* group_scale, void* stream) {
+    if (int rc = check_out_dtype("fie_gemm_bf16_ex", ep, out_dtype)) return rc;
+    return gemm_impl("fie_gemm_bf16_ex", A, lda, A1, lda1, k_split, B, D, ldd, M, N, K, ep, 1, out_dtype, stream, group_scale);
 }
 
 extern "C" int fie_conv3x3_f16(const void* x, const void* wgt, void* out, long long ldd, int n, int h, int w, int cin, int cout,

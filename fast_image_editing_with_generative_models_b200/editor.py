@@ -33,6 +33,7 @@ from PIL import Image
 
 from . import model_zoo, ops
 from . import synthetic as S
+from .pipeline import per_image
 
 _ENV_KEYS = {"root": "FIE_CHECKPOINTS", "controlnet": "FIE_CONTROLNET", "vae": "FIE_VAE", "lora": "FIE_LCM_LORA"}
 
@@ -112,6 +113,16 @@ def resolve_size(size, image_size) -> tuple:
     if w * h > MAX_PIXELS:
         raise ValueError(f"size {w}x{h}: at most {MAX_PIXELS} pixels (1024 x 1024)")
     return (w, h)
+
+
+def micro_batches(sizes: Sequence[tuple], n_exec: Sequence[int], guidance: Sequence[float], mb: int) -> List[tuple]:
+    """edit_many's plan: the image indices grouped by (size, executed step count, guidance > 1) -- the images of one engine call share
+    its launch sequence -- each group cut into micro-batches of at most ``mb`` images in input order -> [((size, n_exec, cfg), [index,
+    ...]), ...]."""
+    groups: Dict[tuple, List[int]] = {}
+    for i, wh in enumerate(sizes):
+        groups.setdefault((tuple(wh), int(n_exec[i]), guidance[i] > 1), []).append(i)
+    return [(key, idx[b0:b0 + mb]) for key, idx in groups.items() for b0 in range(0, len(idx), mb)]
 
 
 class _PipeShim:
@@ -306,6 +317,32 @@ class FastEditor:
                              f"{n_exec} which is < 1 and not appropriate for this pipeline.")
         return n_exec
 
+    @classmethod
+    def _per_image_settings(cls, n: int, strength, num_inference_steps, guidance_scale, controlnet_conditioning_scale, canny_low_threshold,
+                            canny_high_threshold) -> Dict[str, list]:
+        """edit_many's numeric settings, each a scalar or one value per image -> {name: list of n values} plus "n_exec", the denoising
+        steps each image executes.  ValueError (naming the image) for a wrong length, a non-finite value or an invalid strength / step
+        count."""
+        st = dict(strength=strength, num_inference_steps=num_inference_steps, guidance_scale=guidance_scale,
+                  controlnet_conditioning_scale=controlnet_conditioning_scale, canny_low_threshold=canny_low_threshold,
+                  canny_high_threshold=canny_high_threshold)
+        for name, v in st.items():
+            if name == "num_inference_steps" and not isinstance(v, (str, bytes)) and isinstance(v, (Sequence, np.ndarray)):
+                if len(v) != n:
+                    raise ValueError(f"num_inference_steps: {len(v)} values for {n} images")
+                st[name] = list(v)                     # kept as given: _executed_steps checks that each is an int
+            elif name == "num_inference_steps":
+                st[name] = [v] * n
+            else:
+                st[name] = per_image(name, v, n)
+        st["n_exec"] = []
+        for i in range(n):
+            try:
+                st["n_exec"].append(cls._executed_steps(st["strength"][i], st["num_inference_steps"][i]))
+            except ValueError as err:
+                raise ValueError(f"image {i}: {err}") from None
+        return st
+
     def _draw_noises(self, seed, n_exec: int, size=(OUT_SIZE, OUT_SIZE)) -> List[torch.Tensor]:
         """Reference RNG order for one image of ``size`` = (width, height): posterior sample, init noise, then one draw per non-final
         executed step, each [1, 4, height/8, width/8]."""
@@ -338,7 +375,8 @@ class FastEditor:
             img = self._to_device(image, wh)
             pe, pl = self._encode_prompt(prompt, negative_prompt)
             noises = self._draw_noises(seed, n_exec, wh)
-            out = self._engine.edit_batch(img, pe, pl, noises, strength=strength, num_inference_steps=num_inference_steps,
+            # per-image prompt layout [1,2,77,D], as edit_many passes it: warm_up(micro_batch=1) captures the graph edit() replays
+            out = self._engine.edit_batch(img, pe[None], pl[None], noises, strength=strength, num_inference_steps=num_inference_steps,
                                           guidance_scale=guidance_scale, controlnet_conditioning_scale=controlnet_conditioning_scale,
                                           canny_low=int(np.floor(canny_low_threshold)), canny_high=int(np.floor(canny_high_threshold)),
                                           canny_blur=canny_gaussian_blur)
@@ -356,8 +394,13 @@ class FastEditor:
         to Pillow's encoder at ``jpeg_quality``), encoded on the GPU: ~0.1-0.3 MB instead of 3 MB per image cross PCIe and the host
         does no pixel work at all.
 
-        ``size`` as in :meth:`edit`.  With ``"auto"`` the images are grouped by their bucket; each group runs in its own micro-batches
-        and the results come back in input order.
+        ``strength``, ``num_inference_steps``, ``guidance_scale``, ``controlnet_conditioning_scale``, ``canny_low_threshold`` and
+        ``canny_high_threshold`` each take a scalar (every image) or a sequence with one value per image.  The values are device data of
+        the edit, so images with different settings share a micro-batch and its CUDA graph.
+
+        ``size`` as in :meth:`edit`.  The images are grouped by (size, executed step count, guidance > 1): the images of one micro-batch
+        run the same launch sequence (with ``guidance_scale <= 1`` only the positive prompt rows run, as in diffusers).  Each group runs
+        in its own micro-batches and the results come back in input order.
 
         The host side is pipelined: while the GPU runs micro-batch *i* (one CUDA-graph replay), the host converts the outputs of
         micro-batch *i-1* to PIL images and stages the inputs of *i+1* (pinned buffers, asynchronous copies)."""
@@ -373,14 +416,11 @@ class FastEditor:
             raise ValueError("edit_many: seeds must have one entry per image")
         if output not in ("pil", "jpeg"):
             raise ValueError("edit_many: output must be 'pil' or 'jpeg'")
-        n_exec = self._executed_steps(strength, num_inference_steps)
+        st = self._per_image_settings(n, strength, num_inference_steps, guidance_scale, controlnet_conditioning_scale, canny_low_threshold,
+                                      canny_high_threshold)
         mb = int(micro_batch or self.MICRO_BATCH)
-        lo, hi = int(np.floor(canny_low_threshold)), int(np.floor(canny_high_threshold))
         sizes = [resolve_size(size, im.size) for im in images]
-        by_size: Dict[tuple, List[int]] = {}
-        for i, wh in enumerate(sizes):
-            by_size.setdefault(wh, []).append(i)
-        chunks = [(wh, idx[b0:b0 + mb]) for wh, idx in by_size.items() for b0 in range(0, len(idx), mb)]
+        chunks = micro_batches(sizes, st["n_exec"], st["guidance_scale"], mb)
         results: List[Optional[Image.Image]] = [None] * n
         pending = None                                   # (index list, pinned output buffer, event) of the micro-batch in flight
         with torch.cuda.device(self._dev):
@@ -410,7 +450,7 @@ class FastEditor:
                     trace.append((name, _time.perf_counter() - t0))
                 return _time.perf_counter()
 
-            for k, (wh, idx) in enumerate(chunks):
+            for k, ((wh, n_exec, _), idx) in enumerate(chunks):
                 t_ = _time.perf_counter()
                 nb = len(idx)
                 pad_to = mb if nb * 2 >= mb else 1 << (nb - 1).bit_length()       # ragged tail: reuse the full-size graph, or the next power of two
@@ -433,9 +473,10 @@ class FastEditor:
                 per_img += [per_img[-1]] * (pad_to - nb)
                 noises = [torch.cat([p[d] for p in per_img], 0) for d in range(len(per_img[0]))]
                 t_ = mark("noise draws (launch)", t_)
-                out = self._engine.edit_batch(d_img, pe, pl, noises, strength=strength, num_inference_steps=num_inference_steps,
-                                              guidance_scale=guidance_scale, controlnet_conditioning_scale=controlnet_conditioning_scale,
-                                              canny_low=lo, canny_high=hi, canny_blur=canny_gaussian_blur)
+                sel = lambda name: [st[name][i] for i in idx + pad]
+                out = self._engine.edit_batch(d_img, pe, pl, noises, strength=sel("strength"), num_inference_steps=sel("num_inference_steps"),
+                                              guidance_scale=sel("guidance_scale"), controlnet_conditioning_scale=sel("controlnet_conditioning_scale"),
+                                              canny_low=sel("canny_low_threshold"), canny_high=sel("canny_high_threshold"), canny_blur=canny_gaussian_blur)
                 t_ = mark("edit_batch (graph launch)", t_)
                 if output == "jpeg":
                     # Encode on the GPU.  The file sizes are not known on the host yet, so a prefix of every file buffer is copied whose
@@ -468,7 +509,8 @@ class FastEditor:
 
     def warm_up(self, micro_batch: Optional[int] = None, *, size=None, **edit_kwargs) -> float:
         """Runs one dummy micro-batch with the given ``edit`` arguments so that the CUDA graph for that shape / schedule is captured and
-        the pinned staging buffers exist before the first real call (sweeps call this during initialisation).  ``size`` as in
+        the pinned staging buffers exist before the first real call (sweeps call this during initialisation).  The graph serves every
+        setting with the same size, executed step count and CFG on/off (guidance > 1), whatever the guidance, scales, thresholds.  ``size`` as in
         :meth:`edit`; ``"auto"`` warms up the square bucket.  Returns the seconds spent."""
         import time
         t0 = time.perf_counter()

@@ -244,10 +244,16 @@ class _EncoderPart:
         aug = ops.gemm(h, self.a2[0], col_bias=self.a2[1])
         return ctx_kv, aug
 
-    def time_rows(self, t: float, aug: Tensor) -> Tensor:
-        """Per-step: fp32 [B, sum Cout] row biases (time_emb_proj(SiLU(emb)) + conv1.bias) for every resnet."""
+    def time_rows(self, t, aug: Tensor) -> Tensor:
+        """Per-step: fp32 [B, sum Cout] row biases (time_emb_proj(SiLU(emb)) + conv1.bias) for every resnet.  ``t``: one timestep for
+        every row, or an fp32 CUDA tensor [B] with the timestep of each row (read on the device: the edit's parameter block)."""
         b = aug.shape[0]
-        te = ops.sincos_embedding([t], self.cfg.block_out_channels[0], aug.device).expand(b, -1).contiguous()
+        if isinstance(t, Tensor):
+            if t.numel() != b:
+                raise ValueError(f"time_rows: {t.numel()} timesteps for {b} rows")
+            te = ops.sincos_embedding(t, self.cfg.block_out_channels[0], aug.device)
+        else:
+            te = ops.sincos_embedding([t], self.cfg.block_out_channels[0], aug.device).expand(b, -1).contiguous()
         h = ops.gemm(te, self.t1[0], col_bias=self.t1[1], act=ops.ACT_SILU)
         emb = ops.gemm(h, self.t2[0], col_bias=self.t2[1], residual=aug)
         return ops.gemm(ops.silu(emb), self.temb_w, col_bias=self.temb_b, out_f32=True)
@@ -368,20 +374,25 @@ class ControlNet:
         h = ops.conv3x3_c8(ops.pad8(x), self.enc.conv_in[0], col_bias=self.enc.conv_in[1], residual=cond_emb)
         return self.enc.down_mid(h, temb, ctx_kv, nctx)
 
-    def merge_into(self, feats, scale: float):
+    def merge_into(self, feats, scale):
         """-> merge(unet_skips, unet_h): every zero convolution writes scale * (W f + b) + <the UNet tensor it is added to> in one
         GEMM epilogue, i.e. `down_block_res_samples[i] + down_block_additional_residuals[i]` and the mid-block add of
-        UNet2DConditionModel.forward without separate element-wise kernels (and with one rounding instead of two)."""
+        UNet2DConditionModel.forward without separate element-wise kernels (and with one rounding instead of two).
+        ``scale``: one conditioning scale, or an fp32 CUDA tensor with one per batch row (image and CFG half), read on the device as
+        the GEMMs' group_scale."""
         cn_h, cn_skips = feats
 
+        def zero_conv(f, w, b, res):
+            n_, hh, ww, c_ = res.shape
+            if isinstance(scale, Tensor):
+                kw = dict(group_scale=scale, rows_per_group=hh * ww)
+            else:
+                kw = dict(scale=scale)
+            return ops.gemm(f.view(-1, f.shape[-1]), w, col_bias=b, residual=res.view(-1, c_), **kw).view(res.shape)
+
         def merge(skips, h):
-            n_, hh, ww, c_ = h.shape
-            merged = []
-            for f, (w, b), s in zip(cn_skips, self.zero, skips):
-                sh = s.shape
-                merged.append(ops.gemm(f.view(-1, f.shape[-1]), w, col_bias=b, scale=scale, residual=s.view(-1, sh[-1])).view(sh))
-            hm = ops.gemm(cn_h.view(-1, c_), self.zero_mid[0], col_bias=self.zero_mid[1], scale=scale, residual=h.view(-1, c_)).view(n_, hh, ww, c_)
-            return merged, hm
+            merged = [zero_conv(f, w, b, s) for f, (w, b), s in zip(cn_skips, self.zero, skips)]
+            return merged, zero_conv(cn_h, self.zero_mid[0], self.zero_mid[1], h)
         return merge
 
 

@@ -7,6 +7,7 @@ input goes to the ``*_bf16`` entry points, an fp16 input to the fp16 ones exactl
 from __future__ import annotations
 
 import ctypes
+import math
 from typing import Optional
 
 import torch
@@ -103,10 +104,31 @@ def _req(t: torch.Tensor, dtype, name: str):
         raise _lib.FieError(f"{name}: expected a contiguous tensor")
 
 
-def canny(img_u8: torch.Tensor, low: int = 100, high: int = 200, out_channels: int = 1, gaussian_blur: bool = False) -> torch.Tensor:
+CANNY_MAX_MAGNITUDE = 2040      # largest L1 Sobel magnitude of an 8-bit image: 4 * 255 per direction
+
+
+def canny_thresholds(low, high):
+    """A cv2.Canny threshold pair as cv2 reads it, normalised for :func:`canny`'s per-image form: floor, swap if low > high, clamp both
+    to [0, 2040].  Magnitudes lie in [0, 2040] and a zero magnitude never survives the non-maximum suppression, so the clamp changes
+    no edge map.  -> (low, high) ints."""
+    lo, hi = math.floor(low), math.floor(high)
+    if lo > hi:
+        lo, hi = hi, lo
+    clamp = lambda v: min(max(v, 0), CANNY_MAX_MAGNITUDE)
+    return clamp(lo), clamp(hi)
+
+
+def canny(img_u8: torch.Tensor, low: int = 100, high: int = 200, out_channels: int = 1, gaussian_blur: bool = False, *,
+          thresholds: Optional[torch.Tensor] = None) -> torch.Tensor:
     """uint8 [N,H,W,3] (RGB) or [N,H,W] (gray) -> uint8 edges [N,H,W] or [N,H,W,3] (0/255); == cv2.Canny.
-    ``gaussian_blur`` (default off, as in the reference): gray -> cv2.GaussianBlur(gray, (5, 5), 0) -> Canny."""
+    ``gaussian_blur`` (default off, as in the reference): gray -> cv2.GaussianBlur(gray, (5, 5), 0) -> Canny.
+    ``thresholds``: int32 [N, 2] CUDA tensor of per-image (low, high) pairs, each normalised by :func:`canny_thresholds`; replaces
+    ``low`` / ``high`` (fie_canny_u8_per_image: the values are read on the device, so a CUDA graph replays with new ones)."""
     _req(img_u8, torch.uint8, "canny")
+    if thresholds is not None:
+        _req(thresholds, torch.int32, "canny")
+        if tuple(thresholds.shape) != (img_u8.shape[0], 2):
+            raise _lib.FieError("canny: thresholds must be int32 [N, 2]")
     if gaussian_blur:
         gray = rgb_to_gray(img_u8) if img_u8.dim() == 4 else img_u8
         img_u8 = gaussian_blur5(gray)
@@ -117,7 +139,11 @@ def canny(img_u8: torch.Tensor, low: int = 100, high: int = 200, out_channels: i
     ws = torch.empty(max(ws_bytes, 16), dtype=torch.uint8, device=img_u8.device)
     out = torch.empty((n, h, w, 3) if out_channels == 3 else (n, h, w), dtype=torch.uint8, device=img_u8.device)
     with _prof("canny", float(n) * h * w * (in_ch + out_channels), "B"):
-        check(L.fie_canny_u8(_p(img_u8), _p(out), n, h, w, in_ch, out_channels, int(low), int(high), _p(ws), ws_bytes, _stream()), "fie_canny_u8")
+        if thresholds is not None:
+            check(L.fie_canny_u8_per_image(_p(img_u8), _p(out), n, h, w, in_ch, out_channels, _p(thresholds), _p(ws), ws_bytes, _stream()),
+                  "fie_canny_u8_per_image")
+        else:
+            check(L.fie_canny_u8(_p(img_u8), _p(out), n, h, w, in_ch, out_channels, int(low), int(high), _p(ws), ws_bytes, _stream()), "fie_canny_u8")
     _count(3)
     return out
 
@@ -442,6 +468,14 @@ def embed_tokens(ids: torch.Tensor, tok: torch.Tensor, pos: torch.Tensor) -> tor
 
 
 def sincos_embedding(vals, dim: int, device) -> torch.Tensor:
+    """Timesteps -> fp16 [count, dim] = cat(cos, sin) (diffusers Timesteps).  ``vals``: host numbers (at most 64), or an fp32 CUDA
+    tensor [count] read on the device (fie_sincos_embedding_dev; bit-identical for the same floats)."""
+    if isinstance(vals, torch.Tensor):
+        _req(vals, torch.float32, "sincos_embedding")
+        out = torch.empty((vals.numel(), dim), dtype=torch.float16, device=vals.device)
+        check(_lib.lib().fie_sincos_embedding_dev(_p(vals), vals.numel(), dim, _p(out), _stream()), "fie_sincos_embedding_dev")
+        _count()
+        return out
     vals = [float(v) for v in vals]
     arr = (ctypes.c_float * len(vals))(*vals)
     out = torch.empty((len(vals), dim), dtype=torch.float16, device=device)
@@ -592,8 +626,9 @@ def _epilogue(col_bias=None, row_bias=None, rows_per_group=1, m_bias=None, resid
 def gemm(a: torch.Tensor, w: torch.Tensor, *, a1: Optional[torch.Tensor] = None, out: Optional[torch.Tensor] = None, n_valid: Optional[int] = None,
          col_bias=None, row_bias=None, rows_per_group=1, m_bias=None, residual=None, scale=1.0, act=ACT_NONE, out_f32=False,
          gn_groups: int = 0, gn_rows: int = 0, ln_out: Optional[torch.Tensor] = None, ln_in=None,
-         row_scale: Optional[torch.Tensor] = None, out_dtype: Optional[torch.dtype] = None) -> torch.Tensor:
+         row_scale: Optional[torch.Tensor] = None, out_dtype: Optional[torch.dtype] = None, group_scale: Optional[torch.Tensor] = None) -> torch.Tensor:
     """D = epilogue(A @ W^T).  a: [..., K] fp16 rows (row stride may exceed K), w: [N, K] fp16; optional a1 continues K.
+    group_scale: fp32 [ceil(M / rows_per_group)] CUDA tensor that replaces ``scale`` per group of rows (fie_gemm_f16_ex).
     ln_out: zeroed int64 [M, 2] that receives the LayerNorm statistics of the output rows.  ln_in = (stats, eps): the A rows are
     layer-normalised on the fly (w / col_bias from weights.fold_layernorm).
     bf16 a / w (/ a1): fie_gemm_bf16, whose output is bf16 by default, else ``out_dtype`` / the dtype of ``out`` (fp16, bf16, fp32)."""
@@ -632,14 +667,25 @@ def gemm(a: torch.Tensor, w: torch.Tensor, *, a1: Optional[torch.Tensor] = None,
         raise _lib.FieError("gemm: ln_in = (contiguous int64 [M, 2] statistics, eps)")
     if row_scale is not None and (row_scale.dtype != torch.float32 or row_scale.numel() != m or not row_scale.is_contiguous()):
         raise _lib.FieError("gemm: row_scale must be a contiguous fp32 [M] tensor")
+    if group_scale is not None:
+        _req(group_scale, torch.float32, "gemm group_scale")
+        if group_scale.numel() != -(-m // int(rows_per_group)):
+            raise _lib.FieError("gemm: group_scale must hold one fp32 value per group of rows_per_group rows")
     ep = _epilogue(col_bias, row_bias, rows_per_group, m_bias, residual, scale, act, out_f32, gn, ln_out, ln_in, row_scale)
     ep.ln_dim = k
     with _prof("gemm", 2.0 * m * n * k, "FLOP", f"M{m} N{n} K{k} act{act} res{int(residual is not None)} f32{int(out_f32)}" + (" bf16" if bf else "")):
-        if bf:
-            check(_lib.lib().fie_gemm_bf16(_p(a), lda, _p(a1), lda1, k_split, _p(w), _p(out), ldd, m, n, k, ctypes.byref(ep), _DT[out.dtype], _stream()),
+        L = _lib.lib()
+        if bf and group_scale is not None:
+            check(L.fie_gemm_bf16_ex(_p(a), lda, _p(a1), lda1, k_split, _p(w), _p(out), ldd, m, n, k, ctypes.byref(ep), _DT[out.dtype], _p(group_scale),
+                                     _stream()), "fie_gemm_bf16_ex")
+        elif bf:
+            check(L.fie_gemm_bf16(_p(a), lda, _p(a1), lda1, k_split, _p(w), _p(out), ldd, m, n, k, ctypes.byref(ep), _DT[out.dtype], _stream()),
                   "fie_gemm_bf16")
+        elif group_scale is not None:
+            check(L.fie_gemm_f16_ex(_p(a), lda, _p(a1), lda1, k_split, _p(w), _p(out), ldd, m, n, k, ctypes.byref(ep), _p(group_scale), _stream()),
+                  "fie_gemm_f16_ex")
         else:
-            check(_lib.lib().fie_gemm_f16(_p(a), lda, _p(a1), lda1, k_split, _p(w), _p(out), ldd, m, n, k, ctypes.byref(ep), _stream()), "fie_gemm_f16")
+            check(L.fie_gemm_f16(_p(a), lda, _p(a1), lda1, k_split, _p(w), _p(out), ldd, m, n, k, ctypes.byref(ep), _stream()), "fie_gemm_f16")
     _count()
     return out
 
@@ -819,5 +865,38 @@ def cfg_lcm_step(eps_u: torch.Tensor, eps_c: torch.Tensor, x32: torch.Tensor, no
     check(_lib.lib().fie_cfg_lcm_step(_p(eps_u), _p(eps_c), eps_u.stride(-2), _p(x32), _p(noise), _p(out32), _p(out16), npx, float(guidance), float(c["sqrt_a"]),
                                        float(c["sqrt_1ma"]), float(c["c_skip"]), float(c["c_out"]), float(c["sqrt_a_prev"]), float(c["sqrt_1ma_prev"]),
                                        int(bool(c["last"])), _stream()), "fie_cfg_lcm_step")
+    _count()
+    return out32, out16
+
+
+def vae_sample_add_noise_batched(moments: torch.Tensor, xi: torch.Tensor, noise: torch.Tensor, scaling: float, coef: torch.Tensor):
+    """:func:`vae_sample_add_noise` with per-image add-noise coefficients: coef fp32 [N, 2] = (sqrt_a, sqrt_1ma) CUDA tensor."""
+    _req(moments, torch.float16, "vae_sample_add_noise_batched")
+    _req(coef, torch.float32, "vae_sample_add_noise_batched")
+    n = xi.shape[0]
+    if coef.numel() != 2 * n:
+        raise _lib.FieError("vae_sample_add_noise_batched: coef must be fp32 [N, 2]")
+    out32 = torch.empty(xi.shape, dtype=torch.float32, device=xi.device)
+    out16 = torch.empty_like(xi)
+    npx = xi.numel() // 4
+    check(_lib.lib().fie_vae_sample_add_noise_batched(_p(moments), moments.shape[-1], _p(xi), _p(noise), _p(out32), _p(out16), npx, npx // n,
+                                                       float(scaling), _p(coef), _stream()), "fie_vae_sample_add_noise_batched")
+    _count()
+    return out32, out16
+
+
+def cfg_lcm_step_batched(eps_u: torch.Tensor, eps_c: torch.Tensor, x32: torch.Tensor, noise: Optional[torch.Tensor], coef: torch.Tensor, last: bool):
+    """:func:`cfg_lcm_step` with per-image coefficients: coef fp32 [N, 7] = (guidance, sqrt_a, sqrt_1ma, c_skip, c_out, sqrt_a_prev,
+    sqrt_1ma_prev) CUDA tensor (LCMSchedule.batch_tables); ``last``: the final step of every image (no noise)."""
+    _req(x32, torch.float32, "cfg_lcm_step_batched")
+    _req(coef, torch.float32, "cfg_lcm_step_batched")
+    n = x32.shape[0]
+    if coef.numel() != 7 * n:
+        raise _lib.FieError("cfg_lcm_step_batched: coef must be fp32 [N, 7]")
+    out32 = torch.empty_like(x32)
+    out16 = torch.empty(x32.shape, dtype=torch.float16, device=x32.device)
+    npx = x32.numel() // 4
+    check(_lib.lib().fie_cfg_lcm_step_batched(_p(eps_u), _p(eps_c), eps_u.stride(-2), _p(x32), _p(noise), _p(out32), _p(out16), npx, npx // n, _p(coef),
+                                               int(bool(last)), _stream()), "fie_cfg_lcm_step_batched")
     _count()
     return out32, out16

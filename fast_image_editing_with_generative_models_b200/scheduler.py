@@ -5,7 +5,7 @@ scaled_linear betas 0.00085..0.012 over 1000 steps, epsilon prediction, original
 timestep_scaling 10, sigma_data 0.5."""
 from __future__ import annotations
 
-from typing import Dict, List, Tuple
+from typing import Dict, List, Sequence, Tuple
 
 import numpy as np
 
@@ -38,6 +38,26 @@ class LCMSchedule:
     def add_noise_coeffs(self, t: int) -> Tuple[float, float]:
         a = float(self.alphas_cumprod[t])
         return a ** 0.5, (1.0 - a) ** 0.5
+
+    STEP_COLUMNS = ("guidance", "sqrt_a", "sqrt_1ma", "c_skip", "c_out", "sqrt_a_prev", "sqrt_1ma_prev")
+
+    def batch_tables(self, steps: Sequence[int], strengths: Sequence[float], guidance: Sequence[float]):
+        """Per-image schedules of one batch, every image with its own ``(num_inference_steps, strength)`` and guidance (pass 1.0 for a
+        batch without CFG) -> (timesteps [B][n_exec], add-noise coefficients fp32 [B, 2] = (sqrt_a, sqrt_1ma) at each image's first
+        timestep, step table fp32 [n_exec, B, 7] in the columns of ``STEP_COLUMNS``), the values of :meth:`add_noise_coeffs` and
+        :meth:`step_coeffs` rounded to fp32.  Every image must execute the same number of steps (one launch sequence)."""
+        ts, add, rows = [], [], []
+        for i, (n, st) in enumerate(zip(steps, strengths)):
+            t, begin = self.img2img_timesteps(int(n), float(st))
+            if ts and len(t) != len(ts[0]):
+                raise ValueError(f"image {i}: {n} steps at strength {st} execute {len(t)} steps, image 0 executes {len(ts[0])}; "
+                                 "the images of one batch must execute the same number of steps")
+            ts.append(t)
+            add.append(self.add_noise_coeffs(t[0]))
+            cs = [self.step_coeffs(begin + k) for k in range(len(t))]
+            rows.append([[float(guidance[i])] + [c[name] for name in self.STEP_COLUMNS[1:]] for c in cs])
+        table = np.asarray(rows, dtype=np.float32).transpose(1, 0, 2) if rows else np.zeros((0, 0, 7), np.float32)
+        return ts, np.asarray(add, dtype=np.float32).reshape(-1, 2), np.ascontiguousarray(table)
 
     def step_coeffs(self, step_index: int) -> Dict[str, float]:
         t = self.timesteps[step_index]

@@ -39,6 +39,12 @@ int fie_device_supported(void);
 size_t fie_canny_workspace_bytes(int n, int h, int w);
 int fie_canny_u8(const void* img, void* edges, int n, int h, int w, int in_channels, int out_channels,
                  int low, int high, void* workspace, size_t workspace_bytes, void* stream);
+/* Per-image thresholds (EditEngine.edit_batch with a threshold per image, pipeline.py): thresholds int32 [n][2] = (low, high) of
+ * image i in DEVICE memory, so that a CUDA graph replays with new values.  Each pair must be normalised on the host as
+ * cv2.Canny reads it: floor, swap if low > high, clamp both to [0, 2040] (ops.canny_thresholds).  L1 Sobel magnitudes lie in
+ * [0, 2040] and a pixel of magnitude 0 never survives NMS, so the clamp changes no result.  Same kernels as fie_canny_u8. */
+int fie_canny_u8_per_image(const void* img, void* edges, int n, int h, int w, int in_channels, int out_channels,
+                           const int* thresholds, void* workspace, size_t workspace_bytes, void* stream);
 
 /* ---- optional Canny pre-stage (DEFAULT OFF in the path: the reference's cv2.Canny call, src/pipeline.py:205, has no blur;
  * BASELINE.json's north_star lists a Gaussian stage, so it exists as an opt-in: FastEditor.preprocess_image(..., gaussian_blur=True)) ----
@@ -131,6 +137,9 @@ int fie_upsample2x_f16(const void* x, void* out, int n, int h, int w, int c, voi
 /* sinusoidal embedding (diffusers Timesteps, flip_sin_to_cos, shift 0): vals fp32 [count] (HOST pointer,
  * count <= 64) -> fp16 [count, dim] = cat(cos, sin) */
 int fie_sincos_embedding(const float* host_vals, int count, int dim, void* out_f16, void* stream);
+/* the same from DEVICE values fp32 [count] (no count limit): the per-row timesteps of the time embedding (engine._EncoderPart.time_rows,
+ * read from the graph's parameter block).  Bit-identical to fie_sincos_embedding for the same floats. */
+int fie_sincos_embedding_dev(const float* dev_vals, int count, int dim, void* out_f16, void* stream);
 /* softmax over rows: fp32 [rows, cols] (ld_in) * scale -> fp16 [rows, cols] (ld_out) */
 int fie_softmax_rows_f32_to_f16(const void* s_f32, long long ld_in, void* p_f16, long long ld_out,
                                 long long rows, int cols, float scale, void* stream);
@@ -225,6 +234,13 @@ void fie_gemm_trace(long long* device_buf);
 int fie_gemm_f16(const void* A, long long lda, const void* A1, long long lda1, int k_split,
                  const void* B, void* D, long long ldd, long long M, int N, int K,
                  const fie_epilogue* ep, void* stream);
+/* fie_gemm_f16 with a per-row-group scale: group_scale fp32 [ceil(M / ep->rows_per_group)] in device memory multiplies the
+ * value where ep->scale does (after the activation, before the residual add), row m using group_scale[m / rows_per_group];
+ * ep->scale is then ignored.  NULL: exactly fie_gemm_f16.  The ControlNet zero convolutions (engine.ControlNet.merge_into): one
+ * conditioning scale per image and CFG half, rows_per_group = h*w. */
+int fie_gemm_f16_ex(const void* A, long long lda, const void* A1, long long lda1, int k_split,
+                    const void* B, void* D, long long ldd, long long M, int N, int K,
+                    const fie_epilogue* ep, const float* group_scale, void* stream);
 
 /* 3x3 convolution as implicit GEMM, NHWC fp16.  x: [n,h,w,cin] (cin multiple of 64), wgt: [cout][3][3][cin],
  * out: [n,oh,ow,cout].  stride 1: pad 1.  stride 2: pad_mode 0 = symmetric pad 1 (UNet Downsample2D),
@@ -265,6 +281,10 @@ enum { FIE_DT_F16 = 0, FIE_DT_BF16 = 1, FIE_DT_F32 = 2 };
 int fie_gemm_bf16(const void* A, long long lda, const void* A1, long long lda1, int k_split,
                   const void* B, void* D, long long ldd, long long M, int N, int K,
                   const fie_epilogue* ep, int out_dtype, void* stream);
+/* fie_gemm_bf16 with group_scale as in fie_gemm_f16_ex */
+int fie_gemm_bf16_ex(const void* A, long long lda, const void* A1, long long lda1, int k_split,
+                     const void* B, void* D, long long ldd, long long M, int N, int K,
+                     const fie_epilogue* ep, int out_dtype, const float* group_scale, void* stream);
 int fie_conv3x3_bf16(const void* x, const void* wgt, void* out, long long ldd, int n, int h, int w, int cin, int cout,
                      int cout_valid, int stride, int pad_mode, const fie_epilogue* ep, int out_dtype, void* stream);
 int fie_conv_up2x_bf16(const void* x, const void* wgt, void* out, long long ldd, int n, int h, int w, int cin, int cout,
@@ -345,6 +365,15 @@ int fie_vae_sample_add_noise(const void* moments, int ld_m, const void* xi, cons
 int fie_cfg_lcm_step(const void* eps_u, const void* eps_c, int ld_e, const float* x_f32, const void* noise, float* x_out_f32, void* x_out_f16,
                      long long count_px, float guidance, float sqrt_a, float sqrt_1ma, float c_skip, float c_out,
                      float sqrt_a_prev, float sqrt_1ma_prev, int last, void* stream);
+/* Per-image forms (EditEngine.edit_batch, pipeline.py: every image of a batch with its own strength, step count and guidance).  The
+ * coefficients are DEVICE arrays, so that one CUDA graph serves every setting; image i covers pixels [i px_per_img, (i+1) px_per_img).
+ * coef of fie_vae_sample_add_noise_batched: fp32 [n][2] = (sqrt_a, sqrt_1ma); of fie_cfg_lcm_step_batched: fp32 [n][7] = (guidance,
+ * sqrt_a, sqrt_1ma, c_skip, c_out, sqrt_a_prev, sqrt_1ma_prev).  Same kernels and arithmetic as the scalar forms: an image's result is
+ * bit-identical to the scalar call with that image's values. */
+int fie_vae_sample_add_noise_batched(const void* moments, int ld_m, const void* xi, const void* noise, float* x_out_f32, void* x_out_f16,
+                                     long long count_px, long long px_per_img, float scaling, const float* coef, void* stream);
+int fie_cfg_lcm_step_batched(const void* eps_u, const void* eps_c, int ld_e, const float* x_f32, const void* noise, float* x_out_f32,
+                             void* x_out_f16, long long count_px, long long px_per_img, const float* coef, int last, void* stream);
 
 #ifdef __cplusplus
 }
