@@ -89,14 +89,71 @@ def load_model_dir(folder: str):
     return cfg, {k: v.float() for k, v in load_file(_weights_file(folder)).items()}
 
 
-def lora_to_peft(sd: Dict[str, Tensor], param_names: Sequence[str]) -> Dict[str, Tensor]:
-    """LCM-LoRA state dict (kohya or peft/diffusers keys) -> {param}.lora_A.weight / {param}.lora_B.weight, ``alpha / rank`` folded into B."""
+# model part -> (kohya prefix, peft / diffusers prefix) of the keys of a LoRA file
+LORA_PARTS = {"unet": ("lora_unet_", "unet."), "text_encoder": ("lora_te1_", "text_encoder."), "text_encoder_2": ("lora_te2_", "text_encoder_2.")}
+_UNSUPPORTED_LORA = ("dora_scale", "hada_", "lokr_")          # DoRA, LyCORIS LoHa / LoKr: not a plain B A delta
+
+
+def read_lora(src, weight_name: Optional[str] = None) -> Dict[str, Tensor]:
+    """``load_lora_weights``' first argument -> a state dict: a dict as it is, a local ``.safetensors`` file, or a folder holding
+    ``weight_name`` (default ``pytorch_lora_weights.safetensors``).  Anything else (a hub id) is a ValueError: nothing is downloaded."""
+    if isinstance(src, dict):
+        return dict(src)
+    if not isinstance(src, (str, os.PathLike)):
+        raise ValueError(f"LoRA: expected a state dict, a .safetensors file or a folder, not {type(src).__name__}")
+    path = os.fspath(src)
+    if os.path.isdir(path):
+        path = os.path.join(path, weight_name or "pytorch_lora_weights.safetensors")
+    if not (path.endswith(".safetensors") and os.path.isfile(path)):
+        raise ValueError(f"LoRA: {path!r} is not a local .safetensors file or a folder holding one (hub ids are not supported)")
+    from safetensors.torch import load_file
+    return load_file(path)
+
+
+def split_lora(sd: Dict[str, Tensor]) -> Dict[str, Dict[str, Tensor]]:
+    """A LoRA state dict -> {part: its keys} for the parts of :data:`LORA_PARTS` that occur.  Keys with no part prefix belong to the UNet
+    (peft files saved from a bare UNet).  ValueError for DoRA (``dora_scale``) and LyCORIS LoHa / LoKr keys, and for any key that is not
+    a LoRA factor of one of the parts in a layout :func:`lora_to_peft` reads (e.g. SD 1.x ``lora_te_`` keys), or whose partner is missing."""
+    bad = [k for k in sd if any(t in k for t in _UNSUPPORTED_LORA)]
+    if bad:
+        raise ValueError(f"LoRA: unsupported format (DoRA / LyCORIS LoHa / LoKr keys, first: {bad[:2]}); only plain LoRA (B A) deltas are supported")
+    parts: Dict[str, Dict[str, Tensor]] = {}
+    unknown = []
+    for k, v in sd.items():
+        part = next((p for p, pre in LORA_PARTS.items() if k.startswith(pre)), "unet")
+        if not _lora_key_ok(k, sd, LORA_PARTS[part][0]):
+            unknown.append(k)
+        parts.setdefault(part, {})[k] = v
+    if unknown:             # a key lora_to_peft would skip: a silently dropped tensor would give a quietly different model
+        raise ValueError(f"LoRA: {len(unknown)} tensors are not LoRA factors of the UNet or a text encoder in a known layout, or lack their "
+                         f"partner (first: {unknown[:3]})")
+    return parts
+
+
+def _lora_key_ok(k: str, sd: Dict[str, Tensor], kohya: str) -> bool:
+    """Whether :func:`lora_to_peft` consumes key ``k``: a kohya down / up / alpha key of the part (down and up both present), or a peft
+    ``lora_A`` / ``lora_B`` (``lora.down`` / ``lora.up``) weight with its partner.  peft files carry no alpha (it is folded into B)."""
+    if k.startswith(kohya):
+        for role, other in ((".lora_down.weight", ".lora_up.weight"), (".lora_up.weight", ".lora_down.weight"), (".alpha", ".lora_down.weight")):
+            if k.endswith(role):
+                return k[: -len(role)] + other in sd
+        return False
+    for role, other in ((".lora_A.", ".lora_B."), (".lora_B.", ".lora_A."), (".lora.down.", ".lora.up."), (".lora.up.", ".lora.down.")):
+        if role in k and k.endswith(".weight"):
+            return k.replace(role, other) in sd
+    return False
+
+
+def lora_to_peft(sd: Dict[str, Tensor], param_names: Sequence[str], part: str = "unet") -> Dict[str, Tensor]:
+    """LoRA state dict (kohya or peft/diffusers keys) of one model part (:data:`LORA_PARTS`) -> {param}.lora_A.weight /
+    {param}.lora_B.weight, ``alpha / rank`` folded into B."""
+    kohya, peft = LORA_PARTS[part]
     by_flat = {n[: -len(".weight")].replace(".", "_"): n[: -len(".weight")] for n in param_names if n.endswith(".weight")}
     out: Dict[str, Tensor] = {}
     unmapped = []
     for k, v in sd.items():
-        if k.endswith(".lora_down.weight") and k.startswith("lora_unet_"):              # kohya
-            flat = k[len("lora_unet_"): -len(".lora_down.weight")]
+        if k.endswith(".lora_down.weight") and k.startswith(kohya):                     # kohya
+            flat = k[len(kohya): -len(".lora_down.weight")]
             name = by_flat.get(flat)
             if name is None:
                 unmapped.append(k)
@@ -107,14 +164,15 @@ def lora_to_peft(sd: Dict[str, Tensor], param_names: Sequence[str]) -> Dict[str,
             out[name + ".lora_A.weight"], out[name + ".lora_B.weight"] = v.float(), up * scale
         elif ".lora_A" in k or ".lora.down" in k:                                         # peft / old diffusers
             name = k.split(".lora")[0]
-            name = name[len("unet."):] if name.startswith("unet.") else name
+            name = name[len(peft):] if name.startswith(peft) else name
             kb = k.replace(".lora_A", ".lora_B").replace(".lora.down", ".lora.up")
             if name + ".weight" in param_names or name in by_flat.values():
                 out[name + ".lora_A.weight"], out[name + ".lora_B.weight"] = v.float(), sd[kb].float()
             else:
                 unmapped.append(k)
     if unmapped:            # a silently skipped adapter layer would give a quietly different model
-        raise ValueError(f"LoRA: {len(unmapped)} adapter tensors do not match any UNet parameter (first: {unmapped[:3]})")
+        what = "UNet" if part == "unet" else part
+        raise ValueError(f"LoRA: {len(unmapped)} adapter tensors do not match any {what} parameter (first: {unmapped[:3]})")
     return out
 
 

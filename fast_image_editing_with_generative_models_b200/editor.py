@@ -33,6 +33,7 @@ from PIL import Image
 
 from . import model_zoo, ops
 from . import synthetic as S
+from .lora import LoraAdapters
 from .pipeline import per_image
 
 _ENV_KEYS = {"root": "FIE_CHECKPOINTS", "controlnet": "FIE_CONTROLNET", "vae": "FIE_VAE", "lora": "FIE_LCM_LORA"}
@@ -126,14 +127,41 @@ def micro_batches(sizes: Sequence[tuple], n_exec: Sequence[int], guidance: Seque
 
 
 class _PipeShim:
-    """What callers touch on ``editor.pipe``: ``run_batch.py:157-158`` calls ``set_progress_bar_config(disable=True)``."""
+    """What callers touch on ``editor.pipe``: ``run_batch.py:157-158`` calls ``set_progress_bar_config(disable=True)``, and users of
+    diffusers' pipeline add style LoRAs with ``load_lora_weights`` / ``set_adapters`` (as the reference adds its LCM-LoRA,
+    ``src/pipeline.py:154``).  The adapters are fused into the packed weights in place (:mod:`.lora`): every edit after a change uses
+    them, captured CUDA graphs included.  An adapter is active at weight 1.0 once loaded; with SDXL the load-time LCM-LoRA is adapter
+    ``"default_0"``."""
 
-    def __init__(self, engine):
+    def __init__(self, engine, adapters: Optional[LoraAdapters] = None):
         self.engine = engine
         self.progress_bar_config: Dict = {}
+        self.adapters = adapters or LoraAdapters(engine)
 
     def set_progress_bar_config(self, **kwargs):
         self.progress_bar_config.update(kwargs)
+
+    def load_lora_weights(self, pretrained_model_name_or_path_or_dict, adapter_name: Optional[str] = None, weight_name: Optional[str] = None):
+        """A local ``.safetensors`` file, a folder holding ``pytorch_lora_weights.safetensors`` (or ``weight_name``), or a state dict (kohya
+        or peft / diffusers keys) -> adapter ``adapter_name`` (default: the next ``default_<i>``), active at 1.0 next to the active ones."""
+        self.adapters.load_lora_weights(pretrained_model_name_or_path_or_dict, adapter_name, weight_name)
+
+    def set_adapters(self, adapter_names, adapter_weights=None):
+        """Make exactly these adapters active, with these weights (default 1.0; one number for all, or one per adapter)."""
+        self.adapters.set_adapters(adapter_names, adapter_weights)
+
+    def get_active_adapters(self) -> List[str]:
+        return self.adapters.get_active_adapters()
+
+    def get_list_adapters(self) -> Dict[str, List[str]]:
+        return self.adapters.get_list_adapters()
+
+    def delete_adapters(self, adapter_names):
+        self.adapters.delete_adapters(adapter_names)
+
+    def unload_lora_weights(self):
+        """Remove every adapter loaded after the editor was built: the weights are again, byte for byte, the ones it was built with."""
+        self.adapters.unload_lora_weights()
 
 
 class FastEditor:
@@ -213,7 +241,10 @@ class FastEditor:
             self._engine = model_zoo.build_engine(state, self._dev)
         self._engine.use_graphs = True      # every edit has the same shapes: replay it as one CUDA graph after the first call
         self.controlnet = self._engine.cn
-        self.pipe = _PipeShim(self._engine)
+        # the LoRA fused at build time is adapter "default_0" (diffusers' name for an unnamed first adapter): its factors (no copy; B is
+        # scaled as it was fused only when they move to the device at the first change) are what re-weighting or deleting it subtracts
+        base = {"default_0": (state["lora"], float(state.get("lora_scale", 1.0)))} if state.get("lora") else None
+        self.pipe = _PipeShim(self._engine, LoraAdapters(self._engine, base, text=lambda: self._text, on_change=self._prompt_cache_clear))
         self._prompt_encoder = prompt_encoder
         self._prompt_cache: "OrderedDict" = OrderedDict()
         self._text = None
@@ -249,6 +280,29 @@ class FastEditor:
             warnings.warn("FastEditor: checkpoints without text_encoder / text_encoder_2 folders — prompts are mapped to seeded RANDOM "
                           "embeddings (pass prompt_encoder= or add the CLIP folders)", RuntimeWarning, stacklevel=2)
         self._say("[FastEditor] Initialization complete!")
+
+    # ---- LoRA adapters (diffusers' names; see _PipeShim) ----
+    def load_lora_weights(self, pretrained_model_name_or_path_or_dict, adapter_name: Optional[str] = None, weight_name: Optional[str] = None):
+        self.pipe.load_lora_weights(pretrained_model_name_or_path_or_dict, adapter_name, weight_name)
+
+    def set_adapters(self, adapter_names, adapter_weights=None):
+        self.pipe.set_adapters(adapter_names, adapter_weights)
+
+    def get_active_adapters(self) -> List[str]:
+        return self.pipe.get_active_adapters()
+
+    def get_list_adapters(self) -> Dict[str, List[str]]:
+        return self.pipe.get_list_adapters()
+
+    def delete_adapters(self, adapter_names):
+        self.pipe.delete_adapters(adapter_names)
+
+    def unload_lora_weights(self):
+        self.pipe.unload_lora_weights()
+
+    def _prompt_cache_clear(self):
+        """Adapters changed: cached prompt embeddings may come from the old text-encoder weights."""
+        self._prompt_cache.clear()
 
     # ---- prompt -> embeddings ----
     def _encode_prompt(self, prompt: str, negative_prompt: str):
@@ -546,6 +600,9 @@ class FastEditor:
                 torch.cuda.empty_cache()
 
     def get_memory_usage(self):
+        """``lora_pristine_gb``: the part of ``allocated_gb`` held by the pristine weight copies of active LoRA adapters (0 when the
+        adapters are the ones the editor was built with)."""
         if str(self.device).startswith("cuda"):
-            return {"allocated_gb": torch.cuda.memory_allocated(self._dev) / 1024 ** 3, "reserved_gb": torch.cuda.memory_reserved(self._dev) / 1024 ** 3}
+            return {"allocated_gb": torch.cuda.memory_allocated(self._dev) / 1024 ** 3, "reserved_gb": torch.cuda.memory_reserved(self._dev) / 1024 ** 3,
+                    "lora_pristine_gb": self.pipe.adapters.pristine_bytes() / 1024 ** 3}
         return {"allocated_gb": 0, "reserved_gb": 0}

@@ -21,7 +21,7 @@ import torch
 
 from . import ops
 from .configs import ControlNetConfig, UNetConfig, VAEConfig, skip_channels
-from .weights import cast_f16, fold_layernorm, fuse_lora, pack_conv3x3, pack_conv3x3_c8, pack_conv_up2x, pack_geglu
+from .weights import LoraTarget, cast_f16, geglu_rows, fold_layernorm, fuse_lora, pack_conv3x3, pack_conv3x3_c8, pack_conv_up2x, pack_geglu
 
 Tensor = torch.Tensor
 Params = Dict[str, Tensor]
@@ -123,6 +123,15 @@ class Resnet:
             self.b1 = None
         self.sc = pk.conv1(pre + ".conv_shortcut") if pk.has(pre + ".conv_shortcut") else None
 
+    def lora_targets(self, pre: str, temb_w: Tensor, out: Dict[str, LoraTarget]):
+        cin = self.w1.shape[1] // 9
+        out[pre + ".conv1"] = LoraTarget("conv3", self.w1, self.cout, cin)
+        out[pre + ".conv2"] = LoraTarget("conv3", self.w2, self.cout, self.cout)
+        if self.sc is not None:
+            out[pre + ".conv_shortcut"] = LoraTarget("rows", self.sc[0], self.cout, self.sc[0].shape[1])
+        if self.temb_off is not None:
+            out[pre + ".time_emb_proj"] = LoraTarget("rows", temb_w, self.cout, temb_w.shape[1], row0=self.temb_off)
+
     def __call__(self, x: Tensor, temb_all: Optional[Tensor] = None, skip: Optional[Tensor] = None) -> Tensor:
         n, h, w, _ = x.shape
         hcur = ops.groupnorm(x, self.n1[0], self.n1[1], self.eps, True, self.groups, skip)
@@ -150,6 +159,7 @@ class TransformerBlock:
     def __init__(self, pk: _Packer, pre: str, c: int, kv_slot: List):
         self.c = c
         ln1, ln2, ln3 = pk.norm(pre + ".norm1"), pk.norm(pre + ".norm2"), pk.norm(pre + ".norm3")
+        self.ln = (ln1, ln2, ln3)          # kept for LoRA deltas of the folded projections (lora_targets)
         wqkv = torch.cat([pk.w(f"{pre}.attn1.{n}") for n in ("to_q", "to_k", "to_v")], 0)
         self.wo1 = pk.linear(pre + ".attn1.to_out.0")
         self.kv_off = sum(t.shape[0] for t in kv_slot)
@@ -159,6 +169,19 @@ class TransformerBlock:
         self.wqkv, self.bqkv = fold_layernorm(wqkv, None, *ln1)
         self.wq2, self.bq2 = fold_layernorm(pk.w(pre + ".attn2.to_q"), pk.b(pre + ".attn2.to_q"), *ln2)
         self.wg, self.bg = pack_geglu(*fold_layernorm(pk.w(pre + ".ff.net.0.proj"), pk.b(pre + ".ff.net.0.proj"), *ln3))
+
+    def lora_targets(self, pre: str, kv_w: Tensor, out: Dict[str, LoraTarget]):
+        c = self.c
+        for i, n in enumerate(("to_q", "to_k", "to_v")):
+            out[f"{pre}.attn1.{n}"] = LoraTarget("rows", self.wqkv, c, c, row0=i * c, ln=self.ln[0], bias=self.bqkv)
+        out[pre + ".attn1.to_out.0"] = LoraTarget("rows", self.wo1[0], c, c)
+        out[pre + ".attn2.to_q"] = LoraTarget("rows", self.wq2, c, c, ln=self.ln[1], bias=self.bq2)
+        out[pre + ".attn2.to_k"] = LoraTarget("rows", kv_w, c, kv_w.shape[1], row0=self.kv_off)
+        out[pre + ".attn2.to_v"] = LoraTarget("rows", kv_w, c, kv_w.shape[1], row0=self.kv_off + c)
+        out[pre + ".attn2.to_out.0"] = LoraTarget("rows", self.wo2[0], c, c)
+        out[pre + ".ff.net.0.proj"] = LoraTarget("rows", self.wg, self.wg.shape[0], c, ln=self.ln[2], bias=self.bg,
+                                                 perm=geglu_rows(self.wg.shape[0], self.wg.device))
+        out[pre + ".ff.net.2"] = LoraTarget("rows", self.wf[0], c, self.wf[0].shape[1])
 
     def __call__(self, h: Tensor, b: int, ntok: int, ctx_kv: Tensor, nctx: int, st: Tensor, st_next: Optional[Tensor] = None) -> Tensor:
         """st: int64 [3, M, 2] row statistics (st[0] already holds those of h); st_next receives those of the result."""
@@ -183,6 +206,12 @@ class Transformer2D:
         self.pin = pk.linear(pre + ".proj_in")
         self.blocks = [TransformerBlock(pk, f"{pre}.transformer_blocks.{k}", c, kv_slot) for k in range(depth)]
         self.pout = pk.linear(pre + ".proj_out")
+
+    def lora_targets(self, pre: str, kv_w: Tensor, out: Dict[str, LoraTarget]):
+        out[pre + ".proj_in"] = LoraTarget("rows", self.pin[0], self.c, self.c)
+        out[pre + ".proj_out"] = LoraTarget("rows", self.pout[0], self.c, self.c)
+        for k, blk in enumerate(self.blocks):
+            blk.lora_targets(f"{pre}.transformer_blocks.{k}", kv_w, out)
 
     def __call__(self, x: Tensor, ctx_kv: Tensor, nctx: int) -> Tensor:
         n, hh, ww, c = x.shape
@@ -232,6 +261,26 @@ class _EncoderPart:
         self.temb_b = torch.cat([t[1] for t in self.temb_slot], 0).contiguous()
         self.kv_w = torch.cat(self.kv_slot, 0).contiguous() if self.kv_slot else None
         self.temb_slot = self.kv_slot = None
+
+    def lora_targets(self, out: Dict[str, LoraTarget]):
+        """{diffusers module name: where its packed weight lives} for conv_in, the embeddings, down and mid blocks."""
+        w = self.conv_in[0]
+        out["conv_in"] = LoraTarget("c8", w, self.cfg.block_out_channels[0], self.cfg.in_channels)
+        for name, lin in (("time_embedding.linear_1", self.t1), ("time_embedding.linear_2", self.t2), ("add_embedding.linear_1", self.a1),
+                          ("add_embedding.linear_2", self.a2)):
+            out[name] = LoraTarget("rows", lin[0], lin[0].shape[0], lin[0].shape[1])
+        for i, blk in enumerate(self.down):
+            for j, r in enumerate(blk["res"]):
+                r.lora_targets(f"down_blocks.{i}.resnets.{j}", self.temb_w, out)
+                if blk["attn"]:
+                    blk["attn"][j].lora_targets(f"down_blocks.{i}.attentions.{j}", self.kv_w, out)
+            if blk["down"] is not None:
+                d = blk["down"][0]
+                out[f"down_blocks.{i}.downsamplers.0.conv"] = LoraTarget("conv3", d, d.shape[0], d.shape[1] // 9)
+        self.mid_res0.lora_targets("mid_block.resnets.0", self.temb_w, out)
+        if self.mid_attn is not None:
+            self.mid_attn.lora_targets("mid_block.attentions.0", self.kv_w, out)
+            self.mid_res1.lora_targets("mid_block.resnets.1", self.temb_w, out)
 
     # ---- step-invariant (per prompt) work ----
     def prepare_prompt(self, ctx: Tensor, text_embeds: Tensor, time_ids: Sequence[float]):
@@ -300,6 +349,22 @@ class UNet:
 
     def prepare_prompt(self, ctx, text_embeds, time_ids):
         return self.enc.prepare_prompt(ctx, text_embeds, time_ids)
+
+    def lora_targets(self) -> Dict[str, LoraTarget]:
+        """{diffusers module name: :class:`weights.LoraTarget`} for every Linear / Conv2d of the UNet whose packed weight can take a LoRA
+        delta in place (every one of them: the norms are the only parameters left out)."""
+        out: Dict[str, LoraTarget] = {}
+        self.enc.lora_targets(out)
+        for i, blk in enumerate(self.up):
+            for j, r in enumerate(blk["res"]):
+                r.lora_targets(f"up_blocks.{i}.resnets.{j}", self.enc.temb_w, out)
+                if blk["attn"]:
+                    blk["attn"][j].lora_targets(f"up_blocks.{i}.attentions.{j}", self.enc.kv_w, out)
+            if blk["up"] is not None:
+                u = blk["up"][0]
+                out[f"up_blocks.{i}.upsamplers.0.conv"] = LoraTarget("up2x", u, u.shape[1], u.shape[2] // 4)
+        out["conv_out"] = LoraTarget("conv3", self.conv_out[0], self.cfg.out_channels, self.conv_out[0].shape[1] // 9)
+        return out
 
     def forward(self, x: Tensor, t: float, prompt_state, down_res: Optional[List[Tensor]] = None, mid_res: Optional[Tensor] = None,
                 nctx: int = 77, merge=None) -> Tensor:

@@ -14,6 +14,7 @@ from typing import Dict, List, Optional, Tuple
 import torch
 
 from . import ops
+from .weights import LoraTarget
 
 Tensor = torch.Tensor
 
@@ -82,6 +83,7 @@ class CLIPTextEncoder:
         if cfg.hidden_size % 64 or cfg.hidden_size // cfg.num_heads != 64:
             raise ValueError("CLIPTextEncoder: head_dim must be 64")
         self.cfg, self.dev = cfg, torch.device(device)
+        self.param_names = list(params)
         h16 = lambda k: params[k].to(self.dev, torch.float16).contiguous()
         f32 = lambda k: params[k].to(self.dev, torch.float32).contiguous()
         self.tok, self.pos = h16("text_model.embeddings.token_embedding.weight"), h16("text_model.embeddings.position_embedding.weight")
@@ -97,6 +99,20 @@ class CLIPTextEncoder:
         self.lnf = (f32("text_model.final_layer_norm.weight"), f32("text_model.final_layer_norm.bias"))
         self.proj = h16("text_projection.weight") if cfg.projection_dim else None
         self.act = ops.ACT_QUICKGELU if cfg.hidden_act == "quick_gelu" else ops.ACT_GELU
+
+    def lora_targets(self) -> Dict[str, LoraTarget]:
+        """{transformers module name: :class:`weights.LoraTarget`} of the projections a text-encoder LoRA adapts (plain rows; q/k/v fused)."""
+        c, out = self.cfg.hidden_size, {}
+        for i, L in enumerate(self.layers):
+            pre = f"text_model.encoder.layers.{i}."
+            for j, n in enumerate(("q_proj", "k_proj", "v_proj")):
+                out[pre + "self_attn." + n] = LoraTarget("rows", L["wqkv"], c, c, row0=j * c)
+            out[pre + "self_attn.out_proj"] = LoraTarget("rows", L["wo"], c, c)
+            out[pre + "mlp.fc1"] = LoraTarget("rows", L["w1"], self.cfg.intermediate_size, c)
+            out[pre + "mlp.fc2"] = LoraTarget("rows", L["w2"], c, self.cfg.intermediate_size)
+        if self.proj is not None:
+            out["text_projection"] = LoraTarget("rows", self.proj, self.cfg.projection_dim, c)
+        return out
 
     @torch.no_grad()
     def forward(self, ids: Tensor) -> Tuple[Tensor, Tensor, Optional[Tensor]]:

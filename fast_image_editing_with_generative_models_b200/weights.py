@@ -8,6 +8,7 @@ runs at load time), on CPU tensors plain torch ops (``EditEngine(pack_on_host=Tr
 VAE; ``fie_pack_*_bf16``)."""
 from __future__ import annotations
 
+from dataclasses import dataclass
 from typing import Optional, Tuple
 
 import torch
@@ -56,8 +57,17 @@ def pack_conv3x3(w: torch.Tensor, pad_cout_to: Optional[int] = None, pad_cin_to:
         with torch.cuda.device(w.device):
             _lib.check(getattr(_lib.lib(), fn)(w.data_ptr(), out.data_ptr(), cout, cin, op, cp, _stream(w)), fn)
         return out
-    out = torch.zeros((op, 3, 3, cp), dtype=dtype, device=w.device)
-    out[:cout, :, :, :cin] = w.permute(0, 2, 3, 1).to(dtype)
+    return conv3x3_layout(w, op, cp).to(dtype)
+
+
+def conv3x3_layout(w: torch.Tensor, pad_cout_to: Optional[int] = None, pad_cin_to: Optional[int] = None) -> torch.Tensor:
+    """The K order of :func:`pack_conv3x3` in the element type of ``w``: [Cout, Cin, 3, 3] -> [Cout_p, 9*Cin_p], (kh, kw, cin).
+    Linear in ``w``, so it is also the LoRA factor transform: conv3x3_layout(A) of A [r, Cin, 3, 3] gives the rows whose product with B
+    [Cout, r] is the packed delta."""
+    cout, cin = w.shape[:2]
+    op, cp = pad_cout_to or cout, pad_cin_to or cin
+    out = torch.zeros((op, 3, 3, cp), dtype=w.dtype, device=w.device)
+    out[:cout, :, :, :cin] = w.permute(0, 2, 3, 1)
     return out.reshape(op, 9 * cp).contiguous()
 
 
@@ -83,6 +93,13 @@ def pack_conv3x3_c8(w: torch.Tensor, pad_cout_to: Optional[int] = None) -> torch
     return out.reshape(op, 3 * 2 * 64).contiguous()
 
 
+def unpack_conv3x3_c8(packed: torch.Tensor, cout: int, cin: int) -> torch.Tensor:
+    """Inverse of :func:`pack_conv3x3_c8`: fp16 [Cout_p, 384] -> fp32 [cout, cin, 3, 3] = hi + lo (exact in fp32).  The hi/lo split is
+    not linear in the weight, so a LoRA delta on this layer is added here and the sum packed again."""
+    p = packed.float().reshape(packed.shape[0], 3, 2, 8, 8)[:cout, :, :, :3, :cin]       # [co][kh][hi|lo][kw][c]
+    return (p[:, :, 0] + p[:, :, 1]).permute(0, 3, 1, 2).contiguous()
+
+
 def pack_conv_up2x(w: torch.Tensor, dtype=torch.float16) -> torch.Tensor:
     """[Cout, Cin, 3, 3] -> fp16 (or bf16) [4, Cout, 4*Cin]: phase (a, b) weights of nearest-2x-upsample + conv3x3.
     Output row 2i+a reads input rows {i-1, i} (a = 0) or {i, i+1} (a = 1); the 3x3 taps that fall on the same input row are
@@ -96,7 +113,12 @@ def pack_conv_up2x(w: torch.Tensor, dtype=torch.float16) -> torch.Tensor:
         with torch.cuda.device(w.device):
             _lib.check(getattr(_lib.lib(), fn)(w.data_ptr(), out.data_ptr(), cout, cin, _stream(w)), fn)
         return out
-    w = w.float()
+    return conv_up2x_layout(w.float()).to(dtype).contiguous()
+
+
+def conv_up2x_layout(w: torch.Tensor) -> torch.Tensor:
+    """The phase filters of :func:`pack_conv_up2x` in the element type of ``w``: [Cout, Cin, 3, 3] -> [4, Cout, 4*Cin].  Linear in
+    ``w``: for a LoRA A [r, Cin, 3, 3] it gives the four phase-summed factors [4, r, 4*Cin] (one product B A'' per phase)."""
     rows = {0: [w[:, :, 0], w[:, :, 1] + w[:, :, 2]], 1: [w[:, :, 0] + w[:, :, 1], w[:, :, 2]]}   # each [Cout, Cin, 3(kw)]
     out = []
     for a in (0, 1):
@@ -107,20 +129,24 @@ def pack_conv_up2x(w: torch.Tensor, dtype=torch.float16) -> torch.Tensor:
                 cols = [r[:, :, 0], r[:, :, 1] + r[:, :, 2]] if b == 0 else [r[:, :, 0] + r[:, :, 1], r[:, :, 2]]
                 taps += cols                                   # (ty, tx) order, each [Cout, Cin]
             out.append(torch.stack(taps, dim=1).reshape(w.shape[0], -1))
-    return torch.stack(out, 0).to(dtype).contiguous()
+    return torch.stack(out, 0).contiguous()
 
 
 def pack_geglu(w: torch.Tensor, b: Optional[torch.Tensor]) -> Tuple[torch.Tensor, Optional[torch.Tensor]]:
     """GEGLU projection [8C, C] (value rows first, gate rows second) -> rows interleaved per accumulator tile:
     tile j = [value rows j*h..(j+1)*h | gate rows 4C+j*h..], h = fie_geglu_block_n(8C)/2."""
-    n = w.shape[0]
-    half = n // 2
-    h = _lib.lib().fie_geglu_block_n(n) // 2
-    assert half % h == 0
-    idx = torch.arange(n, device=w.device).view(2, half // h, h).permute(1, 0, 2).reshape(-1)
+    idx = geglu_rows(w.shape[0], w.device)
     wp = w.index_select(0, idx).contiguous()
     bp = None if b is None else b.index_select(0, idx).float().contiguous()
     return wp, bp
+
+
+def geglu_rows(n: int, device=None) -> torch.Tensor:
+    """Row order of :func:`pack_geglu` for N = 8C rows: packed row i is source row idx[i] (also the row order of a LoRA B factor)."""
+    half = n // 2
+    h = _lib.lib().fie_geglu_block_n(n) // 2
+    assert half % h == 0
+    return torch.arange(n, device=device).view(2, half // h, h).permute(1, 0, 2).reshape(-1)
 
 
 def fold_layernorm(w: torch.Tensor, b: Optional[torch.Tensor], gamma: torch.Tensor, beta: Optional[torch.Tensor]):
@@ -141,12 +167,41 @@ def fold_layernorm(w: torch.Tensor, b: Optional[torch.Tensor], gamma: torch.Tens
                                                          None if be32 is None else be32.data_ptr(), w16.data_ptr(), bias.data_ptr(), n, k, _stream(w)),
                        "fie_fold_layernorm_f16")
         return w16, bias
-    w32 = w.float() * gamma.float()[None, :]
-    w16 = (w32 - w32.mean(dim=1, keepdim=True)).to(torch.float16).contiguous()
+    w16 = _centre_rows(w.float() * gamma.float()[None, :]).to(torch.float16).contiguous()
     bias = torch.zeros(w.shape[0], dtype=torch.float32, device=w.device) if b is None else b.float().clone()
     if beta is not None:
         bias = bias + w.float() @ beta.float()
     return w16, bias.contiguous()
+
+
+def _centre_rows(w: torch.Tensor) -> torch.Tensor:
+    return w - w.mean(dim=1, keepdim=True)
+
+
+def fold_layernorm_lora(a: torch.Tensor, gamma: torch.Tensor, beta: Optional[torch.Tensor]):
+    """LoRA factor transform of :func:`fold_layernorm`: for a delta B A of W, the folded weight changes by B A'' with
+    A'' = centre_rows(A (.) gamma) (centring over K commutes with the product by B) and the bias by B (A beta).
+    Returns (A'' [r, K], A beta [r] or None) in the element type of ``a``."""
+    ag = _centre_rows(a * gamma.to(a)[None, :])
+    return ag, (None if beta is None else a @ beta.to(a))
+
+
+@dataclass
+class LoraTarget:
+    """Where the packed form of one diffusers Linear / Conv2d lives, for applying LoRA deltas in place.
+
+    kind: "rows" (packed weight rows = the module's output rows, K as in the source), "conv3" (:func:`conv3x3_layout`), "up2x"
+    (:func:`conv_up2x_layout`, ``weight`` [4, Cout, 4 Cin]) or "c8" (:func:`pack_conv3x3_c8`, rebuilt from hi + lo + delta).
+    The module's rows are ``weight[row0:row0 + out]``; ``ln`` = (gamma, beta): the LayerNorm folded by :func:`fold_layernorm` (then
+    ``bias`` is the fp32 folded bias and changes too); ``perm``: the :func:`geglu_rows` order of the whole buffer."""
+    kind: str
+    weight: torch.Tensor
+    out: int
+    inp: int
+    row0: int = 0
+    ln: Optional[Tuple[torch.Tensor, Optional[torch.Tensor]]] = None
+    bias: Optional[torch.Tensor] = None
+    perm: Optional[torch.Tensor] = None
 
 
 def fuse_lora(w: torch.Tensor, lora_a: torch.Tensor, lora_b: torch.Tensor, scale: float) -> torch.Tensor:

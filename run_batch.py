@@ -65,6 +65,7 @@ def build_parser():
                    "(the files are byte-identical either way)")
     add_checkpoint_args(p)
     add_size_arg(p)
+    add_lora_arg(p)
     return p
 
 
@@ -97,6 +98,37 @@ def add_checkpoint_args(p):
     p.add_argument("--lcm_lora", type=str, default=None, help="LCM-LoRA safetensors file (SDXL)")
     p.add_argument("--vae_dtype", choices=("auto", "fp16", "bf16"), default="auto",
                    help="VAE storage type: auto = bf16 if the VAE config.json says force_upcast: true (e.g. stabilityai/sdxl-vae), else fp16")
+
+
+def parse_lora(text: str):
+    """--lora PATH[=WEIGHT] -> (path, weight); the weight defaults to 1.0."""
+    path, sep, w = text.rpartition("=")
+    if sep:
+        try:
+            return path, float(w)
+        except ValueError:
+            pass
+    return text, 1.0
+
+
+def add_lora_arg(p):
+    p.add_argument("--lora", type=parse_lora, action="append", default=[], metavar="PATH[=WEIGHT]",
+                   help="style LoRA (.safetensors file or folder), repeatable: loaded after the editor is built and active next to the "
+                        "LCM-LoRA at WEIGHT (default 1.0); editor.pipe.load_lora_weights / set_adapters")
+
+
+def apply_lora_args(editor, args):
+    """Loads every --lora adapter and activates them, at their weights, next to the adapters the editor was built with."""
+    if not args.lora:
+        return
+    names = editor.pipe.get_active_adapters()
+    weights = [1.0] * len(names)
+    for i, (path, w) in enumerate(args.lora):
+        name = f"lora_{i}"
+        editor.pipe.load_lora_weights(path, adapter_name=name)
+        names.append(name)
+        weights.append(w)
+    editor.pipe.set_adapters(names, weights)
 
 
 def vae_dtype_from_args(args):
@@ -169,6 +201,7 @@ def main(argv=None):
                         checkpoints=checkpoints_from_args(args), vae_dtype=vae_dtype_from_args(args))
     if hasattr(editor, "pipe"):
         editor.pipe.set_progress_bar_config(disable=True)
+    apply_lora_args(editor, args)
     processed = skipped = failed = 0
     total_time = 0.0
     # ---- per-entry admission (the reference's checks, run_batch.py:185-207), then micro-batches of --micro_batch images ----

@@ -12,7 +12,7 @@ from datetime import datetime
 
 from PIL import Image
 
-from run_batch import checkpoints_from_args, vae_dtype_from_args
+from run_batch import apply_lora_args, checkpoints_from_args, vae_dtype_from_args
 from src.pipeline import FastEditor
 
 
@@ -36,8 +36,9 @@ def build_parser():
     p.add_argument("--full_controlnet", action="store_true")
     p.add_argument("--compute_metrics", action="store_true")
     p.add_argument("--show_plot", action="store_true")
-    from run_batch import add_checkpoint_args, add_size_arg
+    from run_batch import add_checkpoint_args, add_lora_arg, add_size_arg
     add_checkpoint_args(p)
+    add_lora_arg(p)
     add_size_arg(p)
     return p
 
@@ -72,6 +73,7 @@ def main(argv=None):
     editor = FastEditor(model_name=args.model, device="cuda", enable_cpu_offload=not args.no_cpu_offload,
                         use_full_precision=args.full_precision, use_full_controlnet=args.full_controlnet,
                         checkpoints=checkpoints_from_args(args), vae_dtype=vae_dtype_from_args(args))
+    apply_lora_args(editor, args)
     mem = editor.get_memory_usage()
     print(f"      GPU Memory: {mem['allocated_gb']:.2f}GB allocated, {mem['reserved_gb']:.2f}GB reserved")
     print("\n[3/4] Running image editing...")
