@@ -52,13 +52,10 @@ SIGNATURES = {
     "fie_im2col3x3_f16": (c_int, [c_void_p, c_int, c_ll, c_void_p, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_void_p]),
     "fie_maxpool3s2_ceil_f16": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p]),
     "fie_lpips_layer_f16": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_ll, c_int, c_void_p, c_void_p]),
-    "fie_preprocess_u8_to_f16": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p]),
     "fie_preprocess_u8_to_f16_pad8": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p]),
     "fie_pad8_f16": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_void_p]),
     "fie_postprocess_f16_to_u8": (c_int, [c_void_p, c_int, c_void_p, c_int, c_int, c_int, c_void_p]),
-    "fie_add_f16": (c_int, [c_void_p, c_void_p, c_void_p, c_ll, c_void_p]),
     "fie_silu_f16": (c_int, [c_void_p, c_void_p, c_ll, c_void_p]),
-    "fie_upsample2x_f16": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p]),
     "fie_sincos_embedding": (c_int, [ctypes.POINTER(c_float), c_int, c_int, c_void_p, c_void_p]),
     "fie_softmax_rows_f32_to_f16": (c_int, [c_void_p, c_ll, c_void_p, c_ll, c_ll, c_int, c_float, c_void_p]),
     "fie_softmax_rows_f16": (c_int, [c_void_p, c_ll, c_void_p, c_ll, c_ll, c_int, c_float, c_void_p]),
@@ -87,7 +84,6 @@ SIGNATURES = {
     "fie_attention_d64_f16": (c_int, [c_void_p, c_ll, c_void_p, c_ll, c_void_p, c_ll, c_void_p, c_ll, c_int, c_int, c_int, c_int, c_float, c_void_p]),
     "fie_attention_d64_causal_f16": (c_int, [c_void_p, c_ll, c_void_p, c_ll, c_void_p, c_ll, c_void_p, c_ll, c_int, c_int, c_int, c_int, c_float, c_void_p]),
     "fie_embed_tokens_f16": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_ll, c_int, c_int, c_int, c_void_p]),
-    "fie_vae_sample_add_noise": (c_int, [c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_ll, c_float, c_float, c_float, c_void_p]),
     "fie_gemm_bf16": (c_int, [c_void_p, c_ll, c_void_p, c_ll, c_int, c_void_p, c_void_p, c_ll, c_ll, c_int, c_int, ctypes.POINTER(Epilogue), c_int, c_void_p]),
     "fie_conv3x3_bf16": (c_int, [c_void_p, c_void_p, c_void_p, c_ll, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int, ctypes.POINTER(Epilogue), c_int,
                                  c_void_p]),
@@ -101,7 +97,6 @@ SIGNATURES = {
     "fie_pack_conv3x3_bf16": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p]),
     "fie_pack_conv_up2x_bf16": (c_int, [c_void_p, c_void_p, c_int, c_int, c_void_p]),
     "fie_pack_rows_bf16": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_void_p]),
-    "fie_cfg_lcm_step":(c_int, [c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_ll] + [c_float] * 7 + [c_int, c_void_p]),
     "fie_canny_u8_per_image": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p, c_void_p, c_size_t, c_void_p]),
     "fie_sincos_embedding_dev": (c_int, [c_void_p, c_int, c_int, c_void_p, c_void_p]),
     "fie_gemm_f16_ex": (c_int, [c_void_p, c_ll, c_void_p, c_ll, c_int, c_void_p, c_void_p, c_ll, c_ll, c_int, c_int, ctypes.POINTER(Epilogue), c_void_p,

@@ -1,5 +1,4 @@
-// Memory-bound helper kernels: pre/post-processing, residual adds, nearest upsample, sinusoidal embedding,
-// row softmax, VAE posterior sample + add_noise, fused CFG + LCMScheduler.step.
+// Memory-bound helper kernels: pre/post-processing, sinusoidal embedding, row softmax, VAE posterior sample + add_noise, fused CFG + LCMScheduler.step.
 // All use 128-bit accesses where the layout allows and grid-stride loops sized to the SM count.
 #include "fie_common.cuh"
 
@@ -11,25 +10,9 @@ static inline int grid_for(long long work_items, int block) {
     return (int)(b < 1 ? 1 : (b > cap ? cap : b));
 }
 
-// ---- VaeImageProcessor.preprocess: u8 HWC -> fp16 NHWC (x/127.5 - 1 computed as 2*(x/255)-1 in fp32) ----
-__global__ void __launch_bounds__(256) k_pre(const uint8_t* __restrict__ in, __half* __restrict__ out, long long npix, int c_out, int normalize) {
-    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < npix; i += (long long)gridDim.x * blockDim.x) {
-        float v[3];
-#pragma unroll
-        for (int c = 0; c < 3; ++c) { float x = (float)in[i * 3 + c] / 255.0f; v[c] = normalize ? 2.0f * x - 1.0f : x; }
-        __half* o = out + i * c_out;
-        if (c_out == 4) {
-            __half2 a = __floats2half2_rn(v[0], v[1]), b = __floats2half2_rn(v[2], 0.0f);
-            uint2 u; u.x = *reinterpret_cast<uint32_t*>(&a); u.y = *reinterpret_cast<uint32_t*>(&b);
-            *reinterpret_cast<uint2*>(o) = u;
-        } else {
-            for (int c = 0; c < c_out; ++c) o[c] = __float2half_rn(c < 3 ? v[c] : 0.0f);
-        }
-    }
-}
-
-// Same conversion into the zero-padded 8-channel layout [n][h+2][w+8][8] the tensor-core conv_in reads (real pixel (y, x) at
-// (y+1, x+1)); one thread writes one 16-byte padded pixel, borders and channels 3..7 as zeros.
+// ---- VaeImageProcessor.preprocess: u8 HWC (x/127.5 - 1 computed as 2*(x/255)-1 in fp32) -> fp16 in the zero-padded 8-channel
+// layout [n][h+2][w+8][8] the tensor-core conv_in reads (real pixel (y, x) at (y+1, x+1)); one thread writes one 16-byte padded
+// pixel, borders and channels 3..7 as zeros.
 __global__ void __launch_bounds__(256) k_pre_pad8(const uint8_t* __restrict__ in, uint4* __restrict__ out, int n, int h, int w, int normalize) {
     const int wp = w + 8, hp = h + 2;
     const long long total = (long long)n * hp * wp;
@@ -74,17 +57,6 @@ __global__ void __launch_bounds__(256) k_post(const __half* __restrict__ in, int
     }
 }
 
-__global__ void __launch_bounds__(256) k_add(const uint4* __restrict__ a, const uint4* __restrict__ b, uint4* __restrict__ o, long long n8) {
-    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n8; i += (long long)gridDim.x * blockDim.x) {
-        uint4 x = __ldg(a + i), y = __ldg(b + i), r;
-        const __half2* xh = reinterpret_cast<const __half2*>(&x); const __half2* yh = reinterpret_cast<const __half2*>(&y);
-        __half2* rh = reinterpret_cast<__half2*>(&r);
-#pragma unroll
-        for (int j = 0; j < 4; ++j) { float2 fa = __half22float2(xh[j]), fb = __half22float2(yh[j]); rh[j] = __floats2half2_rn(fa.x + fb.x, fa.y + fb.y); }
-        o[i] = r;
-    }
-}
-
 __global__ void __launch_bounds__(256) k_silu(const uint4* __restrict__ a, uint4* __restrict__ o, long long n8) {
     for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n8; i += (long long)gridDim.x * blockDim.x) {
         uint4 x = __ldg(a + i), r;
@@ -92,16 +64,6 @@ __global__ void __launch_bounds__(256) k_silu(const uint4* __restrict__ a, uint4
 #pragma unroll
         for (int j = 0; j < 4; ++j) { float2 f = __half22float2(xh[j]); rh[j] = __floats2half2_rn(silu_f(f.x), silu_f(f.y)); }
         o[i] = r;
-    }
-}
-
-__global__ void __launch_bounds__(256) k_up2x(const uint4* __restrict__ x, uint4* __restrict__ o, int n, int h, int w, int c8) {
-    const long long total = (long long)n * 2 * h * 2 * w * c8;
-    for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (long long)gridDim.x * blockDim.x) {
-        int cv = (int)(i % c8); long long t = i / c8;
-        int ox = (int)(t % (2 * w)); t /= (2 * w);
-        int oy = (int)(t % (2 * h)); int img = (int)(t / (2 * h));
-        o[i] = __ldg(x + (((long long)img * h + (oy >> 1)) * w + (ox >> 1)) * c8 + cv);
     }
 }
 
@@ -277,13 +239,13 @@ __global__ void __launch_bounds__(256) k_softmax_rows(const T* __restrict__ s, l
 // z0 = (mean + exp(0.5*clamp(logvar,-30,20))*xi)*scaling ; x = sqrt_a*z0 + sqrt_1ma*noise.  The latent STATE is kept in fp32
 // across the scheduler steps (out32); out16 is the fp16 copy the UNet / ControlNet read.  (diffusers keeps the state in the model
 // dtype; the fp32 state removes one fp16 rounding of |x| <= 16, i.e. up to 4e-3, per step from the final latents.)
-// coef: per-image (sqrt_a, sqrt_1ma) [npx / px_per_img] in device memory, or NULL -> the by-value sa, s1.
+// coef: per-image (sqrt_a, sqrt_1ma) [npx / px_per_img] in device memory.
 __global__ void __launch_bounds__(256) k_vae_sample(const __half* __restrict__ mom, int ld_m, const __half* __restrict__ xi, const __half* __restrict__ noise,
-                                                    float* __restrict__ out32, __half* __restrict__ out16, long long npx, float scaling, float sa, float s1,
+                                                    float* __restrict__ out32, __half* __restrict__ out16, long long npx, float scaling,
                                                     const float2* __restrict__ coef, long long px_per_img) {
     for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < npx * 4; i += (long long)gridDim.x * blockDim.x) {
         long long px = i >> 2; int c = (int)(i & 3);
-        if (coef) { const float2 k = __ldg(coef + px / px_per_img); sa = k.x; s1 = k.y; }
+        const float2 k = __ldg(coef + px / px_per_img); const float sa = k.x, s1 = k.y;
         const float mean = __half2float(mom[px * ld_m + c]);
         const float logvar = fminf(fmaxf(__half2float(mom[px * ld_m + 4 + c]), -30.0f), 20.0f);
         const float z = (mean + expf(0.5f * logvar) * __half2float(xi[i])) * scaling;
@@ -293,15 +255,12 @@ __global__ void __launch_bounds__(256) k_vae_sample(const __half* __restrict__ m
 }
 
 __global__ void __launch_bounds__(256) k_cfg_lcm(const __half* __restrict__ eu, const __half* __restrict__ ec, int ld_e, const float* __restrict__ x,
-                                                 const __half* __restrict__ noise, float* __restrict__ out32, __half* __restrict__ out16, long long npx, float g,
-                                                 float sa, float s1, float c_skip, float c_out, float sap, float s1p, int last,
-                                                 const float* __restrict__ coef, long long px_per_img) {
+                                                 const __half* __restrict__ noise, float* __restrict__ out32, __half* __restrict__ out16, long long npx,
+                                                 int last, const float* __restrict__ coef, long long px_per_img) {
     for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < npx * 4; i += (long long)gridDim.x * blockDim.x) {
         long long px = i >> 2; int c = (int)(i & 3);
-        if (coef) {                                     // per-image (g, sa, s1, c_skip, c_out, sap, s1p) [npx / px_per_img][7]
-            const float* k = coef + (px / px_per_img) * 7;
-            g = __ldg(k); sa = __ldg(k + 1); s1 = __ldg(k + 2); c_skip = __ldg(k + 3); c_out = __ldg(k + 4); sap = __ldg(k + 5); s1p = __ldg(k + 6);
-        }
+        const float* k = coef + (px / px_per_img) * 7;  // per-image (g, sa, s1, c_skip, c_out, sap, s1p) [npx / px_per_img][7]
+        const float g = __ldg(k), sa = __ldg(k + 1), s1 = __ldg(k + 2), c_skip = __ldg(k + 3), c_out = __ldg(k + 4), sap = __ldg(k + 5), s1p = __ldg(k + 6);
         float u = __half2float(eu[px * ld_e + c]), cc = __half2float(ec[px * ld_e + c]);
         float eps = u + g * (cc - u);
         float xv = x[i];
@@ -336,12 +295,6 @@ extern "C" int fie_embed_tokens_f16(const int* ids, const void* tok, const void*
     return check_launch("fie_embed_tokens_f16");
 }
 
-extern "C" int fie_preprocess_u8_to_f16(const void* img, void* out, int n, int h, int w, int c_out, int normalize, void* stream) {
-    FIE_REQUIRE(img && out && n > 0 && h > 0 && w > 0 && c_out >= 3, "fie_preprocess_u8_to_f16: bad args");
-    long long npix = (long long)n * h * w;
-    k_pre<<<grid_for(npix, 256), 256, 0, (cudaStream_t)stream>>>((const uint8_t*)img, (__half*)out, npix, c_out, normalize);
-    return check_launch("fie_preprocess_u8_to_f16");
-}
 extern "C" int fie_preprocess_u8_to_f16_pad8(const void* img, void* out, int n, int h, int w, int normalize, void* stream) {
     FIE_REQUIRE(img && out && n > 0 && h > 0 && w > 0, "fie_preprocess_u8_to_f16_pad8: bad args");
     const long long total = (long long)n * (h + 2) * (w + 8);
@@ -360,21 +313,10 @@ extern "C" int fie_postprocess_f16_to_u8(const void* x, int ld, void* out, int n
     k_post<<<grid_for(npix, 256), 256, 0, (cudaStream_t)stream>>>((const __half*)x, ld, (uint8_t*)out, npix);
     return check_launch("fie_postprocess_f16_to_u8");
 }
-extern "C" int fie_add_f16(const void* a, const void* b, void* out, long long count, void* stream) {
-    FIE_REQUIRE(a && b && out && count > 0 && (count % 8) == 0, "fie_add_f16: count must be a positive multiple of 8");
-    k_add<<<grid_for(count / 8, 256), 256, 0, (cudaStream_t)stream>>>((const uint4*)a, (const uint4*)b, (uint4*)out, count / 8);
-    return check_launch("fie_add_f16");
-}
 extern "C" int fie_silu_f16(const void* a, void* out, long long count, void* stream) {
     FIE_REQUIRE(a && out && count > 0 && (count % 8) == 0, "fie_silu_f16: count must be a positive multiple of 8");
     k_silu<<<grid_for(count / 8, 256), 256, 0, (cudaStream_t)stream>>>((const uint4*)a, (uint4*)out, count / 8);
     return check_launch("fie_silu_f16");
-}
-extern "C" int fie_upsample2x_f16(const void* x, void* out, int n, int h, int w, int c, void* stream) {
-    FIE_REQUIRE(x && out && n > 0 && h > 0 && w > 0 && c > 0 && (c % 8) == 0, "fie_upsample2x_f16: c must be a multiple of 8");
-    long long total = (long long)n * 4 * h * w * (c / 8);
-    k_up2x<<<grid_for(total, 256), 256, 0, (cudaStream_t)stream>>>((const uint4*)x, (uint4*)out, n, h, w, c / 8);
-    return check_launch("fie_upsample2x_f16");
 }
 extern "C" int fie_sincos_embedding(const float* host_vals, int count, int dim, void* out, void* stream) {
     FIE_REQUIRE(host_vals && out && count > 0 && count <= 64 && dim > 0 && (dim % 2) == 0, "fie_sincos_embedding: bad args");
@@ -412,37 +354,19 @@ extern "C" int fie_softmax_rows_exp_f16(const void* s, long long ld_in, void* p,
     k_softmax_rows_exp<16><<<(unsigned)rows, 256, 0, (cudaStream_t)stream>>>((const __half*)s, ld_in, (__half*)p, ld_out, inv_sum, cols, scale);
     return check_launch("fie_softmax_rows_exp_f16");
 }
-extern "C" int fie_vae_sample_add_noise(const void* moments, int ld_m, const void* xi, const void* noise, float* x_out_f32, void* x_out_f16,
-                                        long long count_px, float scaling, float sqrt_a, float sqrt_1ma, void* stream) {
-    FIE_REQUIRE(moments && xi && noise && x_out_f32 && x_out_f16 && count_px > 0 && ld_m >= 8, "fie_vae_sample_add_noise: bad args");
-    k_vae_sample<<<grid_for(count_px * 4, 256), 256, 0, (cudaStream_t)stream>>>((const __half*)moments, ld_m, (const __half*)xi, (const __half*)noise,
-                                                                                x_out_f32, (__half*)x_out_f16, count_px, scaling, sqrt_a, sqrt_1ma, nullptr, 1);
-    return check_launch("fie_vae_sample_add_noise");
-}
 extern "C" int fie_vae_sample_add_noise_batched(const void* moments, int ld_m, const void* xi, const void* noise, float* x_out_f32, void* x_out_f16,
                                                 long long count_px, long long px_per_img, float scaling, const float* coef, void* stream) {
     FIE_REQUIRE(moments && xi && noise && x_out_f32 && x_out_f16 && coef && count_px > 0 && px_per_img > 0 && (count_px % px_per_img) == 0 && ld_m >= 8,
                 "fie_vae_sample_add_noise_batched: bad args");
     k_vae_sample<<<grid_for(count_px * 4, 256), 256, 0, (cudaStream_t)stream>>>((const __half*)moments, ld_m, (const __half*)xi, (const __half*)noise,
-                                                                                x_out_f32, (__half*)x_out_f16, count_px, scaling, 0.f, 0.f,
-                                                                                (const float2*)coef, px_per_img);
+                                                                                x_out_f32, (__half*)x_out_f16, count_px, scaling, (const float2*)coef, px_per_img);
     return check_launch("fie_vae_sample_add_noise_batched");
-}
-extern "C" int fie_cfg_lcm_step(const void* eps_u, const void* eps_c, int ld_e, const float* x_f32, const void* noise, float* x_out_f32, void* x_out_f16,
-                                long long count_px, float guidance, float sqrt_a, float sqrt_1ma, float c_skip, float c_out,
-                                float sqrt_a_prev, float sqrt_1ma_prev, int last, void* stream) {
-    FIE_REQUIRE(eps_u && eps_c && x_f32 && x_out_f32 && x_out_f16 && count_px > 0 && ld_e >= 4 && (last || noise), "fie_cfg_lcm_step: bad args");
-    k_cfg_lcm<<<grid_for(count_px * 4, 256), 256, 0, (cudaStream_t)stream>>>((const __half*)eps_u, (const __half*)eps_c, ld_e, x_f32,
-                                                                              (const __half*)noise, x_out_f32, (__half*)x_out_f16, count_px, guidance, sqrt_a, sqrt_1ma,
-                                                                              c_skip, c_out, sqrt_a_prev, sqrt_1ma_prev, last, nullptr, 1);
-    return check_launch("fie_cfg_lcm_step");
 }
 extern "C" int fie_cfg_lcm_step_batched(const void* eps_u, const void* eps_c, int ld_e, const float* x_f32, const void* noise, float* x_out_f32, void* x_out_f16,
                                         long long count_px, long long px_per_img, const float* coef, int last, void* stream) {
     FIE_REQUIRE(eps_u && eps_c && x_f32 && x_out_f32 && x_out_f16 && coef && count_px > 0 && px_per_img > 0 && (count_px % px_per_img) == 0 && ld_e >= 4 &&
                 (last || noise), "fie_cfg_lcm_step_batched: bad args");
     k_cfg_lcm<<<grid_for(count_px * 4, 256), 256, 0, (cudaStream_t)stream>>>((const __half*)eps_u, (const __half*)eps_c, ld_e, x_f32,
-                                                                              (const __half*)noise, x_out_f32, (__half*)x_out_f16, count_px, 0.f, 0.f, 0.f,
-                                                                              0.f, 0.f, 0.f, 0.f, last, coef, px_per_img);
+                                                                              (const __half*)noise, x_out_f32, (__half*)x_out_f16, count_px, last, coef, px_per_img);
     return check_launch("fie_cfg_lcm_step_batched");
 }

@@ -34,7 +34,7 @@ from PIL import Image
 from . import model_zoo, ops
 from . import synthetic as S
 from .lora import LoraAdapters
-from .pipeline import per_image
+from .pipeline import executed_steps, per_image_settings
 
 _ENV_KEYS = {"root": "FIE_CHECKPOINTS", "controlnet": "FIE_CONTROLNET", "vae": "FIE_VAE", "lora": "FIE_LCM_LORA"}
 
@@ -358,45 +358,6 @@ class FastEditor:
             edges = ops.canny(d, int(np.floor(low_threshold)), int(np.floor(high_threshold)), out_channels=3, gaussian_blur=gaussian_blur)
             return Image.fromarray(edges[0].cpu().numpy())
 
-    # ---- argument checks shared by edit / edit_many (diffusers img2img check_inputs + get_timesteps) ----
-    @staticmethod
-    def _executed_steps(strength: float, num_inference_steps: int) -> int:
-        if strength < 0 or strength > 1:
-            raise ValueError(f"The value of strength should in [0.0, 1.0] but is {strength}")
-        if not isinstance(num_inference_steps, int) or num_inference_steps <= 0:
-            raise ValueError(f"`num_inference_steps` has to be a positive integer but is {num_inference_steps}")
-        n_exec = min(int(num_inference_steps * strength), num_inference_steps)
-        if n_exec < 1:
-            raise ValueError(f"After adjusting the num_inference_steps by strength parameter: {strength}, the number of pipeline steps is "
-                             f"{n_exec} which is < 1 and not appropriate for this pipeline.")
-        return n_exec
-
-    @classmethod
-    def _per_image_settings(cls, n: int, strength, num_inference_steps, guidance_scale, controlnet_conditioning_scale, canny_low_threshold,
-                            canny_high_threshold) -> Dict[str, list]:
-        """edit_many's numeric settings, each a scalar or one value per image -> {name: list of n values} plus "n_exec", the denoising
-        steps each image executes.  ValueError (naming the image) for a wrong length, a non-finite value or an invalid strength / step
-        count."""
-        st = dict(strength=strength, num_inference_steps=num_inference_steps, guidance_scale=guidance_scale,
-                  controlnet_conditioning_scale=controlnet_conditioning_scale, canny_low_threshold=canny_low_threshold,
-                  canny_high_threshold=canny_high_threshold)
-        for name, v in st.items():
-            if name == "num_inference_steps" and not isinstance(v, (str, bytes)) and isinstance(v, (Sequence, np.ndarray)):
-                if len(v) != n:
-                    raise ValueError(f"num_inference_steps: {len(v)} values for {n} images")
-                st[name] = list(v)                     # kept as given: _executed_steps checks that each is an int
-            elif name == "num_inference_steps":
-                st[name] = [v] * n
-            else:
-                st[name] = per_image(name, v, n)
-        st["n_exec"] = []
-        for i in range(n):
-            try:
-                st["n_exec"].append(cls._executed_steps(st["strength"][i], st["num_inference_steps"][i]))
-            except ValueError as err:
-                raise ValueError(f"image {i}: {err}") from None
-        return st
-
     def _draw_noises(self, seed, n_exec: int, size=(OUT_SIZE, OUT_SIZE)) -> List[torch.Tensor]:
         """Reference RNG order for one image of ``size`` = (width, height): posterior sample, init noise, then one draw per non-final
         executed step, each [1, 4, height/8, width/8]."""
@@ -422,19 +383,12 @@ class FastEditor:
              controlnet_conditioning_scale=0.5, canny_low_threshold=100, canny_high_threshold=200, seed=None, *, canny_gaussian_blur=False,
              size=None):
         """Edit an image with a text prompt, preserving structure via Canny conditioning -> PIL RGB image of ``size`` (default
-        1024x1024; see :func:`resolve_size`)."""
-        wh = resolve_size(size, image.size)
-        n_exec = self._executed_steps(strength, num_inference_steps)
-        with torch.cuda.device(self._dev):
-            img = self._to_device(image, wh)
-            pe, pl = self._encode_prompt(prompt, negative_prompt)
-            noises = self._draw_noises(seed, n_exec, wh)
-            # per-image prompt layout [1,2,77,D], as edit_many passes it: warm_up(micro_batch=1) captures the graph edit() replays
-            out = self._engine.edit_batch(img, pe[None], pl[None], noises, strength=strength, num_inference_steps=num_inference_steps,
-                                          guidance_scale=guidance_scale, controlnet_conditioning_scale=controlnet_conditioning_scale,
-                                          canny_low=int(np.floor(canny_low_threshold)), canny_high=int(np.floor(canny_high_threshold)),
-                                          canny_blur=canny_gaussian_blur)
-            return Image.fromarray(out.images[0].cpu().numpy())
+        1024x1024; see :func:`resolve_size`).  One image through :meth:`edit_many`: warm_up(micro_batch=1) captures the graph it
+        replays."""
+        executed_steps(strength, num_inference_steps)         # diffusers' check_inputs / get_timesteps messages, naming no image
+        return self.edit_many([image], [prompt], [negative_prompt], strength, num_inference_steps, guidance_scale, controlnet_conditioning_scale,
+                              canny_low_threshold, canny_high_threshold, seeds=[seed], micro_batch=1, canny_gaussian_blur=canny_gaussian_blur,
+                              size=size)[0]
 
     def edit_many(self, images: Sequence, prompts: Union[str, Sequence[str]], negative_prompt: Union[str, Sequence[str]] = "", strength=0.80,
                   num_inference_steps=4, guidance_scale=1.5, controlnet_conditioning_scale=0.5, canny_low_threshold=100, canny_high_threshold=200,
@@ -470,8 +424,8 @@ class FastEditor:
             raise ValueError("edit_many: seeds must have one entry per image")
         if output not in ("pil", "jpeg"):
             raise ValueError("edit_many: output must be 'pil' or 'jpeg'")
-        st = self._per_image_settings(n, strength, num_inference_steps, guidance_scale, controlnet_conditioning_scale, canny_low_threshold,
-                                      canny_high_threshold)
+        st = per_image_settings(n, strength, num_inference_steps, guidance_scale, controlnet_conditioning_scale, canny_low_threshold,
+                                canny_high_threshold)
         mb = int(micro_batch or self.MICRO_BATCH)
         sizes = [resolve_size(size, im.size) for im in images]
         chunks = micro_batches(sizes, st["n_exec"], st["guidance_scale"], mb)

@@ -293,16 +293,13 @@ class _EncoderPart:
         aug = ops.gemm(h, self.a2[0], col_bias=self.a2[1])
         return ctx_kv, aug
 
-    def time_rows(self, t, aug: Tensor) -> Tensor:
-        """Per-step: fp32 [B, sum Cout] row biases (time_emb_proj(SiLU(emb)) + conv1.bias) for every resnet.  ``t``: one timestep for
-        every row, or an fp32 CUDA tensor [B] with the timestep of each row (read on the device: the edit's parameter block)."""
+    def time_rows(self, t: Tensor, aug: Tensor) -> Tensor:
+        """Per-step: fp32 [B, sum Cout] row biases (time_emb_proj(SiLU(emb)) + conv1.bias) for every resnet.  ``t``: an fp32 CUDA
+        tensor [B] with the timestep of each row (read on the device: the edit's parameter block)."""
         b = aug.shape[0]
-        if isinstance(t, Tensor):
-            if t.numel() != b:
-                raise ValueError(f"time_rows: {t.numel()} timesteps for {b} rows")
-            te = ops.sincos_embedding(t, self.cfg.block_out_channels[0], aug.device)
-        else:
-            te = ops.sincos_embedding([t], self.cfg.block_out_channels[0], aug.device).expand(b, -1).contiguous()
+        if t.numel() != b:
+            raise ValueError(f"time_rows: {t.numel()} timesteps for {b} rows")
+        te = ops.sincos_embedding(t, self.cfg.block_out_channels[0], aug.device)
         h = ops.gemm(te, self.t1[0], col_bias=self.t1[1], act=ops.ACT_SILU)
         emb = ops.gemm(h, self.t2[0], col_bias=self.t2[1], residual=aug)
         return ops.gemm(ops.silu(emb), self.temb_w, col_bias=self.temb_b, out_f32=True)
@@ -366,11 +363,10 @@ class UNet:
         out["conv_out"] = LoraTarget("conv3", self.conv_out[0], self.cfg.out_channels, self.conv_out[0].shape[1] // 9)
         return out
 
-    def forward(self, x: Tensor, t: float, prompt_state, down_res: Optional[List[Tensor]] = None, mid_res: Optional[Tensor] = None,
-                nctx: int = 77, merge=None) -> Tensor:
-        """x [B,H,W,4] fp16 -> eps [B,H,W,4] fp16 (UNet2DConditionModel.forward with ControlNet residuals).
-        The residuals come either as tensors (down_res, mid_res: added here) or through ``merge(skips, h) -> (skips, h)``
-        (ControlNet.merge_into: the zero-convolution GEMMs add this UNet's skip tensors in their epilogue -- no add kernels)."""
+    def forward(self, x: Tensor, t: Tensor, prompt_state, nctx: int = 77, merge=None) -> Tensor:
+        """x [B,H,W,4] fp16, t fp32 CUDA [B] per-row timesteps -> eps [B,H,W,4] fp16 (UNet2DConditionModel.forward with ControlNet
+        residuals).  The residuals come through ``merge(skips, h) -> (skips, h)`` (ControlNet.merge_into: the zero-convolution GEMMs
+        add this UNet's skip tensors in their epilogue -- no add kernels)."""
         ctx_kv, aug = prompt_state
         cfg = self.cfg
         temb = self.enc.time_rows(t, aug)
@@ -378,10 +374,6 @@ class UNet:
         h, skips = self.enc.down_mid(h, temb, ctx_kv, nctx)
         if merge is not None:
             skips, h = merge(skips, h)
-        if down_res is not None:
-            skips = [ops.add(s, r) for s, r in zip(skips, down_res)]
-        if mid_res is not None:
-            h = ops.add(h, mid_res)
         for blk in self.up:
             for j, r in enumerate(blk["res"]):
                 h = r(h, temb, skip=skips.pop())
@@ -422,38 +414,26 @@ class ControlNet:
             h = ops.conv3x3(h, w, stride=stride, pad_mode=0, col_bias=b, act=ops.ACT_SILU)
         return ops.conv3x3(h, self.cond_out[0], col_bias=self.cond_out[1])
 
-    def forward(self, x: Tensor, t: float, prompt_state, cond_emb: Tensor, scale: float, nctx: int = 77):
-        """-> (down residuals, mid residual), each already multiplied by the conditioning scale."""
+    def encode(self, x: Tensor, t: Tensor, prompt_state, cond_emb: Tensor, nctx: int = 77):
+        """The ControlNet up to (not including) its zero convolutions -> (skip features, mid feature); see merge_into.
+        t: fp32 CUDA [B] per-row timesteps."""
         ctx_kv, aug = prompt_state
         temb = self.enc.time_rows(t, aug)
         h = ops.conv3x3_c8(ops.pad8(x), self.enc.conv_in[0], col_bias=self.enc.conv_in[1], residual=cond_emb)     # conv_in(x) + conditioning embedding
-        h, skips = self.enc.down_mid(h, temb, ctx_kv, nctx)
-        down = [ops.gemm(s, w, col_bias=b, scale=scale) for s, (w, b) in zip(skips, self.zero)]
-        mid = ops.gemm(h, self.zero_mid[0], col_bias=self.zero_mid[1], scale=scale)
-        return down, mid
-
-    def encode(self, x: Tensor, t: float, prompt_state, cond_emb: Tensor, nctx: int = 77):
-        """The ControlNet up to (not including) its zero convolutions -> (skip features, mid feature); see merge_into."""
-        ctx_kv, aug = prompt_state
-        temb = self.enc.time_rows(t, aug)
-        h = ops.conv3x3_c8(ops.pad8(x), self.enc.conv_in[0], col_bias=self.enc.conv_in[1], residual=cond_emb)
         return self.enc.down_mid(h, temb, ctx_kv, nctx)
 
-    def merge_into(self, feats, scale):
+    def merge_into(self, feats, scale: Tensor):
         """-> merge(unet_skips, unet_h): every zero convolution writes scale * (W f + b) + <the UNet tensor it is added to> in one
         GEMM epilogue, i.e. `down_block_res_samples[i] + down_block_additional_residuals[i]` and the mid-block add of
         UNet2DConditionModel.forward without separate element-wise kernels (and with one rounding instead of two).
-        ``scale``: one conditioning scale, or an fp32 CUDA tensor with one per batch row (image and CFG half), read on the device as
-        the GEMMs' group_scale."""
+        ``scale``: an fp32 CUDA tensor with one conditioning scale per batch row (image and CFG half), read on the device as the
+        GEMMs' group_scale."""
         cn_h, cn_skips = feats
 
         def zero_conv(f, w, b, res):
             n_, hh, ww, c_ = res.shape
-            if isinstance(scale, Tensor):
-                kw = dict(group_scale=scale, rows_per_group=hh * ww)
-            else:
-                kw = dict(scale=scale)
-            return ops.gemm(f.view(-1, f.shape[-1]), w, col_bias=b, residual=res.view(-1, c_), **kw).view(res.shape)
+            return ops.gemm(f.view(-1, f.shape[-1]), w, col_bias=b, residual=res.view(-1, c_), group_scale=scale,
+                            rows_per_group=hh * ww).view(res.shape)
 
         def merge(skips, h):
             merged = [zero_conv(f, w, b, s) for f, (w, b), s in zip(cn_skips, self.zero, skips)]

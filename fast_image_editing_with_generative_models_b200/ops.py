@@ -388,15 +388,6 @@ def lpips_layer(f0: torch.Tensor, f1: torch.Tensor, lin: torch.Tensor) -> torch.
     return out / float(h * w)
 
 
-def preprocess(img_u8: torch.Tensor, c_out: int = 4, normalize: bool = True) -> torch.Tensor:
-    _req(img_u8, torch.uint8, "preprocess")
-    n, h, w, _ = img_u8.shape
-    out = torch.empty((n, h, w, c_out), dtype=torch.float16, device=img_u8.device)
-    check(_lib.lib().fie_preprocess_u8_to_f16(_p(img_u8), _p(out), n, h, w, c_out, int(normalize), _stream()), "fie_preprocess_u8_to_f16")
-    _count()
-    return out
-
-
 def preprocess_pad8(img_u8: torch.Tensor, normalize: bool = True) -> torch.Tensor:
     """uint8 [N,H,W,3] -> fp16 zero-padded [N,H+2,W+8,8] (input layout of :func:`conv3x3_c8`)."""
     _req(img_u8, torch.uint8, "preprocess_pad8")
@@ -429,29 +420,10 @@ def postprocess(x: torch.Tensor) -> torch.Tensor:
     return out
 
 
-def add(a: torch.Tensor, b: torch.Tensor, out: Optional[torch.Tensor] = None) -> torch.Tensor:
-    _req(a, torch.float16, "add"); _req(b, torch.float16, "add")
-    out = torch.empty_like(a) if out is None else out
-    with _prof("add", 6.0 * a.numel(), "B"):
-        check(_lib.lib().fie_add_f16(_p(a), _p(b), _p(out), a.numel(), _stream()), "fie_add_f16")
-    _count()
-    return out
-
-
 def silu(a: torch.Tensor) -> torch.Tensor:
     _req(a, torch.float16, "silu")
     out = torch.empty_like(a)
     check(_lib.lib().fie_silu_f16(_p(a), _p(out), a.numel(), _stream()), "fie_silu_f16")
-    _count()
-    return out
-
-
-def upsample2x(x: torch.Tensor) -> torch.Tensor:
-    _req(x, torch.float16, "upsample2x")
-    n, h, w, c = x.shape
-    out = torch.empty((n, 2 * h, 2 * w, c), dtype=torch.float16, device=x.device)
-    with _prof("upsample2x", 2.0 * out.numel() + 2.0 * x.numel(), "B"):
-        check(_lib.lib().fie_upsample2x_f16(_p(x), _p(out), n, h, w, c, _stream()), "fie_upsample2x_f16")
     _count()
     return out
 
@@ -843,39 +815,14 @@ def attention_vae(q: torch.Tensor, k: torch.Tensor, vt: torch.Tensor, scale: flo
     return out
 
 
-def vae_sample_add_noise(moments: torch.Tensor, xi: torch.Tensor, noise: torch.Tensor, scaling: float, sqrt_a: float, sqrt_1ma: float):
-    """moments [N,H,W,>=8] fp16, xi/noise [N,H,W,4] fp16 -> noisy latents [N,H,W,4] as (fp32 state, fp16 copy for the UNet)."""
+def vae_sample_add_noise(moments: torch.Tensor, xi: torch.Tensor, noise: torch.Tensor, scaling: float, coef: torch.Tensor):
+    """moments [N,H,W,>=8] fp16, xi/noise [N,H,W,4] fp16, per-image add-noise coefficients coef fp32 [N, 2] = (sqrt_a, sqrt_1ma) CUDA
+    tensor -> noisy latents [N,H,W,4] as (fp32 state, fp16 copy for the UNet)."""
     _req(moments, torch.float16, "vae_sample_add_noise")
-    out32 = torch.empty(xi.shape, dtype=torch.float32, device=xi.device)
-    out16 = torch.empty_like(xi)
-    npx = xi.numel() // 4
-    check(_lib.lib().fie_vae_sample_add_noise(_p(moments), moments.shape[-1], _p(xi), _p(noise), _p(out32), _p(out16), npx, float(scaling), float(sqrt_a),
-                                               float(sqrt_1ma), _stream()), "fie_vae_sample_add_noise")
-    _count()
-    return out32, out16
-
-
-def cfg_lcm_step(eps_u: torch.Tensor, eps_c: torch.Tensor, x32: torch.Tensor, noise: Optional[torch.Tensor], guidance: float, c: dict):
-    """eps_u/eps_c: [N,H,W,ld] fp16 views (first 4 channels used); x32 [N,H,W,4] fp32 latent state; c = LCM step coefficients
-    -> (fp32 state, fp16 copy)."""
-    _req(x32, torch.float32, "cfg_lcm_step")
-    out32 = torch.empty_like(x32)
-    out16 = torch.empty(x32.shape, dtype=torch.float16, device=x32.device)
-    npx = x32.numel() // 4
-    check(_lib.lib().fie_cfg_lcm_step(_p(eps_u), _p(eps_c), eps_u.stride(-2), _p(x32), _p(noise), _p(out32), _p(out16), npx, float(guidance), float(c["sqrt_a"]),
-                                       float(c["sqrt_1ma"]), float(c["c_skip"]), float(c["c_out"]), float(c["sqrt_a_prev"]), float(c["sqrt_1ma_prev"]),
-                                       int(bool(c["last"])), _stream()), "fie_cfg_lcm_step")
-    _count()
-    return out32, out16
-
-
-def vae_sample_add_noise_batched(moments: torch.Tensor, xi: torch.Tensor, noise: torch.Tensor, scaling: float, coef: torch.Tensor):
-    """:func:`vae_sample_add_noise` with per-image add-noise coefficients: coef fp32 [N, 2] = (sqrt_a, sqrt_1ma) CUDA tensor."""
-    _req(moments, torch.float16, "vae_sample_add_noise_batched")
-    _req(coef, torch.float32, "vae_sample_add_noise_batched")
+    _req(coef, torch.float32, "vae_sample_add_noise")
     n = xi.shape[0]
     if coef.numel() != 2 * n:
-        raise _lib.FieError("vae_sample_add_noise_batched: coef must be fp32 [N, 2]")
+        raise _lib.FieError("vae_sample_add_noise: coef must be fp32 [N, 2]")
     out32 = torch.empty(xi.shape, dtype=torch.float32, device=xi.device)
     out16 = torch.empty_like(xi)
     npx = xi.numel() // 4
@@ -885,14 +832,15 @@ def vae_sample_add_noise_batched(moments: torch.Tensor, xi: torch.Tensor, noise:
     return out32, out16
 
 
-def cfg_lcm_step_batched(eps_u: torch.Tensor, eps_c: torch.Tensor, x32: torch.Tensor, noise: Optional[torch.Tensor], coef: torch.Tensor, last: bool):
-    """:func:`cfg_lcm_step` with per-image coefficients: coef fp32 [N, 7] = (guidance, sqrt_a, sqrt_1ma, c_skip, c_out, sqrt_a_prev,
-    sqrt_1ma_prev) CUDA tensor (LCMSchedule.batch_tables); ``last``: the final step of every image (no noise)."""
-    _req(x32, torch.float32, "cfg_lcm_step_batched")
-    _req(coef, torch.float32, "cfg_lcm_step_batched")
+def cfg_lcm_step(eps_u: torch.Tensor, eps_c: torch.Tensor, x32: torch.Tensor, noise: Optional[torch.Tensor], coef: torch.Tensor, last: bool):
+    """CFG combine + LCMScheduler.step.  eps_u/eps_c: [N,H,W,ld] fp16 views (first 4 channels used); x32 [N,H,W,4] fp32 latent state;
+    per-image coefficients coef fp32 [N, 7] = (guidance, sqrt_a, sqrt_1ma, c_skip, c_out, sqrt_a_prev, sqrt_1ma_prev) CUDA tensor
+    (LCMSchedule.batch_tables); ``last``: the final step of every image (no noise) -> (fp32 state, fp16 copy)."""
+    _req(x32, torch.float32, "cfg_lcm_step")
+    _req(coef, torch.float32, "cfg_lcm_step")
     n = x32.shape[0]
     if coef.numel() != 7 * n:
-        raise _lib.FieError("cfg_lcm_step_batched: coef must be fp32 [N, 7]")
+        raise _lib.FieError("cfg_lcm_step: coef must be fp32 [N, 7]")
     out32 = torch.empty_like(x32)
     out16 = torch.empty(x32.shape, dtype=torch.float16, device=x32.device)
     npx = x32.numel() // 4

@@ -52,11 +52,31 @@ def executed_steps(strength, num_inference_steps) -> int:
     """diffusers img2img ``check_inputs`` + ``get_timesteps``: the number of denoising steps an image executes (ValueError if none)."""
     if strength < 0 or strength > 1:
         raise ValueError(f"The value of strength should in [0.0, 1.0] but is {strength}")
+    if not isinstance(num_inference_steps, int) or num_inference_steps <= 0:
+        raise ValueError(f"`num_inference_steps` has to be a positive integer but is {num_inference_steps}")
     n_exec = min(int(num_inference_steps * strength), num_inference_steps)
     if n_exec < 1:                   # diffusers: get_timesteps leaves no step to run
         raise ValueError(f"After adjusting the num_inference_steps by strength parameter: {strength}, the number of pipeline steps is "
                          f"{n_exec} which is < 1 and not appropriate for this pipeline.")
     return n_exec
+
+
+def per_image_settings(n: int, strength, num_inference_steps, guidance_scale, controlnet_conditioning_scale, canny_low_threshold,
+                       canny_high_threshold) -> Dict[str, list]:
+    """The numeric settings of an edit, each a scalar (every image) or a sequence with one value per image -> {name: list of ``n``
+    values} plus "n_exec", the denoising steps each image executes.  ValueError (naming the image) for a wrong length, a non-finite
+    value or an invalid strength / step count."""
+    st = dict(strength=strength, num_inference_steps=num_inference_steps, guidance_scale=guidance_scale,
+              controlnet_conditioning_scale=controlnet_conditioning_scale, canny_low_threshold=canny_low_threshold,
+              canny_high_threshold=canny_high_threshold)
+    st = {name: per_image(name, v, n) for name, v in st.items()}
+    st["n_exec"] = []
+    for i in range(n):
+        try:
+            st["n_exec"].append(executed_steps(st["strength"][i], st["num_inference_steps"][i]))
+        except ValueError as err:
+            raise ValueError(f"image {i}: {err}") from None
+    return st
 
 
 @dataclass
@@ -76,28 +96,22 @@ class EditParams:
         """Each setting a scalar (the whole batch) or a sequence with one value per image.  All images must execute the same number of
         steps and agree on CFG (guidance > 1 for all, or for none: diffusers runs the positive rows only at guidance <= 1)."""
         B = n_images
-        strength = per_image("strength", strength, B)
-        steps = per_image("num_inference_steps", num_inference_steps, B)
-        guidance = per_image("guidance_scale", guidance_scale, B)
-        scale = per_image("controlnet_conditioning_scale", controlnet_conditioning_scale, B)
-        low, high = per_image("canny_low", canny_low, B), per_image("canny_high", canny_high, B)
-        n_exec = None
-        for i in range(B):
-            try:
-                e = executed_steps(strength[i], steps[i])
-            except ValueError as err:
-                raise ValueError(f"image {i}: {err}") from None
-            if n_exec is not None and e != n_exec:
+        st = per_image_settings(B, strength, num_inference_steps, guidance_scale, controlnet_conditioning_scale, canny_low, canny_high)
+        n_exec = st["n_exec"][0]
+        for i, e in enumerate(st["n_exec"]):
+            if e != n_exec:
                 raise ValueError(f"image {i} executes {e} denoising steps, image 0 executes {n_exec}: the images of one batch must execute "
                                  "the same number of steps")
-            n_exec = e
+        guidance = st["guidance_scale"]
         cfg = guidance[0] > 1
         if any((g > 1) != cfg for g in guidance):
             raise ValueError("guidance_scale: the images of one batch must all be > 1 (classifier-free guidance) or all <= 1")
-        ts, add, table = sched.batch_tables(steps, strength, [g if cfg else 1.0 for g in guidance])
+        ts, add, table = sched.batch_tables(st["num_inference_steps"], st["strength"], [g if cfg else 1.0 for g in guidance])
         nrow = 2 if cfg else 1
-        thr = np.array([ops.canny_thresholds(lo, hi) for lo, hi in zip(low, high)], dtype=np.int32).reshape(B, 2)
+        thr = np.array([ops.canny_thresholds(lo, hi) for lo, hi in zip(st["canny_low_threshold"], st["canny_high_threshold"])],
+                       dtype=np.int32).reshape(B, 2)
         tsr = np.array(ts, dtype=np.float32).T                               # [n_exec, B]
+        scale = st["controlnet_conditioning_scale"]
         block = np.concatenate([thr.view(np.float32).ravel(), add.ravel(), np.tile(np.asarray(scale, np.float32), nrow),
                                 np.tile(tsr, (1, nrow)).ravel(), table.ravel()])
         return EditParams(B, n_exec, cfg, np.ascontiguousarray(block, dtype=np.float32))
@@ -287,7 +301,7 @@ class EditEngine:
         # ---- VAE encode -> posterior sample -> scale -> add_noise ----
         ops.stage("vae_encode")
         moments = self.vae.encode_moments(ops.preprocess_pad8(images_u8, normalize=True))
-        x32, x = ops.vae_sample_add_noise_batched(moments, nz[0], nz[1], self.vae.cfg.scaling_factor, v["add"])    # fp32 state, fp16 copy
+        x32, x = ops.vae_sample_add_noise(moments, nz[0], nz[1], self.vae.cfg.scaling_factor, v["add"])    # fp32 state, fp16 copy
         # ---- prompt conditioning (step-invariant): rows [neg]*B + [pos]*B as diffusers ----
         ops.stage("prompt_kv")
         if pe.dim() == 3:
@@ -316,7 +330,7 @@ class EditEngine:
             eu, ec = (eps[:B], eps[B:]) if do_cfg else (eps, eps)
             if return_extras:
                 eps_list.append(eps)
-            x32, x = ops.cfg_lcm_step_batched(eu, ec, x32, z, v["step"][k], last)
+            x32, x = ops.cfg_lcm_step(eu, ec, x32, z, v["step"][k], last)
         # ---- VAE decode (latents / scaling folded into post_quant_conv) + postprocess ----
         ops.stage("vae_decode")
         decoded = self.vae.decode(x)

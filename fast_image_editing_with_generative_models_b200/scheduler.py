@@ -1,5 +1,5 @@
-"""Host-side LCMScheduler logic (timestep table and per-step scalars); the arithmetic on latents runs in
-``fie_cfg_lcm_step`` / ``fie_vae_sample_add_noise``.  Mirrors diffusers ``LCMScheduler`` as configured by the
+"""Host-side LCMScheduler logic (timestep table and per-image coefficient tables); the arithmetic on latents runs in
+``fie_cfg_lcm_step_batched`` / ``fie_vae_sample_add_noise_batched``.  Mirrors diffusers ``LCMScheduler`` as configured by the
 reference (``LCMScheduler.from_config(..., timestep_spacing="trailing")``, ``src/pipeline.py:138-141,158-161``):
 scaled_linear betas 0.00085..0.012 over 1000 steps, epsilon prediction, original_inference_steps 50,
 timestep_scaling 10, sigma_data 0.5."""

@@ -117,9 +117,7 @@ int fie_lpips_layer_f16(const void* f0, const void* f1, const float* lin, int n,
 
 /* ---- Pre/post-processing: replaces VaeImageProcessor.preprocess/postprocess inside the diffusers call
  *      at reference src/pipeline.py:261-272 ---- */
-/* uint8 [n,h,w,3] -> fp16 [n,h,w,c_out] (c_out >= 3, extra channels zero): x/127.5-1 (normalize=1) or x/255 */
-int fie_preprocess_u8_to_f16(const void* img_u8, void* out_f16, int n, int h, int w, int c_out, int normalize, void* stream);
-/* uint8 [n,h,w,3] -> fp16 [n,h+2,w+8,8]: the same conversion written into the zero-padded 8-channel layout read by
+/* uint8 [n,h,w,3] -> fp16 [n,h+2,w+8,8]: x/127.5-1 (normalize=1) or x/255, written into the zero-padded 8-channel layout read by
  * fie_conv3x3_c8_f16 (real pixel (y,x) at (y+1,x+1); borders and channels 3..7 are zero) */
 int fie_preprocess_u8_to_f16_pad8(const void* img_u8, void* out_f16, int n, int h, int w, int normalize, void* stream);
 /* fp16 [n,h,w,4] (latents) -> the same zero-padded layout fp16 [n,h+2,w+8,8] (channels 4..7 and borders zero) */
@@ -128,12 +126,8 @@ int fie_pad8_f16(const void* x4_f16, void* out_f16, int n, int h, int w, void* s
 int fie_postprocess_f16_to_u8(const void* x_f16, int ld, void* out_u8, int n, int h, int w, void* stream);
 
 /* ---- Elementwise helpers ---- */
-/* out = a + b (fp16, count elements, multiple of 8) */
-int fie_add_f16(const void* a, const void* b, void* out, long long count, void* stream);
-/* out = silu(a) */
+/* out = silu(a) (fp16, count elements, multiple of 8) */
 int fie_silu_f16(const void* a, void* out, long long count, void* stream);
-/* nearest 2x upsample, NHWC fp16: [n,h,w,c] -> [n,2h,2w,c] */
-int fie_upsample2x_f16(const void* x, void* out, int n, int h, int w, int c, void* stream);
 /* sinusoidal embedding (diffusers Timesteps, flip_sin_to_cos, shift 0): vals fp32 [count] (HOST pointer,
  * count <= 64) -> fp16 [count, dim] = cat(cos, sin) */
 int fie_sincos_embedding(const float* host_vals, int count, int dim, void* out_f16, void* stream);
@@ -356,22 +350,16 @@ int fie_embed_tokens_f16(const int* ids, const void* tok, const void* pos, void*
 /* ---- Scheduler / latent math: replaces DiagonalGaussianDistribution.sample, LCMScheduler.add_noise,
  *      the CFG combine and LCMScheduler.step inside the diffusers call ---- */
 /* The latent state is carried in fp32 between the scheduler steps; each call also writes the fp16 copy the UNet / ControlNet read.
- * moments fp16 [n,hw,ld_m] (mean = ch 0..3, logvar = ch 4..7), xi/noise fp16 [n,hw,4]:
+ * Every image of a batch has its own strength, step count and guidance (EditEngine.edit_batch, pipeline.py): the coefficients are
+ * DEVICE arrays, so that one CUDA graph serves every setting; image i covers pixels [i px_per_img, (i+1) px_per_img).
+ * moments fp16 [n,hw,ld_m] (mean = ch 0..3, logvar = ch 4..7), xi/noise fp16 [n,hw,4], coef fp32 [n][2] = (sqrt_a, sqrt_1ma):
  * z0 = (mean + exp(0.5*clamp(logvar,-30,20))*xi)*scaling; x = sqrt_a*z0 + sqrt_1ma*noise. Writes x as fp32 and fp16 [n,hw,4] */
-int fie_vae_sample_add_noise(const void* moments, int ld_m, const void* xi, const void* noise, float* x_out_f32, void* x_out_f16,
-                             long long count_px, float scaling, float sqrt_a, float sqrt_1ma, void* stream);
-/* eps_u/eps_c fp16 [count_px, ld_e] (first 4 ch), x fp32 [count_px,4], noise fp16 or NULL:
- * eps = eps_u + g*(eps_c-eps_u); x0 = (x - s1*eps)/sa; den = c_out*x0 + c_skip*x; x' = sap*den + s1p*noise (fp32 and fp16 out) */
-int fie_cfg_lcm_step(const void* eps_u, const void* eps_c, int ld_e, const float* x_f32, const void* noise, float* x_out_f32, void* x_out_f16,
-                     long long count_px, float guidance, float sqrt_a, float sqrt_1ma, float c_skip, float c_out,
-                     float sqrt_a_prev, float sqrt_1ma_prev, int last, void* stream);
-/* Per-image forms (EditEngine.edit_batch, pipeline.py: every image of a batch with its own strength, step count and guidance).  The
- * coefficients are DEVICE arrays, so that one CUDA graph serves every setting; image i covers pixels [i px_per_img, (i+1) px_per_img).
- * coef of fie_vae_sample_add_noise_batched: fp32 [n][2] = (sqrt_a, sqrt_1ma); of fie_cfg_lcm_step_batched: fp32 [n][7] = (guidance,
- * sqrt_a, sqrt_1ma, c_skip, c_out, sqrt_a_prev, sqrt_1ma_prev).  Same kernels and arithmetic as the scalar forms: an image's result is
- * bit-identical to the scalar call with that image's values. */
 int fie_vae_sample_add_noise_batched(const void* moments, int ld_m, const void* xi, const void* noise, float* x_out_f32, void* x_out_f16,
                                      long long count_px, long long px_per_img, float scaling, const float* coef, void* stream);
+/* eps_u/eps_c fp16 [count_px, ld_e] (first 4 ch), x fp32 [count_px,4], noise fp16 or NULL (last step), coef fp32 [n][7] =
+ * (g, sa, s1, c_skip, c_out, sap, s1p) = (guidance, sqrt_a, sqrt_1ma, c_skip, c_out, sqrt_a_prev, sqrt_1ma_prev):
+ * eps = eps_u + g*(eps_c-eps_u); x0 = (x - s1*eps)/sa; den = c_out*x0 + c_skip*x; x' = sap*den + s1p*noise, or den when last
+ * (fp32 and fp16 out) */
 int fie_cfg_lcm_step_batched(const void* eps_u, const void* eps_c, int ld_e, const float* x_f32, const void* noise, float* x_out_f32,
                              void* x_out_f16, long long count_px, long long px_per_img, const float* coef, int last, void* stream);
 

@@ -13,7 +13,7 @@ run() { # name, pytest args...
 }
 : > gpurun_out/gpu_check.log
 run canny tests/test_gpu_canny.py
-run elementwise tests/test_gpu_kernels.py -k "pre_post or add_silu or sincos or groupnorm or layernorm or softmax or scheduler or cin4"
+run elementwise tests/test_gpu_kernels.py -k "pre_post or test_silu or sincos or groupnorm or layernorm or softmax or scheduler or cin4"
 run gemm_plain tests/test_gpu_kernels.py -k "gemm_plain"
 run gemm_epi tests/test_gpu_kernels.py -k "gemm_epilogue or folded_layernorm"
 run gemm_geglu tests/test_gpu_kernels.py -k "gemm_geglu"

@@ -44,12 +44,14 @@ else:
     cond = eng.cn.cond_embedding(ops.preprocess_pad8(ops.canny(imgs, 100, 200, out_channels=3), normalize=False))
     cond = torch.cat([cond, cond], 0)
     x2 = torch.randn((2 * B, 128, 128, 4), device=dev).half()
+    t = torch.full((2 * B,), 499.0, dtype=torch.float32, device=dev)          # per-row timesteps and ControlNet scales, as the edit
+    scale = torch.full((2 * B,), 0.5, dtype=torch.float32, device=dev)        # reads them from its parameter block
     for it in range(2):
         if it == 1:
             torch.cuda.synchronize()
             torch.cuda.profiler.start()
-        feats = eng.cn.encode(x2, 499.0, ps_cn, cond, 77)
-        eps = eng.unet.forward(x2, 499.0, ps_un, nctx=77, merge=eng.cn.merge_into(feats, 0.5))
+        feats = eng.cn.encode(x2, t, ps_cn, cond, 77)
+        eps = eng.unet.forward(x2, t, ps_un, nctx=77, merge=eng.cn.merge_into(feats, scale))
     torch.cuda.synchronize()
     torch.cuda.profiler.stop()
 print("probe done", mode, ops.LAUNCHES)

@@ -8,8 +8,8 @@ import pytest
 import torch
 
 from fast_image_editing_with_generative_models_b200 import ops
-from fast_image_editing_with_generative_models_b200.editor import FastEditor, micro_batches
-from fast_image_editing_with_generative_models_b200.pipeline import EditParams, graph_key, per_image
+from fast_image_editing_with_generative_models_b200.editor import micro_batches
+from fast_image_editing_with_generative_models_b200.pipeline import EditParams, graph_key, per_image, per_image_settings
 from fast_image_editing_with_generative_models_b200.scheduler import LCMSchedule
 
 
@@ -27,20 +27,20 @@ def test_per_image_broadcasts_scalars_and_checks_sequences():
         per_image("strength", "0.5", 2)
 
 
-def test_edit_many_settings_validation_names_the_image():
-    st = FastEditor._per_image_settings(3, [0.5, 0.25, 1.0], [4, 8, 2], 1.5, [0.3, 0.4, 0.5], 100, [200, 150, 250])
+def test_per_image_settings_validation_names_the_image():
+    st = per_image_settings(3, [0.5, 0.25, 1.0], [4, 8, 2], 1.5, [0.3, 0.4, 0.5], 100, [200, 150, 250])
     assert st["n_exec"] == [2, 2, 2]
     assert st["controlnet_conditioning_scale"] == [0.3, 0.4, 0.5] and st["canny_low_threshold"] == [100] * 3
     with pytest.raises(ValueError, match=r"image 1: The value of strength should in \[0.0, 1.0\] but is 1.5"):
-        FastEditor._per_image_settings(2, [0.5, 1.5], 4, 1.5, 0.5, 100, 200)
+        per_image_settings(2, [0.5, 1.5], 4, 1.5, 0.5, 100, 200)
     with pytest.raises(ValueError, match="image 2: `num_inference_steps` has to be a positive integer"):
-        FastEditor._per_image_settings(3, 0.5, [4, 4, 2.5], 1.5, 0.5, 100, 200)
+        per_image_settings(3, 0.5, [4, 4, 2.5], 1.5, 0.5, 100, 200)
     with pytest.raises(ValueError, match="image 0: After adjusting the num_inference_steps by strength parameter: 0.1"):
-        FastEditor._per_image_settings(2, [0.1, 0.5], 4, 1.5, 0.5, 100, 200)
+        per_image_settings(2, [0.1, 0.5], 4, 1.5, 0.5, 100, 200)
     with pytest.raises(ValueError, match="1 values for 2 images"):
-        FastEditor._per_image_settings(2, 0.5, [4], 1.5, 0.5, 100, 200)
+        per_image_settings(2, 0.5, [4], 1.5, 0.5, 100, 200)
     with pytest.raises(ValueError, match="canny_high_threshold of image 1"):
-        FastEditor._per_image_settings(2, 0.5, 4, 1.5, 0.5, 100, [200, float("nan")])
+        per_image_settings(2, 0.5, 4, 1.5, 0.5, 100, [200, float("nan")])
 
 
 def test_micro_batches_group_by_size_steps_and_cfg_in_input_order():

@@ -1,4 +1,4 @@
-"""GPU: per-image edit settings read from device memory -- the kernels' device-parameter forms against their scalar forms, cv2 and a
+"""GPU: per-image edit settings read from device memory -- the kernels' batched calls against one-image calls, cv2 and a
 float64 reference, and the engine: per-image results independent of the other images' settings, one CUDA graph for every setting of
 one (size, executed steps, CFG), edit_many's grouping and staging."""
 import cv2
@@ -24,7 +24,7 @@ def test_sincos_from_device_equals_host_form(cuda_dev):
             assert torch.equal(got[r0:r0 + 50].view(torch.int16), ref.view(torch.int16))
 
 
-def test_cfg_lcm_and_vae_sample_per_image_equal_scalar_forms(cuda_dev):
+def test_cfg_lcm_and_vae_sample_per_image_equal_one_image_calls(cuda_dev):
     from fast_image_editing_with_generative_models_b200 import ops
     from fast_image_editing_with_generative_models_b200.scheduler import LCMSchedule
     g = torch.Generator().manual_seed(5)
@@ -33,18 +33,19 @@ def test_cfg_lcm_and_vae_sample_per_image_equal_scalar_forms(cuda_dev):
     xi, nz = (torch.randn((B, h, w, 4), generator=g).half().to(cuda_dev) for _ in range(2))
     steps, strengths, guidance = [4, 8, 5, 4], [0.5, 0.25, 0.4, 0.5], [1.5, 2.25, 1.0, 7.5]
     ts, add, table = LCMSchedule().batch_tables(steps, strengths, guidance)
-    x32, x16 = ops.vae_sample_add_noise_batched(mom, xi, nz, 0.13025, torch.from_numpy(add).to(cuda_dev))
+    add = torch.from_numpy(add).to(cuda_dev)
+    x32, x16 = ops.vae_sample_add_noise(mom, xi, nz, 0.13025, add)
     for i in range(B):
-        r32, r16 = ops.vae_sample_add_noise(mom[i:i + 1], xi[i:i + 1], nz[i:i + 1], 0.13025, *[float(v) for v in add[i]])
+        r32, r16 = ops.vae_sample_add_noise(mom[i:i + 1], xi[i:i + 1], nz[i:i + 1], 0.13025, add[i:i + 1])
         assert torch.equal(x32[i:i + 1], r32) and torch.equal(x16[i:i + 1].view(torch.int16), r16.view(torch.int16))
     eps = torch.randn((2 * B, h, w, 8), generator=g).half().to(cuda_dev)[..., :4]
     tab = torch.from_numpy(table).to(cuda_dev)
     for k in range(table.shape[0]):
         last = k == table.shape[0] - 1
-        y32, y16 = ops.cfg_lcm_step_batched(eps[:B], eps[B:], x32, None if last else nz, tab[k], last)
+        y32, y16 = ops.cfg_lcm_step(eps[:B], eps[B:], x32, None if last else nz, tab[k], last)
         for i in range(B):
-            c = dict(zip(LCMSchedule.STEP_COLUMNS, [float(v) for v in table[k, i]]), last=last)
-            r32, r16 = ops.cfg_lcm_step(eps[i:i + 1], eps[B + i:B + i + 1], x32[i:i + 1].contiguous(), None if last else nz[i:i + 1], c["guidance"], c)
+            r32, r16 = ops.cfg_lcm_step(eps[i:i + 1], eps[B + i:B + i + 1], x32[i:i + 1].contiguous(), None if last else nz[i:i + 1],
+                                        tab[k, i:i + 1], last)
             assert torch.equal(y32[i:i + 1], r32) and torch.equal(y16[i:i + 1].view(torch.int16), r16.view(torch.int16))
         x32 = y32
 

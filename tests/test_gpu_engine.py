@@ -53,7 +53,10 @@ def test_vae_encode_decode_tiny(cuda_dev):
 
 
 @pytest.mark.parametrize("mid_depth,lora", [(1, False), (None, True)])
-def test_unet_controlnet_tiny(cuda_dev, mid_depth, lora):
+def test_unet_controlnet_merge_tiny(cuda_dev, mid_depth, lora):
+    """The ControlNet residuals (its zero convolutions at scale 0.5) against the oracle's, and the UNet eps with those residuals merged
+    by the zero-convolution GEMM epilogues (ControlNet.merge_into, the edit's path) against the oracle's UNet given the oracle's."""
+    from fast_image_editing_with_generative_models_b200 import ops
     from fast_image_editing_with_generative_models_b200.engine import ControlNet, UNet
     ucfg, up, ccfg, cp, vcfg, vp, lp = _models(cuda_dev, lora=lora, full_cn=lora, mid_depth=mid_depth)
     unet = UNet(up, ucfg, cuda_dev, lp, 1.0)
@@ -71,8 +74,12 @@ def test_unet_controlnet_tiny(cuda_dev, mid_depth, lora):
     cond_p8 = torch.zeros((B, 8 * h + 2, 8 * h + 8, 8), dtype=torch.float16, device=cuda_dev)   # layout of ops.preprocess_pad8
     cond_p8[:, 1:-1, 1:8 * h + 1, :3] = _nhwc(cond)
     cemb = cn.cond_embedding(cond_p8)
-    down, mid = cn.forward(_nhwc(x), t, ps_cn, cemb, 0.5)
-    eps = unet.forward(_nhwc(x), t, ps_un, down, mid)
+    t_rows = torch.full((B,), t, dtype=torch.float32, device=cuda_dev)
+    feats = cn.encode(_nhwc(x), t_rows, ps_cn, cemb)
+    fh, fskips = feats
+    down = [ops.gemm(f, w, col_bias=b, scale=0.5) for f, (w, b) in zip(fskips, cn.zero)]
+    mid = ops.gemm(fh, cn.zero_mid[0], col_bias=cn.zero_mid[1], scale=0.5)
+    eps = unet.forward(_nhwc(x), t_rows, ps_un, merge=cn.merge_into(feats, torch.full((B,), 0.5, dtype=torch.float32, device=cuda_dev)))
     # oracle, fp32 on the GPU
     up32, cp32 = O.to_dtype(up, torch.float32, cuda_dev), O.to_dtype(cp, torch.float32, cuda_dev)
     lora32 = O._LoRA(O.to_dtype(lp, torch.float32, cuda_dev), 1.0) if lp else None
